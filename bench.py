@@ -20,6 +20,8 @@ all histories full length, synthetic precomputed modality embeddings.
                  row-sharded ID table at seq len 512 (train step) and 10k x 10M retrieval.
 `--impl reference` runs the UNMODIFIED reference (baseline/_ref, installed by __graft_entry__.build()) for the same
 metric and config on the host cores; rank 0 only.
+`--dump-outputs DIR` (one GPU) runs the timed c2 step once more from the seeded start and writes what it computed as
+DIR/<name>.npy (dump_train_outputs): the same every run, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -42,6 +44,8 @@ C2_WORKLOAD = ("c2: two-tower train step (fwd+bwd+InfoNCE+dense AdamW), batch 25
                "100k-item ID table, dropout 0.1")
 C4 = dict(batch=512, seq_len=200, vocab=100_001)                 # BASELINE.json configs[3]: 8 x 512 = 4096 global
 C5 = dict(batch=512, seq_len=512, vocab=10_000_001, users=10_000, k=100)   # BASELINE.json configs[4]
+DUMP_TABLE_ROWS = 16_384      # --dump-outputs: seeded row sample of the ID table (all 100k rows are 102 MB)
+DUMP_MAX_BYTES = 64 << 20
 
 
 def flops_per_sample_fwd(L, B_neg, D=256, FF=1024, NL=2):
@@ -355,6 +359,8 @@ def run_ours(args, rank, world, local_rank):
     e2e_value = world * B * args.steps / e2e_s.item()
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    if args.dump_outputs:
+        dump_train_outputs(args.dump_outputs, runner, eng, synthetic.make_state_dict(cfg, seed=0), host_batches[0])
 
     # ---- forward + backward only (no optimizer step; SURVEY.md §8d) -------------------------
     fb = None
@@ -368,11 +374,11 @@ def run_ours(args, rank, world, local_rank):
         torch.cuda.synchronize()
         f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         f0.record()
-        for _ in range(20):
+        for _ in range(args.steps):
             r2.step_resident()
         f1.record()
         torch.cuda.synchronize()
-        fb_ms = f0.elapsed_time(f1) / 20
+        fb_ms = f0.elapsed_time(f1) / args.steps
         fb = {"ms_per_step": fb_ms, "samples_per_s": B * 1e3 / fb_ms,
               "what": "forward + backward + InfoNCE, gradient buffer cleared instead of the AdamW step"}
         del r2, eng2
@@ -483,6 +489,45 @@ def run_ours(args, rank, world, local_rank):
         print(json.dumps(line), flush=True)
 
 
+def dump_train_outputs(out_dir, runner, eng, state, batch):
+    """--dump-outputs: the timed step (the runner's captured graph) once more from the benchmark's seeded start —
+    parameters and BatchNorm statistics `state`, zero AdamW moments, step and dropout counters, input `batch` — and
+    what it computed, as out_dir/<name>.npy in float32: `loss`, `logits`, `user_emb` and `item_emb` as
+    TwoTowerEngine.forward returns them, and `grad.<parameter name>` for every parameter gradient (of the ID table a
+    fixed seeded sample of DUMP_TABLE_ROWS rows, with their ids as float64 `grad.<name>.row_ids`).
+    Gradients are summed with fp32 atomics, so their last bits vary from run to run (on one B200 at 1000 W, by at
+    most 7e-7 of each array's largest element); everything else is the same every run. That is why the step starts from the seeded state and not from where the timed loop left the model,
+    and why the updated parameters are not written: AdamW turns that rounding noise into updates of up to lr
+    wherever the exact gradient is zero (the biases ahead of BatchNorm, the key bias), and over many steps the
+    whole state drifts apart. The gradient is read back from AdamW's first moment, which after the first step is
+    (1 - beta1) * gradient. Leaves the model in the state after that one step."""
+    import numpy as np
+    eng.load_state_dict(state)
+    eng.refresh_shadow()
+    for t in (eng.grad, eng.exp_avg, eng.exp_avg_sq, eng.step_dev, eng.seed_dev):
+        t.zero_()
+    runner.load_batch(batch)
+    runner.step_resident()
+    torch.cuda.synchronize()
+    ws = eng.workspace(runner.B, runner.L)
+    out = {"loss": ws["loss"].view(1), "logits": ws["S"], "user_emb": ws["un"], "item_emb": ws["in"]}
+    grad = eng.exp_avg / (1.0 - runner.betas[0])
+    for name, (o, shape) in eng.layout.items():
+        g = grad[o:o + torch.Size(shape).numel()].view(shape)
+        if name == "user_tower.item_embedding.weight":
+            rows = torch.randperm(shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_TABLE_ROWS].sort().values
+            out[f"grad.{name}.row_ids"] = rows
+            g = g[rows.to(g.device)]
+        out[f"grad.{name}"] = g
+    arrays = {k: v.detach().cpu().numpy().astype(np.float32 if v.is_floating_point() else np.float64)
+              for k, v in out.items()}
+    nbytes = sum(a.nbytes for a in arrays.values())
+    assert nbytes <= DUMP_MAX_BYTES, f"--dump-outputs would write {nbytes} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def bench_parity_train(cfg, host_batch, dev):
     """The bench batch through a fresh engine with dropout 0 against the oracle's fp32 CPU forward."""
     import dataclasses
@@ -582,8 +627,7 @@ def bench_c5(rank, world, dev, peaks, args):
     table.weight[:table.rows].copy_(torch.randn(table.rows, 256, device=dev, generator=g) * (2.0 / (V + 256)) ** 0.5)
     runner = TrainStepRunner(eng, B, L, world_size=world, sharded_table=table)
     hb = [pin(synthetic.make_batch(cfg, B, seed=600 + rank * 17 + i, full_length=True, num_users=1_000_000)) for i in range(2)]
-    steps = max(5, args.steps // 2)
-    ms = _time_train(runner, hb, steps, args.warmup, dev, world)
+    ms = _time_train(runner, hb, args.steps, args.warmup, dev, world)
     flops = 3.0 * flops_per_sample_fwd(L, world * B) * B
     peak_tf = peaks.get("bf16_tflops_sustained", peaks.get("bf16_tflops"))
     train = {"workload": f"c5 train: {V - 1} items, ID table row-sharded over {world} ranks ({table.rows} rows/rank), "
@@ -923,10 +967,18 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--skip-retrieval", action="store_true", help="skip the c3 retrieval section (A/B timing runs)")
     ap.add_argument("--skip-c45", action="store_true", help="skip the c4 / c5 blocks of multi-GPU runs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed c2 step computes from the seeded start to DIR/<name>.npy (one GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        ap.error("--dump-outputs runs on one GPU")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
