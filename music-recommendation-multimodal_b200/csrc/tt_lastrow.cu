@@ -4,7 +4,11 @@
 // 122-132); nothing else of that layer's output is ever read, and its pad/other rows carry zero
 // gradient. So in the last layer only K and V are needed for every position; the query, the
 // attention output, out_proj, both residual adds, norm2 and the FFN are needed for ONE row per
-// sequence. These kernels implement that exactly (same results as the full computation):
+// sequence. These kernels implement that exactly: without dropout, the same results as the full
+// computation. With dropout the masks differ: the out_proj / linear1 / linear2 GEMMs of the pruned
+// layer run on the compact [B, .] rows, so their epilogues hash the compact row b where the full
+// schedule hashes the token row b*L + last_b (tt_attn_lastq_* keep the full-sequence index). Both
+// are valid draws of the same dropout, not the same draw.
 //   tt_gather_rows        : rows[b] = x[b*L + last_idx[b]]  (fp32 and/or bf16 copies)
 //   tt_scatter_rows_add   : x[b*L + last_idx[b]] (+)= rows[b]
 //   tt_attn_lastq_fwd/bwd : causal attention for the single query row len-1 of every

@@ -45,10 +45,13 @@ def l2_normalize(x: torch.Tensor, eps: float = 1e-12) -> torch.Tensor:
 
 
 def encoder_layer(x: torch.Tensor, p: Params, prefix: str, num_heads: int,
-                  key_is_pad: torch.Tensor) -> torch.Tensor:
-    """One pre-LN nn.TransformerEncoderLayer(d, nhead, 4d, batch_first, norm_first=True),
-    dropout disabled (user_tower.py:37-45, called at :111-116 with a causal mask and a
-    key-padding mask). torch semantics: x += OutProj(Attn(LN1(x))); x += W2 ReLU(W1 LN2(x))."""
+                  key_is_pad: torch.Tensor, drop: Optional[Params] = None) -> torch.Tensor:
+    """One pre-LN nn.TransformerEncoderLayer(d, nhead, 4d, batch_first, norm_first=True)
+    (user_tower.py:37-45, called at :111-116 with a causal mask and a key-padding mask).
+    torch semantics: x += OutProj(Attn(LN1(x))); x += W2 ReLU(W1 LN2(x)).
+    Dropout is off unless ``drop`` gives this layer's scaled masks (keep / (1 - p)), applied where
+    nn.TransformerEncoderLayer applies its dropouts: "attn" (B,H,L,L) on the softmax probabilities,
+    "out_proj" (B,L,D) and "linear2" (B,L,D) before the residual adds, "ffn" (B,L,4D) after the ReLU."""
     B, L, D = x.shape
     dh = D // num_heads
     h = layer_norm(x, p[prefix + "norm1.weight"], p[prefix + "norm1.bias"])
@@ -63,23 +66,35 @@ def encoder_layer(x: torch.Tensor, p: Params, prefix: str, num_heads: int,
     s = s.masked_fill(causal, neg)
     s = s.masked_fill(key_is_pad[:, None, None, :], neg)
     a = torch.softmax(s, dim=-1)
+    if drop is not None:
+        a = a * drop["attn"]
     ctx = (a @ v).transpose(1, 2).reshape(B, L, D)
-    x = x + ctx @ p[prefix + "self_attn.out_proj.weight"].t() + p[prefix + "self_attn.out_proj.bias"]
+    if drop is None:
+        x = x + ctx @ p[prefix + "self_attn.out_proj.weight"].t() + p[prefix + "self_attn.out_proj.bias"]
+    else:
+        x = x + (ctx @ p[prefix + "self_attn.out_proj.weight"].t() + p[prefix + "self_attn.out_proj.bias"]) * drop["out_proj"]
     h2 = layer_norm(x, p[prefix + "norm2.weight"], p[prefix + "norm2.bias"])
     f = torch.relu(h2 @ p[prefix + "linear1.weight"].t() + p[prefix + "linear1.bias"])
-    x = x + f @ p[prefix + "linear2.weight"].t() + p[prefix + "linear2.bias"]
+    if drop is None:
+        x = x + f @ p[prefix + "linear2.weight"].t() + p[prefix + "linear2.bias"]
+    else:
+        f = f * drop["ffn"]
+        x = x + (f @ p[prefix + "linear2.weight"].t() + p[prefix + "linear2.bias"]) * drop["linear2"]
     return x
 
 
 def user_tower(p: Params, history_ids: torch.Tensor, user_gender: torch.Tensor,
                user_country: torch.Tensor, history_mask: Optional[torch.Tensor] = None,
-               num_heads: int = 4, prefix: str = "user_tower.") -> torch.Tensor:
-    """SequentialUserEncoder.forward (user_tower.py:73-144), dropout off.
+               num_heads: int = 4, prefix: str = "user_tower.", drop: Optional[Params] = None) -> torch.Tensor:
+    """SequentialUserEncoder.forward (user_tower.py:73-144). Dropout is off unless ``drop`` holds the
+    scaled masks "emb" (B,L,D), after the embedding LayerNorm, and "layers.{l}.<site>" of encoder_layer.
     Returns the un-normalised (B, D) user embedding."""
     B, L = history_ids.shape
     E = p[prefix + "item_embedding.weight"]
     x = E[history_ids] + p[prefix + "position_embedding.weight"][:L].unsqueeze(0)     # :86-92
     x = layer_norm(x, p[prefix + "layer_norm.weight"], p[prefix + "layer_norm.bias"])  # :93
+    if drop is not None:
+        x = x * drop["emb"]
     if history_mask is not None:                                                        # :100-103
         key_is_pad = history_mask == 0
         lengths = history_mask.sum(dim=1).long() - 1                                    # :122-125
@@ -90,7 +105,8 @@ def user_tower(p: Params, history_ids: torch.Tensor, user_gender: torch.Tensor,
     while f"{prefix}transformer_encoder.layers.{num_layers}.norm1.weight" in p:
         num_layers += 1
     for l in range(num_layers):                                                         # :111-116
-        x = encoder_layer(x, p, f"{prefix}transformer_encoder.layers.{l}.", num_heads, key_is_pad)
+        ld = None if drop is None else {k: drop[f"layers.{l}.{k}"] for k in ("attn", "out_proj", "ffn", "linear2")}
+        x = encoder_layer(x, p, f"{prefix}transformer_encoder.layers.{l}.", num_heads, key_is_pad, ld)
     lengths = lengths.clamp(min=0)                                                      # :128
     seq = x[torch.arange(B), lengths]                                                   # :132
     g = p[prefix + "gender_embedding.weight"][user_gender]                              # :135-136
@@ -104,10 +120,12 @@ def user_tower(p: Params, history_ids: torch.Tensor, user_gender: torch.Tensor,
 
 def item_fusion(p: Params, audio: torch.Tensor, visual: torch.Tensor, text: torch.Tensor,
                 tabular: torch.Tensor, training: bool, bn_eps: float = 1e-5,
-                prefix: str = "item_tower.fusion_layer.") -> Tuple[torch.Tensor, Optional[Tuple[torch.Tensor, torch.Tensor]]]:
+                prefix: str = "item_tower.fusion_layer.", drop: Optional[torch.Tensor] = None,
+                ) -> Tuple[torch.Tensor, Optional[Tuple[torch.Tensor, torch.Tensor]]]:
     """MultimodalItemEncoder.forward from the concat on (item_tower.py:147-150) with
-    fusion_layer = Linear(512,512) -> BatchNorm1d -> ReLU -> Dropout(off) -> Linear(512,256)
+    fusion_layer = Linear(512,512) -> BatchNorm1d -> ReLU -> Dropout -> Linear(512,256)
     -> LayerNorm (item_tower.py:121-129). Concat order: audio, visual, text, tabular.
+    The Dropout is off unless ``drop`` gives its scaled (B, 512) mask.
     Returns (un-normalised item embedding, (batch_mean, batch_var_biased) in training mode)."""
     x = torch.cat([audio, visual, text, tabular], dim=1)
     y = x @ p[prefix + "0.weight"].t() + p[prefix + "0.bias"]
@@ -120,6 +138,8 @@ def item_fusion(p: Params, audio: torch.Tensor, visual: torch.Tensor, text: torc
         mu, var = p[prefix + "1.running_mean"].to(y.dtype), p[prefix + "1.running_var"].to(y.dtype)
     y = (y - mu) / torch.sqrt(var + bn_eps) * p[prefix + "1.weight"] + p[prefix + "1.bias"]
     y = torch.relu(y)
+    if drop is not None:
+        y = y * drop
     y = y @ p[prefix + "4.weight"].t() + p[prefix + "4.bias"]
     return layer_norm(y, p[prefix + "5.weight"], p[prefix + "5.bias"]), stats
 
@@ -149,16 +169,18 @@ def infonce(user_emb: torch.Tensor, item_emb: torch.Tensor, temperature: float,
 
 
 def two_tower_forward(p: Params, batch: Dict[str, torch.Tensor], temperature: float = 0.07,
-                      num_heads: int = 4, training: bool = True):
+                      num_heads: int = 4, training: bool = True, drop: Optional[Params] = None):
     """TwoTowerModel.forward (two_tower.py:68-142) with the four modality encoders replaced
     by identity (north_star): batch['target_audio'|'target_image'|'target_input_ids'|
-    'target_tabular'] carry precomputed (B,128) embeddings.
+    'target_tabular'] carry precomputed (B,128) embeddings. ``drop``: every dropout site's
+    scaled mask (user_tower's keys and "item"); None runs without dropout.
     Returns (loss, logits, user_emb, item_emb, bn_stats)."""
     u = user_tower(p, batch["history_ids"], batch["user_gender"], batch["user_country"],
-                   batch.get("history_mask"), num_heads)
+                   batch.get("history_mask"), num_heads, drop=drop)
     dt = u.dtype
     i, stats = item_fusion(p, batch["target_audio"].to(dt), batch["target_image"].to(dt),
-                           batch["target_input_ids"].to(dt), batch["target_tabular"].to(dt), training)
+                           batch["target_input_ids"].to(dt), batch["target_tabular"].to(dt), training,
+                           drop=None if drop is None else drop["item"])
     u = l2_normalize(u)
     i = l2_normalize(i)
     loss, logits = infonce(u, i, temperature, batch.get("user_idx"))
@@ -169,16 +191,17 @@ TRAINABLE_SKIP = ("running_mean", "running_var", "num_batches_tracked")
 
 
 def loss_and_grads(p: Params, batch, temperature: float = 0.07, num_heads: int = 4,
-                   dtype: torch.dtype = torch.float32):
+                   dtype: torch.dtype = torch.float32, drop: Optional[Params] = None):
     """Forward + autograd backward of the restated path (train.py:57-63 without AMP:
-    on a CPU host autocast/GradScaler disable themselves, SURVEY.md App. A)."""
+    on a CPU host autocast/GradScaler disable themselves, SURVEY.md App. A). ``drop``: the
+    scaled dropout masks of two_tower_forward (None: dropout off)."""
     q = {}
     for k, v in p.items():
         if k.endswith(TRAINABLE_SKIP):
             q[k] = v.clone()
         else:
             q[k] = v.detach().to(dtype).clone().requires_grad_(True)
-    loss, logits, u, i, stats = two_tower_forward(q, batch, temperature, num_heads, training=True)
+    loss, logits, u, i, stats = two_tower_forward(q, batch, temperature, num_heads, training=True, drop=drop)
     loss.backward()
     grads = {k: v.grad for k, v in q.items() if isinstance(v, torch.Tensor) and v.requires_grad}
     for k, g in list(grads.items()):

@@ -233,8 +233,10 @@ def test_gathered_negatives_two_virtual_ranks_match_global_oracle():
 
 
 def test_pruned_last_layer_equals_full_computation():
-    """The single-row last layer (SURVEY §8 a5) is exact: same loss / embeddings / gradients as running
-    the last layer on every position (differences are bf16 rounding of different but equivalent paths)."""
+    """The single-row last layer (SURVEY §8 a5) is exact at dropout 0: same loss / embeddings / gradients as running
+    the last layer on every position (differences are bf16 rounding of different but equivalent paths). With dropout
+    the two schedules draw different masks (compact vs token rows in the last layer's GEMM epilogues); each is checked
+    against the oracle with its own masks in test_dropout_parity.py."""
     gold, cfg, sd, batch, eng, dbatch = _setup("train_l200.pt")
     from mrm_b200.engine import TwoTowerEngine
     full = TwoTowerEngine(cfg)
