@@ -342,6 +342,19 @@ int tt_infonce_loss(const float* lse_a, const float* pos_a, const float* lse_b, 
  * tt_topk_merge_lists : the same with input lists of K_in entries and K_out outputs (-1 / -inf padded).
  * tt_exact_topk     : brute-force exact top K of one user (fallback for flagged users);
  *                     key_scratch = N * 8 bytes.
+ *
+ * Excluding seen items (src/inference.py:296-302: scores[0] = -inf and scores[h] = -inf for every
+ * history item h, before the top k). Excluded ids are dropped from the candidate lists before any
+ * prune and before the lists are handed over, so pruning, finalize, the certificate, the bounded shard protocol and the merges all speak about the
+ * admissible items only; a user with fewer than K admissible items gets a -1 / -inf tail.
+ * tt_exclusions_build : ids [U, m] int64 with row pitch ld_in (0 = empty slot; ids <= 0 or >= vocab_size
+ *                     are dropped), m <= 4096 -> per user a sorted, de-duplicated int32 list out_ids [U, ld]
+ *                     (ld >= m), its length out_cnt [U] and a 4096-bit hashed bitmap out_bits [U, 128].
+ * tt_score_topk_excl : tt_score_topk that never admits user u's excluded ids (ex_* from
+ *                     tt_exclusions_build, ex_ld = its ld; all NULL = tt_score_topk). The sample pass
+ *                     raises each user's rank by its excluded ids inside the sampled item steps.
+ * tt_exact_topk_excl : tt_exact_topk without the ids ex_ids[0 .. *ex_cnt) (one user's row of
+ *                     tt_exclusions_build's output; NULL = tt_exact_topk).
  * tt_rank_metrics   : per-row Recall@k / NDCG@k (:159-185); gain_table[r] = 1/log2(r+2) comes
  *                     from the host so rows are bit-identical to the reference's; outputs [nk][U].
  */
@@ -383,6 +396,14 @@ int tt_topk_merge_lists(const float* scores, const int32_t* idx, int G, int U, i
                         int32_t* out_idx, void* stream);
 int tt_exact_topk(const float* user_f32, const float* items_f32, int N, int item_base, int mask_item0, int K,
                   void* key_scratch, float* out_score, int32_t* out_idx, void* stream);
+int tt_exclusions_build(const int64_t* ids, int U, int m, int ld_in, int vocab_size, int32_t* out_ids, int ld,
+                        int32_t* out_cnt, uint32_t* out_bits, void* stream);
+int tt_score_topk_excl(const void* users_bf16, const void* items_bf16, int item_base, const tt_topk_plan* plan,
+                       void* cand, int32_t* cand_cnt, void* thr, void* smax, int mask_item0, const int32_t* ex_ids,
+                       const int32_t* ex_cnt, const uint32_t* ex_bits, int ex_ld, void* stream);
+int tt_exact_topk_excl(const float* user_f32, const float* items_f32, int N, int item_base, int mask_item0, int K,
+                       const int32_t* ex_ids, const int32_t* ex_cnt, void* key_scratch, float* out_score,
+                       int32_t* out_idx, void* stream);
 int tt_rank_metrics(const int32_t* topk_idx, const int64_t* targets, int U, int K, const int32_t* k_list, int nk,
                     const float* gain_table, float* recall, float* ndcg, void* stream);
 

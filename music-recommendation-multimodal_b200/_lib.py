@@ -181,6 +181,12 @@ _SIGNATURES = {
     "tt_topk_merge": [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p],
     "tt_topk_merge_lists": [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p],
     "tt_exact_topk": [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p],
+    "tt_exclusions_build": [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_int32, c_void_p, c_void_p,
+                            c_void_p],
+    "tt_score_topk_excl": [c_void_p, c_void_p, c_int32, ctypes.POINTER(TopkPlan), c_void_p, c_void_p, c_void_p,
+                           c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p],
+    "tt_exact_topk_excl": [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
+                           c_void_p, c_void_p, c_void_p],
     "tt_rank_metrics": [c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_int32, c_void_p, c_void_p, c_void_p,
                         c_void_p],
     "tt_cast_bf16": [c_void_p, c_void_p, _I64, c_void_p],

@@ -26,6 +26,7 @@
 // a certificate that no non-candidate can belong to the exact top K.
 #include "../../include/tt_b200.h"
 #include "tt_common.cuh"
+#include <climits>
 #include <math.h>
 
 namespace tt {
@@ -42,6 +43,8 @@ static constexpr int kTopkThreads = 640;   // TMA, MMA, TMEM-alloc, spare + 16 e
 static constexpr int kCap = 512;       // candidate list capacity per (range, row)
 static constexpr int kMaxLists = 1216;  // finalize: lists per user (ranges x kLists) the offset table holds
 static constexpr int kPoolCap = 4096;  // finalize: per-user key pool in shared memory
+static constexpr int kExclMax = 4096;  // excluded ids per user (tt_exclusions_build: one shared-memory bitonic sort)
+static constexpr int kExclWords = 128; // per-user hashed bitmap of excluded ids: 4096 bits
 
 __device__ __forceinline__ uint32_t f2ord(float f) {
   const uint32_t u = __float_as_uint(f + 0.0f);  // -0 -> +0
@@ -68,7 +71,55 @@ struct TopkParams {
   int* cand_cnt;             // [n_ranges * kLists][u_pad]
   unsigned long long* thr;   // [u_pad]
   int mask_item0;
+  // score_topk_kernel<false, true>: per-user excluded global ids (tt_exclusions_build)
+  const int* ex_ids;         // [U][ex_ld] sorted ascending, distinct
+  const int* ex_cnt;         // [U]
+  const uint32_t* ex_bits;   // [U][kExclWords] hashed bitmap: a clear bit proves an id is not excluded
+  int ex_ld;
 };
+
+// Bit of the exclusion bitmap that stands for global id `id` (Fibonacci hashing: the top 12 bits of id * 2^32/phi).
+__device__ __forceinline__ uint32_t excl_hash(uint32_t id) { return (id * 2654435761u) >> 20; }
+
+// Drop the keys of excluded items from one lane's candidate list buf[0, n) in place; returns the new count. A key
+// whose bitmap bit is clear is kept after one L2-resident load; only the ~m/4096 others pay for a binary search of
+// the sorted list. Candidates (about one score in a thousand) enter the list unchecked and the list is filtered here,
+// once per work unit and before a prune — testing each candidate as it is admitted put an L2 round trip into the
+// epilogue's chunk chain, whose latency bounds an item step (measured on a B200: 1.48x the plain pass at m = 50).
+__device__ __noinline__ int drop_excluded(unsigned long long* buf, int n, const uint32_t* __restrict__ bits,
+                                          const int* __restrict__ ids, int n_ids) {
+  constexpr int kBatch = 8;   // keys whose list and bitmap loads are in flight together (the writes trail the reads)
+  int w = 0;
+  for (int i0 = 0; i0 < n; i0 += kBatch) {
+    unsigned long long k[kBatch];
+    uint32_t word[kBatch];
+#pragma unroll
+    for (int e = 0; e < kBatch; ++e) k[e] = i0 + e < n ? buf[i0 + e] : 0ull;
+#pragma unroll
+    for (int e = 0; e < kBatch; ++e) word[e] = i0 + e < n ? __ldg(bits + (excl_hash(key_idx(k[e])) >> 5)) : 0u;
+#pragma unroll
+    for (int e = 0; e < kBatch; ++e) {
+      if (i0 + e >= n) break;
+      const uint32_t gidx = key_idx(k[e]);
+      bool ex = false;
+      if ((word[e] >> (excl_hash(gidx) & 31u)) & 1u) {
+        int lo = 0, hi = n_ids;                          // first position whose id is >= gidx
+        while (lo < hi) {
+          const int mid = (lo + hi) >> 1;
+          if (__ldg(ids + mid) < static_cast<int>(gidx)) lo = mid + 1; else hi = mid;
+        }
+        ex = lo < n_ids && __ldg(ids + lo) == static_cast<int>(gidx);
+      }
+      if (!ex) buf[w++] = k[e];
+    }
+  }
+  return w;
+}
+
+__device__ __forceinline__ int drop_excluded_row(unsigned long long* buf, int n, const TopkParams& p, int row) {
+  return drop_excluded(buf, n, p.ex_bits + static_cast<size_t>(row) * kExclWords,
+                       p.ex_ids + static_cast<size_t>(row) * p.ex_ld, __ldg(p.ex_cnt + row));
+}
 
 // Warp-cooperative prune of one row's candidate list to its kprime largest keys.
 // Returns the new count; T receives a threshold with count(keys >= T) == new count.
@@ -135,6 +186,7 @@ __device__ __forceinline__ uint32_t chunk_group_mask(const uint32_t (&r)[32], fl
   return gm;
 }
 
+template <bool kExclude>
 __device__ __forceinline__ void collect_groups(uint32_t gm, uint32_t t_chunk, int idx0, const TopkParams& p, int lane,
                                                int row, unsigned long long* buf, int& cnt,
                                                unsigned long long& thr_key, float& thr_s) {
@@ -161,6 +213,9 @@ __device__ __forceinline__ void collect_groups(uint32_t gm, uint32_t t_chunk, in
       }
     }
   }
+  if constexpr (kExclude) {
+    if (cnt > kCap - 64) cnt = drop_excluded_row(buf, cnt, p, row);   // prune thresholds count admissible keys only
+  }
   unsigned full = __ballot_sync(0xffffffffu, cnt > kCap - 64)   /* a call appends at most 64 keys per lane */;
   while (full) {
     const int src = __ffs(full) - 1;
@@ -178,7 +233,10 @@ __device__ __forceinline__ void collect_groups(uint32_t gm, uint32_t t_chunk, in
   }
 }
 
-template <bool kSample>
+// kExclude (main pass only): the user's excluded items are removed from its candidate lists before every prune and
+// before the lists are handed over, so the pruning thresholds, finalize and its certificate all speak about the
+// admissible items only.
+template <bool kSample, bool kExclude>
 __global__ void __launch_bounds__(kTopkThreads, 1)
 score_topk_kernel(const __grid_constant__ CUtensorMap tmU, const __grid_constant__ CUtensorMap tmI,
                   const TopkParams p) {
@@ -328,7 +386,7 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmU, const __grid_constant
           const uint32_t gm1 = chunk_group_mask(r1, thr_s);
           if (__any_sync(0xffffffffu, (gm0 | gm1) != 0u)) {
             const int idx0 = tile * kIT + colq * 64;
-            collect_groups(gm0 | (gm1 << 8), t_base, idx0, p, lane, row, buf, cnt, thr_key, thr_s);
+            collect_groups<kExclude>(gm0 | (gm1 << 8), t_base, idx0, p, lane, row, buf, cnt, thr_key, thr_s);
           }
         }
         tc_fence_before();
@@ -336,6 +394,9 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmU, const __grid_constant
         if (lane == 0) mbar_arrive_cluster(&t_empty[acc], 0);
         acc ^= 1;
         if (acc == 0) acc_phase ^= 1u;
+      }
+      if constexpr (kExclude) {
+        if (active && cnt > 0) cnt = drop_excluded_row(buf, cnt, p, row);
       }
       if constexpr (!kSample) p.cand_cnt[list * p.u_pad + row] = active ? cnt : 0;
     }
@@ -358,14 +419,35 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmU, const __grid_constant
 // only scores above it (no pruning, mostly the fast path). It is a heuristic STARTING point only:
 // tt_topk_finalize verifies that enough candidates were found plus the exactness certificate, and
 // users for which that fails go to the exact fallback. One warp per user, maxima held in registers.
+// With exclusions (ex_cnt != nullptr) the sample still scores every item, and an excluded item can own a chunk
+// maximum: the rank rises by the number of the user's excluded ids inside the sampled item steps (step index a
+// multiple of tile_stride, below sample_tiles * tile_stride). Each lifts at most one chunk maximum, so the
+// (rank + e)-th raw maximum is at most the rank-th maximum over admissible items.
 // --------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) sample_threshold_kernel(const float* __restrict__ smax, int U, int n_chunks,
-                                                               int rank, unsigned long long* __restrict__ thr) {
+                                                               int rank, unsigned long long* __restrict__ thr,
+                                                               const int* __restrict__ ex_ids,
+                                                               const int* __restrict__ ex_cnt, int ex_ld,
+                                                               int item_base, int N, int tile_stride,
+                                                               int sample_tiles) {
   pdl_launch_dependents();
   pdl_wait();
   constexpr int kMaxPerLane = 32;   // up to 1024 chunk maxima per user
   const int u = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (u >= U) return;
+  if (ex_cnt != nullptr) {
+    const int* ids = ex_ids + static_cast<size_t>(u) * ex_ld;
+    const int n = ex_cnt[u];
+    int e = 0;
+    for (int i = lane; i < n; i += 32) {
+      const int local = ids[i] - item_base;
+      const int tile = local / kIT;
+      e += (local >= 0 && local < N && tile % tile_stride == 0 && tile < sample_tiles * tile_stride) ? 1 : 0;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) e += __shfl_xor_sync(0xffffffffu, e, o);
+    rank += e;
+  }
   const float* row = smax + static_cast<size_t>(u) * n_chunks;
   uint32_t v[kMaxPerLane];
 #pragma unroll
@@ -728,6 +810,19 @@ __global__ void __launch_bounds__(256) exact_keys_kernel(const float* __restrict
   }
 }
 
+// Exact fallback with exclusions: zero the keys of the user's excluded ids that lie in this shard. A key of 0 is
+// never selected (the same way mask_item0 removes item 0).
+__global__ void __launch_bounds__(256) exact_exclude_kernel(const int* __restrict__ ex_ids, const int* __restrict__ ex_cnt,
+                                                            int N, int item_base, unsigned long long* __restrict__ keys) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const int n = *ex_cnt;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    const int local = ex_ids[i] - item_base;
+    if (local >= 0 && local < N) keys[local] = 0ull;
+  }
+}
+
 __global__ void __launch_bounds__(256) exact_select_kernel(const unsigned long long* __restrict__ keys, int N, int K,
                                                            float* __restrict__ out_score, int* __restrict__ out_idx) {
   pdl_launch_dependents();
@@ -823,9 +918,91 @@ __global__ void __launch_bounds__(256) users_prepare_kernel(const float* __restr
   }
 }
 
+// --------------------------------------------------------------------------------------------
+// Per-user exclusion lists (the history masking of src/inference.py:296-302) in the form the selection epilogue
+// probes: ids sorted ascending and de-duplicated, their count, and a 4096-bit hashed bitmap. One block per user;
+// the row (0 = empty slot, ids <= 0 or >= vocab dropped) is padded with INT_MAX to a power of two >= 256, bitonic
+// sorted in shared memory, and compacted with a block scan (each thread owns n_pad / 256 consecutive slots).
+// --------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) exclusions_build_kernel(const int64_t* __restrict__ in, int m, int ld_in,
+                                                               int vocab, int n_pad, int* __restrict__ out_ids,
+                                                               int ld, int* __restrict__ out_cnt,
+                                                               uint32_t* __restrict__ out_bits) {
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ int s[kExclMax];
+  __shared__ uint32_t s_bits[kExclWords];
+  __shared__ int s_scan[8];
+  const int u = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int64_t* row = in + static_cast<size_t>(u) * ld_in;
+  for (int i = tid; i < n_pad; i += 256) {
+    const int64_t v = i < m ? row[i] : 0;
+    s[i] = (v > 0 && v < vocab) ? static_cast<int>(v) : INT_MAX;
+  }
+  for (int i = tid; i < kExclWords; i += 256) s_bits[i] = 0u;
+  for (int size = 2; size <= n_pad; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      __syncthreads();
+      for (int i = tid; i < n_pad; i += 256) {
+        const int j = i ^ stride;
+        if (j > i) {
+          const int a = s[i], b = s[j];
+          if (((i & size) == 0) ? (a > b) : (a < b)) { s[i] = b; s[j] = a; }
+        }
+      }
+    }
+  }
+  __syncthreads();
+  const int per = n_pad >> 8, b0 = tid * per;
+  int c = 0;
+  for (int e = 0; e < per; ++e) {
+    const int i = b0 + e, v = s[i];
+    c += (v != INT_MAX && (i == 0 || s[i - 1] != v)) ? 1 : 0;
+  }
+  int incl = c;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int v = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += v;
+  }
+  if (lane == 31) s_scan[warp] = incl;
+  __syncthreads();
+  int pos = incl - c, total = 0;
+  for (int w = 0; w < 8; ++w) {
+    pos += w < warp ? s_scan[w] : 0;
+    total += s_scan[w];
+  }
+  int* dst = out_ids + static_cast<size_t>(u) * ld;
+  for (int e = 0; e < per; ++e) {
+    const int i = b0 + e, v = s[i];
+    if (v != INT_MAX && (i == 0 || s[i - 1] != v)) {
+      dst[pos++] = v;
+      const uint32_t h = excl_hash(static_cast<uint32_t>(v));
+      atomicOr(&s_bits[h >> 5], 1u << (h & 31u));
+    }
+  }
+  __syncthreads();
+  for (int i = tid; i < kExclWords; i += 256) out_bits[static_cast<size_t>(u) * kExclWords + i] = s_bits[i];
+  if (tid == 0) out_cnt[u] = total;
+}
+
 }  // namespace tt
 
 using namespace tt;
+
+extern "C" int tt_exclusions_build(const int64_t* ids, int U, int m, int ld_in, int vocab_size, int32_t* out_ids,
+                                   int ld, int32_t* out_cnt, uint32_t* out_bits, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  TT_REQUIRE(out_ids && out_cnt && out_bits && U > 0 && m >= 0 && vocab_size > 0 && ld >= m && ld >= 1 &&
+             (m == 0 || (ids && ld_in >= m)), "tt_exclusions_build: bad arguments");
+  TT_REQUIRE(m <= kExclMax, "tt_exclusions_build: %d ids per user exceed %d", m, kExclMax);
+  int n_pad = 256;
+  while (n_pad < m) n_pad <<= 1;
+  TT_CHECK_CUDA(launch_k(exclusions_build_kernel, dim3(U), dim3(256), 0, stream, ids, m, ld_in, vocab_size, n_pad,
+                         out_ids, ld, out_cnt, out_bits));
+  TT_LAUNCH_CHECK();
+  return TT_OK;
+}
 
 extern "C" int tt_users_prepare(const float* users_f32, void* users_bf16, int U, float* stats, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
@@ -926,8 +1103,9 @@ static int launch_score_topk(const void* users_bf16, const void* items_bf16, Top
   const size_t smem = 1024 + (kKB + kBStages) * kTile16K + 256;
   static bool configured = false;
   if (!configured) {
-    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
     configured = true;
   }
   const int units = p.n_ut * p.n_ranges;
@@ -945,17 +1123,30 @@ static int launch_score_topk(const void* users_bf16, const void* items_bf16, Top
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   if (p.smax != nullptr)
-    TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, score_topk_kernel<true>, tmU, tmI, p));
+    TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, score_topk_kernel<true, false>, tmU, tmI, p));
+  else if (p.ex_ids != nullptr)
+    TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, score_topk_kernel<false, true>, tmU, tmI, p));
   else
-    TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, score_topk_kernel<false>, tmU, tmI, p));
+    TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, score_topk_kernel<false, false>, tmU, tmI, p));
   TT_LAUNCH_CHECK();
   return TT_OK;
 }
 
 extern "C" int tt_score_topk(const void* users_bf16, const void* items_bf16, int item_base, const tt_topk_plan* plan,
                              void* cand, int32_t* cand_cnt, void* thr, void* smax, int mask_item0, void* stream_) {
+  return tt_score_topk_excl(users_bf16, items_bf16, item_base, plan, cand, cand_cnt, thr, smax, mask_item0, nullptr,
+                            nullptr, nullptr, 0, stream_);
+}
+
+extern "C" int tt_score_topk_excl(const void* users_bf16, const void* items_bf16, int item_base,
+                                  const tt_topk_plan* plan, void* cand, int32_t* cand_cnt, void* thr, void* smax,
+                                  int mask_item0, const int32_t* ex_ids, const int32_t* ex_cnt,
+                                  const uint32_t* ex_bits, int ex_ld, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   TT_REQUIRE(users_bf16 && items_bf16 && plan && cand && cand_cnt && thr, "tt_score_topk: null pointer");
+  const bool excl = ex_ids != nullptr;
+  TT_REQUIRE(excl == (ex_cnt != nullptr) && excl == (ex_bits != nullptr) && (!excl || ex_ld >= 1),
+             "tt_score_topk_excl: exclusion ids, counts and bits must be given together (ex_ld >= 1)");
   TopkParams p;
   p.U = plan->U; p.N = plan->N; p.item_base = item_base;
   p.n_ut = plan->n_ut;
@@ -966,6 +1157,7 @@ extern "C" int tt_score_topk(const void* users_bf16, const void* items_bf16, int
   p.cand_cnt = cand_cnt;
   p.thr = static_cast<unsigned long long*>(thr);
   p.mask_item0 = mask_item0;
+  p.ex_ids = ex_ids; p.ex_cnt = ex_cnt; p.ex_bits = ex_bits; p.ex_ld = ex_ld;
   TT_CHECK_CUDA(cudaMemsetAsync(thr, 0, static_cast<size_t>(plan->thr_bytes), stream));
 
   // ---- sample pass: chunk maxima of every sample_stride-th item step -> per-user start thresholds
@@ -981,7 +1173,7 @@ extern "C" int tt_score_topk(const void* users_bf16, const void* items_bf16, int
     p.smax = static_cast<float*>(smax);
     int rc = launch_score_topk(users_bf16, items_bf16, p, plan->N, stream);
     if (rc) return rc;
-    TT_CHECK_CUDA(launch_k(sample_threshold_kernel, dim3((plan->U * 32 + 255) / 256), dim3(256), 0, stream, p.smax, plan->U, sample_tiles * kChunks, plan->sample_rank, p.thr));
+    TT_CHECK_CUDA(launch_k(sample_threshold_kernel, dim3((plan->U * 32 + 255) / 256), dim3(256), 0, stream, p.smax, plan->U, sample_tiles * kChunks, plan->sample_rank, p.thr, ex_ids, ex_cnt, ex_ld, item_base, plan->N, plan->sample_stride, sample_tiles));
     TT_LAUNCH_CHECK();
     p.total_tiles = total_saved;
     p.smax = nullptr;
@@ -1068,13 +1260,25 @@ extern "C" int tt_topk_merge_packed(const int32_t* packed, int ld, int G, int U,
 
 extern "C" int tt_exact_topk(const float* user_f32, const float* items_f32, int N, int item_base, int mask_item0,
                              int K, void* key_scratch, float* out_score, int32_t* out_idx, void* stream_) {
+  return tt_exact_topk_excl(user_f32, items_f32, N, item_base, mask_item0, K, nullptr, nullptr, key_scratch, out_score,
+                            out_idx, stream_);
+}
+
+extern "C" int tt_exact_topk_excl(const float* user_f32, const float* items_f32, int N, int item_base, int mask_item0,
+                                  int K, const int32_t* ex_ids, const int32_t* ex_cnt, void* key_scratch,
+                                  float* out_score, int32_t* out_idx, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   TT_REQUIRE(user_f32 && items_f32 && key_scratch && out_score && out_idx && N > 0 && K > 0 && K <= 256,
              "tt_exact_topk: bad arguments");
+  TT_REQUIRE((ex_ids != nullptr) == (ex_cnt != nullptr), "tt_exact_topk_excl: exclusion ids and count go together");
   int grid = (N + 7) / 8;
   if (grid > num_sms() * 8) grid = num_sms() * 8;
   TT_CHECK_CUDA(launch_k(exact_keys_kernel, dim3(grid), dim3(256), 0, stream, user_f32, items_f32, N, item_base, mask_item0, static_cast<unsigned long long*>(key_scratch)));
   TT_LAUNCH_CHECK();
+  if (ex_ids != nullptr) {
+    TT_CHECK_CUDA(launch_k(exact_exclude_kernel, dim3(1), dim3(256), 0, stream, ex_ids, ex_cnt, N, item_base, static_cast<unsigned long long*>(key_scratch)));
+    TT_LAUNCH_CHECK();
+  }
   TT_CHECK_CUDA(launch_k(exact_select_kernel, dim3(1), dim3(256), 0, stream, static_cast<const unsigned long long*>(key_scratch), N, K, out_score, out_idx));
   TT_LAUNCH_CHECK();
   return TT_OK;

@@ -5,6 +5,9 @@ against the item index, exclusion of the padding id and of the history items, to
 metadata / printing around it stays with the caller. Everything runs on the CUDA kernels of the catalog
 retrieval path: the exclusion is applied AFTER an exact top-(k + |history|) selection, which contains the
 top-k of the non-excluded items whatever the history is.
+
+`recommend_batch` is the batched form for serving: histories of any model window, exclusion lists of up to 4096
+ids per user, sharded catalogs; the exclusion happens inside the selection kernels (`retrieval.Exclusions`).
 """
 from __future__ import annotations
 
@@ -67,3 +70,53 @@ def recommend_for_user(model, index: retrieval.CatalogIndex, history_ids: Sequen
     ex[0, :len(hist)] = torch.tensor(hist, dtype=torch.long)
     idx, score = recommend_topk(u, index, ex.to(dev), k)
     return idx[0], score[0]
+
+
+#: users per user-tower call in `recommend_batch`: bounds the tower's workspace (B = 10 k at L = 512 would otherwise
+#: size every activation buffer for all users at once)
+_TOWER_CHUNK = 1024
+
+
+def recommend_batch(model, index: retrieval.CatalogIndex, history_ids: torch.Tensor,
+                    history_mask: Optional[torch.Tensor] = None, user_gender: Optional[torch.Tensor] = None,
+                    user_country: Optional[torch.Tensor] = None, k: int = 10, exclude_ids: Optional[torch.Tensor] = None,
+                    group=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """`recommend_for_user` (src/inference.py:283-306) for a batch of B users.
+
+    ``history_ids`` (B, L) int64, L <= the model's max_seq_len, right-padded with 0; ``history_mask`` (B, L), default
+    ``history_ids != 0``; ``user_gender`` / ``user_country`` (B,), default 0. The eval-mode user tower runs in chunks of
+    1024 users, its output is re-normalised (eps 1e-8, :286), and the padding id 0 and every excluded item are
+    masked (:296-302) inside the selection kernels. The excluded items are ``exclude_ids`` (B, m) int64 (0 = empty
+    slot, m <= 4096: e.g. a full listening history longer than the tower's window) if given, otherwise the valid
+    history positions. On a sharded ``index`` the top k is taken over the whole catalog across ``group``
+    (collective: every rank passes its copy of the same users).
+
+    Returns (item ids int64 (B, k), scores fp32 (B, k)), best first in the canonical order (score descending, item id
+    ascending). When a user has fewer than k admissible items, the tail is id -1 with score -inf."""
+    chunk = _TOWER_CHUNK
+    if not 1 <= k <= 256:
+        raise ValueError(f"recommend_batch: k = {k} outside [1, 256]")
+    dev = model.engine.device
+    ids = history_ids.to(dev).long()
+    B, L = ids.shape
+    if L > model.engine.cfg.max_seq_len:
+        raise ValueError(f"history window {L} exceeds the model's max_seq_len {model.engine.cfg.max_seq_len}")
+    mask = (ids != 0).long() if history_mask is None else history_mask.to(dev).long()
+    gender = torch.zeros(B, dtype=torch.long, device=dev) if user_gender is None else user_gender.to(dev).long()
+    country = torch.zeros(B, dtype=torch.long, device=dev) if user_country is None else user_country.to(dev).long()
+    was_training = model.training
+    model.eval()
+    with torch.no_grad():
+        u = torch.cat([model.get_user_embedding(ids[s:s + chunk], mask[s:s + chunk], gender[s:s + chunk],
+                                                country[s:s + chunk]) for s in range(0, B, chunk)])
+    model.train(was_training)
+    u = F.normalize(u.float(), p=2, dim=1, eps=1e-8)                     # src/inference.py:286
+    ex = ids * (mask != 0) if exclude_ids is None else exclude_ids.to(dev).long()
+    if ex.shape[0] != B:
+        raise ValueError(f"exclude_ids has {ex.shape[0]} rows for {B} users")
+    exclude = retrieval.Exclusions(ex, index.vocab_size)
+    if index.is_sharded:
+        idx, score = retrieval.sharded_topk(u, index, k, group=group, exclude=exclude)
+    else:
+        idx, score, _ = retrieval.retrieve_topk(u, index, k, exclude=exclude)
+    return idx.long(), score

@@ -119,6 +119,52 @@ class CatalogIndex:
         return self._plans[key]
 
 
+class Exclusions:
+    """Per-user sets of item ids that retrieval must never return (a user's listening history: the masking of
+    src/inference.py:296-302), in the device form the selection kernels probe (tt_exclusions_build): a sorted,
+    de-duplicated int32 list per user, its length and a 4096-bit hashed bitmap. Build it once per batch.
+
+    ``ids`` (U, m) integer tensor, m <= 4096; 0 marks an empty slot and ids <= 0 or >= ``vocab_size`` are dropped.
+    The selection kernel drops excluded items from the candidate lists before it prunes or hands them over, so the
+    result is the exact top K of the admissible items; rows of a sharded catalog may name items of any shard."""
+
+    def __init__(self, ids: torch.Tensor, vocab_size: int):
+        assert ids.dim() == 2 and ids.is_cuda
+        U, m = ids.shape
+        if m > 4096:
+            raise ValueError(f"Exclusions: {m} ids per user exceed 4096")
+        ids = ids.long().contiguous()
+        dev = ids.device
+        self.ld = max(m, 1)
+        self.ids = torch.empty(U, self.ld, device=dev, dtype=torch.int32)
+        self.cnt = torch.empty(U, device=dev, dtype=torch.int32)
+        self.bits = torch.empty(U, 128, device=dev, dtype=torch.int32)
+        check(lib().tt_exclusions_build(ids.data_ptr(), U, m, max(m, 1), vocab_size, self.ids.data_ptr(), self.ld,
+                                        self.cnt.data_ptr(), self.bits.data_ptr(), _stream()), "tt_exclusions_build")
+
+    @property
+    def num_users(self) -> int:
+        return self.cnt.shape[0]
+
+    def rows(self, sel: torch.Tensor) -> "Exclusions":
+        """The exclusions of users ``sel`` (index tensor), in that order: no rebuild."""
+        out = Exclusions.__new__(Exclusions)
+        out.ld = self.ld
+        out.ids, out.cnt, out.bits = self.ids[sel].contiguous(), self.cnt[sel].contiguous(), self.bits[sel].contiguous()
+        return out
+
+
+def _check_exclude(exclude: Optional[Exclusions], U: int) -> None:
+    if exclude is not None and exclude.num_users != U:
+        raise ValueError(f"exclusions for {exclude.num_users} users, {U} user embeddings")
+
+
+def _exclude_kw(exclude: Optional[Exclusions]) -> dict:
+    """keyword arguments that pass ``exclude`` on only when it is set: without exclusions the sharded protocol makes
+    exactly the calls it always made"""
+    return {} if exclude is None else {"exclude": exclude}
+
+
 def exchange_buffers(index, U: int, ld: int, world: int, group=None) -> Dict[str, torch.Tensor]:
     """Reused buffers of the sharded protocol: this shard's packed rows [U, ld] int32, the gathered ones
     [world * U, ld], the certificate flags. On an NCCL group of one NVLink domain the gathered buffer lives in a
@@ -159,8 +205,10 @@ def exchange(buf: Dict[str, torch.Tensor], group=None) -> None:
 
 
 def retrieve_topk(user_emb: torch.Tensor, index: CatalogIndex, K: int, kprime: int = 256,
-                  mask_item0: bool = True, exact_fallback: bool = True, flags_out: Optional[torch.Tensor] = None):
-    """Top-K items of this shard for every user, canonical order.
+                  mask_item0: bool = True, exact_fallback: bool = True, flags_out: Optional[torch.Tensor] = None,
+                  exclude: Optional[Exclusions] = None):
+    """Top-K items of this shard for every user, canonical order; ``exclude``: per-user item ids never returned
+    (a user with fewer than K admissible items gets id -1 / score -inf in the tail).
 
     Returns (idx int32 (U, K) global item ids, score fp32 (U, K), n_fallback). Scores are the
     exact fp32 dot products (fp64-accumulated, rounded once). Users whose exactness certificate
@@ -171,7 +219,8 @@ def retrieve_topk(user_emb: torch.Tensor, index: CatalogIndex, K: int, kprime: i
     user_emb = user_emb.contiguous()
     U = user_emb.shape[0]
     kprime = max(kprime, K)
-    plan, sc = _score_pass(user_emb, index, kprime, mask_item0)
+    _check_exclude(exclude, U)
+    plan, sc = _score_pass(user_emb, index, kprime, mask_item0, exclude)
     dev = user_emb.device
     out_idx = torch.empty(U, K, device=dev, dtype=torch.int32)
     out_score = torch.empty(U, K, device=dev, dtype=torch.float32)
@@ -190,13 +239,17 @@ def retrieve_topk(user_emb: torch.Tensor, index: CatalogIndex, K: int, kprime: i
             if sc["keys"] is None:
                 sc["keys"] = torch.empty(index.num_rows, device=dev, dtype=torch.int64)
             for u in bad:
-                check(lib().tt_exact_topk(user_emb[u].data_ptr(), index.table.data_ptr(), index.num_rows,
-                                          index.item_base, int(mask_item0), K, sc["keys"].data_ptr(),
-                                          out_score[u].data_ptr(), out_idx[u].data_ptr(), _stream()), "tt_exact_topk")
+                ex_ids, ex_cnt = (None, None) if exclude is None else (exclude.ids[u].data_ptr(),
+                                                                       exclude.cnt[u:].data_ptr())
+                check(lib().tt_exact_topk_excl(user_emb[u].data_ptr(), index.table.data_ptr(), index.num_rows,
+                                               index.item_base, int(mask_item0), K, ex_ids, ex_cnt,
+                                               sc["keys"].data_ptr(), out_score[u].data_ptr(), out_idx[u].data_ptr(),
+                                               _stream()), "tt_exact_topk_excl")
     return out_idx, out_score, n_fallback
 
 
-def _score_pass(user_emb: torch.Tensor, index: "CatalogIndex", kprime: int, mask_item0: bool):
+def _score_pass(user_emb: torch.Tensor, index: "CatalogIndex", kprime: int, mask_item0: bool,
+                exclude: Optional[Exclusions] = None):
     """bf16 scoring + streaming candidate selection of this shard (tt_score_topk); returns (plan, scratch).
     The user-side terms of the certificate's error bound (max ||bf16(u) - u||, max ||u||) are reduced on the device by
     the cast kernel into scratch['eps_stats'] and combined with the index's item-side terms inside the finalize kernel
@@ -207,26 +260,30 @@ def _score_pass(user_emb: torch.Tensor, index: "CatalogIndex", kprime: int, mask
     sc = index._scratch[(U, kprime)]
     check(lib().tt_users_prepare(user_emb.data_ptr(), sc["users_bf16"].data_ptr(), U, sc["eps_stats"].data_ptr(),
                                  _stream()), "tt_users_prepare")
-    check(lib().tt_score_topk(sc["users_bf16"].data_ptr(), index.table_bf16.data_ptr(), index.item_base,
-                              ctypes.byref(plan), sc["cand"].data_ptr(), sc["cnt"].data_ptr(), sc["thr"].data_ptr(),
-                              None if sc["smax"] is None else sc["smax"].data_ptr(), int(mask_item0), _stream()),
-          "tt_score_topk")
+    ex = (None, None, None, 0) if exclude is None else (exclude.ids.data_ptr(), exclude.cnt.data_ptr(),
+                                                         exclude.bits.data_ptr(), exclude.ld)
+    check(lib().tt_score_topk_excl(sc["users_bf16"].data_ptr(), index.table_bf16.data_ptr(), index.item_base,
+                                   ctypes.byref(plan), sc["cand"].data_ptr(), sc["cnt"].data_ptr(),
+                                   sc["thr"].data_ptr(), None if sc["smax"] is None else sc["smax"].data_ptr(),
+                                   int(mask_item0), *ex, _stream()), "tt_score_topk_excl")
     return plan, sc
 
 
 def retrieve_candidates(user_emb: torch.Tensor, index: "CatalogIndex", kprime: int, mask_item0: bool = True,
-                        pack: Optional[torch.Tensor] = None):
+                        pack: Optional[torch.Tensor] = None, exclude: Optional[Exclusions] = None):
     """Sharded catalogs: ALL ``kprime`` candidates of this shard per user, re-scored exactly.
 
     Returns (idx int32 (U, kprime) global ids, -1 padded; score fp32 (U, kprime); bound fp32 (U,): every item of
     the shard that is not in the list has exact score <= bound; overflow int32 (U,): 1 = tie flood, use the exact
     path). With G shards a shard needs about 1/G of the single-GPU candidate budget (`shard_kprime`).
     ``pack`` int32 (U, >= 2 * kprime + 2): the kernel writes the exchange layout [scores | ids | bound | flag] of
-    `sharded_topk` directly and the four results are views of it."""
+    `sharded_topk` directly and the four results are views of it. ``exclude``: as in `retrieve_topk`; the lists and
+    bounds then cover the admissible items only."""
     assert user_emb.is_cuda and user_emb.dtype == torch.float32 and user_emb.shape[1] == 256
     user_emb = user_emb.contiguous()
     U = user_emb.shape[0]
-    plan, sc = _score_pass(user_emb, index, kprime, mask_item0)
+    _check_exclude(exclude, U)
+    plan, sc = _score_pass(user_emb, index, kprime, mask_item0, exclude)
     dev = user_emb.device
     if pack is None:
         pack = torch.empty(U, 2 * kprime + 2, device=dev, dtype=torch.int32)
@@ -272,14 +329,15 @@ def merge_bounded(scores: torch.Tensor, idx: torch.Tensor, bounds: torch.Tensor,
 
 
 def sharded_topk(user_emb: torch.Tensor, index: "CatalogIndex", K: int, kprime: int = 256, group=None,
-                 bounded: Optional[bool] = None, defer_check: bool = False):
+                 bounded: Optional[bool] = None, defer_check: bool = False, exclude: Optional[Exclusions] = None):
     """Exact global top K over a catalog sharded across the ranks of ``group`` (every rank gets the result).
 
     bounded protocol (default from 4 shards): per-shard candidate lists of `shard_kprime` entries +
     completeness bounds, one all-gather, merge + certificate; users whose certificate fails (and only those) go
     through the per-shard exact top-K protocol. ``bounded=False`` (default below 4 shards) always uses the latter.
     ``defer_check=True`` (bounded protocol only) returns (idx, score, bad) without reading the certificate back:
-    the caller checks ``bad`` together with its own read-back and calls `finish_sharded_topk` if any flag is set."""
+    the caller checks ``bad`` together with its own read-back and calls `finish_sharded_topk` if any flag is set.
+    ``exclude`` (`Exclusions` of these users, built against the global vocabulary): never return those items."""
     import torch.distributed as dist
     ws = dist.get_world_size(group)
     index.check_group(user_emb.shape[0], group)
@@ -291,7 +349,7 @@ def sharded_topk(user_emb: torch.Tensor, index: "CatalogIndex", K: int, kprime: 
         bounded = (ws >= 4) if env == "" else (env != "0")
 
     def per_shard_exact(users):
-        i, s, _ = retrieve_topk(users, index, K, kprime)
+        i, s, _ = retrieve_topk(users, index, K, kprime, **_exclude_kw(exclude))
         n = s.shape[0]
         # one exchange of [scores | ids | bound = -inf | flag = 0] rows, merged in place like the bounded protocol
         # (every shard's list IS its exact top K, so the certificate is trivially satisfied)
@@ -315,13 +373,13 @@ def sharded_topk(user_emb: torch.Tensor, index: "CatalogIndex", K: int, kprime: 
     buf = exchange_buffers(index, U, _pitch(kps), ws, group)
     # the finalize kernel writes this shard's lists, bounds and flags in the exchange layout; ONE all-gather; the merge
     # kernel reads the gathered buffer in place and emits the certificate
-    retrieve_candidates(user_emb, index, kps, pack=buf["pack"])
+    retrieve_candidates(user_emb, index, kps, pack=buf["pack"], **_exclude_kw(exclude))
     exchange(buf, group)
     bad = buf["bad"]
     out_i, out_s = merge_packed(buf["all"], ws, U, kps, K, bad)
     if defer_check:
         return out_i, out_s, bad
-    finish_sharded_topk(user_emb, index, K, out_i, out_s, bad, kprime, group)
+    finish_sharded_topk(user_emb, index, K, out_i, out_s, bad, kprime, group, exclude)
     return out_i, out_s
 
 
@@ -335,7 +393,8 @@ def merge_packed(allp: torch.Tensor, G: int, U: int, kps: int, K: int, bad: torc
     return out_i, out_s
 
 
-def finish_sharded_topk(user_emb, index, K, out_i, out_s, bad, kprime: int = 256, group=None) -> int:
+def finish_sharded_topk(user_emb, index, K, out_i, out_s, bad, kprime: int = 256, group=None,
+                        exclude: Optional[Exclusions] = None) -> int:
     """Second half of the bounded protocol: users whose merged list is not certified (`bad`, identical on every rank
     because it was computed from all-gathered data) go through the per-shard exact top-K + merge, in place. One host
     read of the flags; returns the number of such users. Collective."""
@@ -351,7 +410,7 @@ def finish_sharded_topk(user_emb, index, K, out_i, out_s, bad, kprime: int = 256
     # a long evaluation with a few uncertified users per batch does not accumulate one scratch set per count
     padded = torch.cat([sel, sel[:1].expand((-n) % 256)])
     users = user_emb[padded].contiguous()
-    i, s, _ = retrieve_topk(users, index, K, kprime)
+    i, s, _ = retrieve_topk(users, index, K, kprime, **_exclude_kw(None if exclude is None else exclude.rows(padded)))
     m = s.shape[0]
     all_s = torch.empty(ws * m, K, device=s.device, dtype=s.dtype)
     all_i = torch.empty(ws * m, K, device=i.device, dtype=i.dtype)
