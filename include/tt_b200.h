@@ -95,7 +95,9 @@ int tt_gemm_bf16(const tt_gemm_args* args, void* stream);
  *   ctx  : bf16 [B*L, H*64]     attention output before out_proj
  *   lse  : fp32 [B, H, L]       natural-log sum-exp of the scaled scores (for backward)
  * Dropout (p > 0) is applied to the attention probabilities with the counter-based hash
- * (seed + *seed_dev, site, ((b*H+h)*L+i)*L+j). L <= 512.
+ * (seed + *seed_dev, site, ((b*H+h)*L+i)*L+j). L <= 4096: L <= 512 keeps every tile of a sequence on chip;
+ * 512 < L <= 4096 runs the tiled kernels (online-softmax forward; a deterministic backward in two kernels, one per key
+ * tile for dK / dV and one per query tile for dQ), which hash the element index in 64 bits. B*L <= 2^31 - 1.
  */
 int tt_attn_causal_fwd(const void* qkv, void* ctx, float* lse, int B, int L, int H, float drop_p,
                        uint64_t drop_seed, const uint64_t* drop_seed_dev, uint32_t drop_site, void* stream);
@@ -280,6 +282,7 @@ int tt_step_counters_advance(int64_t* step_dev, uint64_t* seed_dev, void* stream
  *                         lse fp32 [B, H]; keys 0..last_idx[b]
  *   tt_attn_lastq_bwd   : -> dq bf16 [B, H*64] and the K/V thirds of dqkv for EVERY position
  *                         (zeros beyond last_idx[b])
+ *                         L <= 4096 for both.
  */
 int tt_gather_rows(const float* x_f32, const void* x_bf16, const int32_t* last_idx, int B, int L, int W,
                    float* out_f32, void* out_bf16, void* stream);

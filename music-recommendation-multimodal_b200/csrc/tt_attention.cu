@@ -1472,6 +1472,582 @@ attn_bwd_persist_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_
   if (warp == 16) tmem_dealloc(tmem_base, 512);
 }
 
+// ============================================================================================
+// Long histories, 512 < L <= 4096. The kernels above keep every S tile (forward) or every dQ accumulator (backward)
+// of a sequence in TMEM, which caps L at 512. The kernels below walk the key / query tiles of one 128-row tile with
+// TMEM and shared memory that do not depend on L. Dropout hashes the 64-bit element index ((b*H + h)*L + q)*L + k
+// (B*H*L^2 passes 2^32 from B = 65 at L = 4096), exactly as drop_keep_k and the single-query kernels do.
+// ============================================================================================
+static constexpr int kLongMaxL = 4096;
+
+__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&r)[8]) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];\n"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+               : "r"(taddr)
+               : "memory");
+}
+
+// drop_keepmask32 for a 64-bit element index
+__device__ __forceinline__ uint32_t drop_keepmask32_64(uint32_t dkey, uint64_t didx0, uint32_t thresh) {
+  uint32_t keepmask = 0u;
+  if ((didx0 & 3u) == 0u) {
+#pragma unroll
+    for (int t = 0; t < 32; t += 4) {
+      bool k[4];
+      drop_keep_quad64(dkey, didx0 + t, thresh, k);
+#pragma unroll
+      for (int e = 0; e < 4; ++e) keepmask |= (k[e] ? 1u : 0u) << (t + e);
+    }
+  } else if ((didx0 & 1u) == 0u) {
+#pragma unroll
+    for (int t = 0; t < 32; t += 2) {
+      bool k0, k1;
+      drop_keep_pair64(dkey, didx0 + t, thresh, k0, k1);
+      keepmask |= (k0 ? 1u : 0u) << t;
+      keepmask |= (k1 ? 1u : 0u) << (t + 1);
+    }
+  } else {
+#pragma unroll
+    for (int t = 0; t < 32; ++t) keepmask |= (drop_keep_k(dkey, didx0 + t, thresh) ? 1u : 0u) << t;
+  }
+  return keepmask;
+}
+
+// Forward, L > 512. One CTA (256 threads) per (sequence, head, 128-row query tile), heavy tiles first; thread (row,
+// hf) as in attn_fwd_kernel. Online softmax over the key tiles j = 0..qt:
+//   S_j = Q K_j^T -> TMEM columns [0, 128); the row max of S_j raises the running max m;
+//   P_j = dropout(exp2((S_j - m) * scale * log2e)) -> bf16, 128B-swizzled smem tile; O_j = P_j V_j -> TMEM columns
+//   [128, 192), a fresh accumulator per tile;
+//   O_{j-1} is folded into the thread's 32 output columns in registers (O = O * exp2((m_old - m_new) * c) + O_{j-1})
+//   while S_{j+1} and P_j V_j are under way.
+// TMEM: 256 columns. Shared memory: Q, K, V[2], P (two 64-column chunks) = 96 KB. Two CTAs per SM. K_{j+1} is
+// requested once S_j has retired, V_{j+1} once P_{j-1} V_{j-1} has.
+__global__ void __launch_bounds__(256, 2)
+attn_fwd_long_kernel(const __grid_constant__ CUtensorMap tmQKV, const AttnParams p) {
+  extern __shared__ uint8_t smem_raw[];
+  const uint32_t pad = (1024u - (smem_u32(smem_raw) & 1023u)) & 1023u;
+  uint8_t* smem = smem_raw + pad;
+
+  const int tid = threadIdx.x;
+  const int warp = tid >> 5, lane = tid & 31;
+  const int q = warp & 3, hf = warp >> 2;
+  const int row = q * 32 + lane;
+  const int bh_count = p.B * p.H;
+  const int qt = p.nq - 1 - static_cast<int>(blockIdx.x) / bh_count;  // heavy tiles first
+  const int bh = static_cast<int>(blockIdx.x) % bh_count;
+  const int b = bh / p.H, h = bh % p.H;
+  const int n_kv = qt + 1;
+  const int D = p.H * kDh;
+  constexpr uint32_t kCols = 256, T_O = 128;
+
+  uint8_t* sQ = smem;
+  uint8_t* sK = sQ + kTileBytes;
+  uint8_t* sV = sK + kTileBytes;          // [2]
+  uint8_t* sP = sV + 2 * kTileBytes;      // 2 chunks
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sP + 2 * kTileBytes);
+  uint64_t* bar_k = bars + 0;    // Q + K_0, then K_j: phase j
+  uint64_t* bar_v = bars + 1;    // [2] V slot j & 1: phase j >> 1
+  uint64_t* bar_s = bars + 3;    // S_j retired: phase j
+  uint64_t* bar_pv = bars + 4;   // P_j V_j retired: phase j
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 5);
+  float* s_red = reinterpret_cast<float*>(bars + 6);  // [2][128]
+
+  if (tid == 0) {
+    tma_prefetch_desc(&tmQKV);
+    for (int i = 0; i < 5; ++i) mbar_init(bars + i, 1);
+    fence_barrier_init();
+  }
+  __syncwarp();
+  if (warp == 0) {
+    tmem_alloc(tmem_slot, kCols);
+    tmem_relinquish();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+  pdl_launch_dependents();
+  pdl_wait();
+
+  const int seq_row0 = b * p.L;
+  const uint32_t idesc_s = umma_idesc_bf16(kTile, kTile, false, false);
+  const uint32_t idesc_pv = umma_idesc_bf16(kTile, kDh, false, true);
+  const uint64_t q_desc = umma_desc_kmajor(smem_u32(sQ));
+  const uint64_t k_desc = umma_desc_kmajor(smem_u32(sK));
+  auto issue_s = [&]() {
+#pragma unroll
+    for (int k = 0; k < kDh / 16; ++k)
+      umma_bf16(tmem_base, q_desc + (k * 32 >> 4), k_desc + (k * 32 >> 4), idesc_s, k > 0 ? 1u : 0u);
+    umma_commit(bar_s);
+  };
+  auto load_v = [&](int j) {
+    mbar_arrive_expect_tx(bar_v + (j & 1), kTileBytes);
+    tma_load_2d(sV + static_cast<size_t>(j & 1) * kTileBytes, &tmQKV, bar_v + (j & 1), 2 * D + h * kDh,
+                seq_row0 + j * kTile);
+  };
+  if (tid == 0) {
+    mbar_arrive_expect_tx(bar_k, 2 * kTileBytes);
+    tma_load_2d(sQ, &tmQKV, bar_k, h * kDh, seq_row0 + qt * kTile);
+    tma_load_2d(sK, &tmQKV, bar_k, D + h * kDh, seq_row0);
+    load_v(0);
+    if (n_kv > 1) load_v(1);
+    mbar_wait(bar_k, 0);
+    tc_fence_after();
+    issue_s();
+  }
+
+  const uint32_t lane_base = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
+  const int q_pos = qt * kTile + row;
+  const bool dead_rows = qt * kTile + q * 32 >= p.L;   // warp-uniform: all 32 rows beyond the sequence
+  const float c1 = p.scale * kLog2e;
+  const uint64_t seed = p.drop_seed + ((p.drop_thresh && p.drop_seed_dev) ? *p.drop_seed_dev : 0ull);
+  const uint32_t dkey = drop_key(seed, p.drop_site);
+  const uint64_t didx_row = (static_cast<uint64_t>(bh) * p.L + q_pos) * p.L;
+  uint8_t* chunk = sP + static_cast<size_t>(hf) * kTileBytes;
+  float m = -INFINITY;      // running row max of the raw scores
+  float l = 0.f;            // this thread's half of the row sum, relative to m
+  float m_o = -INFINITY;    // the max that o[] is relative to
+  float o[32];
+#pragma unroll
+  for (int t = 0; t < 32; ++t) o[t] = 0.f;
+  // o = o * exp2((m_o - m_new) * c1) + (the thread's 32 columns of P_{j} V_{j}, relative to m_new)
+  auto fold = [&](float m_new) {
+    uint32_t r[32];
+    tmem_ld32(lane_base + T_O + hf * 32, r);
+    tmem_ld_wait();
+    const float a = fast_exp2((m_o - m_new) * c1);
+#pragma unroll
+    for (int t = 0; t < 32; ++t) o[t] = fmaf(o[t], a, __uint_as_float(r[t]));
+    m_o = m_new;
+  };
+
+  for (int j = 0; j < n_kv; ++j) {
+    const bool diag = (j == qt);
+    mbar_wait(bar_s, j & 1);
+    __syncwarp();
+    tc_fence_after();
+    if (tid == 0 && j + 1 < n_kv) {   // S_j retired: the K slot is free
+      mbar_arrive_expect_tx(bar_k, kTileBytes);
+      tma_load_2d(sK, &tmQKV, bar_k, D + h * kDh, seq_row0 + (j + 1) * kTile);
+    }
+    // ---- row max of S_j (each thread: its column half) ----
+    float mt = -INFINITY;
+    if (!dead_rows) {
+#pragma unroll
+      for (int cc = 0; cc < 2; ++cc) {
+        const int cg = 2 * hf + cc;
+        const int kv0 = j * kTile + cg * 32;
+        if ((diag && cg > q) || kv0 >= p.L) continue;
+        uint32_t r[32];
+        tmem_ld32(lane_base + cg * 32, r);
+        tmem_ld_wait();
+#pragma unroll
+        for (int t = 0; t < 32; ++t)
+          if (!diag || kv0 + t <= q_pos) mt = fmaxf(mt, __uint_as_float(r[t]));
+      }
+    }
+    s_red[hf * 128 + row] = mt;
+    __syncthreads();
+    const float m_prev = m;
+    m = fmaxf(m, fmaxf(s_red[row], s_red[128 + row]));
+    // ---- P_{j-1} V_{j-1} retired: fold it in; the P tile and its V slot are free ----
+    if (j >= 1) {
+      mbar_wait(bar_pv, (j - 1) & 1);
+      __syncwarp();
+      tc_fence_after();
+      if (!dead_rows) fold(m_prev);
+    }
+    const float mc = m * c1;
+    if (!dead_rows) l *= fast_exp2((m_prev - m) * c1);
+    // ---- P_j -> shared memory ----
+#pragma unroll
+    for (int cc = 0; cc < 2; ++cc) {
+      const int cg = 2 * hf + cc;
+      const int u0 = cc * 4;
+      const int kv0 = j * kTile + cg * 32;
+      if (!((diag && cg > q) || dead_rows || kv0 >= p.L)) {
+        uint32_t r[32];
+        tmem_ld32(lane_base + cg * 32, r);
+        tmem_ld_wait();
+        const uint32_t keep = p.drop_thresh ? drop_keepmask32_64(dkey, didx_row + kv0, p.drop_thresh) : 0xFFFFFFFFu;
+        float pv[32];
+#pragma unroll
+        for (int t = 0; t < 32; ++t) {
+          float e = fast_exp2(__uint_as_float(r[t]) * c1 - mc);
+          if (diag && kv0 + t > q_pos) e = 0.f;
+          l += e;
+          pv[t] = ((keep >> t) & 1u) ? e * p.drop_scale : 0.f;
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          uint4 v;
+          v.x = pack_bf16(pv[u * 8 + 0], pv[u * 8 + 1]);
+          v.y = pack_bf16(pv[u * 8 + 2], pv[u * 8 + 3]);
+          v.z = pack_bf16(pv[u * 8 + 4], pv[u * 8 + 5]);
+          v.w = pack_bf16(pv[u * 8 + 6], pv[u * 8 + 7]);
+          st_swizzled_unit(chunk, row, u0 + u, v);
+        }
+      } else {
+#pragma unroll
+        for (int u = 0; u < 4; ++u) st_swizzled_unit(chunk, row, u0 + u, make_uint4(0, 0, 0, 0));
+      }
+    }
+    fence_proxy_async_smem();
+    tc_fence_before();
+    __syncthreads();
+    if (tid == 0) {
+      tc_fence_after();
+      if (j + 1 < n_kv) {
+        mbar_wait(bar_k, (j + 1) & 1);
+        tc_fence_after();
+        issue_s();
+        if (j >= 1) load_v(j + 1);   // P_{j-1} V_{j-1} retired: slot (j + 1) & 1 is free
+      }
+      mbar_wait(bar_v + (j & 1), (j >> 1) & 1);
+      tc_fence_after();
+      const uint64_t p_desc = umma_desc_kmajor(smem_u32(sP));
+      const uint64_t v_desc = umma_desc_mnmajor(smem_u32(sV + static_cast<size_t>(j & 1) * kTileBytes), kTileBytes);
+#pragma unroll
+      for (int k = 0; k < kTile / 16; ++k)
+        umma_bf16(tmem_base + T_O, p_desc + (((k >> 2) * kTileBytes + (k & 3) * 32) >> 4), v_desc + (k * 2048 >> 4),
+                  idesc_pv, k > 0 ? 1u : 0u);
+      umma_commit(bar_pv);
+    }
+  }
+
+  // ---- epilogue: O / l -> ctx, log-sum-exp -> lse ----
+  mbar_wait(bar_pv, (n_kv - 1) & 1);
+  __syncwarp();
+  tc_fence_after();
+  if (!dead_rows) fold(m);
+  s_red[hf * 128 + row] = l;
+  __syncthreads();
+  l = s_red[row] + s_red[128 + row];
+  if (q_pos < p.L) {
+    const float inv_l = 1.f / l;
+    uint32_t r[32];
+#pragma unroll
+    for (int t = 0; t < 32; ++t) r[t] = __float_as_uint(o[t] * inv_l);
+    store_row32_bf16(p.ctx + static_cast<size_t>(seq_row0 + q_pos) * D + h * kDh + hf * 32, r);
+    if (hf == 0 && p.lse) p.lse[static_cast<size_t>(bh) * p.L + q_pos] = m * p.scale + __logf(l);
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 0) tmem_dealloc(tmem_base, kCols);
+}
+
+// Backward, L > 512: two kernels, no atomics, so dqkv is the same bit for bit from run to run.
+//   DQ = false: one CTA per (sequence, head, key tile j) walks the query tiles i = j..nq-1 and accumulates dV_j, dK_j;
+//   DQ = true:  one CTA per (sequence, head, query tile i) walks the key tiles j = 0..i and accumulates dQ_i.
+// Both recompute S = Q_i K_j^T and dP = dO_i V_j^T and form P, Pd and dS exactly as attn_bwd_kernel does, so the two
+// halves of the gradient see the same dS. The tile of the CTA (K_j / V_j, or Q_i / dO_i) stays in shared memory, the
+// walked tiles stream through two slots. Warp roles as in attn_bwd_persist_kernel:
+//   * warps 0-15: the element-wise phase, thread (row, 32-column chunk); they arrive at bar_drain once S / dP of the
+//     iteration sit in registers, so the next iteration's S / dP MMAs run under the element-wise phase;
+//   * warp 16, one lane: TMA loads and MMAs;
+//   * warp 17: delta_i = rowsum(dO_i * O_i) and the log-sum-exps of the coming query tile, double-buffered (DQ: once,
+//     the query tile is fixed). O_i arrives by TMA with the walked dO_i (DQ: with the CTA's own tiles), so delta is
+//     formed from shared memory.
+// TMEM: S [0,128), dP [128,256), accumulators [256,384); 512 allocated, one CTA per SM.
+static constexpr int kLongBwdThreads = kBwdComputeThreads + 64;
+
+template <bool DQ>
+__global__ void __launch_bounds__(kLongBwdThreads, 1)
+attn_bwd_long_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmDO,
+                     const __grid_constant__ CUtensorMap tmO, const AttnBwdParams p) {
+  extern __shared__ uint8_t smem_raw[];
+  const uint32_t pad = (1024u - (smem_u32(smem_raw) & 1023u)) & 1023u;
+  uint8_t* smem = smem_raw + pad;
+
+  const int tid = threadIdx.x;
+  const int warp = tid >> 5, lane = tid & 31;
+  const int D = p.H * kDh;
+  const int bh_count = p.B * p.H;
+  const int tile = DQ ? p.nq - 1 - static_cast<int>(blockIdx.x) / bh_count   // heavy tiles first
+                      : static_cast<int>(blockIdx.x) / bh_count;
+  const int bh = static_cast<int>(blockIdx.x) % bh_count;
+  const int b = bh / p.H, h = bh % p.H;
+  const int n_it = DQ ? tile + 1 : p.nq - tile;
+  const int seq_row0 = b * p.L;
+  // iteration it: query tile i, key tile j
+  auto qtile = [&](int it) { return DQ ? tile : tile + it; };
+  auto ktile = [&](int it) { return DQ ? it : tile; };
+
+  uint8_t* sF = smem;                        // [2] the CTA's own tiles: K_j, V_j (DQ: Q_i, dO_i)
+  uint8_t* sX = sF + 2 * kTileBytes;         // [2 slots] walked Q_i (DQ: K_j)
+  uint8_t* sY = sX + 2 * kTileBytes;         // [2 slots] walked dO_i (DQ: V_j)
+  uint8_t* sDS = sY + 2 * kTileBytes;        // 2 chunks
+  uint8_t* sPd = sDS + 2 * kTileBytes;       // 2 chunks (not DQ)
+  uint8_t* sO = sPd + (DQ ? 0 : 2) * kTileBytes;   // [2 slots] O_i of the walked query tiles (DQ: [1], the own one)
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sO + (DQ ? 1 : 2) * kTileBytes);
+  uint64_t* bar_fix = bars + 0;    // own tiles landed
+  uint64_t* bar_ld = bars + 1;     // [2] slot it & 1 landed: phase it >> 1
+  uint64_t* bar_mm1 = bars + 3;    // S / dP of iteration it ready
+  uint64_t* bar_drain = bars + 4;  // every compute thread holds S / dP of iteration it
+  uint64_t* bar_stage = bars + 5;  // Pd / dS of iteration it staged
+  uint64_t* bar_mm2 = bars + 6;    // accumulator MMAs of iteration it retired
+  uint64_t* bar_dfull = bars + 7;  // [2] delta / lse buffer filled
+  uint64_t* bar_dfree = bars + 9;  // [2] delta / lse buffer read
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 11);
+  float* sDelta = reinterpret_cast<float*>(bars + 12);  // [2][128]
+  float* sLse = sDelta + 2 * kTile;                     // [2][128], times log2e
+
+  if (tid == 0) {
+    tma_prefetch_desc(&tmQKV);
+    tma_prefetch_desc(&tmDO);
+    tma_prefetch_desc(&tmO);
+    for (int i = 0; i < 4; ++i) mbar_init(bars + i, 1);
+    mbar_init(bar_drain, kBwdComputeThreads);
+    mbar_init(bar_stage, kBwdComputeThreads);
+    mbar_init(bar_mm2, 1);
+    mbar_init(bar_dfull + 0, 32);
+    mbar_init(bar_dfull + 1, 32);
+    mbar_init(bar_dfree + 0, kBwdComputeThreads);
+    mbar_init(bar_dfree + 1, kBwdComputeThreads);
+    fence_barrier_init();
+  }
+  __syncwarp();
+  if (warp == 16) {
+    tmem_alloc(tmem_slot, 512);
+    tmem_relinquish();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+  pdl_launch_dependents();
+  pdl_wait();
+  constexpr uint32_t T_S = 0, T_DP = 128, T_ACC = 256;   // dV_j | dK_j, or dQ_i
+
+  if (warp >= 16) {
+    if (warp == 16) {
+      // ======================= issuer: TMA loads and MMAs, one lane ==============================
+      if (lane == 0) {
+        const uint32_t idesc_s = umma_idesc_bf16(kTile, kTile, false, false);    // Q K^T, dO V^T
+        const uint32_t idesc_t = umma_idesc_bf16(kTile, kDh, true, true);        // X^T Y (dV, dK)
+        const uint32_t idesc_q = umma_idesc_bf16(kTile, kDh, false, true);       // dS K
+        auto load_walk = [&](int it) {
+          const int s = it & 1;
+          mbar_arrive_expect_tx(bar_ld + s, (DQ ? 2 : 3) * kTileBytes);
+          if (DQ) {
+            const int j = ktile(it);
+            tma_load_2d(sX + static_cast<size_t>(s) * kTileBytes, &tmQKV, bar_ld + s, D + h * kDh, seq_row0 + j * kTile);
+            tma_load_2d(sY + static_cast<size_t>(s) * kTileBytes, &tmQKV, bar_ld + s, 2 * D + h * kDh, seq_row0 + j * kTile);
+          } else {
+            const int i = qtile(it);
+            tma_load_2d(sX + static_cast<size_t>(s) * kTileBytes, &tmQKV, bar_ld + s, h * kDh, seq_row0 + i * kTile);
+            tma_load_2d(sY + static_cast<size_t>(s) * kTileBytes, &tmDO, bar_ld + s, h * kDh, seq_row0 + i * kTile);
+            tma_load_2d(sO + static_cast<size_t>(s) * kTileBytes, &tmO, bar_ld + s, h * kDh, seq_row0 + i * kTile);
+          }
+        };
+        mbar_arrive_expect_tx(bar_fix, (DQ ? 3 : 2) * kTileBytes);
+        if (DQ) {
+          tma_load_2d(sF, &tmQKV, bar_fix, h * kDh, seq_row0 + tile * kTile);
+          tma_load_2d(sF + kTileBytes, &tmDO, bar_fix, h * kDh, seq_row0 + tile * kTile);
+          tma_load_2d(sO, &tmO, bar_fix, h * kDh, seq_row0 + tile * kTile);
+        } else {
+          tma_load_2d(sF, &tmQKV, bar_fix, D + h * kDh, seq_row0 + tile * kTile);
+          tma_load_2d(sF + kTileBytes, &tmQKV, bar_fix, 2 * D + h * kDh, seq_row0 + tile * kTile);
+        }
+        load_walk(0);
+        if (n_it > 1) load_walk(1);
+        // Q, dO, K, V of iteration it (slot it & 1)
+        auto tq = [&](int it) { return smem_u32(DQ ? sF : sX + static_cast<size_t>(it & 1) * kTileBytes); };
+        auto tdo = [&](int it) { return smem_u32(DQ ? sF + kTileBytes : sY + static_cast<size_t>(it & 1) * kTileBytes); };
+        auto tk = [&](int it) { return smem_u32(DQ ? sX + static_cast<size_t>(it & 1) * kTileBytes : sF); };
+        auto tv = [&](int it) { return smem_u32(DQ ? sY + static_cast<size_t>(it & 1) * kTileBytes : sF + kTileBytes); };
+        auto issue_mm1 = [&](int it) {
+          const uint64_t dq = umma_desc_kmajor(tq(it)), dd = umma_desc_kmajor(tdo(it));
+          const uint64_t dk = umma_desc_kmajor(tk(it)), dv = umma_desc_kmajor(tv(it));
+#pragma unroll
+          for (int k = 0; k < kDh / 16; ++k)
+            umma_bf16(tmem_base + T_S, dq + (k * 32 >> 4), dk + (k * 32 >> 4), idesc_s, k > 0 ? 1u : 0u);
+#pragma unroll
+          for (int k = 0; k < kDh / 16; ++k)
+            umma_bf16(tmem_base + T_DP, dd + (k * 32 >> 4), dv + (k * 32 >> 4), idesc_s, k > 0 ? 1u : 0u);
+          umma_commit(bar_mm1);
+        };
+        auto issue_mm2 = [&](int it) {
+          const uint32_t acc = it > 0 ? 1u : 0u;
+          if (DQ) {
+            const uint64_t ddsk = umma_desc_kmajor(smem_u32(sDS));
+            const uint64_t dk = umma_desc_mnmajor(tk(it), kTileBytes);
+#pragma unroll
+            for (int k = 0; k < kTile / 16; ++k)   // dQ_i += dS K_j
+              umma_bf16(tmem_base + T_ACC, ddsk + (((k >> 2) * kTileBytes + (k & 3) * 32) >> 4), dk + (k * 2048 >> 4),
+                        idesc_q, (acc || k > 0) ? 1u : 0u);
+          } else {
+            const uint64_t dpd = umma_desc_mnmajor(smem_u32(sPd), kTileBytes);
+            const uint64_t dds = umma_desc_mnmajor(smem_u32(sDS), kTileBytes);
+            const uint64_t dq = umma_desc_mnmajor(tq(it), kTileBytes);
+            const uint64_t dd = umma_desc_mnmajor(tdo(it), kTileBytes);
+#pragma unroll
+            for (int k = 0; k < kTile / 16; ++k)   // dV_j += Pd^T dO_i
+              umma_bf16(tmem_base + T_ACC, dpd + (k * 2048 >> 4), dd + (k * 2048 >> 4), idesc_t, (acc || k > 0) ? 1u : 0u);
+#pragma unroll
+            for (int k = 0; k < kTile / 16; ++k)   // dK_j += dS^T Q_i
+              umma_bf16(tmem_base + T_ACC + kDh, dds + (k * 2048 >> 4), dq + (k * 2048 >> 4), idesc_t,
+                        (acc || k > 0) ? 1u : 0u);
+          }
+          umma_commit(bar_mm2);
+        };
+        mbar_wait(bar_fix, 0);
+        mbar_wait(bar_ld + 0, 0);
+        tc_fence_after();
+        issue_mm1(0);
+        for (int it = 0; it < n_it; ++it) {
+          mbar_wait(bar_drain, it & 1);          // S / dP(it) sit in registers: their columns are free
+          tc_fence_after();
+          if (it + 1 < n_it) {
+            mbar_wait(bar_ld + ((it + 1) & 1), ((it + 1) >> 1) & 1);
+            tc_fence_after();
+            issue_mm1(it + 1);
+          }
+          mbar_wait(bar_stage, it & 1);
+          tc_fence_after();
+          issue_mm2(it);
+          mbar_wait(bar_mm2, it & 1);            // slot it & 1 is read for the last time
+          if (it + 2 < n_it) load_walk(it + 2);
+        }
+      }
+    } else {
+      // ======================= warp 17: delta / lse of the coming query tiles ====================
+      const int n_fill = DQ ? 1 : n_it;
+      for (int it = 0; it < n_fill; ++it) {
+        const int s = it & 1;
+        if (it >= 2) mbar_wait(bar_dfree + s, ((it >> 1) - 1) & 1);
+        if (DQ) mbar_wait(bar_fix, 0);
+        else mbar_wait(bar_ld + s, (it >> 1) & 1);
+        const uint8_t* to = sO + static_cast<size_t>(DQ ? 0 : s) * kTileBytes;
+        const uint8_t* tg = DQ ? sF + kTileBytes : sY + static_cast<size_t>(s) * kTileBytes;
+        const int i = qtile(it);
+        float lse[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+          const int pos = i * kTile + lane + 32 * k;
+          lse[k] = pos < p.L ? p.lse[static_cast<size_t>(bh) * p.L + pos] : 0.f;
+        }
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+          const int r = lane + 32 * k;
+          float delta = 0.f;
+          if (i * kTile + r < p.L) {
+#pragma unroll
+            for (int u = 0; u < 8; ++u) {
+              const int off = r * 128 + ((u ^ (r & 7)) << 4);
+              const uint4 a = *reinterpret_cast<const uint4*>(to + off), c = *reinterpret_cast<const uint4*>(tg + off);
+              const uint32_t aw[4] = {a.x, a.y, a.z, a.w}, cw[4] = {c.x, c.y, c.z, c.w};
+#pragma unroll
+              for (int w = 0; w < 4; ++w) {
+                const float2 x = unpack_bf16(aw[w]), y = unpack_bf16(cw[w]);
+                delta += x.x * y.x + x.y * y.y;
+              }
+            }
+          }
+          sDelta[s * kTile + r] = delta;
+          sLse[s * kTile + r] = lse[k] * kLog2e;
+        }
+        mbar_arrive(bar_dfull + s);
+      }
+    }
+  } else {
+    // ======================= compute warps ====================================================
+    const int q = warp & 3, cg = warp >> 2;   // TMEM lane quarter, 32-column chunk of the key tile
+    const int row = q * 32 + lane;
+    const uint32_t lane_base = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
+    const float c1 = p.scale * kLog2e;
+    const uint64_t seed = p.drop_seed + ((p.drop_thresh && p.drop_seed_dev) ? *p.drop_seed_dev : 0ull);
+    const uint32_t dkey = drop_key(seed, p.drop_site);
+    const int u0 = (cg & 1) * 4;
+    for (int it = 0; it < n_it; ++it) {
+      const int i = qtile(it), j = ktile(it);
+      const int s = DQ ? 0 : (it & 1);
+      const int q_pos = i * kTile + row;
+      const int kv0 = j * kTile + cg * 32;
+      const bool diag = (i == j);
+      const bool row_ok = q_pos < p.L;
+      // inactive (warp-uniform): above the diagonal, or all 32 query rows / all 32 key columns beyond the sequence
+      const bool active = !(diag && cg > q) && (i * kTile + q * 32 < p.L) && (kv0 < p.L);
+      const uint32_t keepmask = (active && p.drop_thresh)
+          ? drop_keepmask32_64(dkey, (static_cast<uint64_t>(bh) * p.L + q_pos) * p.L + kv0, p.drop_thresh)
+          : 0xFFFFFFFFu;
+      mbar_wait(bar_dfull + s, DQ ? 0u : static_cast<uint32_t>((it >> 1) & 1));
+      const float lse2 = sLse[s * kTile + row];
+      const float delta = sDelta[s * kTile + row];
+      if (!DQ) mbar_arrive(bar_dfree + s);
+      mbar_wait(bar_mm1, it & 1);
+      __syncwarp();
+      tc_fence_after();
+      uint4 vp[4], vd[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) vp[u] = vd[u] = make_uint4(0, 0, 0, 0);
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {     // four 8-column quarters: 16 raw registers live
+        uint32_t rs[8], rp[8];
+        if (active) {
+          tmem_ld8(lane_base + T_S + cg * 32 + u * 8, rs);
+          tmem_ld8(lane_base + T_DP + cg * 32 + u * 8, rp);
+          tmem_ld_wait();
+        }
+        if (u == 3) {
+          tc_fence_before();
+          mbar_arrive(bar_drain);
+        }
+        if (active) {
+          {
+            float pd[8], ds[8];
+#pragma unroll
+            for (int e = 0; e < 8; ++e) {
+              const int t = u * 8 + e;
+              float pr = fast_exp2(__uint_as_float(rs[e]) * c1 - lse2);
+              if ((diag && kv0 + t > q_pos) || !row_ok) pr = 0.f;
+              const bool keep = (keepmask >> t) & 1u;
+              const float dp = keep ? __uint_as_float(rp[e]) * p.drop_scale : 0.f;
+              pd[e] = keep ? pr * p.drop_scale : 0.f;
+              ds[e] = pr * (dp - delta) * p.scale;
+            }
+            vp[u].x = pack_bf16(pd[0], pd[1]);
+            vp[u].y = pack_bf16(pd[2], pd[3]);
+            vp[u].z = pack_bf16(pd[4], pd[5]);
+            vp[u].w = pack_bf16(pd[6], pd[7]);
+            vd[u].x = pack_bf16(ds[0], ds[1]);
+            vd[u].y = pack_bf16(ds[2], ds[3]);
+            vd[u].z = pack_bf16(ds[4], ds[5]);
+            vd[u].w = pack_bf16(ds[6], ds[7]);
+          }
+        }
+      }
+      if (it > 0) mbar_wait(bar_mm2, (it - 1) & 1);   // the previous MMAs no longer read Pd / dS
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        if (!DQ) st_swizzled_unit(sPd + (cg >> 1) * kTileBytes, row, u0 + u, vp[u]);
+        st_swizzled_unit(sDS + (cg >> 1) * kTileBytes, row, u0 + u, vd[u]);
+      }
+      fence_proxy_async_smem();
+      mbar_arrive(bar_stage);
+    }
+    // ---- accumulators complete: TMEM -> dqkv (groups 0,1: the two 32-column halves of dV_j / dQ_i; 2,3: of dK_j) ----
+    mbar_wait(bar_mm2, (n_it - 1) & 1);
+    __syncwarp();
+    tc_fence_after();
+    if (!DQ || cg < 2) {
+      const int hf = cg & 1;
+      const int pos = tile * kTile + row;
+      uint32_t r[32];
+      tmem_ld32(lane_base + T_ACC + (cg >> 1) * kDh + hf * 32, r);
+      tmem_ld_wait();
+      // dQ -> the Q third; dV_j (cg < 2) -> the V third, dK_j -> the K third
+      const int third = DQ ? 0 : (cg < 2 ? 2 : 1);
+      if (pos < p.L)
+        store_row32_bf16(p.dqkv + static_cast<size_t>(seq_row0 + pos) * (3 * D) + third * D + h * kDh + hf * 32, r);
+    }
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 16) tmem_dealloc(tmem_base, 512);
+}
+
 static int make_rows_map(CUtensorMap* m, const void* base, int rows, int cols) {
   uint64_t dims[2] = {static_cast<uint64_t>(cols), static_cast<uint64_t>(rows)};
   uint64_t str[1] = {static_cast<uint64_t>(cols) * 2};
@@ -1495,7 +2071,9 @@ extern "C" int tt_attn_causal_fwd(const void* qkv, void* ctx, float* lse, int B,
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   TT_REQUIRE(qkv && ctx, "tt_attn_causal_fwd: null pointer");
   TT_REQUIRE(B > 0 && L > 0 && H > 0, "tt_attn_causal_fwd: empty problem");
-  TT_REQUIRE(L <= 512, "tt_attn_causal_fwd: L=%d > 512 unsupported", L);
+  TT_REQUIRE(L <= kLongMaxL, "tt_attn_causal_fwd: L=%d > %d unsupported", L, kLongMaxL);
+  TT_REQUIRE(static_cast<int64_t>(B) * L <= INT32_MAX, "tt_attn_causal_fwd: B*L=%lld rows too many",
+             static_cast<long long>(B) * L);
   TT_REQUIRE(drop_p >= 0.f && drop_p < 1.f, "tt_attn_causal_fwd: drop_p out of range");
   const int D = H * kDh;
   AttnParams p;
@@ -1512,6 +2090,17 @@ extern "C" int tt_attn_causal_fwd(const void* qkv, void* ctx, float* lse, int B,
   CUtensorMap tm;
   int rc = make_rows_map(&tm, qkv, B * L, 3 * D);
   if (rc) return rc;
+  if (L > 512) {
+    const size_t lsmem = 1024 + 6 * static_cast<size_t>(kTileBytes) + 48 + 2 * 128 * sizeof(float);
+    static bool lconfigured = false;
+    if (!lconfigured) {
+      TT_CHECK_CUDA(cudaFuncSetAttribute(attn_fwd_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lsmem));
+      lconfigured = true;
+    }
+    TT_CHECK_CUDA(launch_k(attn_fwd_long_kernel, dim3(B * H * p.nq), dim3(256), lsmem, stream, tm, p));
+    TT_LAUNCH_CHECK();
+    return TT_OK;
+  }
   const size_t smem = 1024 + static_cast<size_t>(1 + p.nq + 1 + 2) * kTileBytes + 64 + 2 * 128 * sizeof(float);
   static bool configured = false;
   if (!configured) {
@@ -1546,7 +2135,9 @@ extern "C" int tt_attn_causal_bwd(const void* qkv, const void* ctx, const void* 
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   TT_REQUIRE(qkv && ctx && dctx && lse && dqkv, "tt_attn_causal_bwd: null pointer");
   TT_REQUIRE(B > 0 && L > 0 && H > 0, "tt_attn_causal_bwd: empty problem");
-  TT_REQUIRE(L <= 512, "tt_attn_causal_bwd: L=%d > 512 unsupported", L);
+  TT_REQUIRE(L <= kLongMaxL, "tt_attn_causal_bwd: L=%d > %d unsupported", L, kLongMaxL);
+  TT_REQUIRE(static_cast<int64_t>(B) * L <= INT32_MAX, "tt_attn_causal_bwd: B*L=%lld rows too many",
+             static_cast<long long>(B) * L);
   const int D = H * kDh;
   AttnBwdParams p;
   p.B = B; p.L = L; p.H = H;
@@ -1566,6 +2157,26 @@ extern "C" int tt_attn_causal_bwd(const void* qkv, const void* ctx, const void* 
   if (rc) return rc;
   rc = make_rows_map(&tmDO, dctx, B * L, D);
   if (rc) return rc;
+  if (L > 512) {
+    // dK / dV (a CTA per key tile) and dQ (a CTA per query tile): 12 and 9 tiles of shared memory
+    const size_t ksmem = 1024 + 12 * static_cast<size_t>(kTileBytes) + 96 + 2 * 2 * kTile * sizeof(float);
+    const size_t qsmem = ksmem - 3 * static_cast<size_t>(kTileBytes);
+    CUtensorMap tmO;
+    rc = make_rows_map(&tmO, ctx, B * L, D);
+    if (rc) return rc;
+    static bool lconfigured = false;
+    if (!lconfigured) {
+      TT_CHECK_CUDA(cudaFuncSetAttribute(attn_bwd_long_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ksmem));
+      TT_CHECK_CUDA(cudaFuncSetAttribute(attn_bwd_long_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
+      lconfigured = true;
+    }
+    const dim3 grid(B * H * p.nq);
+    TT_CHECK_CUDA(launch_k(attn_bwd_long_kernel<false>, grid, dim3(kLongBwdThreads), ksmem, stream, tmQ, tmDO, tmO, p));
+    TT_LAUNCH_CHECK();
+    TT_CHECK_CUDA(launch_k(attn_bwd_long_kernel<true>, grid, dim3(kLongBwdThreads), qsmem, stream, tmQ, tmDO, tmO, p));
+    TT_LAUNCH_CHECK();
+    return TT_OK;
+  }
   const int slots = p.nq <= 2 ? p.nq : 1;
   const size_t smem = 1024 + static_cast<size_t>(2 * slots + 2 + 4) * kTileBytes + 128 +
                       static_cast<size_t>(2 * p.nq * kTile) * sizeof(float);

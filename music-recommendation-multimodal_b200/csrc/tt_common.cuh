@@ -200,6 +200,25 @@ __device__ __forceinline__ void drop_keep_quad(uint32_t key, uint32_t idx4, uint
   k[2] = h * kDropMul2 >= thresh;
   k[3] = h * kDropMul3 >= thresh;
 }
+// 64-bit forms of the two above, bit-equal to drop_keep_k at every index (the 32-bit forms agree with it only below
+// 2^32): the high word of the quad number enters the hash exactly as in drop_keep_k.
+__device__ __forceinline__ uint32_t drop_quad_hash64(uint32_t key, uint64_t idx) {
+  const uint64_t quad = idx >> 2;
+  return mix32((static_cast<uint32_t>(quad) ^ (static_cast<uint32_t>(quad >> 32) * 0x85EBCA6Bu)) ^ key);
+}
+__device__ __forceinline__ void drop_keep_pair64(uint32_t key, uint64_t idx_even, uint32_t thresh, bool& k0, bool& k1) {
+  const uint32_t h = drop_quad_hash64(key, idx_even);
+  const bool hi = (idx_even & 2u) != 0;
+  k0 = h * (hi ? kDropMul2 : 1u) >= thresh;
+  k1 = h * (hi ? kDropMul3 : kDropMul1) >= thresh;
+}
+__device__ __forceinline__ void drop_keep_quad64(uint32_t key, uint64_t idx4, uint32_t thresh, bool (&k)[4]) {
+  const uint32_t h = drop_quad_hash64(key, idx4);
+  k[0] = h >= thresh;
+  k[1] = h * kDropMul1 >= thresh;
+  k[2] = h * kDropMul2 >= thresh;
+  k[3] = h * kDropMul3 >= thresh;
+}
 // Packed fp32 pairs (sm_100 FFMA2 / FMUL2): d = a * b + c on two lanes in one issue slot.
 __device__ __forceinline__ void ffma2(float& a0, float& a1, float b0, float b1, float c0, float c1) {
   uint64_t d;

@@ -21,7 +21,10 @@
 namespace tt {
 
 static constexpr int kDh = 64;
-static constexpr int kMaxL = 512;
+// Longest history the single-query kernels take. L <= kShortL keeps the 2 KB shared-memory instantiation it has always
+// run; longer histories take the kMaxL one (16 KB of scores per CTA).
+static constexpr int kShortL = 512;
+static constexpr int kMaxL = 4096;
 static constexpr float kLog2e = 1.4426950408889634f;
 
 __global__ void gather_rows_kernel(const float* __restrict__ x32, const __nv_bfloat16* __restrict__ x16,
@@ -136,10 +139,11 @@ __device__ __forceinline__ float block4_sum(float v, float* s4, int wib, int lan
   return r;
 }
 
+template <int MaxL>
 __global__ void __launch_bounds__(128) attn_lastq_fwd_kernel(const LastQParams p) {
   pdl_launch_dependents();
   pdl_wait();
-  __shared__ float s_p[kMaxL];
+  __shared__ float s_p[MaxL];
   __shared__ float s_acc[4][64];
   __shared__ float s4[4];
   const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -206,10 +210,11 @@ __global__ void __launch_bounds__(128) attn_lastq_fwd_kernel(const LastQParams p
   }
 }
 
+template <int MaxL>
 __global__ void __launch_bounds__(128) attn_lastq_bwd_kernel(const LastQParams p) {
   pdl_launch_dependents();
   pdl_wait();
-  __shared__ float s_ds[kMaxL];
+  __shared__ float s_ds[MaxL];
   __shared__ float s_acc[4][64];
   const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int ks = lane >> 2, dq = lane & 3;
@@ -354,7 +359,8 @@ extern "C" int tt_attn_lastq_fwd(const void* q, const void* qkv, const int32_t* 
   TT_REQUIRE(ctx, "tt_attn_lastq_fwd: null ctx");
   p.ctx = static_cast<__nv_bfloat16*>(ctx);
   p.lse = lse;
-  TT_CHECK_CUDA(launch_k(attn_lastq_fwd_kernel, dim3(B * H), dim3(128), 0, stream, p));
+  if (L <= kShortL) TT_CHECK_CUDA(launch_k(attn_lastq_fwd_kernel<kShortL>, dim3(B * H), dim3(128), 0, stream, p));
+  else TT_CHECK_CUDA(launch_k(attn_lastq_fwd_kernel<kMaxL>, dim3(B * H), dim3(128), 0, stream, p));
   TT_LAUNCH_CHECK();
   return TT_OK;
 }
@@ -372,7 +378,8 @@ extern "C" int tt_attn_lastq_bwd(const void* q, const void* qkv, const int32_t* 
   p.lse = const_cast<float*>(lse);
   p.dq = static_cast<__nv_bfloat16*>(dq);
   p.dqkv = static_cast<__nv_bfloat16*>(dqkv);
-  TT_CHECK_CUDA(launch_k(attn_lastq_bwd_kernel, dim3(B * H), dim3(128), 0, stream, p));
+  if (L <= kShortL) TT_CHECK_CUDA(launch_k(attn_lastq_bwd_kernel<kShortL>, dim3(B * H), dim3(128), 0, stream, p));
+  else TT_CHECK_CUDA(launch_k(attn_lastq_bwd_kernel<kMaxL>, dim3(B * H), dim3(128), 0, stream, p));
   TT_LAUNCH_CHECK();
   return TT_OK;
 }

@@ -74,6 +74,11 @@ def param_shapes(cfg: TwoTowerConfig) -> List[Tuple[str, Tuple[int, ...]]]:
 
 
 _NUM_SPARSE = 4  # table, positions, gender, country come before the dense region
+#: longest history window the attention kernels take (tt_attn_causal_*, tt_attn_lastq_*)
+MAX_SEQ_LEN = 4096
+#: most tokens (B * L) one user-tower call may hold: the bound the kernels' 32-bit indices were checked against
+#: (T * 4D = 2^30; the GEMM epilogues' 32-bit dropout index row * N + col wraps from 2^22 tokens)
+MAX_TOKENS = 1 << 20
 
 
 class TwoTowerEngine:
@@ -81,6 +86,8 @@ class TwoTowerEngine:
         assert cfg.embedding_dim == 256 and cfg.num_heads == 4, \
             "the sm_100a kernels are specialised for d_model=256, 4 heads of 64 (the reference's configuration)"
         assert cfg.fusion_hidden == 512 and 4 * cfg.modality_dim == 512
+        if not 1 <= cfg.max_seq_len <= MAX_SEQ_LEN:
+            raise ValueError(f"max_seq_len = {cfg.max_seq_len} outside [1, {MAX_SEQ_LEN}]")
         self.cfg = cfg
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else device
         shapes = param_shapes(cfg)
@@ -237,12 +244,15 @@ class TwoTowerEngine:
 
     # ------------------------------------------------------------------ workspaces
     def workspace(self, B: int, L: int) -> Dict[str, torch.Tensor]:
+        """Activation buffers of a (B, L) user-tower call; B * L <= MAX_TOKENS, else ValueError."""
         key = (B, L)
         if key in self._ws:
             return self._ws[key]
         cfg, dev = self.cfg, self.device
         D, FF, NL, Hh = cfg.embedding_dim, cfg.ff_dim, cfg.num_layers, cfg.num_heads
         T = B * L
+        if T > MAX_TOKENS:
+            raise ValueError(f"{B} sequences x {L} positions = {T} tokens in one call; at most {MAX_TOKENS}")
         f32 = dict(device=dev, dtype=torch.float32)
         bf = dict(device=dev, dtype=torch.bfloat16)
         ws: Dict[str, torch.Tensor] = {}

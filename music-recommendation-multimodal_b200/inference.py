@@ -75,6 +75,8 @@ def recommend_for_user(model, index: retrieval.CatalogIndex, history_ids: Sequen
 #: users per user-tower call in `recommend_batch`: bounds the tower's workspace (B = 10 k at L = 512 would otherwise
 #: size every activation buffer for all users at once)
 _TOWER_CHUNK = 1024
+#: tokens per user-tower call: the chunk shrinks to `_TOWER_TOKENS // L` users for windows longer than 512
+_TOWER_TOKENS = 1 << 19
 
 
 def recommend_batch(model, index: retrieval.CatalogIndex, history_ids: torch.Tensor,
@@ -85,7 +87,7 @@ def recommend_batch(model, index: retrieval.CatalogIndex, history_ids: torch.Ten
 
     ``history_ids`` (B, L) int64, L <= the model's max_seq_len, right-padded with 0; ``history_mask`` (B, L), default
     ``history_ids != 0``; ``user_gender`` / ``user_country`` (B,), default 0. The eval-mode user tower runs in chunks of
-    1024 users, its output is re-normalised (eps 1e-8, :286), and the padding id 0 and every excluded item are
+    min(1024, 2**19 // L) users, its output is re-normalised (eps 1e-8, :286), and the padding id 0 and every excluded item are
     masked (:296-302) inside the selection kernels. The excluded items are ``exclude_ids`` (B, m) int64 (0 = empty
     slot, m <= 4096: e.g. a full listening history longer than the tower's window) if given, otherwise the valid
     history positions. On a sharded ``index`` the top k is taken over the whole catalog across ``group``
@@ -93,7 +95,6 @@ def recommend_batch(model, index: retrieval.CatalogIndex, history_ids: torch.Ten
 
     Returns (item ids int64 (B, k), scores fp32 (B, k)), best first in the canonical order (score descending, item id
     ascending). When a user has fewer than k admissible items, the tail is id -1 with score -inf."""
-    chunk = _TOWER_CHUNK
     if not 1 <= k <= 256:
         raise ValueError(f"recommend_batch: k = {k} outside [1, 256]")
     dev = model.engine.device
@@ -101,6 +102,7 @@ def recommend_batch(model, index: retrieval.CatalogIndex, history_ids: torch.Ten
     B, L = ids.shape
     if L > model.engine.cfg.max_seq_len:
         raise ValueError(f"history window {L} exceeds the model's max_seq_len {model.engine.cfg.max_seq_len}")
+    chunk = min(_TOWER_CHUNK, _TOWER_TOKENS // L)
     mask = (ids != 0).long() if history_mask is None else history_mask.to(dev).long()
     gender = torch.zeros(B, dtype=torch.long, device=dev) if user_gender is None else user_gender.to(dev).long()
     country = torch.zeros(B, dtype=torch.long, device=dev) if user_country is None else user_country.to(dev).long()
