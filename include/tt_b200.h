@@ -125,6 +125,13 @@ int tt_embed_ln_fwd(const int64_t* ids, const float* E, const float* P, const fl
                     const float* next_w, const float* next_b, int B, int L, float drop_p, uint64_t seed,
                     const uint64_t* seed_dev, uint32_t site, float* x0, void* h_bf16, void* stream);
 
+/* tt_embed_ln_fwd for n rows at explicit positions: row r is item ids[r] at position pos[r] (int32), local table,
+ * no dropout (eval). x0 fp32 [n,256], h bf16 [n,256]; each row equal bit for bit to tt_embed_ln_fwd's row at the same
+ * (id, position). Same reference lines (src/models/user_tower.py:86-93); used by the session append. */
+int tt_embed_ln_fwd_pos(const int64_t* ids, const int32_t* pos, const float* E, const float* P, const float* ln_w,
+                        const float* ln_b, const float* next_w, const float* next_b, int n, float* x0, void* h_bf16,
+                        void* stream);
+
 /* backward of the embedding LayerNorm + lookup: dx0 -> dE (scatter-add, row 0 skipped:
  * padding_idx, src/models/user_tower.py:26), dP, d(ln_w), d(ln_b); all accumulated. */
 int tt_embed_ln_bwd(const int64_t* ids, const float* E, const float* P, const float* ln_w, const float* ln_b,
@@ -293,6 +300,18 @@ int tt_attn_lastq_fwd(const void* q, const void* qkv, const int32_t* last_idx, v
 int tt_attn_lastq_bwd(const void* q, const void* qkv, const int32_t* last_idx, const void* ctx, const void* dctx,
                       const float* lse, void* dq, void* dqkv, int B, int L, int H, float drop_p, uint64_t seed,
                       const uint64_t* seed_dev, uint32_t site, void* stream);
+
+/* ---- user sessions: one new row per user over cached keys/values -------------------------
+ * Appending item p to a right-padded history of length p < L leaves every earlier position of the causal encoder
+ * unchanged (src/models/user_tower.py:95-120: causal mask, key padding beyond the history), so each layer needs the
+ * new row's attention over the stored K/V of positions 0..p only.
+ *   tt_session_attn : qkv bf16 [n, 3*H*64] (Q | K | V of the new rows), K/V caches bf16 [capacity, H, L, 64] each,
+ *                     slots / pos int32 [n]. For row r: cache[slots[r], :, pos[r]] = its K / V, then ctx bf16 [n, H*64]
+ *                     = softmax(q K[0..pos]^T / 8) V[0..pos]. No dropout (eval). L <= 4096; rows with a slot outside
+ *                     [0, capacity) or pos outside [0, L) touch no cache and get ctx = 0. Slots must be distinct
+ *                     within a call. Bit-identical from run to run. */
+int tt_session_attn(const void* qkv, void* k_cache, void* v_cache, const int32_t* slots, const int32_t* pos, int n,
+                    int H, int L, int capacity, void* ctx, void* stream);
 
 /* ---- symmetric InfoNCE (src/models/two_tower.py:106-140) --------------------------------
  * Row formulation: S [R, C] fp32 holds logits of R local rows against C (all-gathered)

@@ -193,6 +193,8 @@ _SIGNATURES = {
     "tt_last_index": [c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p],
     "tt_embed_ln_fwd": [c_void_p] * 7 + [c_int32, c_int32, c_float, c_uint64, c_void_p, c_uint32,
                                          c_void_p, c_void_p, c_void_p],
+    "tt_embed_ln_fwd_pos": [c_void_p] * 8 + [c_int32, c_void_p, c_void_p, c_void_p],
+    "tt_session_attn": [c_void_p] * 5 + [c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p],
     "tt_embed_ln_bwd": [c_void_p] * 6 + [c_int32, c_int32, c_float, c_uint64, c_void_p, c_uint32,
                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
     "tt_embed_ln_bwd_norm1": [ctypes.POINTER(Norm1Bwd)] + [c_void_p] * 5 + [c_int32, c_int32, c_float, c_uint64, c_void_p,

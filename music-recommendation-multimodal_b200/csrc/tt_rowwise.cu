@@ -148,6 +148,30 @@ struct EmbedParams {
   __nv_bfloat16* h;
 };
 
+// One token row of embed_ln_fwd (one warp): table row E[id] and position row P[pos] -> x0, h at output row `row`.
+// Shared by the [B, L] kernel (pos = row % L, dropout, stash) and the explicit-position one (sessions: no dropout).
+__device__ __forceinline__ void embed_ln_row(const EmbedParams& p, int64_t id, int pos, int row, int lane,
+                                             const float (&w)[8], const float (&b)[8], const float (&nw)[8],
+                                             const float (&nb)[8], uint64_t seed) {
+  constexpr int NV = 2;
+  float e[8], q[8];
+  load_row<NV>(p.E.row(id), lane, e);
+  load_row<NV>(p.P + static_cast<size_t>(pos) * 256, lane, q);
+  if (p.stash) store_row<NV>(p.stash + static_cast<size_t>(row) * 256, lane, e);
+#pragma unroll
+  for (int i = 0; i < 8; ++i) e[i] += q[i];
+  float mean, rstd;
+  ln_stats<NV>(e, 1e-5f, mean, rstd);
+#pragma unroll
+  for (int i = 0; i < 8; ++i) e[i] = (e[i] - mean) * rstd * w[i] + b[i];
+  if (p.drop_thresh) row_dropout<NV>(e, drop_key(seed, p.site), row, 256, lane, p.drop_thresh, p.drop_scale, nullptr);
+  store_row<NV>(p.x0 + static_cast<size_t>(row) * 256, lane, e);
+  ln_stats<NV>(e, 1e-5f, mean, rstd);
+#pragma unroll
+  for (int i = 0; i < 8; ++i) e[i] = (e[i] - mean) * rstd * nw[i] + nb[i];
+  store_row_bf16<NV>(p.h + static_cast<size_t>(row) * 256, lane, e);
+}
+
 __global__ void __launch_bounds__(kRowThreads) embed_ln_fwd_kernel(const EmbedParams p) {
   pdl_launch_dependents();
   pdl_wait();
@@ -160,26 +184,25 @@ __global__ void __launch_bounds__(kRowThreads) embed_ln_fwd_kernel(const EmbedPa
   load_row<NV>(p.nw, lane, nw);
   load_row<NV>(p.nb, lane, nb);
   const uint64_t seed = p.drop_thresh ? read_seed(p.seed, p.seed_dev) : 0;
-  for (int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; row < p.T; row += warps_total) {
-    const int64_t id = p.ids[row];
-    const int pos = row % p.L;
-    float e[8], q[8];
-    load_row<NV>(p.E.row(id), lane, e);
-    load_row<NV>(p.P + static_cast<size_t>(pos) * 256, lane, q);
-    if (p.stash) store_row<NV>(p.stash + static_cast<size_t>(row) * 256, lane, e);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) e[i] += q[i];
-    float mean, rstd;
-    ln_stats<NV>(e, 1e-5f, mean, rstd);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) e[i] = (e[i] - mean) * rstd * w[i] + b[i];
-    if (p.drop_thresh) row_dropout<NV>(e, drop_key(seed, p.site), row, 256, lane, p.drop_thresh, p.drop_scale, nullptr);
-    store_row<NV>(p.x0 + static_cast<size_t>(row) * 256, lane, e);
-    ln_stats<NV>(e, 1e-5f, mean, rstd);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) e[i] = (e[i] - mean) * rstd * nw[i] + nb[i];
-    store_row_bf16<NV>(p.h + static_cast<size_t>(row) * 256, lane, e);
-  }
+  for (int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; row < p.T; row += warps_total)
+    embed_ln_row(p, p.ids[row], row % p.L, row, lane, w, b, nw, nb, seed);
+}
+
+// Rows at explicit positions: row r is item ids[r] at position pos[r] (p.T = n rows; no dropout, no stash).
+__global__ void __launch_bounds__(kRowThreads) embed_ln_fwd_pos_kernel(const EmbedParams p,
+                                                                        const int32_t* __restrict__ pos) {
+  pdl_launch_dependents();
+  pdl_wait();
+  constexpr int NV = 2;
+  const int lane = threadIdx.x & 31;
+  const int warps_total = (gridDim.x * blockDim.x) >> 5;
+  float w[8], b[8], nw[8], nb[8];
+  load_row<NV>(p.ln_w, lane, w);
+  load_row<NV>(p.ln_b, lane, b);
+  load_row<NV>(p.nw, lane, nw);
+  load_row<NV>(p.nb, lane, nb);
+  for (int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; row < p.T; row += warps_total)
+    embed_ln_row(p, p.ids[row], pos[row], row, lane, w, b, nw, nb, 0);
 }
 
 // --------------------------------------------------------------------------------------------
@@ -977,6 +1000,24 @@ extern "C" int tt_embed_ln_fwd(const int64_t* ids, const float* E, const float* 
   TT_REQUIRE(E, "tt_embed_ln_fwd: null table");
   return embed_fwd_impl(ids, single_table(E), nullptr, P, ln_w, ln_b, next_w, next_b, B, L, drop_p, seed, seed_dev, site,
                         x0, h_bf16, static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int tt_embed_ln_fwd_pos(const int64_t* ids, const int32_t* pos, const float* E, const float* P,
+                                   const float* ln_w, const float* ln_b, const float* next_w, const float* next_b,
+                                   int n, float* x0, void* h_bf16, void* stream_) {
+  TT_REQUIRE(ids && pos && E && P && ln_w && ln_b && next_w && next_b && x0 && h_bf16,
+             "tt_embed_ln_fwd_pos: null pointer");
+  TT_REQUIRE(n > 0, "tt_embed_ln_fwd_pos: empty batch");
+  EmbedParams p;
+  p.ids = ids; p.E = single_table(E); p.stash = nullptr; p.P = P; p.ln_w = ln_w; p.ln_b = ln_b;
+  p.nw = next_w; p.nb = next_b;
+  p.T = n; p.L = 0;
+  p.drop_thresh = 0; p.drop_scale = 1.f; p.seed = 0; p.seed_dev = nullptr; p.site = 0;
+  p.x0 = x0; p.h = static_cast<__nv_bfloat16*>(h_bf16);
+  TT_CHECK_CUDA(launch_k(embed_ln_fwd_pos_kernel, dim3(row_grid(n)), dim3(kRowThreads), 0,
+                         static_cast<cudaStream_t>(stream_), p, pos));
+  TT_LAUNCH_CHECK();
+  return TT_OK;
 }
 
 extern "C" int tt_embed_ln_bwd(const int64_t* ids, const float* E, const float* P, const float* ln_w,

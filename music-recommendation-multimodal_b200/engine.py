@@ -162,6 +162,9 @@ class TwoTowerEngine:
         #: and 2 KB of accumulator per distinct id and step.
         self.deterministic_table_grad = os.environ.get("TT_DETERMINISTIC", "0") == "1"
         self._det: Dict[int, Dict[str, torch.Tensor]] = {}
+        #: host-side count of parameter updates (load_state_dict, the AdamW steps, TrainStepRunner steps): state derived
+        #: from the weights, such as the K/V caches of sessions.UserSessions, records it and is refused once it moved
+        self.weights_epoch = 0
 
     # ------------------------------------------------------------------ parameters
     def use_external_table(self, B: int, L: int) -> None:
@@ -227,6 +230,7 @@ class TwoTowerEngine:
             self.bn_running_var.copy_(sd[it + "running_var"])
             self.bn_num_batches.copy_(sd[it + "num_batches_tracked"])
         self.shadow_valid = False
+        self.weights_epoch += 1
 
     def state_dict(self) -> Dict[str, torch.Tensor]:
         out = {k: v.detach().clone() for k, v in self.p.items()}
@@ -335,6 +339,66 @@ class TwoTowerEngine:
         ws["dctx"] = torch.empty(T, D, **bf)
         self._ws[key] = ws
         return ws
+
+    def session_workspace(self, n: int) -> Dict[str, torch.Tensor]:
+        """Buffers of a session append (`session_append`): n rows per layer, no (B, L) token buffers."""
+        key = ("session", n)
+        if key in self._ws:
+            return self._ws[key]
+        cfg, dev = self.cfg, self.device
+        D, FF = cfg.embedding_dim, cfg.ff_dim
+        f32 = dict(device=dev, dtype=torch.float32)
+        bf = dict(device=dev, dtype=torch.bfloat16)
+        ws: Dict[str, torch.Tensor] = {"x_in0": torch.empty(n, D, **f32), "zero_idx": torch.zeros(n, device=dev,
+                                                                                                  dtype=torch.int32)}
+        for l in range(cfg.num_layers):
+            ws[f"h1_{l}"] = torch.empty(n, D, **bf)
+            ws[f"qkv_{l}"] = torch.empty(n, 3 * D, **bf)
+            ws[f"ctx_{l}"] = torch.empty(n, D, **bf)
+            ws[f"xmid_{l}"] = torch.empty(n, D, **f32)
+            ws[f"h2_{l}"] = torch.empty(n, D, **bf)
+            ws[f"f_{l}"] = torch.empty(n, FF, **bf)
+            ws[f"xout_{l}"] = torch.empty(n, D, **f32)
+        ws["cat"] = torch.zeros(n + 1, D + 48, **bf)[:n]          # +1 row: ragged MN-major reads
+        ws["z1"] = torch.empty(n, D, **f32)
+        ws["a1"] = torch.empty(n, D, **bf)
+        ws["u"] = torch.empty(n, D, **f32)
+        ws["un"] = torch.empty(n, D, **f32)
+        ws["un_bf"] = torch.empty(n, D, **bf)
+        self._ws[key] = ws
+        return ws
+
+    def session_append(self, ws, item_ids, slots, pos, k_caches, v_caches, gender, country) -> torch.Tensor:
+        """User tower for ONE new history item per row, from the K/V of the earlier positions (eval, no dropout).
+
+        Row r appends ``item_ids[r]`` (int64) at position ``pos[r]`` (int32) of cache slot ``slots[r]`` (int32, distinct);
+        ``k_caches[l]`` / ``v_caches[l]`` are layer l's planes, bf16 [capacity, 4, L, 64], holding that slot's K/V for
+        positions < pos[r]. The new row's K/V are written into them. Returns ws['un'] fp32 [n, 256]: the normalised user
+        embedding of the extended history (user_forward on the whole window gives the same)."""
+        if self.table_rows is not None or self.peer_table is not None:
+            raise NotImplementedError("user sessions need a local ID table (no row-sharded or peer table)")
+        cfg, p, w = self.cfg, self.p, self.w
+        ut = "user_tower."
+        if not self.shadow_valid:
+            self.refresh_shadow()
+        ops.embed_ln_fwd_pos(item_ids, pos, p[ut + "item_embedding.weight"], p[ut + "position_embedding.weight"],
+                             p[ut + "layer_norm.weight"], p[ut + "layer_norm.bias"], p[self._lp(0, "norm1.weight")],
+                             p[self._lp(0, "norm1.bias")], ws["x_in0"], ws["h1_0"])
+        x_in = ws["x_in0"]
+        for l in range(cfg.num_layers):
+            self._gemm(ws[f"h1_{l}"], w[self._lp(l, "self_attn.in_proj_weight")],
+                       bias=p[self._lp(l, "self_attn.in_proj_bias")], out_bf16=ws[f"qkv_{l}"])
+            ops.session_attn(ws[f"qkv_{l}"], k_caches[l], v_caches[l], slots, pos, ws[f"ctx_{l}"])
+            self._layer_tail(l, ws[f"ctx_{l}"], x_in, ws[f"xmid_{l}"], ws[f"h2_{l}"], ws[f"f_{l}"], ws[f"xout_{l}"],
+                             0.0, self.base_seed, None)
+            x_in = ws[f"xout_{l}"]
+            if l + 1 < cfg.num_layers:
+                ops.chain_fwd(x_in, ln=(p[self._lp(l + 1, "norm1.weight")], p[self._lp(l + 1, "norm1.bias")]),
+                              out_bf16=ws[f"h1_{l + 1}"])
+        n = item_ids.shape[0]
+        ops.gather_cat_fwd(x_in, ws["zero_idx"], gender, country, p[ut + "gender_embedding.weight"],
+                           p[ut + "country_embedding.weight"], n, 1, ws["cat"])
+        return self._user_head(ws)
 
     def _sparse_ws(self, T: int) -> Dict[str, torch.Tensor]:
         """Scratch of the id de-duplication for T tokens per step (direct-address flag / slot tables over the
@@ -495,17 +559,8 @@ class TwoTowerEngine:
                        bias=p[self._lp(l, "self_attn.in_proj_bias")], out_bf16=ws[f"qkv_{l}"])
             ops.attn_fwd(ws[f"qkv_{l}"], ws[f"ctx_{l}"], ws[f"lse_{l}"], B, L, cfg.num_heads, drop_p=dp,
                          drop_seed=seed, drop_seed_dev=sdev, drop_site=_site(l, 0))
-            self._gemm(ws[f"ctx_{l}"], w[self._lp(l, "self_attn.out_proj.weight")],
-                       bias=p[self._lp(l, "self_attn.out_proj.bias")], drop_p=dp, drop_seed=seed,
-                       drop_seed_dev=sdev, drop_site=_site(l, 1), residual=x_in, out_f32=ws[f"xmid_{l}"])
-            ops.chain_fwd(ws[f"xmid_{l}"], ln=(p[self._lp(l, "norm2.weight")], p[self._lp(l, "norm2.bias")]),
-                          out_bf16=ws[f"h2_{l}"])
-            self._gemm(ws[f"h2_{l}"], w[self._lp(l, "linear1.weight")], bias=p[self._lp(l, "linear1.bias")],
-                       relu=True, drop_p=dp, drop_seed=seed, drop_seed_dev=sdev, drop_site=_site(l, 2),
-                       out_bf16=ws[f"f_{l}"])
-            self._gemm(ws[f"f_{l}"], w[self._lp(l, "linear2.weight")], bias=p[self._lp(l, "linear2.bias")],
-                       drop_p=dp, drop_seed=seed, drop_seed_dev=sdev, drop_site=_site(l, 3),
-                       residual=ws[f"xmid_{l}"], out_f32=ws[f"xout_{l}"])
+            self._layer_tail(l, ws[f"ctx_{l}"], x_in, ws[f"xmid_{l}"], ws[f"h2_{l}"], ws[f"f_{l}"], ws[f"xout_{l}"],
+                             dp, seed, sdev)
             x_in = ws[f"xout_{l}"]
             if l + 1 < cfg.num_layers:
                 ops.chain_fwd(x_in, ln=(p[self._lp(l + 1, "norm1.weight")], p[self._lp(l + 1, "norm1.bias")]),
@@ -516,12 +571,30 @@ class TwoTowerEngine:
         else:
             ops.gather_cat_fwd(x_in, ws["last_idx"], gender, country, p[ut + "gender_embedding.weight"],
                                p[ut + "country_embedding.weight"], B, L, ws["cat"])
+        return self._user_head(ws)
+
+    def _user_head(self, ws) -> torch.Tensor:
+        """Fusion MLP on ws['cat'] (last encoder row | gender | country) -> L2-normalised user embedding ws['un']."""
+        p, w = self.p, self.w
+        ut = "user_tower."
         self._gemm(ws["cat"], w[ut + "fusion_layer.0.weight"], bias=p[ut + "fusion_layer.0.bias"], out_f32=ws["z1"])
         ops.chain_fwd(ws["z1"], ln=(p[ut + "fusion_layer.1.weight"], p[ut + "fusion_layer.1.bias"]), relu=True,
                       out_bf16=ws["a1"])
         self._gemm(ws["a1"], w[ut + "fusion_layer.3.weight"], bias=p[ut + "fusion_layer.3.bias"], out_f32=ws["u"])
         ops.chain_fwd(ws["u"], l2norm=True, out_f32=ws["un"], out_bf16=ws["un_bf"])
         return ws["un"]
+
+    def _layer_tail(self, l, ctx, x_in, xmid, h2, f, xout, dp, seed, sdev) -> None:
+        """Encoder layer l after the attention, on whichever rows ``ctx`` holds: out_proj + residual x_in -> xmid,
+        norm2 -> h2, linear1 + ReLU -> f, linear2 + residual -> xout."""
+        p, w = self.p, self.w
+        self._gemm(ctx, w[self._lp(l, "self_attn.out_proj.weight")], bias=p[self._lp(l, "self_attn.out_proj.bias")],
+                   drop_p=dp, drop_seed=seed, drop_seed_dev=sdev, drop_site=_site(l, 1), residual=x_in, out_f32=xmid)
+        ops.chain_fwd(xmid, ln=(p[self._lp(l, "norm2.weight")], p[self._lp(l, "norm2.bias")]), out_bf16=h2)
+        self._gemm(h2, w[self._lp(l, "linear1.weight")], bias=p[self._lp(l, "linear1.bias")], relu=True,
+                   drop_p=dp, drop_seed=seed, drop_seed_dev=sdev, drop_site=_site(l, 2), out_bf16=f)
+        self._gemm(f, w[self._lp(l, "linear2.weight")], bias=p[self._lp(l, "linear2.bias")], drop_p=dp,
+                   drop_seed=seed, drop_seed_dev=sdev, drop_site=_site(l, 3), residual=xmid, out_f32=xout)
 
     def _last_layer_forward(self, ws, l, x_in, B, L, dp, seed, sdev) -> None:
         """Last encoder layer, exact single-row form: K/V for every position, everything downstream of
@@ -534,16 +607,7 @@ class TwoTowerEngine:
         self._gemm(ws["hq"], Wqkv[:D], bias=bqkv[:D], out_bf16=ws["qq"])                          # Q, B rows
         ops.attn_lastq_fwd(ws["qq"], ws[f"qkv_{l}"], ws["last_idx"], ws["ctxq"], ws["lseq"], B, L, cfg.num_heads,
                            drop_p=dp, seed=seed, seed_dev=sdev, site=_site(l, 0))
-        self._gemm(ws["ctxq"], w[self._lp(l, "self_attn.out_proj.weight")], bias=p[self._lp(l, "self_attn.out_proj.bias")],
-                   drop_p=dp, drop_seed=seed, drop_seed_dev=sdev, drop_site=_site(l, 1), residual=ws["xq_in"],
-                   out_f32=ws["xmid_q"])
-        ops.chain_fwd(ws["xmid_q"], ln=(p[self._lp(l, "norm2.weight")], p[self._lp(l, "norm2.bias")]),
-                      out_bf16=ws["h2q"])
-        self._gemm(ws["h2q"], w[self._lp(l, "linear1.weight")], bias=p[self._lp(l, "linear1.bias")], relu=True,
-                   drop_p=dp, drop_seed=seed, drop_seed_dev=sdev, drop_site=_site(l, 2), out_bf16=ws["fq"])
-        self._gemm(ws["fq"], w[self._lp(l, "linear2.weight")], bias=p[self._lp(l, "linear2.bias")], drop_p=dp,
-                   drop_seed=seed, drop_seed_dev=sdev, drop_site=_site(l, 3), residual=ws["xmid_q"],
-                   out_f32=ws["xout_q"])
+        self._layer_tail(l, ws["ctxq"], ws["xq_in"], ws["xmid_q"], ws["h2q"], ws["fq"], ws["xout_q"], dp, seed, sdev)
 
     def _last_layer_backward(self, ws, l, x_in, B, L, dp, seed, sdev, dx, dx_other):
         """Backward of _last_layer_forward. ws['dxq'] holds d(loss)/d(xout_q) (B rows). Returns the
@@ -916,6 +980,7 @@ class TwoTowerEngine:
                        eps, weight_decay, shadow=self.shadow, shadow_begin=self.dense_begin, shadow_end=self.numel,
                        zero_grad=zero_grad)
         self.shadow_valid = True
+        self.weights_epoch += 1
 
     def adamw_step_sharded(self, rank: int, world: int, grad_shard: torch.Tensor, lr: float = 1e-4,
                            betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 0.01) -> torch.Tensor:
@@ -935,6 +1000,7 @@ class TwoTowerEngine:
         ops.adamw_step(p_shard, grad_shard, self.exp_avg, self.exp_avg_sq, self.step_dev, lr, betas[0], betas[1],
                        eps, weight_decay, shadow=None, zero_grad=False)
         self.shadow_valid = False
+        self.weights_epoch += 1
         return p_shard
 
     def train_step(self, batch: Dict[str, torch.Tensor], lr: float = 1e-4) -> torch.Tensor:

@@ -112,8 +112,16 @@ def recommend_batch(model, index: retrieval.CatalogIndex, history_ids: torch.Ten
         u = torch.cat([model.get_user_embedding(ids[s:s + chunk], mask[s:s + chunk], gender[s:s + chunk],
                                                 country[s:s + chunk]) for s in range(0, B, chunk)])
     model.train(was_training)
-    u = F.normalize(u.float(), p=2, dim=1, eps=1e-8)                     # src/inference.py:286
     ex = ids * (mask != 0) if exclude_ids is None else exclude_ids.to(dev).long()
+    return recommend_embeddings(u, index, ex, k, group)
+
+
+def recommend_embeddings(u: torch.Tensor, index: retrieval.CatalogIndex, ex: torch.Tensor, k: int,
+                         group=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The selection of `recommend_batch` for given user embeddings ``u`` (B, 256): re-normalise (eps 1e-8), then the
+    top k over plain or sharded ``index`` with item 0 and the ids of ``ex`` (B, m) int64 (0 = empty) excluded."""
+    B = u.shape[0]
+    u = F.normalize(u.float(), p=2, dim=1, eps=1e-8)                     # src/inference.py:286
     if ex.shape[0] != B:
         raise ValueError(f"exclude_ids has {ex.shape[0]} rows for {B} users")
     exclude = retrieval.Exclusions(ex, index.vocab_size)

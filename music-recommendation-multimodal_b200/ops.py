@@ -143,6 +143,35 @@ def embed_ln_fwd(ids, E, P, ln_w, ln_b, next_w, next_b, B, L, x0, h, drop_p=0.0,
                                 x0.data_ptr(), h.data_ptr(), _stream()), "tt_embed_ln_fwd")
 
 
+def embed_ln_fwd_pos(ids, pos, E, P, ln_w, ln_b, next_w, next_b, x0, h) -> None:
+    """tt_embed_ln_fwd_pos: embed_ln_fwd's rows for item ids[r] at position pos[r] (eval, local table)."""
+    _require_cuda(ids, pos, E, P, x0, h)
+    n = ids.numel()
+    assert ids.dtype == torch.int64 and ids.is_contiguous() and pos.dtype == torch.int32 and pos.is_contiguous()
+    assert pos.numel() == n and E.dtype == torch.float32 and E.shape[1] == 256
+    assert x0.dtype == torch.float32 and x0.is_contiguous() and x0.shape == (n, 256)
+    assert h.dtype == torch.bfloat16 and h.is_contiguous() and h.shape == (n, 256)
+    check(lib().tt_embed_ln_fwd_pos(ids.data_ptr(), pos.data_ptr(), E.data_ptr(), P.data_ptr(), ln_w.data_ptr(),
+                                    ln_b.data_ptr(), next_w.data_ptr(), next_b.data_ptr(), n, x0.data_ptr(),
+                                    h.data_ptr(), _stream()), "tt_embed_ln_fwd_pos")
+
+
+def session_attn(qkv, k_cache, v_cache, slots, pos, ctx) -> None:
+    """tt_session_attn: each new row's K/V into cache[slot, :, pos], ctx = its attention over positions 0..pos.
+    qkv bf16 [n, 3*H*64], caches bf16 [capacity, H, L, 64], slots / pos int32 [n] -> ctx bf16 [n, H*64]."""
+    _require_cuda(qkv, k_cache, v_cache, slots, pos, ctx)
+    n = slots.numel()
+    cap, H, L, dh = k_cache.shape
+    assert dh == 64 and v_cache.shape == k_cache.shape
+    for t in (qkv, k_cache, v_cache, ctx):
+        assert t.dtype == torch.bfloat16 and t.is_contiguous()
+    assert qkv.shape == (n, 3 * H * 64) and ctx.shape == (n, H * 64)
+    assert slots.dtype == torch.int32 and pos.dtype == torch.int32 and pos.numel() == n
+    assert slots.is_contiguous() and pos.is_contiguous()
+    check(lib().tt_session_attn(qkv.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), slots.data_ptr(),
+                                pos.data_ptr(), n, H, L, cap, ctx.data_ptr(), _stream()), "tt_session_attn")
+
+
 def embed_ln_bwd(ids, E, P, ln_w, ln_b, dx0, B, L, dE, dP, dgamma, dbeta, drop_p=0.0, seed=0, seed_dev=None, site=0):
     _require_cuda(ids, E, P, dx0, dE, dP, dgamma, dbeta)
     check(lib().tt_embed_ln_bwd(ids.data_ptr(), E.data_ptr(), P.data_ptr(), ln_w.data_ptr(), ln_b.data_ptr(),

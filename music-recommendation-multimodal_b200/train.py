@@ -399,6 +399,7 @@ class TrainStepRunner:
     def step_resident(self) -> torch.Tensor:
         """One step on whatever is in the static buffers; returns the device loss scalar (with gathered
         negatives: this rank's share of the global loss; step_from_host sums it over ranks)."""
+        self.eng.weights_epoch += 1            # a replayed graph updates the parameters without adamw_step's Python
         if not self._warm:
             c0 = _lib.launch_count
             self._eager()                      # allocates workspaces / moments, sets func attributes
