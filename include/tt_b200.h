@@ -138,23 +138,6 @@ int tt_embed_ln_bwd(const int64_t* ids, const float* E, const float* P, const fl
                     const float* dx0, int B, int L, float drop_p, uint64_t seed, const uint64_t* seed_dev,
                     uint32_t site, float* dE, float* dP, float* dgamma, float* dbeta, void* stream);
 
-/* tt_embed_ln_bwd with the first encoder layer's norm1 backward (src/models/user_tower.py:37-45, norm_first=True:
- * x + attn(norm1(x))) in front of it: d(loss)/d(x0) = LayerNorm1'(x0; dh) + resid is formed per token in registers from
- * x0 recomputed out of the table row (same dropout hash as the forward), so neither x0 nor dx0 is read or written.
- * dgamma / dbeta of norm1 are accumulated like the others. */
-typedef struct tt_norm1_bwd {
-  const void* dh_bf16;   /* bf16 [B*L,256]: gradient w.r.t. norm1's output (dX of the packed in_proj) */
-  const float* resid;    /* fp32 [B*L,256]: residual-stream gradient arriving at x0 */
-  const float* ln_w;     /* norm1.weight / norm1.bias */
-  const float* ln_b;
-  float* dgamma;
-  float* dbeta;
-} tt_norm1_bwd;
-int tt_embed_ln_bwd_norm1(const tt_norm1_bwd* n1, const int64_t* ids, const float* E, const float* P,
-                          const float* ln_w, const float* ln_b, int B, int L, float drop_p, uint64_t seed,
-                          const uint64_t* seed_dev, uint32_t site, float* dE, float* dP, float* dgamma, float* dbeta,
-                          void* stream);
-
 /* Deterministic form of tt_embed_ln_bwd for the table gradient (the reference's embedding backward is
  * autograd's embedding_dense_backward, src/models/user_tower.py:26; its CUDA form is deterministic only under
  * torch.use_deterministic_algorithms). Token t adds its gradient row into acc64[slot_of_token[t]] (int64
@@ -264,9 +247,6 @@ typedef struct tt_bn_args {
 } tt_bn_args;
 int tt_bn_relu_fwd(const tt_bn_args* args, void* stream);
 int tt_bn_relu_bwd(const tt_bn_args* args, void* stream);
-
-/* out[n] += sum_r x[r, n] for a bf16 [R, N] matrix (bias gradients). */
-int tt_colsum_bf16(const void* x_bf16, int R, int N, int ld, float* out, void* stream);
 
 /* Fused dense AdamW over a flat fp32 buffer (torch.optim.AdamW as used at src/train.py:302,
  * 64-65): p,g,m,v [n]; the gradient used is grad_scale * g (1 / world for a buffer that holds the SUM of the
@@ -429,26 +409,15 @@ int tt_exact_topk_excl(const float* user_f32, const float* items_f32, int N, int
 int tt_rank_metrics(const int32_t* topk_idx, const int64_t* targets, int U, int K, const int32_t* k_list, int nk,
                     const float* gain_table, float* recall, float* ndcg, void* stream);
 
-/* ---- ID-embedding lookups against a table row-sharded over the ranks of one NVLink domain ----------
+/* ---- ID table row-sharded over the ranks of one NVLink domain ----------
  * (BASELINE.json configs[4]: 10M items; reference: nn.Embedding(vocab_size, 256, padding_idx=0) and its dense
  * gradient, src/models/user_tower.py:26,86.) The table and its gradient live in a symmetric arena (tt_symm_team
  * below): the rows are dealt ROUND-ROBIN (item popularity is Zipfian in the id: contiguous ranges would send most
  * lookups to rank 0): row id is local row id / world of rank id % world, at byte `weight_offset` / `grad_offset` of
- * that rank's copy. Same computation as tt_embed_ln_fwd / tt_embed_ln_bwd; a token's row is read from — and its gradient
- * row added (red.global.add.v4.f32) into — the OWNER's memory over NVLink. No ids or rows are exchanged between
- * ranks. row_stash (nullable, fp32 [B*L, 256]): the forward keeps the gathered rows, the backward reads them
- * instead of crossing NVLink a second time. The caller separates steps with tt_symm_barrier (owners' updates
- * visible before the next gather; all ranks' gradient rows landed before the owner's AdamW). */
+ * that rank's copy. Rows are read from — and gradient rows added (red.global.add.v4.f32) into — the OWNER's memory
+ * over NVLink. The caller separates steps with tt_symm_barrier (owners' updates visible before the next gather; all
+ * ranks' gradient rows landed before the owner's AdamW). */
 struct tt_symm_team;
-int tt_embed_ln_fwd_sharded(const int64_t* ids, const struct tt_symm_team* team, int64_t weight_offset,
-                            float* row_stash, const float* P, const float* ln_w, const float* ln_b,
-                            const float* next_w, const float* next_b, int B, int L, float drop_p, uint64_t seed,
-                            const uint64_t* seed_dev, uint32_t site, float* x0, void* h_bf16, void* stream);
-int tt_embed_ln_bwd_sharded(const int64_t* ids, const struct tt_symm_team* team, int64_t weight_offset,
-                            int64_t grad_offset, const float* row_stash, const float* P,
-                            const float* ln_w, const float* ln_b, const float* dx0, int B, int L, float drop_p,
-                            uint64_t seed, const uint64_t* seed_dev, uint32_t site, float* dP, float* dgamma,
-                            float* dbeta, void* stream);
 
 /* Duplicate-free traffic for a row-sharded (or replicated) ID table. Histories are Zipfian in the item id: at batch
  * 256 x 200 about a third of the tokens carry a distinct id, so a step first reduces its ids to the distinct ones.

@@ -109,13 +109,6 @@ class ChainArgs(ctypes.Structure):
     ]
 
 
-class Norm1Bwd(ctypes.Structure):
-    """Mirror of ``tt_norm1_bwd``."""
-
-    _fields_ = [("dh_bf16", c_void_p), ("resid", c_void_p), ("ln_w", c_void_p), ("ln_b", c_void_p),
-                ("dgamma", c_void_p), ("dbeta", c_void_p)]
-
-
 class BnArgs(ctypes.Structure):
     """Mirror of ``tt_bn_args``."""
 
@@ -197,9 +190,6 @@ _SIGNATURES = {
     "tt_session_attn": [c_void_p] * 5 + [c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p],
     "tt_embed_ln_bwd": [c_void_p] * 6 + [c_int32, c_int32, c_float, c_uint64, c_void_p, c_uint32,
                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
-    "tt_embed_ln_bwd_norm1": [ctypes.POINTER(Norm1Bwd)] + [c_void_p] * 5 + [c_int32, c_int32, c_float, c_uint64, c_void_p,
-                                                                       c_uint32, c_void_p, c_void_p, c_void_p, c_void_p,
-                                                                       c_void_p],
     "tt_embed_ln_bwd_det": [c_void_p] * 6 + [c_int32, c_int32, c_float, c_uint64, c_void_p, c_uint32,
                                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
     "tt_rows_scatter_add_i64": [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p],
@@ -210,17 +200,11 @@ _SIGNATURES = {
     "tt_concat4_bf16": [c_void_p] * 4 + [c_int32, c_int32, c_void_p, c_void_p],
     "tt_bn_relu_fwd": [ctypes.POINTER(BnArgs), c_void_p],
     "tt_bn_relu_bwd": [ctypes.POINTER(BnArgs), c_void_p],
-    "tt_colsum_bf16": [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p],
     "tt_adamw_step": [c_void_p] * 4 + [_I64, c_float, c_float, c_float, c_float, c_float, c_float, c_void_p, c_void_p,
                                        _I64, _I64, c_int32, c_void_p],
     "tt_ids_dedup": [c_void_p, c_int32, _I64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
     "tt_rows_gather": [ctypes.POINTER(SymmTeam), _I64, c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p],
     "tt_rows_scatter_add": [ctypes.POINTER(SymmTeam), _I64, c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p],
-    "tt_embed_ln_fwd_sharded": [c_void_p, ctypes.POINTER(SymmTeam), _I64] + [c_void_p] * 6 +
-                               [c_int32, c_int32, c_float, c_uint64, c_void_p, c_uint32, c_void_p, c_void_p, c_void_p],
-    "tt_embed_ln_bwd_sharded": [c_void_p, ctypes.POINTER(SymmTeam), _I64, _I64] + [c_void_p] * 5 +
-                               [c_int32, c_int32, c_float, c_uint64, c_void_p, c_uint32, c_void_p, c_void_p, c_void_p,
-                                c_void_p],
     "tt_step_counters_advance": [c_void_p, c_void_p, c_void_p],
     "tt_infonce_rows": [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_int32, c_void_p, c_void_p,
                         c_void_p],

@@ -3,7 +3,6 @@
 // has no link-time dependency on libcuda), device properties.
 #include <stdarg.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "../../include/tt_b200.h"
@@ -90,26 +89,6 @@ int make_tmap(CUtensorMap* out, const void* base, int rank, const uint64_t* dims
     return TT_ERR_CUDA;
   }
   return TT_OK;
-}
-
-int pdl_mode() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("TT_PDL");
-    v = e ? atoi(e) : 2;   // measured on the c2 step: 1.308 ms (0), 1.326 ms (1), 1.282 ms (2)
-    if (v < 0 || v > 2) v = 2;
-  }
-  return v;
-}
-
-int pdl_max_ctas() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("TT_PDL_MAX_CTAS");
-    v = e ? atoi(e) : 64;
-    if (v < 1) v = 64;
-  }
-  return v;
 }
 
 int num_sms() {

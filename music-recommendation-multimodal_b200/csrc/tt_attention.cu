@@ -6,15 +6,17 @@
 // for every VALID query row the causal predicate alone is the full mask (keys <= query <
 // length) and no mask tensor exists. Pad-query rows produce finite values nobody reads.
 //
-// Forward: one CTA (128 threads = 128 query rows = 128 TMEM lanes) per (sequence, head,
-// 128-row query tile). All S_j = Q K_j^T tiles (j <= query tile) are issued up front into
-// TMEM (128 columns each, L <= 512), the row max is taken from TMEM, then per key tile
+// Forward (256 < L <= 512; attn_fwd_persist_kernel takes L <= 256, attn_fwd_long_kernel L > 512):
+// one CTA (128 threads = 128 query rows = 128 TMEM lanes) per (sequence, head, 128-row query tile).
+// All S_j = Q K_j^T tiles (j <= query tile) are issued up front into TMEM (128 columns each,
+// L <= 512), the row max is taken from TMEM, then per key tile
 // P_j = exp2(.) is written as bf16 into a 128B-swizzled K-major smem tile (double-buffered)
 // and O += P_j V_j accumulates in TMEM (V consumed MN-major straight from the QKV buffer's
 // layout). O reuses the first 64 columns of S_0 once S_0 has been drained.
 //
-// Backward: one CTA per (sequence, head) walks key tiles j and query tiles i >= j with the
-// five products of the standard attention backward, all on tcgen05 (see attn_bwd_kernel).
+// Backward (256 < L <= 512; attn_bwd_persist_kernel takes L <= 256, attn_bwd_long_kernel L > 512):
+// one CTA per (sequence, head) walks key tiles j and query tiles i >= j with the five products of
+// the standard attention backward, all on tcgen05 (see attn_bwd_kernel).
 #include "../../include/tt_b200.h"
 #include "tt_common.cuh"
 
@@ -628,19 +630,19 @@ attn_fwd_persist_kernel(const __grid_constant__ CUtensorMap tmQKV, const AttnPar
 }
 
 // --------------------------------------------------------------------------------------------
-// Backward. One CTA (256 threads) per (sequence, head). For key tile j and query tile i >= j:
-//   S   = Q_i K_j^T                    (TMEM cols [0,128))
-//   dP  = dO_i V_j^T                   (TMEM cols [128,256))
+// Backward. One CTA per (sequence, head). For key tile j and query tile i >= j:
+//   S   = Q_i K_j^T
+//   dP  = dO_i V_j^T
 //   P   = exp2(scale*log2e*S - lse_i*log2e) under the causal mask; Pd = dropout(P)
 //   dS  = P * (dropout(dP) - delta_i) * scale,  delta_i = rowsum(dO_i * O_i)
 //   dV_j += Pd^T dO_i   (A = Pd stored [q][kv] read MN-major, B = dO_i read MN-major)
 //   dK_j += dS^T Q_i    (A = dS read MN-major,               B = Q_i  read MN-major)
 //   dQ_i += dS K_j      (A = dS K-major,                     B = K_j  read MN-major)
-// dV_j, dK_j live in TMEM (cols [256,320), [320,384)) across the inner loop; dQ_i
-// (cols [384 + 64*i ...)) is kept for every query tile: two tiles (L <= 256) in the fast layout,
-// four (L <= 512) in the LONG layout described at the kernel.
-// Pd and dS are staged as bf16 in 128B-swizzled smem tiles. Thread (row, hf) owns query row
-// `row` and the 64-column half `hf` of the 128-key tile (warp & 3 = TMEM lane quarter).
+// dV_j, dK_j live in TMEM across the inner loop; dQ_i (64 columns) is kept for every query tile.
+// TMEM columns for two query tiles (L <= 256, attn_bwd_persist_kernel): S [0,128), dP [128,256), dV [256,320),
+// dK [320,384), dQ_i [384 + 64*i); for four (L <= 512, attn_bwd_kernel) see that kernel.
+// Pd and dS are staged as bf16 in 128B-swizzled smem tiles. Thread (row, grp) owns query row `row`
+// and the 32-column chunk `grp` of the 128-key tile (warp & 3 = TMEM lane quarter).
 // --------------------------------------------------------------------------------------------
 // Keep decisions of 32 consecutive elements starting at didx0 as a bit mask: one hash per 4 (2, 1) elements
 // depending on the alignment of didx0 — the same decisions drop_keep_k gives element by element.
@@ -683,15 +685,11 @@ struct AttnBwdParams {
   __nv_bfloat16* dqkv;        // [T, 3*H*64]
 };
 
-// LONG = false: L <= 256 (two query tiles): S and dP have their own TMEM columns and are issued
-//   together. LONG = true: L <= 512 (four query tiles): the four dQ accumulators need 256 columns,
-//   so S and dP SHARE one 128-column region — P is formed from S first (un-dropped P parked as bf16
-//   in the dS tile), then dP = dO V^T overwrites S and dS replaces the parked P.
-// CG = column groups: 128*CG threads, thread (row, g) owns 4/CG of the four 32-column chunks of every
-// 128-key tile. The per-iteration element-wise phase between the two MMA groups is latency-bound, so the
-// fast layout runs it with 16 warps (CG = 4); LONG keeps 8 (its register tiles are larger).
-template <bool LONG, int CG>
-__global__ void __launch_bounds__(128 * CG, 1)
+// L <= 512 (up to four query tiles): the four dQ accumulators need 256 TMEM columns, so S and dP SHARE one
+// 128-column region — P is formed from S first (un-dropped P parked as bf16 in the dS tile), then dP = dO V^T
+// overwrites S and dS replaces the parked P. 512 threads: thread (row, grp) owns the 32-column chunk `grp` of
+// every 128-key tile; the element-wise phase between the two MMA groups is latency-bound, so it runs on 16 warps.
+__global__ void __launch_bounds__(512, 1)
 attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmDO,
                 const AttnBwdParams p) {
   extern __shared__ uint8_t smem_raw[];
@@ -701,7 +699,6 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
   const int tid = threadIdx.x;
   const int warp = tid >> 5, lane = tid & 31;
   const int q = warp & 3, grp = warp >> 2;
-  constexpr int CPT = 4 / CG;   // 32-column chunks per thread per key tile
   const int row = q * 32 + lane;
   const int bh = blockIdx.x;
   const int b = bh / p.H, h = bh % p.H;
@@ -709,21 +706,19 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
   const int nq = p.nq;
   const int seq_row0 = b * p.L;
 
-  // smem: Q[slots], dO[slots], K_j, V_j, Pd (2 chunks), dS (2 chunks). The fast layout keeps every
-  // query tile resident; LONG re-loads Q_i / dO_i per (j, i) iteration into a single slot.
-  const int slots = LONG ? 1 : nq;
+  // smem: Q_i, dO_i, K_j, V_j, Pd (2 chunks), dS (2 chunks). Q_i / dO_i are re-loaded per (j, i) iteration.
   uint8_t* sQ = smem;
-  uint8_t* sDO = sQ + static_cast<size_t>(slots) * kTileBytes;
-  uint8_t* sK = sDO + static_cast<size_t>(slots) * kTileBytes;
+  uint8_t* sDO = sQ + kTileBytes;
+  uint8_t* sK = sDO + kTileBytes;
   uint8_t* sV = sK + kTileBytes;
   uint8_t* sPd = sV + kTileBytes;
   uint8_t* sDS = sPd + 2 * kTileBytes;
   uint64_t* bars = reinterpret_cast<uint64_t*>(sDS + 2 * kTileBytes);
   uint64_t* bar_q = bars + 0;    // Q/dO tiles loaded
   uint64_t* bar_kv = bars + 1;   // K_j/V_j loaded (phase per j)
-  uint64_t* bar_mm1 = bars + 2;  // S and dP ready (phase per (j,i))
+  uint64_t* bar_mm1 = bars + 2;  // S ready (phase per (j,i))
   uint64_t* bar_mm2 = bars + 3;  // dV/dK/dQ MMAs of this (j,i) retired
-  uint64_t* bar_mm1b = bars + 4; // LONG: dP ready (after S has been consumed)
+  uint64_t* bar_mm1b = bars + 4; // dP ready (after S has been consumed)
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 5);
   float* sDelta = reinterpret_cast<float*>(bars + 8);  // [nq*128]
   float* sLse = sDelta + nq * kTile;                   // [nq*128], pre-multiplied by log2e
@@ -753,18 +748,10 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
   pdl_launch_dependents();
   pdl_wait();   // prologue (barriers, TMEM, tensor-map prefetch) overlapped the previous kernel's tail
   const uint32_t lane_base = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
-  constexpr uint32_t T_S = 0, T_DP = LONG ? 0 : 128, T_DV = LONG ? 128 : 256, T_DK = LONG ? 192 : 320,
-                     T_DQ = LONG ? 256 : 384;
+  constexpr uint32_t T_S = 0, T_DP = 0, T_DV = 128, T_DK = 192, T_DQ = 256;
 
-  if (!LONG && tid == 0) {
-    mbar_arrive_expect_tx(bar_q, 2 * nq * kTileBytes);
-    for (int i = 0; i < nq; ++i) {
-      tma_load_2d(sQ + static_cast<size_t>(i) * kTileBytes, &tmQKV, bar_q, h * kDh, seq_row0 + i * kTile);
-      tma_load_2d(sDO + static_cast<size_t>(i) * kTileBytes, &tmDO, bar_q, h * kDh, seq_row0 + i * kTile);
-    }
-  }
   // delta_i = rowsum(dO * O), lse -> smem (generic loads; rows beyond L are treated as zero)
-  for (int pos = tid; pos < nq * kTile; pos += 128 * CG) {
+  for (int pos = tid; pos < nq * kTile; pos += 512) {
     float delta = 0.f, lse2 = 0.f;
     if (pos < p.L) {
       const uint4* o = reinterpret_cast<const uint4*>(p.ctx + static_cast<size_t>(seq_row0 + pos) * D + h * kDh);
@@ -803,31 +790,20 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
       tma_load_2d(sV, &tmQKV, bar_kv, 2 * D + h * kDh, seq_row0 + j * kTile);
     }
     for (int i = j; i < nq; ++i, ++it) {
-      const int slot = LONG ? 0 : i;
       if (tid == 0) {
-        if constexpr (LONG) {   // the previous iteration's MMAs retired (bar_mm2): the slot is free
-          mbar_arrive_expect_tx(bar_q, 2 * kTileBytes);
-          tma_load_2d(sQ, &tmQKV, bar_q, h * kDh, seq_row0 + i * kTile);
-          tma_load_2d(sDO, &tmDO, bar_q, h * kDh, seq_row0 + i * kTile);
-          mbar_wait(bar_q, it & 1);
-        } else {
-          if (it == 0) mbar_wait(bar_q, 0);
-        }
+        // the previous iteration's MMAs retired (bar_mm2): the Q / dO slot is free
+        mbar_arrive_expect_tx(bar_q, 2 * kTileBytes);
+        tma_load_2d(sQ, &tmQKV, bar_q, h * kDh, seq_row0 + i * kTile);
+        tma_load_2d(sDO, &tmDO, bar_q, h * kDh, seq_row0 + i * kTile);
+        mbar_wait(bar_q, it & 1);
         if (i == j) mbar_wait(bar_kv, j & 1);
         tc_fence_after();
-        const uint32_t q_base = smem_u32(sQ + static_cast<size_t>(slot) * kTileBytes);
-        const uint32_t do_base = smem_u32(sDO + static_cast<size_t>(slot) * kTileBytes);
-        const uint32_t k_base = smem_u32(sK), v_base = smem_u32(sV);
+        const uint32_t q_base = smem_u32(sQ);
+        const uint32_t k_base = smem_u32(sK);
 #pragma unroll
         for (int k = 0; k < kDh / 16; ++k)
           umma_bf16(tmem_base + T_S, umma_desc_kmajor(q_base + k * 32), umma_desc_kmajor(k_base + k * 32),
                     idesc_s, k > 0 ? 1u : 0u);
-        if constexpr (!LONG) {
-#pragma unroll
-          for (int k = 0; k < kDh / 16; ++k)
-            umma_bf16(tmem_base + T_DP, umma_desc_kmajor(do_base + k * 32), umma_desc_kmajor(v_base + k * 32),
-                      idesc_s, k > 0 ? 1u : 0u);
-        }
         umma_commit(bar_mm1);
       }
       mbar_wait(bar_mm1, it & 1);
@@ -839,156 +815,98 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
       const float delta = sDelta[q_pos];
       const bool diag = (i == j);
       const bool row_ok = q_pos < p.L;
-      if constexpr (LONG) {
-        // ---- part A: P from S. Pd -> sPd, un-dropped P parked (bf16) in the dS tile ---------------
-        uint32_t km[CPT];   // dropout keep bits of this thread's chunks, formed once and reused by part B
+      // ---- part A: P from S. Pd -> sPd, un-dropped P parked (bf16) in the dS tile ---------------
+      uint32_t km;   // dropout keep bits of this thread's chunk, formed once and reused by part B
+      {
+      const int u0 = (grp & 1) * 4;
+      uint8_t* pchunk = sPd + static_cast<size_t>(grp >> 1) * kTileBytes;
+      uint8_t* dchunk = sDS + static_cast<size_t>(grp >> 1) * kTileBytes;
+      if (!(diag && grp > q)) {
+        uint32_t rs[32];
+        tmem_ld32(lane_base + T_S + grp * 32, rs);
+        tmem_ld_wait();
+        const int kv0 = j * kTile + grp * 32;
+        const uint32_t didx0 = (static_cast<uint32_t>(bh) * p.L + q_pos) * p.L + kv0;
+        km = p.drop_thresh ? drop_keepmask32(dkey, didx0, p.drop_thresh) : 0xFFFFFFFFu;
+        float pr[32], pd[32];
 #pragma unroll
-        for (int cc = 0; cc < CPT; ++cc) {
-          const int cg = CPT * grp + cc;
-          const int u0 = (cg & 1) * 4;
-          uint8_t* pchunk = sPd + static_cast<size_t>(cg >> 1) * kTileBytes;
-          uint8_t* dchunk = sDS + static_cast<size_t>(cg >> 1) * kTileBytes;
-          if (!(diag && cg > q)) {
-            uint32_t rs[32];
-            tmem_ld32(lane_base + T_S + cg * 32, rs);
-            tmem_ld_wait();
-            const int kv0 = j * kTile + cg * 32;
-            const uint32_t didx0 = (static_cast<uint32_t>(bh) * p.L + q_pos) * p.L + kv0;
-            km[cc] = p.drop_thresh ? drop_keepmask32(dkey, didx0, p.drop_thresh) : 0xFFFFFFFFu;
-            float pr[32], pd[32];
-#pragma unroll
-            for (int t = 0; t < 32; ++t) {
-              float x = fast_exp2(__uint_as_float(rs[t]) * c1 - lse2);
-              if ((diag && kv0 + t > q_pos) || !row_ok) x = 0.f;
-              pr[t] = x;
-              pd[t] = ((km[cc] >> t) & 1u) ? x * p.drop_scale : 0.f;
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-              uint4 v, w;
-              v.x = pack_bf16(pd[u * 8 + 0], pd[u * 8 + 1]);
-              v.y = pack_bf16(pd[u * 8 + 2], pd[u * 8 + 3]);
-              v.z = pack_bf16(pd[u * 8 + 4], pd[u * 8 + 5]);
-              v.w = pack_bf16(pd[u * 8 + 6], pd[u * 8 + 7]);
-              w.x = pack_bf16(pr[u * 8 + 0], pr[u * 8 + 1]);
-              w.y = pack_bf16(pr[u * 8 + 2], pr[u * 8 + 3]);
-              w.z = pack_bf16(pr[u * 8 + 4], pr[u * 8 + 5]);
-              w.w = pack_bf16(pr[u * 8 + 6], pr[u * 8 + 7]);
-              st_swizzled_unit(pchunk, row, u0 + u, v);
-              st_swizzled_unit(dchunk, row, u0 + u, w);
-            }
-          } else {
-            km[cc] = 0u;
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-              st_swizzled_unit(pchunk, row, u0 + u, make_uint4(0, 0, 0, 0));
-              st_swizzled_unit(dchunk, row, u0 + u, make_uint4(0, 0, 0, 0));
-            }
-          }
+        for (int t = 0; t < 32; ++t) {
+          float x = fast_exp2(__uint_as_float(rs[t]) * c1 - lse2);
+          if ((diag && kv0 + t > q_pos) || !row_ok) x = 0.f;
+          pr[t] = x;
+          pd[t] = ((km >> t) & 1u) ? x * p.drop_scale : 0.f;
         }
-        // ---- dP = dO V^T overwrites S once every thread has drained it --------------------------
-        tc_fence_before();
-        __syncthreads();
-        if (tid == 0) {
-          tc_fence_after();
-          const uint32_t do_base = smem_u32(sDO + static_cast<size_t>(slot) * kTileBytes);
-          const uint32_t v_base = smem_u32(sV);
 #pragma unroll
-          for (int k = 0; k < kDh / 16; ++k)
-            umma_bf16(tmem_base + T_DP, umma_desc_kmajor(do_base + k * 32), umma_desc_kmajor(v_base + k * 32),
-                      idesc_s, k > 0 ? 1u : 0u);
-          umma_commit(bar_mm1b);
-        }
-        mbar_wait(bar_mm1b, it & 1);
-        __syncwarp();
-        tc_fence_after();
-        // ---- part B: dS = P * (dropout(dP) - delta) * scale replaces the parked P ------------------
-#pragma unroll
-        for (int cc = 0; cc < CPT; ++cc) {
-          const int cg = CPT * grp + cc;
-          const int u0 = (cg & 1) * 4;
-          uint8_t* pchunk = sPd + static_cast<size_t>(cg >> 1) * kTileBytes;
-          uint8_t* dchunk = sDS + static_cast<size_t>(cg >> 1) * kTileBytes;
-          if (!(diag && cg > q)) {
-            uint32_t rp[32];
-            tmem_ld32(lane_base + T_DP + cg * 32, rp);
-            tmem_ld_wait();
-            const int kv0 = j * kTile + cg * 32;
-            const uint32_t didx0 = (static_cast<uint32_t>(bh) * p.L + q_pos) * p.L + kv0;
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-              uint4* slot = reinterpret_cast<uint4*>(dchunk + row * 128 + (((u0 + u) ^ (row & 7)) << 4));
-              const uint4 pw = *slot;
-              const uint32_t w[4] = {pw.x, pw.y, pw.z, pw.w};
-              float ds[8];
-#pragma unroll
-              for (int h2 = 0; h2 < 4; ++h2) {
-                const float2 pr2 = unpack_bf16(w[h2]);
-#pragma unroll
-                for (int e = 0; e < 2; ++e) {
-                  const int t = u * 8 + h2 * 2 + e;
-                  const float prv = e ? pr2.y : pr2.x;
-                  const bool keep = (km[cc] >> t) & 1u;
-                  const float dp = keep ? __uint_as_float(rp[t]) * p.drop_scale : 0.f;
-                  ds[h2 * 2 + e] = prv * (dp - delta) * p.scale;
-                }
-              }
-              uint4 o;
-              o.x = pack_bf16(ds[0], ds[1]);
-              o.y = pack_bf16(ds[2], ds[3]);
-              o.z = pack_bf16(ds[4], ds[5]);
-              o.w = pack_bf16(ds[6], ds[7]);
-              *slot = o;
-            }
-          }
+        for (int u = 0; u < 4; ++u) {
+          uint4 v, w;
+          v.x = pack_bf16(pd[u * 8 + 0], pd[u * 8 + 1]);
+          v.y = pack_bf16(pd[u * 8 + 2], pd[u * 8 + 3]);
+          v.z = pack_bf16(pd[u * 8 + 4], pd[u * 8 + 5]);
+          v.w = pack_bf16(pd[u * 8 + 6], pd[u * 8 + 7]);
+          w.x = pack_bf16(pr[u * 8 + 0], pr[u * 8 + 1]);
+          w.y = pack_bf16(pr[u * 8 + 2], pr[u * 8 + 3]);
+          w.z = pack_bf16(pr[u * 8 + 4], pr[u * 8 + 5]);
+          w.w = pack_bf16(pr[u * 8 + 6], pr[u * 8 + 7]);
+          st_swizzled_unit(pchunk, row, u0 + u, v);
+          st_swizzled_unit(dchunk, row, u0 + u, w);
         }
       } else {
+        km = 0u;
 #pragma unroll
-      for (int cc = 0; cc < CPT; ++cc) {
-        const int cg = CPT * grp + cc;
-        const int u0 = (cg & 1) * 4;
-        uint8_t* pchunk = sPd + static_cast<size_t>(cg >> 1) * kTileBytes;
-        uint8_t* dchunk = sDS + static_cast<size_t>(cg >> 1) * kTileBytes;
-        if (!(diag && cg > q)) {
-          uint32_t rs[32], rp[32];
-          tmem_ld32(lane_base + T_S + cg * 32, rs);
-          tmem_ld32(lane_base + T_DP + cg * 32, rp);
-          tmem_ld_wait();
-          const int kv0 = j * kTile + cg * 32;
-          const uint32_t didx0 = (static_cast<uint32_t>(bh) * p.L + q_pos) * p.L + kv0;
-          const uint32_t keepmask = p.drop_thresh ? drop_keepmask32(dkey, didx0, p.drop_thresh) : 0xFFFFFFFFu;
-          float pd[32], ds[32];
-#pragma unroll
-          for (int t = 0; t < 32; ++t) {
-            float pr = fast_exp2(__uint_as_float(rs[t]) * c1 - lse2);
-            if ((diag && kv0 + t > q_pos) || !row_ok) pr = 0.f;
-            const bool keep = (keepmask >> t) & 1u;
-            const float dp = keep ? __uint_as_float(rp[t]) * p.drop_scale : 0.f;
-            pd[t] = keep ? pr * p.drop_scale : 0.f;
-            ds[t] = pr * (dp - delta) * p.scale;
-          }
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            uint4 v, w;
-            v.x = pack_bf16(pd[u * 8 + 0], pd[u * 8 + 1]);
-            v.y = pack_bf16(pd[u * 8 + 2], pd[u * 8 + 3]);
-            v.z = pack_bf16(pd[u * 8 + 4], pd[u * 8 + 5]);
-            v.w = pack_bf16(pd[u * 8 + 6], pd[u * 8 + 7]);
-            w.x = pack_bf16(ds[u * 8 + 0], ds[u * 8 + 1]);
-            w.y = pack_bf16(ds[u * 8 + 2], ds[u * 8 + 3]);
-            w.z = pack_bf16(ds[u * 8 + 4], ds[u * 8 + 5]);
-            w.w = pack_bf16(ds[u * 8 + 6], ds[u * 8 + 7]);
-            st_swizzled_unit(pchunk, row, u0 + u, v);
-            st_swizzled_unit(dchunk, row, u0 + u, w);
-          }
-        } else {
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            st_swizzled_unit(pchunk, row, u0 + u, make_uint4(0, 0, 0, 0));
-            st_swizzled_unit(dchunk, row, u0 + u, make_uint4(0, 0, 0, 0));
-          }
+        for (int u = 0; u < 4; ++u) {
+          st_swizzled_unit(pchunk, row, u0 + u, make_uint4(0, 0, 0, 0));
+          st_swizzled_unit(dchunk, row, u0 + u, make_uint4(0, 0, 0, 0));
         }
       }
+      }
+      // ---- dP = dO V^T overwrites S once every thread has drained it --------------------------
+      tc_fence_before();
+      __syncthreads();
+      if (tid == 0) {
+        tc_fence_after();
+        const uint32_t do_base = smem_u32(sDO);
+        const uint32_t v_base = smem_u32(sV);
+#pragma unroll
+        for (int k = 0; k < kDh / 16; ++k)
+          umma_bf16(tmem_base + T_DP, umma_desc_kmajor(do_base + k * 32), umma_desc_kmajor(v_base + k * 32),
+                    idesc_s, k > 0 ? 1u : 0u);
+        umma_commit(bar_mm1b);
+      }
+      mbar_wait(bar_mm1b, it & 1);
+      __syncwarp();
+      tc_fence_after();
+      // ---- part B: dS = P * (dropout(dP) - delta) * scale replaces the parked P ------------------
+      const int u0 = (grp & 1) * 4;
+      uint8_t* dchunk = sDS + static_cast<size_t>(grp >> 1) * kTileBytes;
+      if (!(diag && grp > q)) {
+        uint32_t rp[32];
+        tmem_ld32(lane_base + T_DP + grp * 32, rp);
+        tmem_ld_wait();
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          uint4* slot = reinterpret_cast<uint4*>(dchunk + row * 128 + (((u0 + u) ^ (row & 7)) << 4));
+          const uint4 pw = *slot;
+          const uint32_t w[4] = {pw.x, pw.y, pw.z, pw.w};
+          float ds[8];
+#pragma unroll
+          for (int h2 = 0; h2 < 4; ++h2) {
+            const float2 pr2 = unpack_bf16(w[h2]);
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+              const int t = u * 8 + h2 * 2 + e;
+              const float prv = e ? pr2.y : pr2.x;
+              const bool keep = (km >> t) & 1u;
+              const float dp = keep ? __uint_as_float(rp[t]) * p.drop_scale : 0.f;
+              ds[h2 * 2 + e] = prv * (dp - delta) * p.scale;
+            }
+          }
+          uint4 o;
+          o.x = pack_bf16(ds[0], ds[1]);
+          o.y = pack_bf16(ds[2], ds[3]);
+          o.z = pack_bf16(ds[4], ds[5]);
+          o.w = pack_bf16(ds[6], ds[7]);
+          *slot = o;
+        }
       }
       fence_proxy_async_smem();
       tc_fence_before();
@@ -996,8 +914,8 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
       if (tid == 0) {
         tc_fence_after();
         const uint32_t pd_base = smem_u32(sPd), ds_base = smem_u32(sDS);
-        const uint32_t q_base = smem_u32(sQ + static_cast<size_t>(slot) * kTileBytes);
-        const uint32_t do_base = smem_u32(sDO + static_cast<size_t>(slot) * kTileBytes);
+        const uint32_t q_base = smem_u32(sQ);
+        const uint32_t do_base = smem_u32(sDO);
         const uint32_t k_base = smem_u32(sK);
         // Pd / dS are stored [q row][kv col] in two 64-column chunks. Read as the TRANSPOSED
         // operand (M = kv, contraction = q) they are MN-major: 16 q rows = 2048 B per K step,
@@ -1025,8 +943,8 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
       tc_fence_after();
     }
     // ---- dK_j, dV_j complete: TMEM -> dqkv (each thread: 32 of the 64 columns) -------------
-    if (CG == 2 || grp < 2) {
-      // 64 output columns = two 32-column halves: warps of groups 0/1 (CG = 4: groups 0,1 take dK, 2,3 dV)
+    // 64 output columns = two 32-column halves: groups 0,1 take dK, 2,3 dV
+    if (grp < 2) {
       const int hf = grp & 1;
       const int pos = j * kTile + row;
       __nv_bfloat16* grow = p.dqkv + static_cast<size_t>(seq_row0 + pos) * (3 * D) + h * kDh + hf * 32;
@@ -1035,7 +953,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
       tmem_ld_wait();
       if (pos < p.L) store_row32_bf16(grow + D, rk);
     }
-    if (CG == 2 || grp >= 2) {
+    if (grp >= 2) {
       const int hf = grp & 1;
       const int pos = j * kTile + row;
       __nv_bfloat16* grow = p.dqkv + static_cast<size_t>(seq_row0 + pos) * (3 * D) + h * kDh + hf * 32;
@@ -1049,8 +967,8 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
     tc_fence_after();
   }
 
-  // ---- dQ_i -> dqkv ---------------------------------------------------------------------
-  for (int i = (CG == 2 ? 0 : (grp >> 1)); i < nq; i += (CG == 2 ? 1 : 2)) {   // CG = 4: groups (0,1) / (2,3) alternate tiles
+  // ---- dQ_i -> dqkv: groups (0,1) / (2,3) alternate tiles --------------------------------
+  for (int i = grp >> 1; i < nq; i += 2) {
     const int hf = grp & 1;
     const int pos = i * kTile + row;
     uint32_t r[32];
@@ -1066,10 +984,11 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
 }
 
 // --------------------------------------------------------------------------------------------
-// Backward, persistent and pipelined (L <= 256: one or two 128-row tiles). The kernel above spends most
-// of a CTA's life in chains of dependent latencies (TMEM allocation -> TMA -> MMA -> element-wise -> MMA,
-// one CTA per SM, nothing to overlap them with). Here a CTA per SM walks (sequence, head) items:
-//   * warps 0-15 (512 threads): the element-wise phase, thread (row, 32-column chunk) as above; they
+// Backward, persistent and pipelined (L <= 256: one or two 128-row tiles). A CTA per (sequence, head) like
+// the kernel above would spend most of its life in chains of dependent latencies (TMEM allocation -> TMA ->
+// MMA -> element-wise -> MMA, one CTA per SM, nothing to overlap them with). Here a CTA per SM walks
+// (sequence, head) items:
+//   * warps 0-15 (512 threads): the element-wise phase, thread (row, 32-column chunk); they
 //     never issue anything, they only wait on / arrive at mbarriers;
 //   * warp 16, one lane: every TMA load and every MMA. S/dP of iteration g+1 are issued as soon as all
 //     512 threads hold S/dP of iteration g in registers (bar_drain), so those MMAs run under the
@@ -1077,8 +996,8 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
 //     as soon as the last MMA reading the slot has retired (Q0/dO0 after iteration 0, K0/V0 after
 //     iteration 1, the rest after iteration 2), so no load latency is exposed between items;
 //   * warp 17: delta = rowsum(dO * O) and the log-sum-exps of the next item, double-buffered.
-// Iterations of an item (key tile j, query tile i): (0,0), (0,1), (1,1); TMEM columns as in the fast
-// layout above. One __syncthreads at each end of the kernel, none inside.
+// Iterations of an item (key tile j, query tile i): (0,0), (0,1), (1,1); TMEM columns as listed above the
+// backward kernels. One __syncthreads at each end of the kernel, none inside.
 // --------------------------------------------------------------------------------------------
 static constexpr int kBwdComputeThreads = 512;
 static constexpr int kBwdCtrlRegs = 56, kBwdComputeRegs = 104;   // 512 * 104 + 128 * 56 <= 640 * 96
@@ -2101,17 +2020,7 @@ extern "C" int tt_attn_causal_fwd(const void* qkv, void* ctx, float* lse, int B,
     TT_LAUNCH_CHECK();
     return TT_OK;
   }
-  const size_t smem = 1024 + static_cast<size_t>(1 + p.nq + 1 + 2) * kTileBytes + 64 + 2 * 128 * sizeof(float);
-  static bool configured = false;
-  if (!configured) {
-    TT_CHECK_CUDA(cudaFuncSetAttribute(attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-    configured = true;
-  }
-  TT_REQUIRE(smem <= 232448, "tt_attn_causal_fwd: shared memory %zu too large", smem);
-  // TT_ATTN_FWD=legacy keeps the one-CTA-per-(sequence, head, query tile) kernel for L <= 256
-  const char* mode = getenv("TT_ATTN_FWD");
-  const bool legacy = mode && mode[0] == 'l';
-  if (p.nq <= 2 && !legacy) {
+  if (p.nq <= 2) {
     const size_t psmem = 1024 + 12 * static_cast<size_t>(kTileBytes) + 256 + 3 * 4 * kTile * sizeof(float);
     static bool pconfigured = false;
     if (!pconfigured) {
@@ -2123,6 +2032,13 @@ extern "C" int tt_attn_causal_fwd(const void* qkv, void* ctx, float* lse, int B,
     TT_LAUNCH_CHECK();
     return TT_OK;
   }
+  const size_t smem = 1024 + static_cast<size_t>(1 + p.nq + 1 + 2) * kTileBytes + 64 + 2 * 128 * sizeof(float);
+  static bool configured = false;
+  if (!configured) {
+    TT_CHECK_CUDA(cudaFuncSetAttribute(attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
+    configured = true;
+  }
+  TT_REQUIRE(smem <= 232448, "tt_attn_causal_fwd: shared memory %zu too large", smem);
   TT_CHECK_CUDA(launch_k(attn_fwd_kernel, dim3(B * H * p.nq), dim3(256), smem, stream, tm, p));
   TT_LAUNCH_CHECK();
   return TT_OK;
@@ -2177,21 +2093,7 @@ extern "C" int tt_attn_causal_bwd(const void* qkv, const void* ctx, const void* 
     TT_LAUNCH_CHECK();
     return TT_OK;
   }
-  const int slots = p.nq <= 2 ? p.nq : 1;
-  const size_t smem = 1024 + static_cast<size_t>(2 * slots + 2 + 4) * kTileBytes + 128 +
-                      static_cast<size_t>(2 * p.nq * kTile) * sizeof(float);
-  static bool configured = false;
-  if (!configured) {
-    TT_CHECK_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<false, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-    TT_CHECK_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<true, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-    TT_CHECK_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<true, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-    configured = true;
-  }
-  TT_REQUIRE(smem <= 232448, "tt_attn_causal_bwd: shared memory %zu too large", smem);
-  // TT_ATTN_BWD=legacy keeps the one-CTA-per-(sequence, head) kernel for L <= 256 (A/B runs, bit-equality test)
-  const char* mode = getenv("TT_ATTN_BWD");
-  const bool legacy = mode && mode[0] == 'l';
-  if (p.nq <= 2 && !legacy) {
+  if (p.nq <= 2) {
     const size_t psmem = 1024 + 12 * static_cast<size_t>(kTileBytes) + 128 + 2 * 2 * 2 * kTile * sizeof(float);
     static bool pconfigured = false;
     if (!pconfigured) {
@@ -2200,15 +2102,19 @@ extern "C" int tt_attn_causal_bwd(const void* qkv, const void* ctx, const void* 
     }
     const int grid = B * H < num_sms() ? B * H : num_sms();
     TT_CHECK_CUDA(launch_k(attn_bwd_persist_kernel, dim3(grid), dim3(kBwdThreads), psmem, stream, tmQ, tmDO, p));
-  } else if (p.nq <= 2) {
-    TT_CHECK_CUDA(launch_k(attn_bwd_kernel<false, 4>, dim3(B * H), dim3(512), smem, stream, tmQ, tmDO, p));
-  } else {
-    // L <= 512: 16 warps in the element-wise phase (CG = 4) like the fast layout; TT_ATTN_BWD_LONG_CG=2 keeps 8
-    static int long_cg = -1;
-    if (long_cg < 0) { const char* e = getenv("TT_ATTN_BWD_LONG_CG"); long_cg = e ? atoi(e) : 4; }
-    if (long_cg == 4) TT_CHECK_CUDA(launch_k(attn_bwd_kernel<true, 4>, dim3(B * H), dim3(512), smem, stream, tmQ, tmDO, p));
-    else TT_CHECK_CUDA(launch_k(attn_bwd_kernel<true, 2>, dim3(B * H), dim3(256), smem, stream, tmQ, tmDO, p));
+    TT_LAUNCH_CHECK();
+    return TT_OK;
   }
+  // Q_i, dO_i, K_j, V_j, Pd and dS (two tiles each), barriers, delta and lse of every query row
+  const size_t smem = 1024 + static_cast<size_t>(2 + 2 + 4) * kTileBytes + 128 +
+                      static_cast<size_t>(2 * p.nq * kTile) * sizeof(float);
+  static bool configured = false;
+  if (!configured) {
+    TT_CHECK_CUDA(cudaFuncSetAttribute(attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
+    configured = true;
+  }
+  TT_REQUIRE(smem <= 232448, "tt_attn_causal_bwd: shared memory %zu too large", smem);
+  TT_CHECK_CUDA(launch_k(attn_bwd_kernel, dim3(B * H), dim3(512), smem, stream, tmQ, tmDO, p));
   TT_LAUNCH_CHECK();
   return TT_OK;
 }

@@ -53,7 +53,7 @@ int make_tmap(CUtensorMap* out, const void* base, int rank, const uint64_t* dims
 
 int num_sms();
 
-// The ID table as the embedding / sparse kernels see it: one replicated table (world == 0: row `id` lives at
+// The ID table as the sparse kernels (tt_sparse.cu) see it: one replicated table (world == 0: row `id` lives at
 // base[0] + id * 256) or a table row-sharded ROUND-ROBIN over the ranks of one NVLink domain (row id lives at local
 // row id / world of rank id % world; base[r] = rank r's shard as mapped into this process, symmetric arena).
 // Round-robin because item popularity is Zipfian in the id (SURVEY.md §8d): contiguous ranges would put most of
@@ -80,15 +80,14 @@ int make_sharded_table(TableRef& t, const ::tt_symm_team* team, int64_t offset, 
 //     when the previous kernel has completed and its writes are visible.
 // What overlaps with the predecessor is therefore only launch latency and the prologue (barrier
 // init, TMEM allocation, tensor-map prefetch) — semantics stay those of a serialized stream.
-// Opt-in with TT_PDL=1 (without the launch attribute the two instructions are no-ops): inside the
-// replayed CUDA graph the launch gaps are already small and early-resident CTAs cost more than they
-// save — measured 1.576 ms with vs 1.528 ms without on the c2 step — so it is off by default.
+// launch_k sets the programmatic launch attribute only on grids of at most kPdlMaxCtas CTAs (without it
+// the two instructions are no-ops). Measured on the c2 step: 1.308 ms with no programmatic launch,
+// 1.326 ms with it on every launch, 1.282 ms with it on the small grids only.
 // ----------------------------------------------------------------------------
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
-int pdl_mode();       // TT_PDL: 0 = never, 1 = every launch, 2 = small grids only (default)
-int pdl_max_ctas();   // TT_PDL_MAX_CTAS: largest grid that launches programmatically in mode 2
+constexpr size_t kPdlMaxCtas = 64;   // largest grid that launches programmatically
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
@@ -104,11 +103,10 @@ inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
   cfg.attrs = attr;
   // Programmatic dependent launch lets this grid start (and run its prologue up to griddepcontrol.wait)
   // while the previous kernel in the stream drains. Early CTAs of a big grid would sit on SMs the
-  // concurrent weight-gradient / item-tower streams could use, so mode 2 restricts it to the small
-  // latency-bound launches (B-row GEMMs, heads, loss), where launch + prologue latency is the cost.
-  const int mode = pdl_mode();
+  // concurrent weight-gradient / item-tower streams could use, so only the small latency-bound
+  // launches (B-row GEMMs, heads, loss), where launch + prologue latency is the cost, use it.
   const size_t ctas = static_cast<size_t>(grid.x) * grid.y * grid.z;
-  cfg.numAttrs = (mode == 1 || (mode == 2 && ctas <= static_cast<size_t>(pdl_max_ctas()))) ? 1 : 0;
+  cfg.numAttrs = ctas <= kPdlMaxCtas ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 

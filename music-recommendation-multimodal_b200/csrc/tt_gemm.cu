@@ -17,7 +17,6 @@
 // layouts dgrad/wgrad need), selected by template flags and the UMMA descriptors.
 #include "../../include/tt_b200.h"
 #include "tt_common.cuh"
-#include <stdlib.h>
 
 namespace tt {
 
@@ -48,8 +47,6 @@ struct GemmParams {
   int tma_store;    // 1: finished 32 x 32 output blocks leave through TMA tensor stores straight from the (swizzled)
                     // staging tile instead of a transposed LDS + STG pass by the warp
   float* a_colsum;  // optional [K]: += column sums of the (K-major) A operand, taken from the staged tiles by warps 2 and 3
-  int debug;  // profiling knob: low 4 bits 1 = epilogue drains TMEM only (no math, no global IO), 2 = everything but the
-              // global stores; +16 / +32 = operand loads skipped after the first ring revolution (B only / A and B)
 };
 
 static constexpr int kBlockM = 128;
@@ -199,14 +196,14 @@ __device__ __forceinline__ void gemm_epilogue_chunk(const GemmParams& p, const u
       // M / N are clipped by the tensor map
       fence_proxy_async_smem();
       __syncwarp();
-      if (lane == 0 && (p.debug & 15) != 2) { tma_store_2d(tmO32, out, col0, row0); tma_store_commit(); }
+      if (lane == 0) { tma_store_2d(tmO32, out, col0, row0); tma_store_commit(); }
     } else {
     __syncwarp();
 #pragma unroll
     for (int it = 0; it < 8; ++it) {
       const int rr = it * 4 + (lane >> 3), u = lane & 7;
       const int gr = row0 + rr, gc = col0 + u * 4;
-      if (gr < p.M && gc + 4 <= p.N && (p.debug & 15) != 2) {
+      if (gr < p.M && gc + 4 <= p.N) {
         const float4 x = *reinterpret_cast<const float4*>(stg_unit(out, rr, u));
         float* o = p.out_f32 + static_cast<size_t>(gr) * p.ld_f32 + gc;
         if (p.accumulate) red_add_f32x4(o, x.x, x.y, x.z, x.w);
@@ -230,14 +227,14 @@ __device__ __forceinline__ void gemm_epilogue_chunk(const GemmParams& p, const u
     if (p.tma_store) {   // 64-byte TMA swizzle == unit ^ ((row >> 1) & 3)
       fence_proxy_async_smem();
       __syncwarp();
-      if (lane == 0 && (p.debug & 15) != 2) { tma_store_2d(tmO16, out, col0, row0); tma_store_commit(); }
+      if (lane == 0) { tma_store_2d(tmO16, out, col0, row0); tma_store_commit(); }
     } else {
     __syncwarp();
 #pragma unroll
     for (int it = 0; it < 4; ++it) {
       const int rr = it * 8 + (lane >> 2), u = lane & 3;
       const int gr = row0 + rr, gc = col0 + u * 8;
-      if (gr < p.M && gc + 8 <= p.N && (p.debug & 15) != 2)
+      if (gr < p.M && gc + 8 <= p.N)
         *reinterpret_cast<uint4*>(p.out_bf16 + static_cast<size_t>(gr) * p.ld_bf16 + gc) = *stg_unit_bf(out, rr, u);
     }
     __syncwarp();
@@ -333,7 +330,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   auto m_block = [&](int mn) { return pair ? 2 * (mn / tiles_n) + static_cast<int>(rank) : mn / tiles_n; };
   if (warp == 0) {
     if (elect_one()) {
-      int stage = 0, issued = 0;
+      int stage = 0;
       uint32_t phase = 0;
       for (int t = worker; t < num_tiles; t += n_workers) {
         const int split = t % p.k_splits;
@@ -354,16 +351,10 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             else      tma_load_2d_pair(b_dst, &tmB, &full_bar[stage], kb * kBlockK,
                                        n_blk * block_n + static_cast<int>(rank) * (block_n / 2));
           } else {
-            // profiling knobs (results are garbage): +16 = B tiles are fetched for the first ring revolution only
-            // (what a weight-resident form would stream), +32 = neither operand after that
-            const bool skip_b = (p.debug & 48) && issued >= stages, skip_a = (p.debug & 32) && issued >= stages;
-            ++issued;
-            mbar_arrive_expect_tx(&full_bar[stage], (skip_a ? 0u : kABytes) + (skip_b ? 0u : b_bytes));
-            if (skip_a) {}
-            else if (A_MN) tma_load_3d(a_dst, &tmA, &full_bar[stage], 0, kb * kBlockK, m_blk * (kBlockM / 64));
+            mbar_arrive_expect_tx(&full_bar[stage], kABytes + b_bytes);
+            if (A_MN) tma_load_3d(a_dst, &tmA, &full_bar[stage], 0, kb * kBlockK, m_blk * (kBlockM / 64));
             else      tma_load_2d(a_dst, &tmA, &full_bar[stage], kb * kBlockK, m_blk * kBlockM);
-            if (skip_b) {}
-            else if (B_MN) tma_load_3d(b_dst, &tmB, &full_bar[stage], 0, kb * kBlockK, n_blk * (block_n / 64));
+            if (B_MN) tma_load_3d(b_dst, &tmB, &full_bar[stage], 0, kb * kBlockK, n_blk * (block_n / 64));
             else      tma_load_2d(b_dst, &tmB, &full_bar[stage], kb * kBlockK, n_blk * block_n);
           }
           if (++stage == stages) { stage = 0; phase ^= 1u; }
@@ -524,11 +515,9 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         tmem_ld32(t_base + static_cast<uint32_t>(c * 32), r);
         tmem_ld_wait();
         const int cn = c + kEpiWarps / 4;
-        if ((p.debug & 15) != 1)
-          gemm_epilogue_chunk(p, r, stg, stg, sbias + k * 32, lane, row0, colbase + c * 32,
-                              cn < nchunks ? colbase + cn * 32 : -1, dkey, &tmO32, &tmO16);
+        gemm_epilogue_chunk(p, r, stg, stg, sbias + k * 32, lane, row0, colbase + c * 32,
+                            cn < nchunks ? colbase + cn * 32 : -1, dkey, &tmO32, &tmO16);
       }
-      if ((p.debug & 15) == 1) cp_async_wait_all();
       tc_fence_before();
       __syncwarp();
       if (lane == 0) {
@@ -665,22 +654,15 @@ extern "C" int tt_gemm_bf16(const tt_gemm_args* a, void* stream_) {
   TT_REQUIRE(ks == 1 || a->accumulate, "tt_gemm_bf16: k_splits > 1 requires accumulate");
   p.k_splits = ks;
 
-  // CTA pairs (see the kernel): for launches where every pair of SMs still gets (nearly) a full share of
-  // work items AND the contraction per tile is deep (>= 8 k-blocks): measured on the c2 step, the K >= 512
-  // launches gain 7-15 % (dgrad 1024: 39.3 -> 33.3 us, wgrads 36.9 -> 32.8 / 45.0 -> 38.8 us) while the
-  // epilogue-bound K = 256 ones lose 10-20 % to the lockstep of the pair (QKV 37.1 -> 42.9 us).
-  // Since the epilogue stores through TMA (round 2, third session) the pair no longer loses on the K = 256 launches
-  // (c2 step 1.160 -> 1.146 ms with every eligible launch on pairs), so that is the default now.
-  // TT_GEMM_PAIR=0 disables, =1 takes only the deep launches, =2 (default) every eligible launch.
+  // CTA pairs (see the kernel) for every launch where each pair of SMs still gets (nearly) a full share of work
+  // items. Measured on the c2 step with the earlier LDS + STG epilogue, the deep (K >= 512) launches gained 7-15 %
+  // (dgrad 1024: 39.3 -> 33.3 us, wgrads 36.9 -> 32.8 / 45.0 -> 38.8 us) while the epilogue-bound K = 256 ones lost
+  // 10-20 % to the lockstep of the pair (QKV 37.1 -> 42.9 us). Since the epilogue stores through TMA the pair no
+  // longer loses on the K = 256 launches (c2 step 1.160 -> 1.146 ms with every eligible launch on pairs).
   const int pairs = num_sms() / 2 > 0 ? num_sms() / 2 : 1;
   const long pair_items = static_cast<long>((tiles_m + 1) / 2) * tiles_n * ks;
-  {
-    static int pair_env = -1;
-    if (pair_env < 0) { const char* e = getenv("TT_GEMM_PAIR"); pair_env = e ? atoi(e) : 2; }
-    const bool eligible = bn >= 128 && tiles_m >= 2 && pair_items * 10 >= static_cast<long>(pairs) * 9;
-    const bool deep = kblocks / ks >= 8;
-    p.pair = (pair_env != 0 && eligible && (deep || pair_env == 2)) ? 1 : 0;
-  }
+  const bool eligible = bn >= 128 && tiles_m >= 2 && pair_items * 10 >= static_cast<long>(pairs) * 9;
+  p.pair = eligible ? 1 : 0;
   const size_t b_bytes = (static_cast<size_t>(bn) * kBlockK * 2) >> (p.pair ? 1 : 0);   // per CTA
   // bf16-only epilogues stage 64-byte rows: half the staging, more pipeline stages
   p.stg_bytes = static_cast<int>((a->out_f32 || a->residual) ? kStageBytesF32 : kStageBytesBf16);
@@ -718,11 +700,6 @@ extern "C" int tt_gemm_bf16(const tt_gemm_args* a, void* stream_) {
   p.out_bf16 = static_cast<__nv_bfloat16*>(a->out_bf16);
   p.ld_bf16 = a->ld_bf16;
   p.accumulate = a->accumulate;
-  {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("TT_GEMM_DEBUG"); dbg = e ? atoi(e) : 0; }
-    p.debug = dbg;
-  }
 
   CUtensorMap tmA, tmB;
   int rc;
@@ -753,11 +730,7 @@ extern "C" int tt_gemm_bf16(const tt_gemm_args* a, void* stream_) {
 
   // Output tensor maps (32 x 32 blocks, the staging tile's swizzle): plain stores only — split-K keeps red.add
   CUtensorMap tmO32 = tmA, tmO16 = tmA;   // placeholders when unused
-  {
-    static int tma_env = -1;
-    if (tma_env < 0) { const char* e = getenv("TT_GEMM_TMA_STORE"); tma_env = e ? atoi(e) : 1; }
-    p.tma_store = (tma_env != 0 && !a->accumulate) ? 1 : 0;
-  }
+  p.tma_store = a->accumulate ? 0 : 1;
   if (p.tma_store && a->out_f32) {
     uint64_t dims[2] = {static_cast<uint64_t>(a->N), static_cast<uint64_t>(a->M)};
     uint64_t str[1] = {static_cast<uint64_t>(a->ld_f32) * 4};

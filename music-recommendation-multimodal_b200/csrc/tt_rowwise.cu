@@ -1,7 +1,7 @@
 // Bandwidth-bound row-wise kernels of the two-tower path: embedding gather + positional add +
 // LayerNorm, LayerNorm / ReLU / dropout / L2-normalise chains and their backward passes,
 // last-valid-step gather + demographic concat, BatchNorm1d (batch or running statistics),
-// column sums (bias gradients), scatter-add of ID-embedding gradients.
+// scatter-add of ID-embedding gradients.
 //
 // Layout rule: one warp per row, each lane owns NV float4 columns strided by 32 lanes
 // (col = (k*32 + lane)*4 + c), so every load/store instruction of a warp covers 512
@@ -9,7 +9,6 @@
 // cross-warp parameter-gradient combine.
 #include "../../include/tt_b200.h"
 #include "tt_common.cuh"
-#include <stdlib.h>
 
 namespace tt {
 
@@ -131,14 +130,9 @@ __global__ void last_index_kernel(const int64_t* __restrict__ ids, const int64_t
 // x0 = dropout(LN_emb(E[id] + P[pos]));  h = LN_next(x0) as bf16       (user_tower.py:86-93 and
 // the first norm1 of the encoder). D = 256.
 // --------------------------------------------------------------------------------------------
-// TableRef (tt_common.cuh): one replicated table, or a table row-sharded round-robin over the ranks of one
-// NVLink domain — then a gather / scatter-add goes straight to the owner's memory, no id or row exchange.
-
 struct EmbedParams {
   const int64_t* ids;
-  TableRef E;
-  float* stash;        // nullable [T, 256]: the gathered table rows, kept for the backward pass (sharded tables:
-                       // saves the second trip over NVLink)
+  const float* E;
   const float* P;
   const float* ln_w; const float* ln_b;
   const float* nw; const float* nb;
@@ -149,15 +143,14 @@ struct EmbedParams {
 };
 
 // One token row of embed_ln_fwd (one warp): table row E[id] and position row P[pos] -> x0, h at output row `row`.
-// Shared by the [B, L] kernel (pos = row % L, dropout, stash) and the explicit-position one (sessions: no dropout).
+// Shared by the [B, L] kernel (pos = row % L, dropout) and the explicit-position one (sessions: no dropout).
 __device__ __forceinline__ void embed_ln_row(const EmbedParams& p, int64_t id, int pos, int row, int lane,
                                              const float (&w)[8], const float (&b)[8], const float (&nw)[8],
                                              const float (&nb)[8], uint64_t seed) {
   constexpr int NV = 2;
   float e[8], q[8];
-  load_row<NV>(p.E.row(id), lane, e);
+  load_row<NV>(p.E + static_cast<size_t>(id) * 256, lane, e);
   load_row<NV>(p.P + static_cast<size_t>(pos) * 256, lane, q);
-  if (p.stash) store_row<NV>(p.stash + static_cast<size_t>(row) * 256, lane, e);
 #pragma unroll
   for (int i = 0; i < 8; ++i) e[i] += q[i];
   float mean, rstd;
@@ -188,7 +181,7 @@ __global__ void __launch_bounds__(kRowThreads) embed_ln_fwd_kernel(const EmbedPa
     embed_ln_row(p, p.ids[row], row % p.L, row, lane, w, b, nw, nb, seed);
 }
 
-// Rows at explicit positions: row r is item ids[r] at position pos[r] (p.T = n rows; no dropout, no stash).
+// Rows at explicit positions: row r is item ids[r] at position pos[r] (p.T = n rows; no dropout).
 __global__ void __launch_bounds__(kRowThreads) embed_ln_fwd_pos_kernel(const EmbedParams p,
                                                                         const int32_t* __restrict__ pos) {
   pdl_launch_dependents();
@@ -581,29 +574,6 @@ __global__ void __launch_bounds__(256) bn_bwd_kernel(const BnParams p) {
 }
 
 // --------------------------------------------------------------------------------------------
-// column sums of a bf16 [R, N] matrix, accumulated into fp32 out[N]  (bias gradients)
-// grid = (ceil(N/256), row_blocks); each thread owns one column pair-free column.
-// --------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) colsum_bf16_kernel(const __nv_bfloat16* __restrict__ x, int R, int N, int ld,
-                                                          float* __restrict__ out) {
-  pdl_launch_dependents();
-  pdl_wait();
-  const int c2 = (blockIdx.x * blockDim.x + threadIdx.x) * 2;  // two adjacent columns per thread
-  if (c2 >= N) return;
-  const int rows_per = (R + gridDim.y - 1) / gridDim.y;
-  const int r0 = blockIdx.y * rows_per, r1 = min(R, r0 + rows_per);
-  float a0 = 0.f, a1 = 0.f;
-  for (int r = r0; r < r1; ++r) {
-    const uint32_t u = __ldg(reinterpret_cast<const uint32_t*>(x + static_cast<size_t>(r) * ld + c2));
-    const float2 f = unpack_bf16(u);
-    a0 += f.x;
-    a1 += f.y;
-  }
-  atomicAdd(out + c2, a0);
-  if (c2 + 1 < N) atomicAdd(out + c2 + 1, a1);
-}
-
-// --------------------------------------------------------------------------------------------
 // Backward of embed_ln_fwd w.r.t. its first LayerNorm: dx0 [T,256] -> dE (scatter-add, id 0
 // skipped: padding_idx), dP (per position), d(ln_w), d(ln_b). The pre-LN sum E[id]+P[pos] is
 // re-gathered instead of being stored.
@@ -614,75 +584,50 @@ __global__ void __launch_bounds__(256) colsum_bf16_kernel(const __nv_bfloat16* _
 static constexpr float kGradFixScale = 1099511627776.f;
 
 struct EmbedBwdParams {
-  const int64_t* ids; TableRef E; const float* stash; const float* P; const float* ln_w; const float* ln_b;
+  const int64_t* ids; const float* E; const float* P; const float* ln_w; const float* ln_b;
   const float* dx0; int B, L;
   uint32_t drop_thresh; float drop_scale; uint64_t seed; const uint64_t* seed_dev; uint32_t site;
-  TableRef dE; float* dP; float* dgamma; float* dbeta;
+  float* dE; float* dP; float* dgamma; float* dbeta;
   // deterministic mode (both set): token `row` adds its gradient row into acc64[acc_slot[row]] in 64-bit fixed
   // point instead of dE (slot 0 = padding: skipped); tt_rows_scatter_add_i64 then rounds each sum once
   unsigned long long* acc64; const int64_t* acc_slot;
-  // fused form (n1_dh set, dx0 unused): the first encoder layer's norm1 backward runs in front, on x0 recomputed from
-  // the table row: dx0 = LayerNorm1'(x0; n1_dh) + n1_resid never travels through memory and x0 is not read
-  const __nv_bfloat16* n1_dh; const float* n1_resid; const float* n1_w; const float* n1_b;
-  float* n1_dgamma; float* n1_dbeta;
-  // the table row of token `row` with id `id`: the forward's stash when there is one, else the table itself
-  __device__ __forceinline__ const float* src_row(size_t row, int64_t id) const {
-    return stash ? stash + row * 256 : E.row(id);
-  }
 };
 
-template <bool FUSED>
 __global__ void __launch_bounds__(kRowThreads, 2) embed_ln_bwd_kernel(const EmbedBwdParams p) {
   pdl_launch_dependents();
   pdl_wait();
-  constexpr int NV = 2, E_ = 8, W = 256, NRED = FUSED ? 5 : 3;
-  __shared__ float s_red[NRED][kRowThreads / 32][W];
+  constexpr int NV = 2, E_ = 8, W = 256;
+  __shared__ float s_red[3][kRowThreads / 32][W];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const int pos = blockIdx.x;
-  float w[E_], dg[E_], db[E_], dp[E_], q[E_], dg1[FUSED ? E_ : 1], db1[FUSED ? E_ : 1];
+  float w[E_], dg[E_], db[E_], dp[E_], q[E_];
   load_row<NV>(p.ln_w, lane, w);
   load_row<NV>(p.P + static_cast<size_t>(pos) * W, lane, q);
 #pragma unroll
   for (int i = 0; i < E_; ++i) { dg[i] = 0.f; db[i] = 0.f; dp[i] = 0.f; }
-  if constexpr (FUSED) {
-#pragma unroll
-    for (int i = 0; i < E_; ++i) { dg1[i] = 0.f; db1[i] = 0.f; }
-  }
   const uint64_t seed = p.drop_thresh ? read_seed(p.seed, p.seed_dev) : 0;
   // The id -> table row -> arithmetic chain is two dependent memory latencies per row; the ids run two
-  // rows ahead and the (table row, gradient row[, residual row]) group one row ahead of the arithmetic.
+  // rows ahead and the (table row, gradient row) pair one row ahead of the arithmetic.
   const int stride = (kRowThreads / 32) * gridDim.y;
   int b = wib * gridDim.y + blockIdx.y;
   int64_t id_n = 0, id_nn = 0;
-  float e_n[E_], g_n[E_], r_n[FUSED ? E_ : 1];
-  auto load_grad = [&](size_t row) {
-    if constexpr (FUSED) {
-      load_row_bf16<NV>(p.n1_dh + row * W, lane, g_n);
-      load_row<NV>(p.n1_resid + row * W, lane, r_n);
-    } else {
-      load_row<NV>(p.dx0 + row * W, lane, g_n);
-    }
-  };
+  float e_n[E_], g_n[E_];
   if (b < p.B) {
     id_n = p.ids[static_cast<size_t>(b) * p.L + pos];
-    load_row<NV>(p.src_row(static_cast<size_t>(b) * p.L + pos, id_n), lane, e_n);
-    load_grad(static_cast<size_t>(b) * p.L + pos);
+    load_row<NV>(p.E + static_cast<size_t>(id_n) * W, lane, e_n);
+    load_row<NV>(p.dx0 + (static_cast<size_t>(b) * p.L + pos) * W, lane, g_n);
   }
   if (b + stride < p.B) id_nn = p.ids[static_cast<size_t>(b + stride) * p.L + pos];
   for (; b < p.B; b += stride) {
     const size_t row = static_cast<size_t>(b) * p.L + pos;
     const int64_t id = id_n;
-    float e[E_], g[E_], xhat[E_], r[FUSED ? E_ : 1];
+    float e[E_], g[E_], xhat[E_];
 #pragma unroll
     for (int i = 0; i < E_; ++i) { e[i] = e_n[i]; g[i] = g_n[i]; }
-    if constexpr (FUSED) {
-#pragma unroll
-      for (int i = 0; i < E_; ++i) r[i] = r_n[i];
-    }
     id_n = id_nn;
     if (b + stride < p.B) {
-      load_row<NV>(p.src_row(static_cast<size_t>(b + stride) * p.L + pos, id_n), lane, e_n);
-      load_grad(static_cast<size_t>(b + stride) * p.L + pos);
+      load_row<NV>(p.E + static_cast<size_t>(id_n) * W, lane, e_n);
+      load_row<NV>(p.dx0 + (static_cast<size_t>(b + stride) * p.L + pos) * W, lane, g_n);
     }
     if (b + 2 * stride < p.B) id_nn = p.ids[static_cast<size_t>(b + 2 * stride) * p.L + pos];
 #pragma unroll
@@ -691,37 +636,7 @@ __global__ void __launch_bounds__(kRowThreads, 2) embed_ln_bwd_kernel(const Embe
     ln_stats<NV>(e, 1e-5f, mean, rstd);
 #pragma unroll
     for (int i = 0; i < E_; ++i) xhat[i] = (e[i] - mean) * rstd;
-    if constexpr (FUSED) {
-      // x0 = dropout(LayerNorm_emb(e)) exactly as the forward formed it, then norm1's backward on it
-      float x0[E_], bE[E_], w1[E_];
-      bool keep[E_];
-      load_row<NV>(p.ln_b, lane, bE);
-#pragma unroll
-      for (int i = 0; i < E_; ++i) { x0[i] = xhat[i] * w[i] + bE[i]; keep[i] = true; }
-      if (p.drop_thresh) row_dropout<NV>(x0, drop_key(seed, p.site), row, W, lane, p.drop_thresh, p.drop_scale, keep);
-      float m1, rs1;
-      ln_stats<NV>(x0, 1e-5f, m1, rs1);
-      load_row<NV>(p.n1_w, lane, w1);
-      float t1 = 0.f, t2 = 0.f;
-#pragma unroll
-      for (int i = 0; i < E_; ++i) {
-        x0[i] = (x0[i] - m1) * rs1;          // xhat of norm1
-        dg1[i] += g[i] * x0[i];
-        db1[i] += g[i];
-        g[i] *= w1[i];
-        t1 += g[i];
-        t2 += g[i] * x0[i];
-      }
-      t1 = warp_sum(t1) * (1.f / W);
-      t2 = warp_sum(t2) * (1.f / W);
-#pragma unroll
-      for (int i = 0; i < E_; ++i) {
-        g[i] = rs1 * (g[i] - t1 - x0[i] * t2) + r[i];                 // = d(loss)/d(x0)
-        if (p.drop_thresh) g[i] = keep[i] ? g[i] * p.drop_scale : 0.f;   // the embedding dropout's backward
-      }
-    } else {
-      if (p.drop_thresh) row_dropout<NV>(g, drop_key(seed, p.site), row, W, lane, p.drop_thresh, p.drop_scale, nullptr);
-    }
+    if (p.drop_thresh) row_dropout<NV>(g, drop_key(seed, p.site), row, W, lane, p.drop_thresh, p.drop_scale, nullptr);
     float s1 = 0.f, s2 = 0.f;
 #pragma unroll
     for (int i = 0; i < E_; ++i) {
@@ -752,7 +667,7 @@ __global__ void __launch_bounds__(kRowThreads, 2) embed_ln_bwd_kernel(const Embe
                       static_cast<unsigned long long>(__float2ll_rn(g[4 * k + e] * kGradFixScale)));
       }
     } else if (id != 0) {
-      float* dst = p.dE.row(id);
+      float* dst = p.dE + static_cast<size_t>(id) * W;
 #pragma unroll
       for (int k = 0; k < NV; ++k)
         red_add_f32x4(dst + (k * 32 + lane) * 4, g[4 * k + 0], g[4 * k + 1], g[4 * k + 2], g[4 * k + 3]);
@@ -764,30 +679,18 @@ __global__ void __launch_bounds__(kRowThreads, 2) embed_ln_bwd_kernel(const Embe
     s_red[0][wib][c] = dg[i];
     s_red[1][wib][c] = db[i];
     s_red[2][wib][c] = dp[i];
-    if constexpr (FUSED) {
-      s_red[3][wib][c] = dg1[i];
-      s_red[4][wib][c] = db1[i];
-    }
   }
   __syncthreads();
   for (int c = threadIdx.x; c < W; c += blockDim.x) {
-    float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f, a4 = 0.f;
+    float a0 = 0.f, a1 = 0.f, a2 = 0.f;
 #pragma unroll
     for (int k = 0; k < kRowThreads / 32; ++k) {
       a0 += s_red[0][k][c]; a1 += s_red[1][k][c]; a2 += s_red[2][k][c];
-      if constexpr (FUSED) { a3 += s_red[3][k][c]; a4 += s_red[4][k][c]; }
     }
     atomicAdd(p.dgamma + c, a0);
     atomicAdd(p.dbeta + c, a1);
     atomicAdd(p.dP + static_cast<size_t>(pos) * W + c, a2);  // gridDim.y blocks per position
-    if constexpr (FUSED) {
-      atomicAdd(p.n1_dgamma + c, a3);
-      atomicAdd(p.n1_dbeta + c, a4);
-    }
   }
-  // sharded table: the gradient rows went to other GPUs; make them globally performed before the grid retires
-  // (the optimizer kernels of the owners start after a cross-rank barrier that follows this kernel)
-  if (p.dE.world != 0) __threadfence_system();
 }
 
 // --------------------------------------------------------------------------------------------
@@ -928,26 +831,13 @@ extern "C" int tt_last_index(const int64_t* ids, const int64_t* mask, int B, int
   return TT_OK;
 }
 
-static TableRef single_table(const float* E) {
-  TableRef t;
-  for (int r = 0; r < TT_SYMM_MAX_RANKS; ++r) t.base[r] = nullptr;
-  t.base[0] = const_cast<float*>(E);
-  t.world = 0;
-  return t;
-}
-
-static int sharded_table(TableRef& t, const tt_symm_team* team, int64_t offset, const char* who) {
-  return make_sharded_table(t, team, offset, who);
-}
-
-static int embed_fwd_impl(const int64_t* ids, const TableRef& E, float* stash, const float* P, const float* ln_w,
-                          const float* ln_b, const float* next_w, const float* next_b, int B, int L, float drop_p,
-                          uint64_t seed, const uint64_t* seed_dev, uint32_t site, float* x0, void* h_bf16,
-                          cudaStream_t stream) {
+static int embed_fwd_impl(const int64_t* ids, const float* E, const float* P, const float* ln_w, const float* ln_b,
+                          const float* next_w, const float* next_b, int B, int L, float drop_p, uint64_t seed,
+                          const uint64_t* seed_dev, uint32_t site, float* x0, void* h_bf16, cudaStream_t stream) {
   TT_REQUIRE(ids && P && ln_w && ln_b && next_w && next_b && x0 && h_bf16, "tt_embed_ln_fwd: null pointer");
   TT_REQUIRE(B > 0 && L > 0, "tt_embed_ln_fwd: empty batch");
   EmbedParams p;
-  p.ids = ids; p.E = E; p.stash = stash; p.P = P; p.ln_w = ln_w; p.ln_b = ln_b; p.nw = next_w; p.nb = next_b;
+  p.ids = ids; p.E = E; p.P = P; p.ln_w = ln_w; p.ln_b = ln_b; p.nw = next_w; p.nb = next_b;
   p.T = B * L; p.L = L;
   p.drop_thresh = drop_threshold(drop_p);
   p.drop_scale = drop_p > 0.f ? 1.f / (1.f - drop_p) : 1.f;
@@ -958,37 +848,25 @@ static int embed_fwd_impl(const int64_t* ids, const TableRef& E, float* stash, c
   return TT_OK;
 }
 
-static int embed_bwd_impl(const int64_t* ids, const TableRef& E, const float* stash, const float* P, const float* ln_w,
-                          const float* ln_b, const float* dx0, int B, int L, float drop_p, uint64_t seed,
-                          const uint64_t* seed_dev, uint32_t site, const TableRef& dE, float* dP, float* dgamma,
-                          float* dbeta, cudaStream_t stream, unsigned long long* acc64 = nullptr,
-                          const int64_t* acc_slot = nullptr, const tt_norm1_bwd* n1 = nullptr) {
-  TT_REQUIRE(ids && P && ln_w && ln_b && (dx0 || n1) && dP && dgamma && dbeta, "tt_embed_ln_bwd: null pointer");
-  TT_REQUIRE(!n1 || (n1->dh_bf16 && n1->resid && n1->ln_w && n1->ln_b && n1->dgamma && n1->dbeta),
-             "tt_embed_ln_bwd_norm1: incomplete norm1 description");
+static int embed_bwd_impl(const int64_t* ids, const float* E, const float* P, const float* ln_w, const float* ln_b,
+                          const float* dx0, int B, int L, float drop_p, uint64_t seed, const uint64_t* seed_dev,
+                          uint32_t site, float* dE, float* dP, float* dgamma, float* dbeta, cudaStream_t stream,
+                          unsigned long long* acc64 = nullptr, const int64_t* acc_slot = nullptr) {
+  TT_REQUIRE(ids && P && ln_w && ln_b && dx0 && dP && dgamma && dbeta, "tt_embed_ln_bwd: null pointer");
   EmbedBwdParams p;
-  p.ids = ids; p.E = E; p.stash = stash; p.P = P; p.ln_w = ln_w; p.ln_b = ln_b; p.dx0 = dx0; p.B = B; p.L = L;
+  p.ids = ids; p.E = E; p.P = P; p.ln_w = ln_w; p.ln_b = ln_b; p.dx0 = dx0; p.B = B; p.L = L;
   p.drop_thresh = drop_threshold(drop_p);
   p.drop_scale = drop_p > 0.f ? 1.f / (1.f - drop_p) : 1.f;
   p.seed = seed; p.seed_dev = seed_dev; p.site = site;
   p.dE = dE; p.dP = dP; p.dgamma = dgamma; p.dbeta = dbeta;
   p.acc64 = acc64; p.acc_slot = acc_slot;
-  p.n1_dh = n1 ? static_cast<const __nv_bfloat16*>(n1->dh_bf16) : nullptr;
-  p.n1_resid = n1 ? n1->resid : nullptr; p.n1_w = n1 ? n1->ln_w : nullptr; p.n1_b = n1 ? n1->ln_b : nullptr;
-  p.n1_dgamma = n1 ? n1->dgamma : nullptr; p.n1_dbeta = n1 ? n1->dbeta : nullptr;
   // ~6 blocks per SM in total (three waves at two resident blocks per SM): measured on the c2 step (L = 200), 1 / 2 /
   // 3 / 4 / 6 / 8 blocks per position -> 1.172 / 1.169 / 1.160 / 1.158 / 1.161 / 1.161 ms per step; one block per
   // position left every warp with a 32-row serial id -> row -> atomics chain and the SMs two thirds empty
   int splits = (6 * num_sms() + L / 2) / L;
-  {
-    static int env = -1;
-    if (env < 0) { const char* e = getenv("TT_EMBED_BWD_SPLITS"); env = e ? atoi(e) : 0; }
-    if (env > 0) splits = env;
-  }
   if (splits < 1) splits = 1;
   if (splits > (B + 7) / 8) splits = (B + 7) / 8;
-  if (n1) TT_CHECK_CUDA(launch_k(embed_ln_bwd_kernel<true>, dim3(L, splits), dim3(kRowThreads), 0, stream, p));
-  else TT_CHECK_CUDA(launch_k(embed_ln_bwd_kernel<false>, dim3(L, splits), dim3(kRowThreads), 0, stream, p));
+  TT_CHECK_CUDA(launch_k(embed_ln_bwd_kernel, dim3(L, splits), dim3(kRowThreads), 0, stream, p));
   TT_LAUNCH_CHECK();
   return TT_OK;
 }
@@ -998,8 +876,8 @@ extern "C" int tt_embed_ln_fwd(const int64_t* ids, const float* E, const float* 
                                float drop_p, uint64_t seed, const uint64_t* seed_dev, uint32_t site, float* x0,
                                void* h_bf16, void* stream_) {
   TT_REQUIRE(E, "tt_embed_ln_fwd: null table");
-  return embed_fwd_impl(ids, single_table(E), nullptr, P, ln_w, ln_b, next_w, next_b, B, L, drop_p, seed, seed_dev, site,
-                        x0, h_bf16, static_cast<cudaStream_t>(stream_));
+  return embed_fwd_impl(ids, E, P, ln_w, ln_b, next_w, next_b, B, L, drop_p, seed, seed_dev, site, x0, h_bf16,
+                        static_cast<cudaStream_t>(stream_));
 }
 
 extern "C" int tt_embed_ln_fwd_pos(const int64_t* ids, const int32_t* pos, const float* E, const float* P,
@@ -1009,7 +887,7 @@ extern "C" int tt_embed_ln_fwd_pos(const int64_t* ids, const int32_t* pos, const
              "tt_embed_ln_fwd_pos: null pointer");
   TT_REQUIRE(n > 0, "tt_embed_ln_fwd_pos: empty batch");
   EmbedParams p;
-  p.ids = ids; p.E = single_table(E); p.stash = nullptr; p.P = P; p.ln_w = ln_w; p.ln_b = ln_b;
+  p.ids = ids; p.E = E; p.P = P; p.ln_w = ln_w; p.ln_b = ln_b;
   p.nw = next_w; p.nb = next_b;
   p.T = n; p.L = 0;
   p.drop_thresh = 0; p.drop_scale = 1.f; p.seed = 0; p.seed_dev = nullptr; p.site = 0;
@@ -1025,17 +903,8 @@ extern "C" int tt_embed_ln_bwd(const int64_t* ids, const float* E, const float* 
                                const uint64_t* seed_dev, uint32_t site, float* dE, float* dP, float* dgamma,
                                float* dbeta, void* stream_) {
   TT_REQUIRE(E && dE, "tt_embed_ln_bwd: null table");
-  return embed_bwd_impl(ids, single_table(E), nullptr, P, ln_w, ln_b, dx0, B, L, drop_p, seed, seed_dev, site,
-                        single_table(dE), dP, dgamma, dbeta, static_cast<cudaStream_t>(stream_));
-}
-
-extern "C" int tt_embed_ln_bwd_norm1(const tt_norm1_bwd* n1, const int64_t* ids, const float* E, const float* P,
-                                     const float* ln_w, const float* ln_b, int B, int L, float drop_p, uint64_t seed,
-                                     const uint64_t* seed_dev, uint32_t site, float* dE, float* dP, float* dgamma,
-                                     float* dbeta, void* stream_) {
-  TT_REQUIRE(n1 && E && dE, "tt_embed_ln_bwd_norm1: null pointer");
-  return embed_bwd_impl(ids, single_table(E), nullptr, P, ln_w, ln_b, nullptr, B, L, drop_p, seed, seed_dev, site,
-                        single_table(dE), dP, dgamma, dbeta, static_cast<cudaStream_t>(stream_), nullptr, nullptr, n1);
+  return embed_bwd_impl(ids, E, P, ln_w, ln_b, dx0, B, L, drop_p, seed, seed_dev, site, dE, dP, dgamma, dbeta,
+                        static_cast<cudaStream_t>(stream_));
 }
 
 extern "C" int tt_embed_ln_bwd_det(const int64_t* ids, const float* E, const float* P, const float* ln_w,
@@ -1043,36 +912,9 @@ extern "C" int tt_embed_ln_bwd_det(const int64_t* ids, const float* E, const flo
                                    const uint64_t* seed_dev, uint32_t site, const int64_t* slot_of_token, int64_t* acc64,
                                    float* dP, float* dgamma, float* dbeta, void* stream_) {
   TT_REQUIRE(E && slot_of_token && acc64, "tt_embed_ln_bwd_det: null pointer");
-  TableRef none = single_table(nullptr);
-  return embed_bwd_impl(ids, single_table(E), nullptr, P, ln_w, ln_b, dx0, B, L, drop_p, seed, seed_dev, site, none, dP,
-                        dgamma, dbeta, static_cast<cudaStream_t>(stream_), reinterpret_cast<unsigned long long*>(acc64),
+  return embed_bwd_impl(ids, E, P, ln_w, ln_b, dx0, B, L, drop_p, seed, seed_dev, site, nullptr, dP, dgamma, dbeta,
+                        static_cast<cudaStream_t>(stream_), reinterpret_cast<unsigned long long*>(acc64),
                         slot_of_token);
-}
-
-extern "C" int tt_embed_ln_fwd_sharded(const int64_t* ids, const tt_symm_team* team, int64_t weight_offset,
-                                       float* row_stash, const float* P, const float* ln_w,
-                                       const float* ln_b, const float* next_w, const float* next_b, int B, int L,
-                                       float drop_p, uint64_t seed, const uint64_t* seed_dev, uint32_t site, float* x0,
-                                       void* h_bf16, void* stream_) {
-  TableRef E;
-  int rc = sharded_table(E, team, weight_offset, "tt_embed_ln_fwd_sharded");
-  if (rc) return rc;
-  return embed_fwd_impl(ids, E, row_stash, P, ln_w, ln_b, next_w, next_b, B, L, drop_p, seed, seed_dev, site, x0, h_bf16,
-                        static_cast<cudaStream_t>(stream_));
-}
-
-extern "C" int tt_embed_ln_bwd_sharded(const int64_t* ids, const tt_symm_team* team, int64_t weight_offset,
-                                       int64_t grad_offset, const float* row_stash, const float* P,
-                                       const float* ln_w, const float* ln_b, const float* dx0, int B, int L,
-                                       float drop_p, uint64_t seed, const uint64_t* seed_dev, uint32_t site, float* dP,
-                                       float* dgamma, float* dbeta, void* stream_) {
-  TableRef E, dE;
-  int rc = sharded_table(E, team, weight_offset, "tt_embed_ln_bwd_sharded");
-  if (rc) return rc;
-  rc = sharded_table(dE, team, grad_offset, "tt_embed_ln_bwd_sharded");
-  if (rc) return rc;
-  return embed_bwd_impl(ids, E, row_stash, P, ln_w, ln_b, dx0, B, L, drop_p, seed, seed_dev, site, dE, dP, dgamma, dbeta,
-                        static_cast<cudaStream_t>(stream_));
 }
 
 static int fill_chain(ChainParams& p, const tt_chain_args* a, const char* who) {
@@ -1195,18 +1037,6 @@ extern "C" int tt_bn_relu_bwd(const tt_bn_args* a, void* stream_) {
   if (rc) return rc;
   TT_REQUIRE(p.dout && p.dy && p.dgamma && p.dbeta && p.save_mean && p.save_rstd, "tt_bn_relu_bwd: missing buffers");
   TT_CHECK_CUDA(launch_k(bn_bwd_kernel, dim3((p.C + 31) / 32), dim3(dim3(32, 8)), 0, stream, p));
-  TT_LAUNCH_CHECK();
-  return TT_OK;
-}
-
-extern "C" int tt_colsum_bf16(const void* x, int R, int N, int ld, float* out, void* stream_) {
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  TT_REQUIRE(x && out && R > 0 && N > 0 && N % 2 == 0 && ld % 2 == 0, "tt_colsum_bf16: bad arguments");
-  const int gx = (N / 2 + 255) / 256;
-  int gy = (num_sms() * 4) / gx;
-  if (gy < 1) gy = 1;
-  if (gy > (R + 63) / 64) gy = (R + 63) / 64;
-  TT_CHECK_CUDA(launch_k(colsum_bf16_kernel, dim3(dim3(gx, gy)), dim3(256), 0, stream, static_cast<const __nv_bfloat16*>(x), R, N, ld, out));
   TT_LAUNCH_CHECK();
   return TT_OK;
 }

@@ -130,17 +130,6 @@ class TwoTowerEngine:
         #: run weight-gradient GEMMs / bias column sums on a second stream (see _wg)
         #: measurement aid: issue everything on the current stream (per-kernel event timing without overlap)
         self.serialize = False
-        self.overlap_wgrad = os.environ.get("TT_OVERLAP_WGRAD", "1") != "0"
-        #: bias gradients of the linear layers whose dY is a dgrad GEMM's A operand: column sums taken inside that
-        #: GEMM (tt_gemm_args.a_colsum) instead of a separate pass over dY (tt_colsum_bf16)
-        self.fuse_bias_colsum = os.environ.get("TT_FUSE_BIAS_COLSUM", "1") != "0"
-        #: dX of linear1 / in_proj of the full-sequence layers travels to the LayerNorm backward as bf16 (the dtype
-        #: autograd gives it under the reference's autocast, src/train.py:57-62) instead of fp32
-        self.bf16_linear_dgrad = os.environ.get("TT_BF16_LINEAR_DGRAD", "1") != "0"
-        #: layer 0's norm1 backward inside the embedding backward (tt_embed_ln_bwd_norm1): dx0 never exists in memory.
-        #: Off by default: 156 MB less traffic per c2 step, but the kernel's one-block-per-position grid (200 blocks of
-        #: 8 warps, three dependent row reductions per token) leaves it latency-bound — measured 1.181 vs 1.170 ms.
-        self.fuse_norm1_embed_bwd = os.environ.get("TT_FUSE_NORM1_EMBED_BWD", "0") != "0"
         #: row-sharded ID table (sharding.RowShardedTable, config 5): when set, `table_rows` [1 + B*L, 256] holds
         #: the rows the exchange fetched for this step's tokens (row 0 unused) and the embedding kernels index
         #: it with the token number instead of the item id; `table_rows_grad` receives the per-token gradient
@@ -152,9 +141,6 @@ class TwoTowerEngine:
         #: kernels read rows from / add gradient rows into the OWNER's memory directly (no exchange step). The flat
         #: buffer's own table region is a 2-row dummy.
         self.peer_table = None
-        #: with a peer table: reduce the step's ids to the distinct ones first (TT_TABLE_DEDUP=0: every token's row
-        #: crosses NVLink on its own, kept for A/B timing)
-        self.dedup_ids = os.environ.get("TT_TABLE_DEDUP", "1") != "0"
         self._sparse: Dict[int, Dict[str, torch.Tensor]] = {}
         #: deterministic table gradient (TT_DETERMINISTIC=1): the per-token gradient rows of duplicate ids are summed
         #: in 64-bit fixed point per distinct id (tt_embed_ln_bwd_det), so the result does not depend on the order the
@@ -490,9 +476,6 @@ class TwoTowerEngine:
         ~25 tiny B-row wgrads then overlap the dgrad chain instead of extending it. Every buffer they read
         is written once per backward (no reuse), so the only cross-stream hazard is the read-after-write
         edge this helper orders."""
-        if not self.overlap_wgrad:
-            fn(*a, **kw)
-            return
         main = torch.cuda.current_stream()
         wst = self._wgrad_stream()
         wst.wait_stream(main)
@@ -501,13 +484,8 @@ class TwoTowerEngine:
 
     def _dgrad_bias(self, dy, W, gbias, **kw) -> None:
         """dX = dY W on the main chain together with the bias gradient sum(dY, dim=0) -> gbias (accumulated).
-        By default the GEMM's two idle warps take the column sums from the dY tiles it stages anyway
-        (``a_colsum``); with ``fuse_bias_colsum`` off a separate pass over dY runs on the wgrad stream."""
-        if self.fuse_bias_colsum:
-            self._gemm(dy, W, b_mn=True, a_colsum=gbias, **kw)
-        else:
-            self._wg(ops.colsum_bf16, dy, gbias)
-            self._gemm(dy, W, b_mn=True, **kw)
+        The GEMM's two idle warps take the column sums from the dY tiles it stages anyway (``a_colsum``)."""
+        self._gemm(dy, W, b_mn=True, a_colsum=gbias, **kw)
 
     def _lp(self, l: int, name: str) -> str:
         return f"user_tower.transformer_encoder.layers.{l}.{name}"
@@ -524,7 +502,7 @@ class TwoTowerEngine:
         seed, sdev = self.base_seed, self.seed_dev
         ut = "user_tower."
         ops.last_index(ids, mask, ws["last_idx"])
-        if self.peer_table is not None and self.dedup_ids:
+        if self.peer_table is not None:
             # distinct ids of the step -> each distinct row crosses NVLink once into a compact (L2-resident) cache;
             # the embedding kernel then runs on the cache with the slot numbers as ids
             t, sp = self.peer_table, self._sparse_ws(B * L)
@@ -534,15 +512,6 @@ class TwoTowerEngine:
                              p[ut + "layer_norm.weight"], p[ut + "layer_norm.bias"],
                              p[self._lp(0, "norm1.weight")], p[self._lp(0, "norm1.bias")], B, L,
                              ws["x_in0"], ws["h1_0"], drop_p=dp, seed=seed, seed_dev=sdev, site=SITE_EMB)
-        elif self.peer_table is not None:
-            t = self.peer_table
-            if "row_stash" not in ws:
-                ws["row_stash"] = torch.empty(B * L, cfg.embedding_dim, device=self.device)
-            ops.embed_ln_fwd_sharded(ids.view(-1), t.arena.team, t.arena.offset("weight"), ws["row_stash"],
-                                     p[ut + "position_embedding.weight"], p[ut + "layer_norm.weight"],
-                                     p[ut + "layer_norm.bias"], p[self._lp(0, "norm1.weight")],
-                                     p[self._lp(0, "norm1.bias")], B, L, ws["x_in0"], ws["h1_0"], drop_p=dp, seed=seed,
-                                     seed_dev=sdev, site=SITE_EMB)
         else:
             e_ids, e_table, _ = self._embed_operands(ids)
             ops.embed_ln_fwd(e_ids, e_table, p[ut + "position_embedding.weight"],
@@ -855,13 +824,6 @@ class TwoTowerEngine:
                           seed_dev=sdev, dx_colsum=g[self._lp(top, "linear2.bias")])
 
         # ---- encoder layers, last to first
-        # the single-table embedding backward (local table, or the compact cache of the step's distinct rows) can take
-        # layer 0's norm1 backward with it when that layer runs the full-sequence schedule with a bf16 dX
-        single_table = (self.peer_table is not None and self.dedup_ids) or \
-            (self.peer_table is None and not (self.deterministic_table_grad and self.table_rows is None))
-        fuse_n1 = (self.fuse_norm1_embed_bwd and self.bf16_linear_dgrad and single_table and
-                   not (self.prune_last_layer and top == 0))
-        n1 = None
         for l in range(cfg.num_layers - 1, -1, -1):
             x_in = ws[f"xout_{l - 1}"] if l > 0 else ws["x_in0"]
             if self.prune_last_layer and l == top:
@@ -872,21 +834,18 @@ class TwoTowerEngine:
             if f"dpre_{l}" not in ws:      # prune_last_layer toggled after the workspace was built
                 ws[f"dpre_{l}"] = torch.empty(B * L, cfg.ff_dim, dtype=torch.bfloat16, device=self.device)
             dy2, dy1, dpre, dqkv = ws[f"dy2_{l}"], ws[f"dy1_{l}"], ws[f"dpre_{l}"], ws[f"dqkv_{l}"]
-            # the gradient a Linear hands back to the LayerNorm in front of it: bf16 like the reference's autocast
-            # backward (half the bytes between the dgrad GEMM and the LayerNorm backward), or fp32
-            if self.bf16_linear_dgrad:
-                dh_out, dh_in = dict(out_bf16=ws["dh_bf"]), dict(dout_bf16=ws["dh_bf"])
-            else:
-                dh_out, dh_in = dict(out_f32=ws["dh"]), dict(dout=ws["dh"])
             wg(gemm, dy2, ws[f"f_{l}"], a_mn=True, b_mn=True, out_f32=g[self._lp(l, "linear2.weight")], accumulate=True)
             gemm(dy2, w[self._lp(l, "linear2.weight")], b_mn=True, gate=ws[f"f_{l}"], gate_scale=ffn_scale,
                  out_bf16=dpre)
             wg(gemm, dpre, ws[f"h2_{l}"], a_mn=True, b_mn=True, out_f32=g[self._lp(l, "linear1.weight")],
                accumulate=True)
-            self._dgrad_bias(dpre, w[self._lp(l, "linear1.weight")], g[self._lp(l, "linear1.bias")], **dh_out)
+            # the gradient a Linear hands back to the LayerNorm in front of it is bf16 like the reference's autocast
+            # backward (half the bytes between the dgrad GEMM and the LayerNorm backward)
+            self._dgrad_bias(dpre, w[self._lp(l, "linear1.weight")], g[self._lp(l, "linear1.bias")],
+                             out_bf16=ws["dh_bf"])
             # norm2 backward (+ residual); emits dy for out_proj (dropout-1 mask) and its bias grad
             ops.chain_bwd(ws[f"xmid_{l}"], ln=(p[self._lp(l, "norm2.weight")], p[self._lp(l, "norm2.bias")]),
-                          resid=dx, dx_f32=dx_other, dx_bf16=dy1, drop2_p=dp, **dh_in,
+                          resid=dx, dx_f32=dx_other, dx_bf16=dy1, drop2_p=dp, dout_bf16=ws["dh_bf"],
                           drop2_site=_site(l, 1), seed=seed, seed_dev=sdev,
                           dgamma=g[self._lp(l, "norm2.weight")], dbeta=g[self._lp(l, "norm2.bias")],
                           dx_colsum=g[self._lp(l, "self_attn.out_proj.bias")])
@@ -899,47 +858,28 @@ class TwoTowerEngine:
             wg(gemm, dqkv, ws[f"h1_{l}"], a_mn=True, b_mn=True, out_f32=g[self._lp(l, "self_attn.in_proj_weight")],
                accumulate=True)
             self._dgrad_bias(dqkv, w[self._lp(l, "self_attn.in_proj_weight")], g[self._lp(l, "self_attn.in_proj_bias")],
-                             **dh_out)
+                             out_bf16=ws["dh_bf"])
             # norm1 backward (+ residual); for l > 0 also dy for the previous layer's linear2
             extra = {}
             if l > 0:
                 extra = dict(dx_bf16=ws[f"dy2_{l - 1}"], drop2_p=dp, drop2_site=_site(l - 1, 3),
                              dx_colsum=g[self._lp(l - 1, "linear2.bias")])
-            if l == 0 and fuse_n1:
-                # layer 0's norm1 backward runs inside the embedding backward below (x0 recomputed, dx0 never stored)
-                n1 = (ws["dh_bf"], dx, p[self._lp(0, "norm1.weight")], p[self._lp(0, "norm1.bias")],
-                      g[self._lp(0, "norm1.weight")], g[self._lp(0, "norm1.bias")])
-                continue
-            ops.chain_bwd(x_in, ln=(p[self._lp(l, "norm1.weight")], p[self._lp(l, "norm1.bias")]), **dh_in,
-                          resid=dx, dx_f32=dx_other, seed=seed, seed_dev=sdev,
+            ops.chain_bwd(x_in, ln=(p[self._lp(l, "norm1.weight")], p[self._lp(l, "norm1.bias")]),
+                          dout_bf16=ws["dh_bf"], resid=dx, dx_f32=dx_other, seed=seed, seed_dev=sdev,
                           dgamma=g[self._lp(l, "norm1.weight")], dbeta=g[self._lp(l, "norm1.bias")], **extra)
             dx, dx_other = dx_other, dx
 
         # ---- embedding LayerNorm + lookup
-        if self.peer_table is not None and self.dedup_ids:
+        if self.peer_table is not None:
             # per-token gradient rows are combined in the compact local buffer (atomics on L2-resident memory), then
             # ONE remote reduction per distinct row goes to its owner
             t, sp = self.peer_table, self._sparse_ws(B * L)
-            if n1 is not None:
-                ops.embed_ln_bwd_norm1(sp["inverse"], sp["cache"], p[ut + "position_embedding.weight"],
-                                       p[ut + "layer_norm.weight"], p[ut + "layer_norm.bias"], *n1, B, L,
-                                       sp["gacc"], g[ut + "position_embedding.weight"],
-                                       g[ut + "layer_norm.weight"], g[ut + "layer_norm.bias"], drop_p=dp, seed=seed,
-                                       seed_dev=sdev, site=SITE_EMB)
-            else:
-                ops.embed_ln_bwd(sp["inverse"], sp["cache"], p[ut + "position_embedding.weight"],
-                                 p[ut + "layer_norm.weight"], p[ut + "layer_norm.bias"], dx, B, L,
-                                 sp["gacc"], g[ut + "position_embedding.weight"],
-                                 g[ut + "layer_norm.weight"], g[ut + "layer_norm.bias"], drop_p=dp, seed=seed,
-                                 seed_dev=sdev, site=SITE_EMB)
+            ops.embed_ln_bwd(sp["inverse"], sp["cache"], p[ut + "position_embedding.weight"],
+                             p[ut + "layer_norm.weight"], p[ut + "layer_norm.bias"], dx, B, L,
+                             sp["gacc"], g[ut + "position_embedding.weight"],
+                             g[ut + "layer_norm.weight"], g[ut + "layer_norm.bias"], drop_p=dp, seed=seed,
+                             seed_dev=sdev, site=SITE_EMB)
             ops.rows_scatter_add(sp["uniq"], sp["state"], sp["gacc"], team=t.arena.team, grad_offset=t.arena.offset("grad"))
-        elif self.peer_table is not None:
-            t = self.peer_table
-            ops.embed_ln_bwd_sharded(ids.view(-1), t.arena.team, t.arena.offset("weight"), t.arena.offset("grad"),
-                                     ws["row_stash"], p[ut + "position_embedding.weight"], p[ut + "layer_norm.weight"],
-                                     p[ut + "layer_norm.bias"], dx, B, L, g[ut + "position_embedding.weight"],
-                                     g[ut + "layer_norm.weight"], g[ut + "layer_norm.bias"], drop_p=dp, seed=seed,
-                                     seed_dev=sdev, site=SITE_EMB)
         elif self.deterministic_table_grad and self.table_rows is None:
             dw = self._det_ws(T)
             ops.ids_dedup(ids.view(-1), cfg.vocab_size, dw["flag"], dw["slot"], dw["uniq"], dw["state"], dw["inverse"])
@@ -950,21 +890,13 @@ class TwoTowerEngine:
             ops.rows_scatter_add_i64(dw["uniq"], dw["state"], dw["acc64"], g[ut + "item_embedding.weight"])
         else:
             e_ids, e_table, e_grad = self._embed_operands(ids)
-            if n1 is not None:
-                ops.embed_ln_bwd_norm1(e_ids, e_table, p[ut + "position_embedding.weight"],
-                                       p[ut + "layer_norm.weight"], p[ut + "layer_norm.bias"], *n1, B, L,
-                                       e_grad, g[ut + "position_embedding.weight"],
-                                       g[ut + "layer_norm.weight"], g[ut + "layer_norm.bias"], drop_p=dp, seed=seed,
-                                       seed_dev=sdev, site=SITE_EMB)
-            else:
-                ops.embed_ln_bwd(e_ids, e_table, p[ut + "position_embedding.weight"],
-                                 p[ut + "layer_norm.weight"], p[ut + "layer_norm.bias"], dx, B, L,
-                                 e_grad, g[ut + "position_embedding.weight"],
-                                 g[ut + "layer_norm.weight"], g[ut + "layer_norm.bias"], drop_p=dp, seed=seed,
-                                 seed_dev=sdev, site=SITE_EMB)
+            ops.embed_ln_bwd(e_ids, e_table, p[ut + "position_embedding.weight"],
+                             p[ut + "layer_norm.weight"], p[ut + "layer_norm.bias"], dx, B, L,
+                             e_grad, g[ut + "position_embedding.weight"],
+                             g[ut + "layer_norm.weight"], g[ut + "layer_norm.bias"], drop_p=dp, seed=seed,
+                             seed_dev=sdev, site=SITE_EMB)
         main.wait_stream(side)
-        if self.overlap_wgrad:
-            main.wait_stream(self._wgrad_stream())
+        main.wait_stream(self._wgrad_stream())
 
     # ------------------------------------------------------------------ optimizer
     def adamw_step(self, lr: float = 1e-4, betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 0.01,

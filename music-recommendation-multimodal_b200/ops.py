@@ -179,22 +179,6 @@ def embed_ln_bwd(ids, E, P, ln_w, ln_b, dx0, B, L, dE, dP, dgamma, dbeta, drop_p
                                 dP.data_ptr(), dgamma.data_ptr(), dbeta.data_ptr(), _stream()), "tt_embed_ln_bwd")
 
 
-def embed_ln_bwd_norm1(ids, E, P, ln_w, ln_b, dh_bf16, resid, n1_w, n1_b, n1_dgamma, n1_dbeta, B, L, dE, dP, dgamma, dbeta,
-                       drop_p=0.0, seed=0, seed_dev=None, site=0):
-    """tt_embed_ln_bwd_norm1: the first encoder layer's norm1 backward and the embedding LayerNorm / lookup backward
-    in one pass (x0 is recomputed from the table rows, dx0 never exists in memory)."""
-    from ._lib import Norm1Bwd
-    _require_cuda(ids, E, P, dh_bf16, resid, n1_w, n1_b, n1_dgamma, n1_dbeta, dE, dP, dgamma, dbeta)
-    assert dh_bf16.dtype == torch.bfloat16 and dh_bf16.is_contiguous() and dh_bf16.shape == (B * L, 256)
-    assert resid.dtype == torch.float32 and resid.is_contiguous() and resid.shape == (B * L, 256)
-    n1 = Norm1Bwd(dh_bf16.data_ptr(), resid.data_ptr(), n1_w.data_ptr(), n1_b.data_ptr(), n1_dgamma.data_ptr(),
-                  n1_dbeta.data_ptr())
-    check(lib().tt_embed_ln_bwd_norm1(ctypes.byref(n1), ids.data_ptr(), E.data_ptr(), P.data_ptr(), ln_w.data_ptr(),
-                                      ln_b.data_ptr(), B, L, drop_p, seed, _ptr(seed_dev), site, dE.data_ptr(),
-                                      dP.data_ptr(), dgamma.data_ptr(), dbeta.data_ptr(), _stream()),
-          "tt_embed_ln_bwd_norm1")
-
-
 def embed_ln_bwd_det(ids, E, P, ln_w, ln_b, dx0, B, L, slot_of_token, acc64, dP, dgamma, dbeta, drop_p=0.0, seed=0,
                      seed_dev=None, site=0):
     """tt_embed_ln_bwd_det: the table gradient is accumulated per distinct id in 64-bit fixed point (order-independent,
@@ -214,26 +198,6 @@ def rows_scatter_add_i64(uniq, state, acc64, grad_local) -> None:
     assert grad_local.dtype == torch.float32 and grad_local.is_contiguous()
     check(lib().tt_rows_scatter_add_i64(grad_local.data_ptr(), uniq.data_ptr(), state.data_ptr() + 4, acc64.shape[0],
                                         acc64.data_ptr(), _stream()), "tt_rows_scatter_add_i64")
-
-
-def embed_ln_fwd_sharded(ids, team, weight_offset, stash, P, ln_w, ln_b, next_w, next_b, B, L, x0, h,
-                         drop_p=0.0, seed=0, seed_dev=None, site=0):
-    """tt_embed_ln_fwd_sharded: the ID table is row-sharded over the ranks of a symmetric arena."""
-    _require_cuda(ids, stash, P, x0, h)
-    assert ids.dtype == torch.int64 and P.shape[0] >= L
-    check(lib().tt_embed_ln_fwd_sharded(ids.data_ptr(), ctypes.byref(team), weight_offset, _ptr(stash),
-                                        P.data_ptr(), ln_w.data_ptr(), ln_b.data_ptr(), next_w.data_ptr(),
-                                        next_b.data_ptr(), B, L, drop_p, seed, _ptr(seed_dev), site, x0.data_ptr(),
-                                        h.data_ptr(), _stream()), "tt_embed_ln_fwd_sharded")
-
-
-def embed_ln_bwd_sharded(ids, team, weight_offset, grad_offset, stash, P, ln_w, ln_b, dx0, B, L, dP,
-                         dgamma, dbeta, drop_p=0.0, seed=0, seed_dev=None, site=0):
-    _require_cuda(ids, stash, P, dx0, dP, dgamma, dbeta)
-    check(lib().tt_embed_ln_bwd_sharded(ids.data_ptr(), ctypes.byref(team), weight_offset, grad_offset,
-                                        _ptr(stash), P.data_ptr(), ln_w.data_ptr(), ln_b.data_ptr(), dx0.data_ptr(), B,
-                                        L, drop_p, seed, _ptr(seed_dev), site, dP.data_ptr(), dgamma.data_ptr(),
-                                        dbeta.data_ptr(), _stream()), "tt_embed_ln_bwd_sharded")
 
 
 def ids_dedup(ids, V, flag, slot, uniq, state, inverse) -> None:
@@ -349,13 +313,6 @@ def bn_relu_fwd(y, w, b, running_mean, running_var, num_batches, **kw) -> None:
 def bn_relu_bwd(y, w, b, running_mean, running_var, num_batches, **kw) -> None:
     a = _bn_args(y, w, b, running_mean, running_var, num_batches, **kw)
     check(lib().tt_bn_relu_bwd(ctypes.byref(a), _stream()), "tt_bn_relu_bwd")
-
-
-def colsum_bf16(x: torch.Tensor, out: torch.Tensor) -> None:
-    _require_cuda(x, out)
-    assert x.dtype == torch.bfloat16 and x.stride(1) == 1 and out.dtype == torch.float32
-    check(lib().tt_colsum_bf16(x.data_ptr(), x.shape[0], x.shape[1], x.stride(0), out.data_ptr(), _stream()),
-          "tt_colsum_bf16")
 
 
 def adamw_step(p, g, m, v, step_dev, lr=1e-4, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=0.01,

@@ -345,8 +345,7 @@ def sharded_topk(user_emb: torch.Tensor, index: "CatalogIndex", K: int, kprime: 
         # Measured (tools/dist_retrieval_check.py, 2 GPUs over NCCL, 10 k users x 1 M items): with 2 shards the
         # lists are nearly as long as the single-GPU budget (208 of 256) and the bounded pass is the slower one
         # (3.27 vs 3.06 ms); a 1/8 shard takes 1.14 ms with 64-entry lists against 1.76 ms with K' = 256.
-        env = os.environ.get("TT_SHARD_BOUNDED", "")
-        bounded = (ws >= 4) if env == "" else (env != "0")
+        bounded = ws >= 4
 
     def per_shard_exact(users):
         i, s, _ = retrieve_topk(users, index, K, kprime, **_exclude_kw(exclude))
@@ -475,22 +474,12 @@ def metrics_from_embeddings(user_emb: torch.Tensor, targets: torch.Tensor, index
     happens to be initialised (every rank then evaluates its own users against the whole catalog)."""
     K = max(k_list)
     targets = targets.to(user_emb.device)
-    _dbg = os.environ.get("TT_RETRIEVAL_TRACE", "") == "1"
-    if _dbg:
-        import time as _t
-        _marks = [("enter", _t.perf_counter())]
     if index.is_sharded:
         # the certificate flags travel to the host WITH the metrics: one synchronisation per call; only if a flag is
         # set (rare) the exact per-shard protocol repairs those users and the metrics are taken again
         idx, score, bad = sharded_topk(user_emb, index, K, kprime, group, defer_check=True)
-        if _dbg:
-            _marks.append(("sharded_topk", _t.perf_counter()))
         recall, ndcg = rank_metrics(idx, targets, k_list)
-        if _dbg:
-            _marks.append(("rank_metrics", _t.perf_counter()))
         packed = torch.cat([recall.flatten(), ndcg.flatten(), bad.max().float().view(1)]).cpu()
-        if _dbg:
-            _marks.append(("readback", _t.perf_counter()))
         if packed[-1].item() != 0:
             finish_sharded_topk(user_emb, index, K, idx, score, bad, kprime, group)
             recall, ndcg = rank_metrics(idx, targets, k_list)
@@ -508,9 +497,4 @@ def metrics_from_embeddings(user_emb: torch.Tensor, targets: torch.Tensor, index
         out[f"Recall@{k}"] = r[j].mean().item()
     for j, k in enumerate(k_list):
         out[f"NDCG@{k}"] = n[j].mean().item()
-    if _dbg:
-        _marks.append(("means", _t.perf_counter()))
-        print(f"[rank {os.environ.get('RANK', '0')}] metrics_from_embeddings t0 {_t.time() % 100:.4f} host ms:",
-              ", ".join(f"{b[0]} {1e3 * (b[1] - a[1]):.2f}" for a, b in zip(_marks[:-1], _marks[1:])),
-              file=__import__("sys").stderr, flush=True)
     return out

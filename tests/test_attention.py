@@ -8,10 +8,13 @@ import math
 import pytest
 import torch
 
+import _dropout_ref as R
+
 pytestmark = pytest.mark.gpu
 
 
-def _ref_attention(qkv, B, L, H, dctx=None):
+def _ref_attention(qkv, B, L, H, dctx=None, drop_mask=None):
+    """fp32 causal attention; ``drop_mask`` (B, H, L, L), if given, multiplies the probabilities."""
     D = H * 64
     x = qkv.float().view(B, L, 3, H, 64).requires_grad_(dctx is not None)
     q, k, v = x[:, :, 0].transpose(1, 2), x[:, :, 1].transpose(1, 2), x[:, :, 2].transpose(1, 2)
@@ -19,7 +22,10 @@ def _ref_attention(qkv, B, L, H, dctx=None):
     mask = torch.triu(torch.ones(L, L, dtype=torch.bool, device=qkv.device), 1)
     s = s.masked_fill(mask, float("-inf"))
     lse = torch.logsumexp(s, dim=-1)                         # (B,H,L)
-    o = (torch.softmax(s, dim=-1) @ v).transpose(1, 2).reshape(B * L, D)
+    prob = torch.softmax(s, dim=-1)
+    if drop_mask is not None:
+        prob = prob * drop_mask
+    o = (prob @ v).transpose(1, 2).reshape(B * L, D)
     if dctx is None:
         return o, lse, None
     o.backward(dctx.float())
@@ -91,12 +97,47 @@ def test_attn_dropout_statistics():
     assert diff <= 0.25 * ref, (diff, ref)
 
 
-@pytest.mark.parametrize("B,L,H,drop", [(3, 200, 4, 0.0), (160, 200, 4, 0.1), (150, 50, 4, 0.1), (40, 256, 2, 0.2),
-                                        (37, 129, 4, 0.1), (2, 128, 4, 0.0)])
-def test_attn_bwd_persistent_equals_legacy(B, L, H, drop, monkeypatch):
-    """The persistent, pipelined backward (L <= 256) runs the same arithmetic in the same order as the
-    one-CTA-per-(sequence, head) kernel: bit-identical dq/dk/dv, with and without dropout, with more
-    items than SMs (several items per CTA) and with fewer."""
+# More (sequence, head) items than SMs (a persistent CTA walks several items) and fewer; with and without dropout.
+REPEAT_SHAPES = [(160, 200, 4, 0.1), (150, 50, 4, 0.1), (40, 256, 2, 0.2), (37, 129, 4, 0.1), (3, 200, 4, 0.0),
+                 (2, 128, 4, 0.0)]
+
+
+def _drop_mask(B, L, H, drop, seed, site):
+    """The kernels' dropout mask of the probabilities (index ((b*H + h)*L + q)*L + k), scaled, or None."""
+    if drop == 0.0:
+        return None
+    return torch.from_numpy(R.scaled_mask(seed, site, (B, H, L, L), drop)).cuda()
+
+
+@pytest.mark.parametrize("B,L,H,drop", REPEAT_SHAPES)
+def test_attn_fwd_repeated_launches_match_reference(B, L, H, drop):
+    """Two forward launches give the very same bits (the second must not depend on state the first left behind),
+    finite, and equal to fp32 attention with the kernels' dropout mask."""
+    from mrm_b200 import ops
+    g = torch.Generator().manual_seed(11 * L + B)
+    qkv = (torch.randn(B * L, 3 * H * 64, generator=g) * 1.2).cuda().bfloat16()
+    out = []
+    for _ in range(2):
+        ctx = torch.full((B * L, H * 64), float("nan"), device="cuda", dtype=torch.bfloat16)
+        lse = torch.full((B, H, L), float("nan"), device="cuda")
+        ops.attn_fwd(qkv, ctx, lse, B, L, H, drop_p=drop, drop_seed=11, drop_site=2)
+        out.append((ctx, lse))
+    torch.cuda.synchronize()
+    (ctx, lse), (ctx2, lse2) = out
+    assert torch.isfinite(ctx.float()).all() and torch.isfinite(lse).all()
+    assert torch.equal(ctx, ctx2) and torch.equal(lse, lse2)
+    o, lse_ref, _ = _ref_attention(qkv, B, L, H, drop_mask=_drop_mask(B, L, H, drop, 11, 2))
+    tol = 4e-2 if drop > 0 else 3e-2
+    err = (ctx.float() - o).abs().max().item()
+    lerr = (lse - lse_ref).abs().max().item()
+    assert err <= tol, f"ctx err {err}"
+    assert lerr <= 2e-3, f"lse err {lerr}"
+
+
+@pytest.mark.parametrize("B,L,H,drop", REPEAT_SHAPES)
+def test_attn_bwd_repeated_launches_match_reference(B, L, H, drop):
+    """Two backward launches give the very same bits (the second must not depend on state the first left behind),
+    finite, and equal to fp32 autograd with the kernels' dropout mask."""
     from mrm_b200 import ops
     g = torch.Generator().manual_seed(7 * L + B)
     qkv = (torch.randn(B * L, 3 * H * 64, generator=g) * 1.2).cuda().bfloat16()
@@ -104,42 +145,23 @@ def test_attn_bwd_persistent_equals_legacy(B, L, H, drop, monkeypatch):
     ctx = torch.empty((B * L, H * 64), device="cuda", dtype=torch.bfloat16)
     lse = torch.empty(B, H, L, device="cuda")
     ops.attn_fwd(qkv, ctx, lse, B, L, H, drop_p=drop, drop_seed=11, drop_site=2)
-    out = {}
-    for mode in ("legacy", "persistent"):
-        monkeypatch.setenv("TT_ATTN_BWD", mode)
+    out = []
+    for _ in range(2):
         d = torch.full((B * L, 3 * H * 64), float("nan"), device="cuda", dtype=torch.bfloat16)
-        for _ in range(2):      # twice: the second launch must not depend on state left by the first
-            ops.attn_bwd(qkv, ctx, dctx, lse, d, B, L, H, drop_p=drop, drop_seed=11, drop_site=2)
-        torch.cuda.synchronize()
-        out[mode] = d
-    assert torch.isfinite(out["persistent"].float()).all()
-    assert torch.equal(out["legacy"], out["persistent"])
-
-
-@pytest.mark.parametrize("B,L,H,drop", [(3, 200, 4, 0.0), (160, 200, 4, 0.1), (150, 50, 4, 0.1), (40, 256, 2, 0.2),
-                                        (37, 129, 4, 0.1), (2, 128, 4, 0.0)])
-def test_attn_fwd_persistent_equals_legacy(B, L, H, drop, monkeypatch):
-    """The persistent forward (L <= 256) forms the same P tiles and issues the same MMAs as the per-tile kernel; only the
-    row sums are added in another order (four column groups instead of two halves), so ctx may differ by one bf16
-    rounding and the log-sum-exp by fp32 rounding. With more items than SMs and with fewer; with and without dropout."""
-    from mrm_b200 import ops
-    g = torch.Generator().manual_seed(11 * L + B)
-    qkv = (torch.randn(B * L, 3 * H * 64, generator=g) * 1.2).cuda().bfloat16()
-    out = {}
-    for mode in ("legacy", "persistent"):
-        monkeypatch.setenv("TT_ATTN_FWD", mode)
-        ctx = torch.full((B * L, H * 64), float("nan"), device="cuda", dtype=torch.bfloat16)
-        lse = torch.full((B, H, L), float("nan"), device="cuda")
-        for _ in range(2):
-            ops.attn_fwd(qkv, ctx, lse, B, L, H, drop_p=drop, drop_seed=11, drop_site=2)
-        torch.cuda.synchronize()
-        out[mode] = (ctx, lse)
-    a, b = out["legacy"], out["persistent"]
-    assert torch.isfinite(b[0].float()).all() and torch.isfinite(b[1]).all()
-    assert float((a[1] - b[1]).abs().max()) <= 2e-5
-    diff = (a[0].float() - b[0].float()).abs()
-    assert float(diff.max()) <= 2.0 ** -7 * max(1.0, float(a[0].float().abs().max()))
-    assert float((diff > 0).float().mean()) < 0.02        # almost everywhere the very same bits
+        ops.attn_bwd(qkv, ctx, dctx, lse, d, B, L, H, drop_p=drop, drop_seed=11, drop_site=2)
+        out.append(d)
+    torch.cuda.synchronize()
+    dqkv, dqkv2 = out
+    assert torch.isfinite(dqkv.float()).all()
+    assert torch.equal(dqkv, dqkv2)
+    _, _, dref = _ref_attention(qkv, B, L, H, dctx, drop_mask=_drop_mask(B, L, H, drop, 11, 2))
+    tol = 4e-2 if drop > 0 else 3e-2
+    D = H * 64
+    for name, sl in (("dq", slice(0, D)), ("dk", slice(D, 2 * D)), ("dv", slice(2 * D, 3 * D))):
+        a, r = dqkv[:, sl].float(), dref[:, sl]
+        err = (a - r).abs().max().item()
+        scale = r.abs().max().item()
+        assert err <= tol * max(scale, 1.0), f"{name}: err {err} scale {scale}"
 
 
 @pytest.mark.parametrize("B,L,H", [(2, 200, 2), (2, 384, 2), (1, 512, 2), (2, 300, 4)])

@@ -188,11 +188,9 @@ def test_bn_relu_fwd_mask(B, case):
     _close(out.float()[keep], ref[keep], 1e-2)
 
 
-def _probs_readout(qkv, B, L, H, mode, monkeypatch, **drop):
+def _probs_readout(qkv, B, L, H, **drop):
     """[B, H, L, L] probabilities as attn_fwd forms them (dropout applied), read out through one-hot V blocks."""
     from mrm_b200 import ops
-    if mode is not None:
-        monkeypatch.setenv("TT_ATTN_FWD", mode)
     D = H * 64
     out = torch.zeros(B, H, L, L, device="cuda")
     x = qkv.clone().view(B, L, 3, H, 64)
@@ -219,16 +217,16 @@ def _attn_ref(qkv, B, L, H, mask, dctx):
 
 
 # odd B*H (and L = 50, 129, 300: every alignment of the index, so the quad, pair and single hash forms all run);
-# the persistent and legacy kernels for L <= 256, the four-tile per-item kernels above
+# the persistent kernels for L <= 256, the four-tile per-item kernels for 256 < L <= 512
 ATTN_SHAPES = [(3, 50, 1), (1, 129, 3), (3, 200, 1), (2, 200, 4), (1, 256, 3), (3, 300, 1), (1, 512, 3)]
 
 
 @gpu
 @pytest.mark.parametrize("case", CASES, ids=CASE_IDS)
 @pytest.mark.parametrize("B,L,H", ATTN_SHAPES)
-def test_attention_masks_forward_and_backward(B, L, H, case, monkeypatch):
+def test_attention_masks_forward_and_backward(B, L, H, case):
     """The forward's keep bits, read out through one-hot V, equal the numpy mask wherever the probability is
-    resolvable (P > 1e-5); the backward of every kernel equals fp32 autograd with the numpy mask."""
+    resolvable (P > 1e-5); the backward equals fp32 autograd with the numpy mask."""
     from mrm_b200 import ops
     seed, ctr, site = case
     p = 0.1
@@ -238,29 +236,23 @@ def test_attention_masks_forward_and_backward(B, L, H, case, monkeypatch):
     dctx = torch.randn(B * L, D, generator=g).cuda().bfloat16()
     drop = dict(drop_p=p, drop_seed=seed, drop_seed_dev=_counter(ctr), drop_site=site)
     keep = _keep(case, (B, H, L, L), p)
-    modes = ("legacy", "persistent") if L <= 256 else (None,)
-    for mode in modes:
-        P0 = _probs_readout(qkv, B, L, H, mode, monkeypatch)
-        Pd = _probs_readout(qkv, B, L, H, mode, monkeypatch, **drop)
-        known = P0 > 1e-5
-        assert known.sum().item() > 0.5 * B * H * L * (L + 1) / 2    # most of the causal triangle is resolvable
-        assert torch.equal((Pd > 0.5 * P0)[known], keep[known]), mode
+    P0 = _probs_readout(qkv, B, L, H)
+    Pd = _probs_readout(qkv, B, L, H, **drop)
+    known = P0 > 1e-5
+    assert known.sum().item() > 0.5 * B * H * L * (L + 1) / 2    # most of the causal triangle is resolvable
+    assert torch.equal((Pd > 0.5 * P0)[known], keep[known])
     mask = torch.where(keep, float(R.drop_scale(p)), 0.0)
     o_ref, d_ref = _attn_ref(qkv, B, L, H, mask, dctx)
-    for mode in modes:
-        if mode is not None:
-            monkeypatch.setenv("TT_ATTN_FWD", mode)
-            monkeypatch.setenv("TT_ATTN_BWD", mode)
-        ctx = torch.empty(B * L, D, device="cuda", dtype=torch.bfloat16)
-        lse = torch.empty(B, H, L, device="cuda")
-        ops.attn_fwd(qkv, ctx, lse, B, L, H, **drop)
-        dqkv = torch.full((B * L, 3 * D), float("nan"), device="cuda", dtype=torch.bfloat16)
-        ops.attn_bwd(qkv, ctx, dctx, lse, dqkv, B, L, H, **drop)
-        torch.cuda.synchronize()
-        assert (ctx.float() - o_ref).abs().max().item() <= 4e-2, mode
-        for name, sl in (("dq", slice(0, D)), ("dk", slice(D, 2 * D)), ("dv", slice(2 * D, 3 * D))):
-            err = (dqkv[:, sl].float() - d_ref[:, sl]).abs().max().item()
-            assert err <= 4e-2 * max(d_ref[:, sl].abs().max().item(), 1.0), (mode, name, err)
+    ctx = torch.empty(B * L, D, device="cuda", dtype=torch.bfloat16)
+    lse = torch.empty(B, H, L, device="cuda")
+    ops.attn_fwd(qkv, ctx, lse, B, L, H, **drop)
+    dqkv = torch.full((B * L, 3 * D), float("nan"), device="cuda", dtype=torch.bfloat16)
+    ops.attn_bwd(qkv, ctx, dctx, lse, dqkv, B, L, H, **drop)
+    torch.cuda.synchronize()
+    assert (ctx.float() - o_ref).abs().max().item() <= 4e-2
+    for name, sl in (("dq", slice(0, D)), ("dk", slice(D, 2 * D)), ("dv", slice(2 * D, 3 * D))):
+        err = (dqkv[:, sl].float() - d_ref[:, sl]).abs().max().item()
+        assert err <= 4e-2 * max(d_ref[:, sl].abs().max().item(), 1.0), (name, err)
 
 
 def _lastq_operands(B, L, H, last, seed):
@@ -277,7 +269,7 @@ def _lastq_last(B, L):
 @gpu
 @pytest.mark.parametrize("case", CASES, ids=CASE_IDS)
 @pytest.mark.parametrize("L", [77, 200, 512])
-def test_attn_lastq_fwd_mask_equals_the_full_kernel_row(L, case, monkeypatch):
+def test_attn_lastq_fwd_mask_equals_the_full_kernel_row(L, case):
     """attn_lastq_fwd (the pruned last layer's attention) draws its mask at the full-sequence index
     ((b*H + h)*L + last)*L + k: its probabilities, read out through one-hot V, keep the numpy mask's bits and equal
     row `last` of the full kernel's."""
@@ -308,7 +300,7 @@ def test_attn_lastq_fwd_mask_equals_the_full_kernel_row(L, case, monkeypatch):
     keep_rows = keep[bi, :, last.long()]                              # (B, H, L)
     known = P0 > 1e-5
     assert torch.equal((Pd > 0.5 * P0)[known], keep_rows[known])
-    full = _probs_readout(qkv, B, L, H, None, monkeypatch, drop_p=p, drop_seed=seed, drop_seed_dev=_counter(ctr),
+    full = _probs_readout(qkv, B, L, H, drop_p=p, drop_seed=seed, drop_seed_dev=_counter(ctr),
                           drop_site=site)[bi, :, last.long()]
     assert torch.equal((full > 0)[known], (Pd > 0)[known])
     assert torch.allclose(full, Pd, rtol=1e-2, atol=1e-4)
@@ -357,45 +349,27 @@ def test_attn_lastq_bwd_with_dropout_matches_autograd(L):
 # ----------------------------------------------------------------------------------------------------------------
 @gpu
 @pytest.mark.parametrize("p", [0.1, 0.25])
-def test_embed_ln_bwd_with_dropout_matches_autograd(p):
-    """B = 64, L = 50: several row splits per position (the c2 step runs four), both the plain embedding backward
-    and the one with layer 0's norm1 backward inside."""
+def test_embed_ln_bwd_dropout_matches_autograd(p):
+    """B = 64, L = 50: several row splits per position (the c2 step runs four)."""
     from mrm_b200 import ops
     case = CASES[1]
     seed, ctr, site = case
     B, L = 64, 50
-    ids, E, P, w, b, w1, b1 = _embed_operands(B, L, seed=30)
+    ids, E, P, w, b, _, _ = _embed_operands(B, L, seed=30)
     kw = dict(drop_p=p, seed=seed, seed_dev=_counter(ctr), site=site)
     mask = torch.where(_keep(case, (B * L, 256), p), float(R.drop_scale(p)), 0.0)
     dx0 = _randn(B * L, 256, seed=40)
-    dh = _randn(B * L, 256, seed=41).bfloat16()
-    resid = _randn(B * L, 256, seed=42)
-
-    def zeros():
-        return (torch.zeros_like(E), torch.zeros_like(P), torch.zeros(256, device="cuda"), torch.zeros(256, device="cuda"))
-
-    dE, dP, dg, db = zeros()
+    dE, dP, dg, db = (torch.zeros_like(E), torch.zeros_like(P), torch.zeros(256, device="cuda"),
+                      torch.zeros(256, device="cuda"))
     ops.embed_ln_bwd(ids.view(-1), E, P, w, b, dx0, B, L, dE, dP, dg, db, **kw)
-    dE1, dP1, dg1, db1 = zeros()
-    dgn, dbn = torch.zeros(256, device="cuda"), torch.zeros(256, device="cuda")
-    ops.embed_ln_bwd_norm1(ids.view(-1), E, P, w, b, dh, resid, w1, b1, dgn, dbn, B, L, dE1, dP1, dg1, db1, **kw)
     torch.cuda.synchronize()
-    for fused in (False, True):
-        Er, Pr, wr, br, w1r, b1r = (t.clone().requires_grad_(True) for t in (E, P, w, b, w1, b1))
-        x = F.layer_norm(Er[ids] + Pr[:L].unsqueeze(0), (256,), wr, br).view(B * L, 256) * mask
-        if fused:
-            y = F.layer_norm(x, (256,), w1r, b1r)
-            ((y * dh.float()).sum() + (x * resid).sum()).backward()
-            got = (dE1, dP1, dg1, db1)
-            _close(dgn, w1r.grad, 1e-4)
-            _close(dbn, b1r.grad, 1e-4)
-        else:
-            x.backward(dx0)
-            got = (dE, dP, dg, db)
-        dE_ref = Er.grad.clone()
-        dE_ref[0] = 0                     # padding_idx
-        for a, r in zip(got, (dE_ref, Pr.grad, wr.grad, br.grad)):
-            _close(a, r, 1e-4)
+    Er, Pr, wr, br = (t.clone().requires_grad_(True) for t in (E, P, w, b))
+    x = F.layer_norm(Er[ids] + Pr[:L].unsqueeze(0), (256,), wr, br).view(B * L, 256) * mask
+    x.backward(dx0)
+    dE_ref = Er.grad.clone()
+    dE_ref[0] = 0                     # padding_idx
+    for a, r in zip((dE, dP, dg, db), (dE_ref, Pr.grad, wr.grad, br.grad)):
+        _close(a, r, 1e-4)
 
 
 @gpu

@@ -1,6 +1,5 @@
 #!/usr/bin/env python
-"""Event-timed micro-benchmark of tt_gemm_bf16 on the training step's shapes.
-TT_GEMM_DEBUG=1 makes the epilogue drain TMEM only (mainloop-bound time)."""
+"""Event-timed micro-benchmark of tt_gemm_bf16 on the training step's shapes."""
 import os
 import sys
 
@@ -58,7 +57,6 @@ cases = [
     ("dW2   wgrad 256x1024         ", 256, 1024, T, lambda: ops.gemm(x[:, :256], x, a_mn=True, b_mn=True, out_f32=g32[:256], accumulate=True)),
     ("dWo   wgrad 256x256          ", 256, 256, T, lambda: ops.gemm(x[:, :256], x[:, :256], a_mn=True, b_mn=True, out_f32=g32[:256, :256], accumulate=True)),
 ]
-print(f"TT_GEMM_DEBUG={os.environ.get('TT_GEMM_DEBUG', '0')}")
 for name, M, N, K, fn in cases:
     us = t(fn)
     print(f"{name} M={M:6d} N={N:5d} K={K:6d}  {us:8.1f} us  {2.0 * M * N * K / us / 1e6:8.1f} TFLOP/s")
