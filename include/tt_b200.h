@@ -409,6 +409,31 @@ int tt_exact_topk_excl(const float* user_f32, const float* items_f32, int N, int
 int tt_rank_metrics(const int32_t* topk_idx, const int64_t* targets, int U, int K, const int32_t* k_list, int nk,
                     const float* gain_table, float* recall, float* ndcg, void* stream);
 
+/* ---- diversified recommendations: maximal marginal relevance over each user's candidate pool ----
+ * Extends the selection of src/inference.py:296-306 (masked scores, top k): instead of the k best scores, k picks
+ * from the pool of the exact top P admissible candidates (pool_idx int32 / pool_score fp32 [U, P], canonical order,
+ * -1 / -inf tail, as tt_topk_finalize writes them). lam = 1 - diversity and mu = 1 - lam come from the host.
+ * sim(a, b) = fp32 rows of items a and b, fp64 accumulate, rounded once to fp32; m_j = max sim(c_j, s) over the items
+ * s picked so far (0 before the first). Step t picks the unpicked position j with c_j >= 0 and the largest
+ * obj_j = lam * r_j - mu * m_j (fp64: two correctly rounded products, one subtraction, no FMA); ties go to the smaller
+ * j. out_idx int32 / out_score fp32 [U, k]: picked ids in pick order and their relevances (NOT sorted by score when
+ * mu > 0), -1 / -inf where fewer than k candidates are admissible. Bit-identical from run to run.
+ *   tt_mmr_select : rows from source TT_MMR_ROWS_TABLE (rows = this shard's fp32 table; id's row at id - item_base,
+ *                   ids outside [item_base, item_base + num_rows) count as inadmissible) or TT_MMR_ROWS_GATHERED
+ *                   (rows = fp32 [U, P, 256], row of pool position j of user u at (u * P + j) * 256; item_base and
+ *                   num_rows unused). 1 <= k <= P <= 256, lam and mu in [0, 1]; U = 0 launches nothing (its
+ *                   pointers may be NULL). k = 1 reads no row.
+ *   tt_mmr_gather_rows : sharded catalogs: out fp32 [n, 256] row r = the table row of pool_idx[r] when this shard owns
+ *                   it (item_base <= id < item_base + num_rows), zeros otherwise. The sum of every shard's buffer is
+ *                   the TT_MMR_ROWS_GATHERED input, exactly (one non-zero contributor per element). */
+#define TT_MMR_ROWS_TABLE 0
+#define TT_MMR_ROWS_GATHERED 1
+int tt_mmr_select(const int32_t* pool_idx, const float* pool_score, int U, int P, int k, double lam, double mu,
+                  int source, const float* rows, int item_base, int num_rows, int32_t* out_idx, float* out_score,
+                  void* stream);
+int tt_mmr_gather_rows(const int32_t* pool_idx, int n, const float* table, int item_base, int num_rows, float* out,
+                       void* stream);
+
 /* ---- ID table row-sharded over the ranks of one NVLink domain ----------
  * (BASELINE.json configs[4]: 10M items; reference: nn.Embedding(vocab_size, 256, padding_idx=0) and its dense
  * gradient, src/models/user_tower.py:26,86.) The table and its gradient live in a symmetric arena (tt_symm_team

@@ -180,6 +180,9 @@ _SIGNATURES = {
                            c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p],
     "tt_exact_topk_excl": [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
                            c_void_p, c_void_p, c_void_p],
+    "tt_mmr_select": [c_void_p, c_void_p, c_int32, c_int32, c_int32, ctypes.c_double, ctypes.c_double, c_int32,
+                      c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p],
+    "tt_mmr_gather_rows": [c_void_p, c_int32, c_void_p, c_int32, c_int32, c_void_p, c_void_p],
     "tt_rank_metrics": [c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_int32, c_void_p, c_void_p, c_void_p,
                         c_void_p],
     "tt_cast_bf16": [c_void_p, c_void_p, _I64, c_void_p],

@@ -82,7 +82,8 @@ _TOWER_TOKENS = 1 << 19
 def recommend_batch(model, index: retrieval.CatalogIndex, history_ids: torch.Tensor,
                     history_mask: Optional[torch.Tensor] = None, user_gender: Optional[torch.Tensor] = None,
                     user_country: Optional[torch.Tensor] = None, k: int = 10, exclude_ids: Optional[torch.Tensor] = None,
-                    group=None) -> Tuple[torch.Tensor, torch.Tensor]:
+                    group=None, diversity: float = 0.0,
+                    pool: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """`recommend_for_user` (src/inference.py:283-306) for a batch of B users.
 
     ``history_ids`` (B, L) int64, L <= the model's max_seq_len, right-padded with 0; ``history_mask`` (B, L), default
@@ -94,9 +95,13 @@ def recommend_batch(model, index: retrieval.CatalogIndex, history_ids: torch.Ten
     (collective: every rank passes its copy of the same users).
 
     Returns (item ids int64 (B, k), scores fp32 (B, k)), best first in the canonical order (score descending, item id
-    ascending). When a user has fewer than k admissible items, the tail is id -1 with score -inf."""
+    ascending). When a user has fewer than k admissible items, the tail is id -1 with score -inf.
+
+    ``diversity`` > 0 diversifies each list (`recommend_embeddings`); the result is then in pick order, not sorted by
+    score."""
     if not 1 <= k <= 256:
         raise ValueError(f"recommend_batch: k = {k} outside [1, 256]")
+    pool = check_diversity_args(k, diversity, pool)
     dev = model.engine.device
     ids = history_ids.to(dev).long()
     B, L = ids.shape
@@ -113,20 +118,39 @@ def recommend_batch(model, index: retrieval.CatalogIndex, history_ids: torch.Ten
                                                 country[s:s + chunk]) for s in range(0, B, chunk)])
     model.train(was_training)
     ex = ids * (mask != 0) if exclude_ids is None else exclude_ids.to(dev).long()
-    return recommend_embeddings(u, index, ex, k, group)
+    return recommend_embeddings(u, index, ex, k, group, diversity, pool)
+
+
+def check_diversity_args(k: int, diversity: float, pool: Optional[int]) -> int:
+    """Validate ``diversity`` (in [0, 1]) and ``pool`` (k <= pool <= 256, default min(256, 10 k)); returns the pool."""
+    retrieval.check_diversity(diversity)
+    pool = min(256, 10 * k) if pool is None else int(pool)
+    if not k <= pool <= 256:
+        raise ValueError(f"pool = {pool} outside [k = {k}, 256]")
+    return pool
 
 
 def recommend_embeddings(u: torch.Tensor, index: retrieval.CatalogIndex, ex: torch.Tensor, k: int,
-                         group=None) -> Tuple[torch.Tensor, torch.Tensor]:
+                         group=None, diversity: float = 0.0,
+                         pool: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """The selection of `recommend_batch` for given user embeddings ``u`` (B, 256): re-normalise (eps 1e-8), then the
-    top k over plain or sharded ``index`` with item 0 and the ids of ``ex`` (B, m) int64 (0 = empty) excluded."""
+    top k over plain or sharded ``index`` with item 0 and the ids of ``ex`` (B, m) int64 (0 = empty) excluded.
+
+    ``diversity`` in [0, 1]: 0 (default) is the plain top k. Above 0 the exact top ``pool`` admissible items (default
+    min(256, 10 k), k <= pool <= 256) are taken instead and k of them picked by maximal marginal relevance
+    (`retrieval.diversify`): near-duplicates of an item already picked (e.g. other versions of one song) give way to
+    less similar items. The result is then in pick order, not sorted by score."""
+    pool = check_diversity_args(k, diversity, pool)
     B = u.shape[0]
     u = F.normalize(u.float(), p=2, dim=1, eps=1e-8)                     # src/inference.py:286
     if ex.shape[0] != B:
         raise ValueError(f"exclude_ids has {ex.shape[0]} rows for {B} users")
     exclude = retrieval.Exclusions(ex, index.vocab_size)
+    n = k if diversity == 0 else pool
     if index.is_sharded:
-        idx, score = retrieval.sharded_topk(u, index, k, group=group, exclude=exclude)
+        idx, score = retrieval.sharded_topk(u, index, n, group=group, exclude=exclude)
     else:
-        idx, score, _ = retrieval.retrieve_topk(u, index, k, exclude=exclude)
+        idx, score, _ = retrieval.retrieve_topk(u, index, n, exclude=exclude)
+    if diversity != 0:
+        idx, score = retrieval.diversify(idx, score, index, k, diversity, group)
     return idx.long(), score

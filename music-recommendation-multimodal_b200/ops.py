@@ -172,6 +172,40 @@ def session_attn(qkv, k_cache, v_cache, slots, pos, ctx) -> None:
                                 pos.data_ptr(), n, H, L, cap, ctx.data_ptr(), _stream()), "tt_session_attn")
 
 
+#: row sources of tt_mmr_select (include/tt_b200.h)
+MMR_ROWS_TABLE, MMR_ROWS_GATHERED = 0, 1
+
+
+def mmr_select(pool_idx, pool_score, k: int, lam: float, mu: float, source: int, rows, item_base: int = 0,
+               num_rows: int = 0):
+    """tt_mmr_select: k maximal-marginal-relevance picks per user from its pool (int32 / fp32 [U, P], canonical order).
+    ``rows``: the shard's fp32 table [num_rows, 256] (MMR_ROWS_TABLE) or the gathered pool rows [U, P, 256]
+    (MMR_ROWS_GATHERED). Returns (ids int32 [U, k], relevances fp32 [U, k]) in pick order."""
+    _require_cuda(pool_idx, pool_score, rows)
+    U, P = pool_idx.shape
+    assert pool_idx.dtype == torch.int32 and pool_score.dtype == torch.float32 and pool_score.shape == (U, P)
+    assert pool_idx.is_contiguous() and pool_score.is_contiguous()
+    assert rows.dtype == torch.float32 and rows.is_contiguous() and rows.shape[-1] == 256
+    out_idx = torch.empty(U, k, device=pool_idx.device, dtype=torch.int32)
+    out_score = torch.empty(U, k, device=pool_idx.device, dtype=torch.float32)
+    check(lib().tt_mmr_select(pool_idx.data_ptr(), pool_score.data_ptr(), U, P, k, lam, mu, source, rows.data_ptr(),
+                              item_base, num_rows, out_idx.data_ptr(), out_score.data_ptr(), _stream()),
+          "tt_mmr_select")
+    return out_idx, out_score
+
+
+def mmr_gather_rows(pool_idx, table, item_base: int, out) -> None:
+    """tt_mmr_gather_rows: out [.., 256] row r = table row of pool_idx.flatten()[r] when this shard (rows
+    [item_base, item_base + len(table))) owns it, zeros otherwise."""
+    _require_cuda(pool_idx, table, out)
+    n = pool_idx.numel()
+    assert pool_idx.dtype == torch.int32 and pool_idx.is_contiguous()
+    assert table.dtype == torch.float32 and table.is_contiguous() and table.shape[1] == 256
+    assert out.dtype == torch.float32 and out.is_contiguous() and out.numel() == n * 256
+    check(lib().tt_mmr_gather_rows(pool_idx.data_ptr(), n, table.data_ptr(), item_base, table.shape[0], out.data_ptr(),
+                                   _stream()), "tt_mmr_gather_rows")
+
+
 def embed_ln_bwd(ids, E, P, ln_w, ln_b, dx0, B, L, dE, dP, dgamma, dbeta, drop_p=0.0, seed=0, seed_dev=None, site=0):
     _require_cuda(ids, E, P, dx0, dE, dP, dgamma, dbeta)
     check(lib().tt_embed_ln_bwd(ids.data_ptr(), E.data_ptr(), P.data_ptr(), ln_w.data_ptr(), ln_b.data_ptr(),

@@ -431,6 +431,55 @@ def merge_topk(scores: torch.Tensor, idx: torch.Tensor):
     return out_i, out_s
 
 
+#: bytes of gathered pool rows per `diversify` chunk on a sharded index
+_DIVERSIFY_CHUNK_BYTES = 256 << 20
+
+
+def check_diversity(diversity: float) -> None:
+    if not 0.0 <= diversity <= 1.0:            # also rejects NaN
+        raise ValueError(f"diversity = {diversity} outside [0, 1]")
+
+
+def diversify(idx: torch.Tensor, score: torch.Tensor, index: CatalogIndex, k: int, diversity: float, group=None):
+    """k maximal-marginal-relevance picks from each user's candidate pool: ``idx`` / ``score`` (U, P), P <= 256, the
+    exact top P of `retrieve_topk` / `sharded_topk` in canonical order (-1 / -inf tail).
+
+    With lambda = 1 - diversity and mu = 1 - lambda, each step picks the unpicked candidate with the largest
+    lambda * score - mu * (its largest similarity to the items picked so far), ties to the earlier pool position;
+    similarity is the dot product of the index's fp32 rows (fp64 accumulate, rounded to fp32). diversity = 0 returns
+    the pool's first k; diversity = 1 starts with the best item and then takes the one least similar to the picks.
+
+    Returns (idx int32 (U, k), score fp32 (U, k)): the picks in pick order with their exact scores — NOT sorted by
+    score when diversity > 0 — and -1 / -inf where fewer than k candidates are admissible. On a sharded index this is
+    collective over ``group`` (every rank brings the same users, as in `sharded_topk`): each rank writes the pool rows
+    it owns into a zeroed buffer, one all-reduce (sum) assembles them, and the result is bit-identical to the
+    single-GPU one."""
+    check_diversity(diversity)
+    U, P = idx.shape
+    if not 1 <= k <= P <= 256:
+        raise ValueError(f"diversify: need 1 <= k = {k} <= pool = {P} <= 256")
+    lam = 1.0 - float(diversity)
+    mu = 1.0 - lam
+    idx = idx.to(torch.int32).contiguous()
+    score = score.contiguous()
+    if not index.is_sharded:
+        return ops.mmr_select(idx, score, k, lam, mu, ops.MMR_ROWS_TABLE, index.table, index.item_base,
+                              index.num_rows)
+    import torch.distributed as dist
+    chunk = max(1, _DIVERSIFY_CHUNK_BYTES // (P * 1024))
+    rows = torch.empty(min(U, chunk), P, 256, device=idx.device, dtype=torch.float32)
+    out_i = torch.empty(U, k, device=idx.device, dtype=torch.int32)
+    out_s = torch.empty(U, k, device=idx.device, dtype=torch.float32)
+    for s0 in range(0, U, chunk):
+        n = min(chunk, U - s0)
+        buf = rows[:n]
+        ops.mmr_gather_rows(idx[s0:s0 + n], index.table, index.item_base, buf)
+        dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)     # one non-zero contributor per element: exact
+        out_i[s0:s0 + n], out_s[s0:s0 + n] = ops.mmr_select(idx[s0:s0 + n], score[s0:s0 + n], k, lam, mu,
+                                                            ops.MMR_ROWS_GATHERED, buf)
+    return out_i, out_s
+
+
 def gain_table(K: int) -> torch.Tensor:
     """1/log2(rank+2) exactly as the reference computes it (fp32 torch ops, evaluate_metrics.py:180)."""
     return 1.0 / torch.log2(torch.arange(K).float() + 2.0)

@@ -204,10 +204,12 @@ class UserSessions:
         return out
 
     def recommend(self, slots: IntsLike, index: retrieval.CatalogIndex, k: int = 10,
-                  exclude_ids: Optional[torch.Tensor] = None, group=None) -> Tuple[torch.Tensor, torch.Tensor]:
+                  exclude_ids: Optional[torch.Tensor] = None, group=None, diversity: float = 0.0,
+                  pool: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor]:
         """`inference.recommend_batch`'s selection on the sessions' current embeddings: top k of plain or sharded
         ``index``, excluding ``exclude_ids`` (n, m) int64 or, by default, each slot's window ids. Returns (item ids int64
-        (n, k), scores fp32 (n, k)); id -1 / score -inf where fewer than k items are admissible."""
+        (n, k), scores fp32 (n, k)); id -1 / score -inf where fewer than k items are admissible. ``diversity`` /
+        ``pool``: as in `inference.recommend_embeddings` (diversity > 0: pick order, not sorted by score)."""
         if not 1 <= k <= 256:
             raise ValueError(f"recommend: k = {k} outside [1, 256]")
         s = self._slots(slots)
@@ -216,7 +218,7 @@ class UserSessions:
         self._check_fresh(s)
         sl = self._ids_of(s)
         ex = self.window[sl] if exclude_ids is None else exclude_ids.to(self.engine.device).long()
-        return inference.recommend_embeddings(self.emb[sl], index, ex, k, group)
+        return inference.recommend_embeddings(self.emb[sl], index, ex, k, group, diversity, pool)
 
     def reset(self, slots: IntsLike) -> None:
         """Empty the slots: the next `append` starts a history at position 0 (gender / country 0)."""
