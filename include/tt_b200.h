@@ -316,6 +316,30 @@ int tt_inbatch_recall(const float* S, int R, int C, int ld, int pos0, int k, flo
 int tt_infonce_loss(const float* lse_a, const float* pos_a, const float* lse_b, const float* pos_b, int R, float coef,
                     float* loss, void* stream);
 
+/* ---- logQ correction of in-batch negatives (Yi et al., RecSys 2019) --------------------
+ * The positives of a batch are its negatives, so column j is sampled with its entity's popularity q_j; the
+ * corrected loss subtracts log q_j from every logit of column j. col_off[j] = log q of column j's entity (C values),
+ * row_off[p] = log q of the OTHER side's entity at global row p (indexed pos0 + i).
+ * tt_infonce_rows_off : tt_infonce_rows over x_ij - col_off[j]; masked entries are -1e4 BEFORE the offset, S keeps the
+ *                       uncorrected masked logits; pos_logit[i] = S[i][pos0+i] - col_off[pos0+i].
+ * tt_infonce_grad_off : dS[i][j] = coef * (exp(S-col_off[j]-row_lse[i]) + exp(S-row_off[pos0+i]-col_lse[j])
+ *                       - 2*[j==pos0+i]). With zero offsets both equal the plain kernels bit for bit.
+ * tt_logq_table_gather : off_out[i] = table[ids[i]] for ids in [0, N), floor otherwise.
+ * tt_logq_stream_update : streaming frequency estimator, one CTA. A int64 [h, 2^log2H] (last step seen), Bv fp32
+ *                       [h, 2^log2H] (interval estimate); slot of id y in array k = low log2H bits of
+ *                       splitmix64_finaliser(y + (k+1) * 0x9E3779B97F4A7C15). t = ++*step_dev; every slot hit by the
+ *                       ids is updated once: Bv = fl(fl(one_minus_alpha * Bv) + fl(alpha * (float)(t - A))), A = t;
+ *                       then off_out[i] = -logf(max_k Bv_k[slot_k(ids[i])]). Deterministic, no host reads.
+ *                       1 <= h <= 4, 0 <= log2H <= 28, alpha in (0, 1], n >= 1. */
+int tt_infonce_rows_off(float* S, int R, int C, int ld, const int64_t* uid_rows, const int64_t* uid_cols, int pos0,
+                        const float* col_off, float* row_lse, float* pos_logit, void* stream);
+int tt_infonce_grad_off(const float* S, int R, int C, int ld, const float* row_lse, const float* col_lse, int pos0,
+                        float coef, const float* col_off, const float* row_off, void* dS_bf16, int ld_d, void* stream);
+int tt_logq_table_gather(const int64_t* ids, int n, const float* table, int64_t N, float floor, float* off_out,
+                         void* stream);
+int tt_logq_stream_update(const int64_t* ids, int n, int64_t* A, float* Bv, int h, int log2H, int64_t* step_dev,
+                          float alpha, float one_minus_alpha, float* off_out, void* stream);
+
 /* ---- catalog retrieval (src/evaluate_metrics.py:106-192) ------------------------------
  * Canonical order everywhere: score descending, then item index ascending (torch.topk leaves
  * ties unspecified). Keys are 64-bit: (order-preserving score bits << 32) | (2^32-1 - index).

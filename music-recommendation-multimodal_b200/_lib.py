@@ -214,6 +214,13 @@ _SIGNATURES = {
     "tt_infonce_grad": [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_int32, c_float, c_void_p,
                         c_int32, c_void_p],
     "tt_infonce_loss": [c_void_p] * 4 + [c_int32, c_float, c_void_p, c_void_p],
+    "tt_infonce_rows_off": [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_int32, c_void_p, c_void_p,
+                            c_void_p, c_void_p],
+    "tt_infonce_grad_off": [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_int32, c_float, c_void_p,
+                            c_void_p, c_void_p, c_int32, c_void_p],
+    "tt_logq_table_gather": [c_void_p, c_int32, c_void_p, _I64, c_float, c_void_p, c_void_p],
+    "tt_logq_stream_update": [c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_float, c_float,
+                              c_void_p, c_void_p],
     "tt_inbatch_recall": [c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p],
     "tt_index_rows": [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, _I64, c_void_p, c_void_p, c_void_p],
 }

@@ -14,10 +14,15 @@
 
 namespace tt {
 
+// kOffset: every logit of column j enters the row's log-sum-exp and positive as x - col_off[j] (logQ correction of
+// sampled negatives, tt_infonce_rows_off); masked entries are -1e4 before the offset. The offsets come last in the
+// parameter list so that the kOffset = false instantiation keeps the parameter layout (and code) of the plain kernel.
+template <bool kOffset>
 __global__ void __launch_bounds__(256) infonce_rows_kernel(float* __restrict__ S, int R, int C, int ld,
                                                            const int64_t* __restrict__ uid_rows,
                                                            const int64_t* __restrict__ uid_cols, int pos0,
-                                                           float* __restrict__ row_lse, float* __restrict__ pos_logit) {
+                                                           float* __restrict__ row_lse, float* __restrict__ pos_logit,
+                                                           const float* __restrict__ col_off) {
   pdl_launch_dependents();
   pdl_wait();
   const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
@@ -33,6 +38,7 @@ __global__ void __launch_bounds__(256) infonce_rows_kernel(float* __restrict__ S
       x = -1e4f;  // the reference's fill value (fp16-safe), two_tower.py:124
       s[j] = x;
     }
+    if (kOffset) x -= col_off[j];
     const float nm = fmaxf(m, x);
     l = l * __expf(m - nm) + __expf(x - nm);
     m = nm;
@@ -50,20 +56,26 @@ __global__ void __launch_bounds__(256) infonce_rows_kernel(float* __restrict__ S
   }
   if (lane == 0) {
     row_lse[row] = m + __logf(l);
-    pos_logit[row] = s[pos];
+    pos_logit[row] = kOffset ? s[pos] - col_off[pos] : s[pos];
   }
 }
 
+// kOffset: dS = coef * (exp(S - col_off[j] - row_lse[i]) + exp(S - row_off[pos0 + i] - col_lse[j]) - 2*onehot): the
+// row direction subtracts its columns' offsets, the column direction the offset of this row's own entity.
+template <bool kOffset>
 __global__ void __launch_bounds__(256) infonce_grad_kernel(const float* __restrict__ S, int R, int C, int ld,
                                                            const float* __restrict__ row_lse,
                                                            const float* __restrict__ col_lse, int pos0, float coef,
-                                                           __nv_bfloat16* __restrict__ dS, int ld_d) {
+                                                           __nv_bfloat16* __restrict__ dS, int ld_d,
+                                                           const float* __restrict__ col_off,
+                                                           const float* __restrict__ row_off) {
   pdl_launch_dependents();
   pdl_wait();
   const int row = blockIdx.y;
   const int j = (blockIdx.x * blockDim.x + threadIdx.x) * 2;
   if (j >= C) return;
   const float lr = row_lse[row];
+  const float ro = kOffset ? row_off[pos0 + row] : 0.f;
   const float* s = S + static_cast<size_t>(row) * ld;
   float g[2];
 #pragma unroll
@@ -72,7 +84,11 @@ __global__ void __launch_bounds__(256) infonce_grad_kernel(const float* __restri
     float v = 0.f;
     if (c < C) {
       const float x = s[c];
-      v = __expf(x - lr) + __expf(x - col_lse[c]);
+      if (kOffset) {
+        v = __expf(x - col_off[c] - lr) + __expf(x - ro - col_lse[c]);
+      } else {
+        v = __expf(x - lr) + __expf(x - col_lse[c]);
+      }
       if (c == pos0 + row) v -= 2.f;
       v *= coef;
     }
@@ -155,9 +171,26 @@ extern "C" int tt_infonce_rows(float* S, int R, int C, int ld, const int64_t* ui
   TT_REQUIRE(S && row_lse && pos_logit && R > 0 && C > 0 && ld >= C, "tt_infonce_rows: bad arguments");
   TT_REQUIRE((uid_rows == nullptr) == (uid_cols == nullptr), "tt_infonce_rows: uid_rows/uid_cols come together");
   TT_REQUIRE(pos0 >= 0 && pos0 + R <= C, "tt_infonce_rows: positives [%d, %d) outside %d columns", pos0, pos0 + R, C);
-  TT_CHECK_CUDA(launch_k(infonce_rows_kernel, dim3((R * 32 + 255) / 256), dim3(256), 0, stream, S, R, C, ld, uid_rows, uid_cols, pos0, row_lse, pos_logit));
+  TT_CHECK_CUDA(launch_k(infonce_rows_kernel<false>, dim3((R * 32 + 255) / 256), dim3(256), 0, stream, S, R, C, ld, uid_rows, uid_cols, pos0, row_lse, pos_logit, nullptr));
   TT_LAUNCH_CHECK();
   return TT_OK;
+}
+
+extern "C" int tt_infonce_rows_off(float* S, int R, int C, int ld, const int64_t* uid_rows, const int64_t* uid_cols,
+                                   int pos0, const float* col_off, float* row_lse, float* pos_logit, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  TT_REQUIRE(S && col_off && row_lse && pos_logit && R > 0 && C > 0 && ld >= C, "tt_infonce_rows_off: bad arguments");
+  TT_REQUIRE((uid_rows == nullptr) == (uid_cols == nullptr), "tt_infonce_rows_off: uid_rows/uid_cols come together");
+  TT_REQUIRE(pos0 >= 0 && pos0 + R <= C, "tt_infonce_rows_off: positives [%d, %d) outside %d columns", pos0, pos0 + R, C);
+  TT_CHECK_CUDA(launch_k(infonce_rows_kernel<true>, dim3((R * 32 + 255) / 256), dim3(256), 0, stream, S, R, C, ld, uid_rows, uid_cols, pos0, row_lse, pos_logit, col_off));
+  TT_LAUNCH_CHECK();
+  return TT_OK;
+}
+
+static dim3 infonce_grad_grid(int R, int C) {
+  dim3 grid((C / 2 + 255) / 256 + ((C / 2) % 256 == 0 && C % 2 ? 1 : 0), R);
+  if (grid.x == 0) grid.x = 1;
+  return grid;
 }
 
 extern "C" int tt_infonce_grad(const float* S, int R, int C, int ld, const float* row_lse, const float* col_lse,
@@ -165,9 +198,20 @@ extern "C" int tt_infonce_grad(const float* S, int R, int C, int ld, const float
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   TT_REQUIRE(S && row_lse && col_lse && dS_bf16 && R > 0 && C > 0, "tt_infonce_grad: bad arguments");
   TT_REQUIRE(ld_d % 2 == 0, "tt_infonce_grad: ld_d must be even");
-  dim3 grid((C / 2 + 255) / 256 + ((C / 2) % 256 == 0 && C % 2 ? 1 : 0), R);
-  if (grid.x == 0) grid.x = 1;
-  TT_CHECK_CUDA(launch_k(infonce_grad_kernel, dim3(grid), dim3(256), 0, stream, S, R, C, ld, row_lse, col_lse, pos0, coef, static_cast<__nv_bfloat16*>(dS_bf16), ld_d));
+  TT_CHECK_CUDA(launch_k(infonce_grad_kernel<false>, infonce_grad_grid(R, C), dim3(256), 0, stream, S, R, C, ld, row_lse, col_lse, pos0, coef, static_cast<__nv_bfloat16*>(dS_bf16), ld_d, nullptr, nullptr));
+  TT_LAUNCH_CHECK();
+  return TT_OK;
+}
+
+extern "C" int tt_infonce_grad_off(const float* S, int R, int C, int ld, const float* row_lse, const float* col_lse,
+                                   int pos0, float coef, const float* col_off, const float* row_off, void* dS_bf16,
+                                   int ld_d, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  TT_REQUIRE(S && row_lse && col_lse && col_off && row_off && dS_bf16 && R > 0 && C > 0 && ld >= C,
+             "tt_infonce_grad_off: bad arguments");
+  TT_REQUIRE(ld_d % 2 == 0 && ld_d >= C, "tt_infonce_grad_off: ld_d must be even and at least C");
+  TT_REQUIRE(pos0 >= 0 && pos0 + R <= C, "tt_infonce_grad_off: positives [%d, %d) outside %d columns", pos0, pos0 + R, C);
+  TT_CHECK_CUDA(launch_k(infonce_grad_kernel<true>, infonce_grad_grid(R, C), dim3(256), 0, stream, S, R, C, ld, row_lse, col_lse, pos0, coef, static_cast<__nv_bfloat16*>(dS_bf16), ld_d, col_off, row_off));
   TT_LAUNCH_CHECK();
   return TT_OK;
 }

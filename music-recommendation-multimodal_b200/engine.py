@@ -689,13 +689,17 @@ class TwoTowerEngine:
         return ws[key]
 
     def loss_forward(self, ws, user_idx: Optional[torch.Tensor], gathered: Optional[Dict[str, torch.Tensor]] = None,
-                     rank: int = 0) -> torch.Tensor:
+                     rank: int = 0, offsets: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> torch.Tensor:
         """Logits + masked row log-sum-exps (+ the local loss when not gathered). With `gathered`
         (U_all, I_all, uid_all filled by the caller's all-gather) the caller must all-gather
-        ws['lse_r'] / ws['lse_c'] into gathered['lse_r_all' / 'lse_c_all'] and then call loss_value()."""
+        ws['lse_r'] / ws['lse_c'] into gathered['lse_r_all' / 'lse_c_all'] and then call loss_value().
+        ``offsets`` = (oi, ou), fp32 over the (global) batch rows: log q of each row's item / user (logQ correction,
+        train.LogQCorrection). The row log-sum-exps, positives and backward() then use x_ij - oi[j] (user rows) and
+        x_ij - ou[j] (item rows); the logits in ws / gathered stay the uncorrected masked ones."""
         B = ws["un"].shape[0]
         inv_t = 1.0 / self.cfg.temperature
         self._gathered = None if gathered is None else (gathered, rank)
+        self._offsets = offsets
         if gathered is None:
             S, S2, U_all, I_all, uid_all, pos0 = ws["S"], ws["S2"], ws["un_bf"], ws["in_bf"], user_idx, 0
         else:
@@ -703,8 +707,12 @@ class TwoTowerEngine:
             uid_all = gathered["uid_all"] if user_idx is not None else None
         self._gemm(ws["un_bf"], I_all, alpha=inv_t, out_f32=S)
         self._gemm(ws["in_bf"], U_all, alpha=inv_t, out_f32=S2)
-        ops.infonce_rows(S, user_idx, uid_all, pos0, ws["lse_r"], ws["pos_r"])
-        ops.infonce_rows(S2, user_idx, uid_all, pos0, ws["lse_c"], ws["pos_c"])
+        if offsets is None:
+            ops.infonce_rows(S, user_idx, uid_all, pos0, ws["lse_r"], ws["pos_r"])
+            ops.infonce_rows(S2, user_idx, uid_all, pos0, ws["lse_c"], ws["pos_c"])
+        else:
+            ops.infonce_rows_off(S, user_idx, uid_all, pos0, offsets[0], ws["lse_r"], ws["pos_r"])
+            ops.infonce_rows_off(S2, user_idx, uid_all, pos0, offsets[1], ws["lse_c"], ws["pos_c"])
         if gathered is None:
             self.loss_value(ws, B)
         return ws["loss"]
@@ -735,6 +743,7 @@ class TwoTowerEngine:
         main.wait_stream(side)
         self._last = (ws, batch, training)
         self._gathered = None
+        self._offsets = None
         return ws
 
     def forward(self, batch: Dict[str, torch.Tensor], training: bool = True):
@@ -777,17 +786,27 @@ class TwoTowerEngine:
 
         # ---- InfoNCE -> d(normalised embeddings)
         gath = getattr(self, "_gathered", None)
+        off = getattr(self, "_offsets", None)
         if gath is None:
             coef = 0.5 / B * loss_scale
-            ops.infonce_grad(ws["S"], ws["lse_r"], ws["lse_c"], 0, coef, ws["dS"])
-            ops.infonce_grad(ws["S2"], ws["lse_c"], ws["lse_r"], 0, coef, ws["dS2"])
+            if off is None:
+                ops.infonce_grad(ws["S"], ws["lse_r"], ws["lse_c"], 0, coef, ws["dS"])
+                ops.infonce_grad(ws["S2"], ws["lse_c"], ws["lse_r"], 0, coef, ws["dS2"])
+            else:
+                ops.infonce_grad_off(ws["S"], ws["lse_r"], ws["lse_c"], 0, coef, off[0], off[1], ws["dS"])
+                ops.infonce_grad_off(ws["S2"], ws["lse_c"], ws["lse_r"], 0, coef, off[1], off[0], ws["dS2"])
             gemm(ws["dS"], ws["in_bf"], b_mn=True, alpha=inv_t, out_f32=ws["dun"])
             gemm(ws["dS2"], ws["un_bf"], b_mn=True, alpha=inv_t, out_f32=ws["din"])
         else:
             g_, rank = gath
             coef = 0.5 / B * loss_scale     # per-rank normalisation; the gradient all-reduce AVERAGES
-            ops.infonce_grad(g_["S"], ws["lse_r"], g_["lse_c_all"], rank * B, coef, g_["dS"])
-            ops.infonce_grad(g_["S2"], ws["lse_c"], g_["lse_r_all"], rank * B, coef, g_["dS2"])
+            if off is None:
+                ops.infonce_grad(g_["S"], ws["lse_r"], g_["lse_c_all"], rank * B, coef, g_["dS"])
+                ops.infonce_grad(g_["S2"], ws["lse_c"], g_["lse_r_all"], rank * B, coef, g_["dS2"])
+            else:
+                ops.infonce_grad_off(g_["S"], ws["lse_r"], g_["lse_c_all"], rank * B, coef, off[0], off[1], g_["dS"])
+                ops.infonce_grad_off(g_["S2"], ws["lse_c"], g_["lse_r_all"], rank * B, coef, off[1], off[0],
+                                     g_["dS2"])
             gemm(g_["dS"], g_["I_all"], b_mn=True, alpha=inv_t, out_f32=ws["dun"])
             gemm(g_["dS2"], g_["U_all"], b_mn=True, alpha=inv_t, out_f32=ws["din"])
 

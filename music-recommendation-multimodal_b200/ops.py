@@ -379,6 +379,55 @@ def infonce_grad(S, row_lse, col_lse, pos0, coef, dS) -> None:
           "tt_infonce_grad")
 
 
+def _offsets(off, n: int, what: str) -> None:
+    if off.dtype != torch.float32 or not off.is_contiguous() or off.numel() != n:
+        raise ValueError(f"{what}: offsets must be contiguous fp32 with {n} values, got {off.dtype} {tuple(off.shape)}")
+
+
+def infonce_rows_off(S, uid_rows, uid_cols, pos0, col_off, row_lse, pos_logit) -> None:
+    """tt_infonce_rows over S[i, j] - col_off[j] (logQ correction); S keeps the uncorrected masked logits."""
+    _require_cuda(S, uid_rows, uid_cols, col_off, row_lse, pos_logit)
+    assert S.dtype == torch.float32 and S.stride(1) == 1
+    _offsets(col_off, S.shape[1], "infonce_rows_off")
+    check(lib().tt_infonce_rows_off(S.data_ptr(), S.shape[0], S.shape[1], S.stride(0), _ptr(uid_rows), _ptr(uid_cols),
+                                    pos0, col_off.data_ptr(), row_lse.data_ptr(), pos_logit.data_ptr(), _stream()),
+          "tt_infonce_rows_off")
+
+
+def infonce_grad_off(S, row_lse, col_lse, pos0, coef, col_off, row_off, dS) -> None:
+    """tt_infonce_grad with the logQ offsets of the columns (col_off) and of the other side's rows (row_off)."""
+    _require_cuda(S, row_lse, col_lse, col_off, row_off, dS)
+    assert dS.dtype == torch.bfloat16 and dS.stride(1) == 1
+    _offsets(col_off, S.shape[1], "infonce_grad_off")
+    _offsets(row_off, S.shape[1], "infonce_grad_off")
+    check(lib().tt_infonce_grad_off(S.data_ptr(), S.shape[0], S.shape[1], S.stride(0), row_lse.data_ptr(),
+                                    col_lse.data_ptr(), pos0, coef, col_off.data_ptr(), row_off.data_ptr(),
+                                    dS.data_ptr(), dS.stride(0), _stream()), "tt_infonce_grad_off")
+
+
+def logq_table_gather(ids, table, floor: float, out) -> None:
+    """out[i] = table[ids[i]] for ids in [0, len(table)), ``floor`` otherwise (tt_logq_table_gather)."""
+    _require_cuda(ids, table, out)
+    assert ids.dtype == torch.int64 and ids.is_contiguous() and table.dtype == torch.float32 and table.is_contiguous()
+    _offsets(out, ids.numel(), "logq_table_gather")
+    check(lib().tt_logq_table_gather(ids.data_ptr(), ids.numel(), table.data_ptr(), table.numel(), floor,
+                                     out.data_ptr(), _stream()), "tt_logq_table_gather")
+
+
+def logq_stream_update(ids, A, Bv, step_dev, alpha: float, one_minus_alpha: float, out) -> None:
+    """One step of the streaming frequency estimator (tt_logq_stream_update): A int64 / Bv fp32 [h, 2^b], step_dev
+    int64 [1]; out[i] = log q of ids[i] after the update."""
+    _require_cuda(ids, A, Bv, step_dev, out)
+    h, H = A.shape
+    assert ids.dtype == torch.int64 and ids.is_contiguous() and A.dtype == torch.int64 and A.is_contiguous()
+    assert Bv.dtype == torch.float32 and Bv.is_contiguous() and Bv.shape == A.shape and H & (H - 1) == 0
+    assert step_dev.dtype == torch.int64
+    _offsets(out, ids.numel(), "logq_stream_update")
+    check(lib().tt_logq_stream_update(ids.data_ptr(), ids.numel(), A.data_ptr(), Bv.data_ptr(), h, H.bit_length() - 1,
+                                      step_dev.data_ptr(), alpha, one_minus_alpha, out.data_ptr(), _stream()),
+          "tt_logq_stream_update")
+
+
 def infonce_loss(lse_a, pos_a, lse_b, pos_b, coef, loss) -> None:
     _require_cuda(lse_a, pos_a, lse_b, pos_b, loss)
     check(lib().tt_infonce_loss(lse_a.data_ptr(), pos_a.data_ptr(), lse_b.data_ptr(), pos_b.data_ptr(),

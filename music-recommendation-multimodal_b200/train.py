@@ -12,9 +12,11 @@ autograd node is used (reference-compatible, slower). bf16 needs no GradScaler.
 from __future__ import annotations
 
 import logging
+import math
 import os
 from typing import Dict, Optional
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -25,6 +27,151 @@ logger = logging.getLogger(__name__)
 
 _BATCH_KEYS = ("history_ids", "history_mask", "user_gender", "user_country", "user_idx", "target_audio",
                "target_image", "target_input_ids", "target_tabular")
+
+
+class LogQCorrection:
+    """logQ correction of in-batch negatives (Yi et al., RecSys 2019) for ONE side of the symmetric InfoNCE.
+
+    Every negative of a batch is another row's positive, so an entity is drawn as a negative with its in-batch
+    sampling probability q, and the plain loss learns roughly log p(item | user) - log q(item): retrieval ends up
+    biased against what users play most. The correction subtracts log q_j from every logit of column j in the
+    training loss only (the logits `forward` returns, evaluation and serving are unchanged). One object per side:
+    ``TrainStepRunner(..., logq=<items>, logq_users=<users>)``; the item side reads each row's ``target_id``, the
+    user side its ``user_idx``.
+
+    Sources of log q (all produce the offsets on the device, inside the captured step):
+      * ``from_offsets(table)``: a fixed fp32 log q per id;
+      * ``from_counts(counts, smoothing=1.0)``: log((c + s) / sum(c + s)), computed in fp64 and stored as fp32;
+      * ``streaming(num_ids, ...)``: the paper's streaming frequency estimator over the training ids (no pass over
+        the dataset): h hash arrays of H slots hold the last step each slot was seen (A) and the estimated
+        interval between sightings (Bv); each step updates every slot its ids hit once, then log q = -log(max Bv).
+    Ids outside [0, N) of a table get the offset of the rarest id (a zero count with ``from_counts``).
+
+    The object owns its device state, allocated once: a captured step graph keeps pointing at it, so it survives
+    runner rebuilds (a trailing partial batch) and is restored in place by ``load_state_dict``. With data-parallel
+    gathered negatives every rank updates its replica from the same all-gathered ids (replicas stay bit-identical);
+    with negatives="local" each rank estimates from its own batch, which is what its softmax samples from."""
+
+    def __init__(self, kind: str, device=None):
+        self.kind = kind
+        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        self.table: Optional[torch.Tensor] = None
+        self.floor = 0.0
+        self.A: Optional[torch.Tensor] = None
+        self.Bv: Optional[torch.Tensor] = None
+        self.step: Optional[torch.Tensor] = None
+        self.alpha = self.num_ids = self.init_interval = None
+
+    @staticmethod
+    def _vector(x, what: str) -> torch.Tensor:
+        t = torch.as_tensor(x)
+        if t.dim() != 1 or t.numel() == 0:
+            raise ValueError(f"{what} must be a non-empty 1-D table indexed by id, got shape {tuple(t.shape)}")
+        if not (t.is_floating_point() or t.dtype in (torch.int32, torch.int64)):
+            raise ValueError(f"{what} must be numeric, got {t.dtype}")
+        t = t.detach().cpu().double()
+        if not torch.isfinite(t).all():
+            raise ValueError(f"{what} contains NaN or infinite values")
+        return t
+
+    @classmethod
+    def from_offsets(cls, table, device=None) -> "LogQCorrection":
+        """A fixed log q per id: ``table[id]`` (fp32)."""
+        t = cls._vector(table, "offsets").float()
+        self = cls("offsets", device)
+        self.table = t.to(self.device)
+        self.floor = float(t.min())
+        return self
+
+    @classmethod
+    def from_counts(cls, counts, smoothing: float = 1.0, device=None) -> "LogQCorrection":
+        """log q[id] = log((counts[id] + smoothing) / sum(counts + smoothing)), in fp64, stored as fp32."""
+        c = cls._vector(counts, "counts")
+        if (c < 0).any():
+            raise ValueError("counts must be >= 0")
+        if not (math.isfinite(smoothing) and smoothing > 0):
+            raise ValueError(f"smoothing must be a finite positive number, got {smoothing}")
+        total = float((c + smoothing).sum())
+        self = cls("offsets", device)
+        self.table = torch.log((c + smoothing) / total).float().to(self.device)
+        self.floor = float(np.float32(math.log(smoothing / total)))
+        return self
+
+    @classmethod
+    def streaming(cls, num_ids: int, num_slots: int = 2 ** 20, num_hashes: int = 2, alpha: float = 0.01,
+                  init_interval: Optional[float] = None, device=None) -> "LogQCorrection":
+        """The streaming estimator. ``init_interval``: the starting Bv of every slot; None takes
+        max(1, num_ids / global batch) (the interval of a uniformly sampled id) when a runner first binds it."""
+        if not (isinstance(num_ids, (int, np.integer)) and num_ids >= 1):
+            raise ValueError(f"num_ids must be a positive integer, got {num_ids!r}")
+        if not (isinstance(num_slots, (int, np.integer)) and 1 <= num_slots <= 2 ** 28
+                and num_slots & (num_slots - 1) == 0):
+            raise ValueError(f"num_slots must be a power of two in [1, 2^28], got {num_slots!r}")
+        if not (isinstance(num_hashes, (int, np.integer)) and 1 <= num_hashes <= 4):
+            raise ValueError(f"num_hashes must be in [1, 4], got {num_hashes!r}")
+        if not 0.0 < float(alpha) <= 1.0:                                     # also rejects NaN
+            raise ValueError(f"alpha must be in (0, 1], got {alpha!r}")
+        if init_interval is not None and not (math.isfinite(init_interval) and init_interval > 0):
+            raise ValueError(f"init_interval must be a finite positive number, got {init_interval!r}")
+        self = cls("streaming", device)
+        self.alpha, self.num_ids = float(alpha), int(num_ids)
+        self.A = torch.zeros(num_hashes, num_slots, dtype=torch.int64, device=self.device)
+        self.Bv = torch.empty(num_hashes, num_slots, dtype=torch.float32, device=self.device)
+        self.step = torch.zeros(1, dtype=torch.int64, device=self.device)
+        self.init_interval = None
+        if init_interval is not None:
+            self._init_state(float(init_interval))
+        return self
+
+    def _init_state(self, interval: float) -> None:
+        self.init_interval = interval
+        self.A.zero_()
+        self.Bv.fill_(interval)
+        self.step.zero_()
+
+    def bind(self, global_batch: int) -> None:
+        """Called by the runner before its first step: fixes the default initial interval of a streaming estimator
+        from the number of ids each step sees."""
+        if self.kind == "streaming" and self.init_interval is None:
+            self._init_state(max(1.0, self.num_ids / global_batch))
+
+    def offsets(self, ids: torch.Tensor, out: torch.Tensor) -> None:
+        """out[i] = log q of ids[i], on the current stream (one kernel; the streaming estimator also advances)."""
+        from . import ops
+        if self.kind == "offsets":
+            ops.logq_table_gather(ids, self.table, self.floor, out)
+        else:
+            if self.init_interval is None:
+                raise RuntimeError("streaming LogQCorrection used before bind(global_batch)")
+            ops.logq_stream_update(ids, self.A, self.Bv, self.step, self.alpha,
+                                   float(np.float32(1.0 - self.alpha)), out)
+
+    def state_dict(self) -> Dict[str, object]:
+        """Arrays, step counter and hyper-parameters (CPU copies); separate from the model's state_dict."""
+        if self.kind == "offsets":
+            return {"kind": self.kind, "table": self.table.cpu().clone(), "floor": self.floor}
+        return {"kind": self.kind, "A": self.A.cpu().clone(), "Bv": self.Bv.cpu().clone(),
+                "step": self.step.cpu().clone(), "alpha": self.alpha, "num_ids": self.num_ids,
+                "init_interval": self.init_interval}
+
+    def load_state_dict(self, sd: Dict[str, object]) -> None:
+        """Restores in place (a captured graph keeps its pointers); the shapes must be this object's."""
+        if sd.get("kind") != self.kind:
+            raise ValueError(f"state of a {sd.get('kind')!r} correction loaded into a {self.kind!r} one")
+        if self.kind == "offsets":
+            if tuple(sd["table"].shape) != tuple(self.table.shape):
+                raise ValueError(f"offset table of shape {tuple(sd['table'].shape)}, expected {tuple(self.table.shape)}")
+            self.table.copy_(sd["table"])
+            self.floor = float(sd["floor"])
+            return
+        for k in ("A", "Bv", "step"):
+            if tuple(sd[k].shape) != tuple(getattr(self, k).shape) or sd[k].dtype != getattr(self, k).dtype:
+                raise ValueError(f"estimator state {k} of shape {tuple(sd[k].shape)} / {sd[k].dtype}, expected "
+                                 f"{tuple(getattr(self, k).shape)} / {getattr(self, k).dtype}")
+        self.A.copy_(sd["A"])
+        self.Bv.copy_(sd["Bv"])
+        self.step.copy_(sd["step"])
+        self.alpha, self.num_ids, self.init_interval = float(sd["alpha"]), int(sd["num_ids"]), sd["init_interval"]
 
 
 class FusedAdamW:
@@ -83,14 +230,26 @@ class TrainStepRunner:
         form the exact gradient of the GLOBAL symmetric InfoNCE for its own rows;
       negatives="local": the reference's DDP semantics (per-rank in-batch negatives, src/train.py:300).
     In both cases BatchNorm statistics are per rank (the reference uses no SyncBatchNorm) and the flat
-    gradient buffer is averaged with ONE all-reduce between the backward and optimizer graphs."""
+    gradient buffer is averaged with ONE all-reduce between the backward and optimizer graphs.
+
+    ``logq`` / ``logq_users`` (LogQCorrection): logQ correction of the item / user negatives. The item side adds
+    ``target_id`` to the input buffer; the user side needs ``with_user_idx``. The offsets are computed inside the
+    step, from the global batch's ids when negatives are gathered."""
 
     def __init__(self, engine: TwoTowerEngine, B: int, L: int, world_size: int = 1, lr: float = 1e-4,
                  use_graph: bool = True, with_user_idx: bool = True, negatives: str = "gathered",
                  rank: Optional[int] = None, group=None, shard_optimizer: bool = True,
                  with_optimizer: bool = True, sharded_table=None, betas=(0.9, 0.999), eps: float = 1e-8,
-                 weight_decay: float = 0.01, comm: str = "auto"):
+                 weight_decay: float = 0.01, comm: str = "auto", logq: Optional[LogQCorrection] = None,
+                 logq_users: Optional[LogQCorrection] = None):
         self.eng, self.B, self.L, self.world, self.lr, self.use_graph = engine, B, L, world_size, lr, use_graph
+        if logq_users is not None and not with_user_idx:
+            raise ValueError("logq_users corrects the user negatives by user_idx: it needs with_user_idx=True")
+        for c in (logq, logq_users):
+            if c is not None and (not isinstance(c, LogQCorrection)
+                                  or c.device != torch.empty(0, device=engine.device).device):
+                raise ValueError(f"logq / logq_users must be LogQCorrection objects on {engine.device}")
+        self.logq, self.logq_users = logq, logq_users
         self.betas, self.eps, self.weight_decay = tuple(betas), eps, weight_decay
         self.group = group
         #: False = forward + backward only (the gradient buffer is cleared instead of consumed): the
@@ -143,10 +302,14 @@ class TrainStepRunner:
         if self.shard_opt:
             self._grad_shard = torch.empty(engine.numel // world_size, device=engine.device)
         # packed exchange buffers: one all-gather for (user emb | item emb | user id), one for the two LSE vectors
+        # (+ 8 bytes of target id per row when the item side of the logQ correction is on)
         if self.gathered and self.arena is None:
             D = engine.cfg.embedding_dim
-            self._pack_emb = torch.empty(B, 2 * D * 2 + 8, device=engine.device, dtype=torch.uint8)
-            self._pack_emb_all = torch.empty(world_size * B, 2 * D * 2 + 8, device=engine.device, dtype=torch.uint8)
+            w = 2 * D * 2 + 8 + (8 if logq is not None else 0)
+            self._pack_emb = torch.empty(B, w, device=engine.device, dtype=torch.uint8)
+            self._pack_emb_all = torch.empty(world_size * B, w, device=engine.device, dtype=torch.uint8)
+            if logq is not None:
+                self._tid_all = torch.zeros(world_size * B, device=engine.device, dtype=torch.long)
             self._pack_lse = torch.empty(B, 2, device=engine.device)
             self._pack_lse_all = torch.empty(world_size * B, 2, device=engine.device)
         dev, m = engine.device, engine.cfg.modality_dim
@@ -159,6 +322,8 @@ class TrainStepRunner:
                   ("target_input_ids", (B, m), torch.float32), ("target_tabular", (B, m), torch.float32)]
         if with_user_idx:
             fields.append(("user_idx", (B,), torch.long))
+        if logq is not None:
+            fields.append(("target_id", (B,), torch.long))
         self._fields, off = [], 0
         for name, shape, dt in fields:
             n = 1
@@ -182,6 +347,15 @@ class TrainStepRunner:
         self._staged = False
         self.kernels_per_step = 0
         self._warm = False
+        # logQ offsets over the columns of the logit blocks (global batch when gathered); a side that is off stays 0
+        self._offsets = None
+        if logq is not None or logq_users is not None:
+            n = world_size * B if self.gathered else B
+            self._offsets = (torch.zeros(n, device=dev), torch.zeros(n, device=dev))
+            for c in (logq, logq_users):
+                if c is not None:
+                    c.bind(n)
+            self._logq_stream = torch.cuda.Stream(device=dev)
 
     # ---- symmetric-arena path -----------------------------------------------------------------
     def _setup_symm(self, eng: TwoTowerEngine, B: int, G: int, group) -> None:
@@ -190,6 +364,8 @@ class TrainStepRunner:
         layout = {"flat": eng.numel * 4, "grad": eng.numel * 4, "shadow": eng.shadow.numel() * 2,
                   "U_all": G * B * D * 2, "I_all": G * B * D * 2, "uid_all": G * B * 8,
                   "lse_r_all": G * B * 4, "lse_c_all": G * B * 4, "loss_all": G * 16}
+        if self.logq is not None:
+            layout["tid_all"] = G * B * 8
         self.arena = a = SymmArena(layout, group, eng.device)
         eng.rebind_storage(a.view("flat", torch.float32, (eng.numel,)), a.view("grad", torch.float32, (eng.numel,)),
                            a.view("shadow", torch.bfloat16, (eng.shadow.numel(),)))
@@ -230,8 +406,13 @@ class TrainStepRunner:
         # no leading barrier: the peers' last reads of these blocks (previous step's backward) precede the
         # barrier that ended the previous step's optimizer kernel
         blocks = [(ws["un_bf"], "U_all"), (ws["in_bf"], "I_all")] + ([(uid, "uid_all")] if uid is not None else [])
+        if self.logq is not None:
+            blocks.append((self.static["target_id"], "tid_all"))
         a.allgather(blocks)
-        eng.loss_forward(ws, uid, gathered=g, rank=self.rank)
+        if self._offsets is not None:
+            tid_all = a.view("tid_all", torch.long, (self.world * self.B,)) if self.logq is not None else None
+            self._compute_offsets(tid_all, g["uid_all"])
+        eng.loss_forward(ws, uid, gathered=g, rank=self.rank, offsets=self._offsets)
         eng.loss_value(ws, self.world * self.B)
         self._loss_pad[:1].copy_(ws["loss"].view(1))
         a.allgather([(ws["lse_r"], "lse_r_all"), (ws["lse_c"], "lse_c_all"), (self._loss_pad, "loss_all")])
@@ -250,13 +431,31 @@ class TrainStepRunner:
             dst.copy_(batch[k], non_blocking=True)
 
     # ---- step phases (each is graph-capturable; NCCL calls stay between the graphs) ----------
+    def _compute_offsets(self, item_ids, user_ids):
+        """log q of every column entity into self._offsets (item side, user side)."""
+        if self.logq is not None:
+            self.logq.offsets(item_ids, self._offsets[0])
+        if self.logq_users is not None:
+            self.logq_users.offsets(user_ids, self._offsets[1])
+
     def _phase_towers(self):
+        if self._offsets is not None and not self.gathered:
+            # local negatives: the offsets need only this batch's ids, so they run beside the towers
+            main, side = torch.cuda.current_stream(), self._logq_stream
+            side.wait_stream(main)
+            with torch.cuda.stream(side):
+                self._compute_offsets(self.static.get("target_id"), self.static.get("user_idx"))
+            self._ws = self.eng.forward_towers(self.static, training=True)
+            main.wait_stream(side)
+            return
         self._ws = self.eng.forward_towers(self.static, training=True)
 
     def _phase_loss_rows(self):
         eng, ws = self.eng, self._ws
         g = eng.gathered_workspace(ws, self.world) if self.gathered else None
-        eng.loss_forward(ws, self.static.get("user_idx"), gathered=g, rank=self.rank)
+        if self._offsets is not None and self.gathered:
+            self._compute_offsets(self._tid_all if self.logq is not None else None, g["uid_all"])
+        eng.loss_forward(ws, self.static.get("user_idx"), gathered=g, rank=self.rank, offsets=self._offsets)
 
     def _phase_backward(self):
         if self.gathered:
@@ -287,7 +486,9 @@ class TrainStepRunner:
         pk[:, :2 * D].copy_(ws["un_bf"].view(torch.uint8).view(B, 2 * D))
         pk[:, 2 * D:4 * D].copy_(ws["in_bf"].view(torch.uint8).view(B, 2 * D))
         if "user_idx" in self.static:
-            pk[:, 4 * D:].copy_(self.static["user_idx"].view(torch.uint8).view(B, 8))
+            pk[:, 4 * D:4 * D + 8].copy_(self.static["user_idx"].view(torch.uint8).view(B, 8))
+        if self.logq is not None:
+            pk[:, 4 * D + 8:].copy_(self.static["target_id"].view(torch.uint8).view(B, 8))
 
     def _phase_unpack_emb(self):
         ws, D, B, G = self._ws, self.eng.cfg.embedding_dim, self.B, self.world
@@ -296,7 +497,9 @@ class TrainStepRunner:
         g["U_all"].view(torch.uint8).view(G * B, 2 * D).copy_(pk[:, :2 * D])
         g["I_all"].view(torch.uint8).view(G * B, 2 * D).copy_(pk[:, 2 * D:4 * D])
         if "user_idx" in self.static:
-            g["uid_all"].view(torch.uint8).view(G * B, 8).copy_(pk[:, 4 * D:])
+            g["uid_all"].view(torch.uint8).view(G * B, 8).copy_(pk[:, 4 * D:4 * D + 8])
+        if self.logq is not None:
+            self._tid_all.view(torch.uint8).view(G * B, 8).copy_(pk[:, 4 * D + 8:])
 
     def _comm_embeddings(self):
         dist.all_gather_into_tensor(self._pack_emb_all, self._pack_emb, group=self.group)
@@ -534,12 +737,18 @@ class TrainStepRunner:
         return float(slot["loss"])
 
 
-def train_one_epoch(model, dataloader, optimizer, device, epoch, is_main_process=True, log_interval=50):
-    """Reference signature and return value (mean loss), src/train.py:41-76."""
+def train_one_epoch(model, dataloader, optimizer, device, epoch, is_main_process=True, log_interval=50,
+                    logq: Optional[LogQCorrection] = None, logq_users: Optional[LogQCorrection] = None):
+    """Reference signature and return value (mean loss), src/train.py:41-76. ``logq`` / ``logq_users``: logQ
+    correction of the item / user negatives (LogQCorrection; needs a FusedAdamW optimizer). A streaming estimator
+    keeps its state across epochs and across the runner rebuilt for a batch of another shape."""
     model.train()
     total_loss, num_batches = 0.0, len(dataloader)
     runner: Optional[TrainStepRunner] = None
     fused = isinstance(optimizer, FusedAdamW)
+    if (logq is not None or logq_users is not None) and not fused:
+        raise ValueError("the logQ correction runs in the fused training step only: use a FusedAdamW optimizer")
+    keys = _BATCH_KEYS + (("target_id",) if logq is not None else ())
     staged = False
     world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
     it = iter(dataloader)
@@ -557,14 +766,15 @@ def train_one_epoch(model, dataloader, optimizer, device, epoch, is_main_process
                         total_loss += pending
                 runner = TrainStepRunner(model.engine, B, L, world_size=world, lr=optimizer.lr,
                                          betas=optimizer.betas, eps=optimizer.eps,
-                                         weight_decay=optimizer.weight_decay, with_user_idx="user_idx" in batch)
+                                         weight_decay=optimizer.weight_decay, with_user_idx="user_idx" in batch,
+                                         logq=logq, logq_users=logq_users)
                 staged = False
-            cur = None if staged else {k: v for k, v in batch.items() if k in _BATCH_KEYS}
+            cur = None if staged else {k: v for k, v in batch.items() if k in keys}
             # the next batch goes over PCIe during this step when it is pinned and has the same shape
             pre = None
             if nxt is not None and tuple(nxt["history_ids"].shape) == (B, L) and \
-                    all(v.is_pinned() for k, v in nxt.items() if k in _BATCH_KEYS and isinstance(v, torch.Tensor)):
-                pre = {k: v for k, v in nxt.items() if k in _BATCH_KEYS}
+                    all(v.is_pinned() for k, v in nxt.items() if k in keys and isinstance(v, torch.Tensor)):
+                pre = {k: v for k, v in nxt.items() if k in keys}
             # the loss is read one step behind (the host enqueues step i + 1 while step i runs) except where the
             # reference logs it, so the GPU is not drained every step; every step's loss still reaches the host
             prev_loss = runner.step_from_host(cur, prefetch=pre, defer_loss=True)
