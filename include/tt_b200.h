@@ -95,9 +95,10 @@ int tt_gemm_bf16(const tt_gemm_args* args, void* stream);
  *   ctx  : bf16 [B*L, H*64]     attention output before out_proj
  *   lse  : fp32 [B, H, L]       natural-log sum-exp of the scaled scores (for backward)
  * Dropout (p > 0) is applied to the attention probabilities with the counter-based hash
- * (seed + *seed_dev, site, ((b*H+h)*L+i)*L+j). L <= 4096: L <= 512 keeps every tile of a sequence on chip;
- * 512 < L <= 4096 runs the tiled kernels (online-softmax forward; a deterministic backward in two kernels, one per key
- * tile for dK / dV and one per query tile for dQ), which hash the element index in 64 bits. B*L <= 2^31 - 1.
+ * (seed + *seed_dev, site, ((b*H+h)*L+i)*L+j). L <= 4096: L <= 256 keeps every tile of a sequence on chip;
+ * 256 < L <= 4096 runs the tiled online-softmax forward, which hashes the element index in 64 bits. The backward keeps
+ * a sequence's dQ accumulators on chip up to L = 512; 512 < L <= 4096 runs the tiled backward (deterministic, in two
+ * kernels: one per key tile for dK / dV and one per query tile for dQ; 64-bit element index). B*L <= 2^31 - 1.
  */
 int tt_attn_causal_fwd(const void* qkv, void* ctx, float* lse, int B, int L, int H, float drop_p,
                        uint64_t drop_seed, const uint64_t* drop_seed_dev, uint32_t drop_site, void* stream);

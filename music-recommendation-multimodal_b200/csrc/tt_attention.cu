@@ -6,17 +6,15 @@
 // for every VALID query row the causal predicate alone is the full mask (keys <= query <
 // length) and no mask tensor exists. Pad-query rows produce finite values nobody reads.
 //
-// Forward (256 < L <= 512; attn_fwd_persist_kernel takes L <= 256, attn_fwd_long_kernel L > 512):
-// one CTA (128 threads = 128 query rows = 128 TMEM lanes) per (sequence, head, 128-row query tile).
-// All S_j = Q K_j^T tiles (j <= query tile) are issued up front into TMEM (128 columns each,
-// L <= 512), the row max is taken from TMEM, then per key tile
-// P_j = exp2(.) is written as bf16 into a 128B-swizzled K-major smem tile (double-buffered)
-// and O += P_j V_j accumulates in TMEM (V consumed MN-major straight from the QKV buffer's
-// layout). O reuses the first 64 columns of S_0 once S_0 has been drained.
-//
-// Backward (256 < L <= 512; attn_bwd_persist_kernel takes L <= 256, attn_bwd_long_kernel L > 512):
-// one CTA per (sequence, head) walks key tiles j and query tiles i >= j with the five products of
-// the standard attention backward, all on tcgen05 (see attn_bwd_kernel).
+// Kernels, chosen by sequence length inside tt_attn_causal_fwd / _bwd:
+//   L <= 256 (one or two 128-row tiles): attn_fwd_persist_kernel / attn_bwd_persist_kernel, persistent CTAs that
+//     keep every S tile (forward) and every dQ accumulator (backward) of a sequence in TMEM;
+//   forward, 256 < L <= 4096: attn_fwd_long_kernel, which walks 128-row tiles with TMEM and shared memory that do
+//     not depend on L;
+//   backward, 256 < L <= 512: attn_bwd_kernel, one CTA per (sequence, head) that keeps its four dQ accumulators in
+//     TMEM; 512 < L <= 4096: attn_bwd_long_kernel, tiled like the forward. At 256 < L <= 512 the tiled backward,
+//     which recomputes S and dP in two kernels over one to four tiles, measured slower at every shape (DESIGN.md §7).
+// Every product runs on tcgen05; the five of the backward are listed above the backward kernels.
 #include "../../include/tt_b200.h"
 #include "tt_common.cuh"
 
@@ -68,245 +66,10 @@ __device__ __forceinline__ void store_row32_bf16(__nv_bfloat16* dst, const uint3
   }
 }
 
-// Forward. 256 threads: warp w -> TMEM lane quarter (w & 3), column half (w >> 2). Thread
-// (row, hf) owns query row `row` of the tile and the 64-column half `hf` of every 128-key tile.
-// Shared memory per CTA (nq = 2): Q 16 KB + K slots 32 KB (reused for V_1.. once the S MMAs have retired) + V_0
-// 16 KB + P 32 KB = 96 KB -> two CTAs per SM (TMEM: 128 or 256 columns each).
-__global__ void __launch_bounds__(256, 2)
-attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const AttnParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t pad = (1024u - (smem_u32(smem_raw) & 1023u)) & 1023u;
-  uint8_t* smem = smem_raw + pad;
-
-  const int tid = threadIdx.x;
-  const int warp = tid >> 5, lane = tid & 31;
-  const int q = warp & 3, hf = warp >> 2;
-  const int row = q * 32 + lane;
-  const int bh_count = p.B * p.H;
-  const int qt = p.nq - 1 - static_cast<int>(blockIdx.x) / bh_count;  // heavy tiles first
-  const int bh = static_cast<int>(blockIdx.x) % bh_count;
-  const int b = bh / p.H, h = bh % p.H;
-  const int n_kv = qt + 1;
-  const int D = p.H * kDh;
-
-  uint8_t* sQ = smem;
-  uint8_t* sKV = sQ + kTileBytes;
-  uint8_t* sV0 = sKV + static_cast<size_t>(p.nq) * kTileBytes;   // V_0 has its own slot: loaded with Q / K, not after S
-  uint8_t* sP = sV0 + kTileBytes;                                 // 2 chunks x 16 KB
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sP + 2 * kTileBytes);
-  uint64_t* bar_qk = bars + 0;
-  uint64_t* bar_v = bars + 1;
-  uint64_t* bar_s = bars + 2;
-  uint64_t* bar_pv = bars + 3;
-  uint64_t* bar_v0 = bars + 4;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 5);
-  float* s_red = reinterpret_cast<float*>(bars + 7);  // [2][128]
-
-  uint32_t tmem_cols = 128;
-  while (tmem_cols < static_cast<uint32_t>(n_kv * kTile)) tmem_cols <<= 1;
-
-  if (tid == 0) {
-    tma_prefetch_desc(&tmQKV);
-    mbar_init(bar_qk, 1);
-    mbar_init(bar_v, 1);
-    mbar_init(bar_s, 1);
-    mbar_init(bar_pv, 1);
-    mbar_init(bar_v0, 1);
-    fence_barrier_init();
-  }
-  __syncwarp();
-  if (warp == 0) {
-    tmem_alloc(tmem_slot, tmem_cols);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  // The trigger comes AFTER this CTA owns its TMEM columns: a dependent CTA scheduled early on the same
-  // SM could otherwise take them first and wait forever for this grid to finish.
-  pdl_launch_dependents();
-  pdl_wait();   // prologue (barriers, TMEM, tensor-map prefetch) overlapped the previous kernel's tail
-
-  const int seq_row0 = b * p.L;
-  const int q_row0 = seq_row0 + qt * kTile;
-
-  if (tid == 0) {
-    mbar_arrive_expect_tx(bar_qk, (1 + n_kv) * kTileBytes);
-    tma_load_2d(sQ, &tmQKV, bar_qk, h * kDh, q_row0);
-    for (int j = 0; j < n_kv; ++j)
-      tma_load_2d(sKV + static_cast<size_t>(j) * kTileBytes, &tmQKV, bar_qk, D + h * kDh, seq_row0 + j * kTile);
-    mbar_arrive_expect_tx(bar_v0, kTileBytes);
-    tma_load_2d(sV0, &tmQKV, bar_v0, 2 * D + h * kDh, seq_row0);
-    mbar_wait(bar_qk, 0);
-    tc_fence_after();
-    const uint32_t idesc_s = umma_idesc_bf16(kTile, kTile, false, false);
-    // descriptors once per tile, a k-step adds its byte offset >> 4 to the address field (addresses < 256 KB)
-    const uint64_t q_desc = umma_desc_kmajor(smem_u32(sQ));
-    for (int j = 0; j < n_kv; ++j) {
-      const uint64_t k_desc = umma_desc_kmajor(smem_u32(sKV + static_cast<size_t>(j) * kTileBytes));
-#pragma unroll
-      for (int k = 0; k < kDh / 16; ++k)
-        umma_bf16(tmem_base + j * kTile, q_desc + (k * 32 >> 4), k_desc + (k * 32 >> 4), idesc_s, k > 0 ? 1u : 0u);
-    }
-    umma_commit(bar_s);
-    // the K slots are free once the S MMAs retired: V_1.. take their place (needed one P tile later than V_0)
-    if (n_kv > 1) {
-      mbar_wait(bar_s, 0);
-      mbar_arrive_expect_tx(bar_v, (n_kv - 1) * kTileBytes);
-      for (int j = 1; j < n_kv; ++j)
-        tma_load_2d(sKV + static_cast<size_t>(j - 1) * kTileBytes, &tmQKV, bar_v, 2 * D + h * kDh, seq_row0 + j * kTile);
-    }
-  }
-
-  // ---- pass A: row maximum over the causal prefix (each thread: its column half) ----------
-  mbar_wait(bar_s, 0);
-  __syncwarp();
-  tc_fence_after();
-  const uint32_t lane_base = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
-  const int q_pos = qt * kTile + row;  // position of this thread's query inside the sequence
-  const bool dead_rows = qt * kTile + q * 32 >= p.L;
-  float m = -INFINITY;
-  for (int j = 0; j < n_kv; ++j) {
-    const bool diag = (j == qt);
-#pragma unroll
-    for (int cc = 0; cc < 2; ++cc) {
-      const int cg = 2 * hf + cc;       // 32-column chunk index inside the key tile
-      // nothing to do (warp-uniform): above the diagonal for every row of this warp, or the warp's 32 query rows /
-      // the chunk's 32 keys lie wholly beyond the sequence (L = 200: a quarter of the second tile's warps)
-      if ((diag && cg > q) || dead_rows || j * kTile + cg * 32 >= p.L) continue;
-      uint32_t r[32];
-      tmem_ld32(lane_base + j * kTile + cg * 32, r);
-      tmem_ld_wait();
-      const int kv0 = j * kTile + cg * 32;
-#pragma unroll
-      for (int t = 0; t < 32; ++t) {
-        const float s = __uint_as_float(r[t]);
-        if (!diag || kv0 + t <= q_pos) m = fmaxf(m, s);
-      }
-    }
-  }
-  s_red[hf * 128 + row] = m;
-  __syncthreads();
-  m = fmaxf(s_red[row], s_red[128 + row]);
-  __syncthreads();
-  const float c1 = p.scale * kLog2e;
-  const float mc = m * c1;
-  const uint64_t seed = p.drop_seed + ((p.drop_thresh && p.drop_seed_dev) ? *p.drop_seed_dev : 0ull);
-  const uint32_t dkey = drop_key(seed, p.drop_site);
-
-  // ---- pass B: P_j -> smem (bf16, swizzled), O += P_j V_j ------------------------------
-  float l = 0.f;
-  const uint32_t idesc_pv = umma_idesc_bf16(kTile, kDh, false, true);
-  uint8_t* chunk = sP + static_cast<size_t>(hf) * kTileBytes;  // this thread's 64 key columns
-  for (int j = 0; j < n_kv; ++j) {
-    if (j >= 1) mbar_wait(bar_pv, (j - 1) & 1);  // previous P tile consumed
-    __syncwarp();
-    const bool diag = (j == qt);
-#pragma unroll
-    for (int cc = 0; cc < 2; ++cc) {
-      const int cg = 2 * hf + cc;
-      const int u0 = cc * 4;
-      if (!((diag && cg > q) || dead_rows || j * kTile + cg * 32 >= p.L)) {
-        uint32_t r[32];
-        tmem_ld32(lane_base + j * kTile + cg * 32, r);
-        tmem_ld_wait();
-        const int kv0 = j * kTile + cg * 32;
-        const uint32_t didx0 = (static_cast<uint32_t>(bh) * p.L + q_pos) * p.L + kv0;
-        float pv[32];
-#pragma unroll
-        for (int t = 0; t < 32; ++t) {
-          float e = fast_exp2(__uint_as_float(r[t]) * c1 - mc);
-          if (diag && kv0 + t > q_pos) e = 0.f;
-          l += e;
-          pv[t] = e;
-        }
-        if (p.drop_thresh) {
-          if ((didx0 & 3u) == 0u) {          // L % 4 == 0: four keys per hash word
-#pragma unroll
-            for (int t = 0; t < 32; t += 4) {
-              bool k[4];
-              drop_keep_quad(dkey, didx0 + t, p.drop_thresh, k);
-#pragma unroll
-              for (int e = 0; e < 4; ++e) pv[t + e] = k[e] ? pv[t + e] * p.drop_scale : 0.f;
-            }
-          } else if ((didx0 & 1u) == 0u) {
-#pragma unroll
-            for (int t = 0; t < 32; t += 2) {
-              bool k0, k1;
-              drop_keep_pair(dkey, didx0 + t, p.drop_thresh, k0, k1);
-              pv[t] = k0 ? pv[t] * p.drop_scale : 0.f;
-              pv[t + 1] = k1 ? pv[t + 1] * p.drop_scale : 0.f;
-            }
-          } else {
-#pragma unroll
-            for (int t = 0; t < 32; ++t)
-              pv[t] = drop_keep_k(dkey, didx0 + t, p.drop_thresh) ? pv[t] * p.drop_scale : 0.f;
-          }
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          uint4 v;
-          v.x = pack_bf16(pv[u * 8 + 0], pv[u * 8 + 1]);
-          v.y = pack_bf16(pv[u * 8 + 2], pv[u * 8 + 3]);
-          v.z = pack_bf16(pv[u * 8 + 4], pv[u * 8 + 5]);
-          v.w = pack_bf16(pv[u * 8 + 6], pv[u * 8 + 7]);
-          st_swizzled_unit(chunk, row, u0 + u, v);
-        }
-      } else {
-#pragma unroll
-        for (int u = 0; u < 4; ++u) st_swizzled_unit(chunk, row, u0 + u, make_uint4(0, 0, 0, 0));
-      }
-    }
-    fence_proxy_async_smem();
-    tc_fence_before();
-    __syncthreads();
-    if (tid == 0) {
-      tc_fence_after();
-      if (j == 0) mbar_wait(bar_v0, 0);
-      else if (j == 1) mbar_wait(bar_v, 0);
-      const uint64_t p_desc = umma_desc_kmajor(smem_u32(sP));
-      const uint64_t v_desc = umma_desc_mnmajor(smem_u32(j == 0 ? sV0 : sKV + static_cast<size_t>(j - 1) * kTileBytes), kTileBytes);
-#pragma unroll
-      for (int k = 0; k < kTile / 16; ++k) {
-        // A = P: chunk (k/4), 32 B per 16 kv columns; B = V rows (MN-major): 16 kv rows = 2048 B
-        umma_bf16(tmem_base, p_desc + (((k >> 2) * kTileBytes + (k & 3) * 32) >> 4), v_desc + (k * 2048 >> 4), idesc_pv,
-                  (j > 0 || k > 0) ? 1u : 0u);
-      }
-      umma_commit(bar_pv);
-    }
-  }
-
-  // ---- epilogue: O / l -> ctx, log-sum-exp -> lse ---------------------------------------
-  s_red[hf * 128 + row] = l;
-  mbar_wait(bar_pv, (n_kv - 1) & 1);
-  __syncthreads();
-  tc_fence_after();
-  l = s_red[row] + s_red[128 + row];
-  {
-    const float inv_l = 1.f / l;
-    const bool valid = q_pos < p.L;
-    __nv_bfloat16* orow = p.ctx + static_cast<size_t>(seq_row0 + q_pos) * D + h * kDh + hf * 32;
-    uint32_t r[32];
-    tmem_ld32(lane_base + hf * 32, r);
-    tmem_ld_wait();
-    if (valid) {
-#pragma unroll
-      for (int t = 0; t < 32; ++t) r[t] = __float_as_uint(__uint_as_float(r[t]) * inv_l);
-      store_row32_bf16(orow, r);   // two 32-byte stores: whole sectors (rows are 512 B apart, nothing coalesces)
-      if (hf == 0 && p.lse) p.lse[static_cast<size_t>(bh) * p.L + q_pos] = m * p.scale + __logf(l);
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem_base, tmem_cols);
-}
-
 // --------------------------------------------------------------------------------------------
-// Forward, persistent and pipelined (L <= 256). The kernel above is a chain of dependent latencies per CTA
-// (TMEM allocation -> TMA -> S MMAs -> row max -> P -> PV MMA -> epilogue) with two CTAs per SM to hide them.
-// Here a CTA per SM walks (sequence, head) items; per item the (query tile u, key tile j <= u) pairs are
+// Forward, persistent and pipelined (L <= 256). A CTA per (sequence, head, query tile) is a chain of dependent
+// latencies (TMEM allocation -> TMA -> S MMAs -> row max -> P -> PV MMA -> epilogue) with two CTAs per SM to hide
+// them. Here a CTA per SM walks (sequence, head) items; per item the (query tile u, key tile j <= u) pairs are
 // (0,0), (1,0), (1,1), S tile t = pair index at TMEM columns 128 t, O_u at 384 + 64 u:
 //   * warps 0-15: thread (row, 32-column chunk). Per query tile: row max over its S tiles (combined across the
 //     four chunk groups through shared memory), then per pair P = dropout(exp2(.)) -> bf16 -> one of two
@@ -1392,8 +1155,9 @@ attn_bwd_persist_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_
 }
 
 // ============================================================================================
-// Long histories, 512 < L <= 4096. The kernels above keep every S tile (forward) or every dQ accumulator (backward)
-// of a sequence in TMEM, which caps L at 512. The kernels below walk the key / query tiles of one 128-row tile with
+// Tiled kernels: the forward for 256 < L <= 4096, the backward for 512 < L <= 4096. The kernels above keep every S
+// tile (forward) or every dQ accumulator (backward) of a sequence in TMEM, which caps L at 256 (persistent kernels)
+// and 512 (attn_bwd_kernel). The kernels below walk the key / query tiles of one 128-row tile with
 // TMEM and shared memory that do not depend on L. Dropout hashes the 64-bit element index ((b*H + h)*L + q)*L + k
 // (B*H*L^2 passes 2^32 from B = 65 at L = 4096), exactly as drop_keep_k and the single-query kernels do.
 // ============================================================================================
@@ -1432,8 +1196,9 @@ __device__ __forceinline__ uint32_t drop_keepmask32_64(uint32_t dkey, uint64_t d
   return keepmask;
 }
 
-// Forward, L > 512. One CTA (256 threads) per (sequence, head, 128-row query tile), heavy tiles first; thread (row,
-// hf) as in attn_fwd_kernel. Online softmax over the key tiles j = 0..qt:
+// Forward, L > 256. One CTA (256 threads) per (sequence, head, 128-row query tile), heavy tiles first. Warp w -> TMEM
+// lane quarter (w & 3), column half (w >> 2): thread (row, hf) owns query row `row` of the tile and the 64-column half
+// `hf` of every 128-key tile. Online softmax over the key tiles j = 0..qt:
 //   S_j = Q K_j^T -> TMEM columns [0, 128); the row max of S_j raises the running max m;
 //   P_j = dropout(exp2((S_j - m) * scale * log2e)) -> bf16, 128B-swizzled smem tile; O_j = P_j V_j -> TMEM columns
 //   [128, 192), a fresh accumulator per tile;
@@ -2009,17 +1774,6 @@ extern "C" int tt_attn_causal_fwd(const void* qkv, void* ctx, float* lse, int B,
   CUtensorMap tm;
   int rc = make_rows_map(&tm, qkv, B * L, 3 * D);
   if (rc) return rc;
-  if (L > 512) {
-    const size_t lsmem = 1024 + 6 * static_cast<size_t>(kTileBytes) + 48 + 2 * 128 * sizeof(float);
-    static bool lconfigured = false;
-    if (!lconfigured) {
-      TT_CHECK_CUDA(cudaFuncSetAttribute(attn_fwd_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lsmem));
-      lconfigured = true;
-    }
-    TT_CHECK_CUDA(launch_k(attn_fwd_long_kernel, dim3(B * H * p.nq), dim3(256), lsmem, stream, tm, p));
-    TT_LAUNCH_CHECK();
-    return TT_OK;
-  }
   if (p.nq <= 2) {
     const size_t psmem = 1024 + 12 * static_cast<size_t>(kTileBytes) + 256 + 3 * 4 * kTile * sizeof(float);
     static bool pconfigured = false;
@@ -2032,14 +1786,13 @@ extern "C" int tt_attn_causal_fwd(const void* qkv, void* ctx, float* lse, int B,
     TT_LAUNCH_CHECK();
     return TT_OK;
   }
-  const size_t smem = 1024 + static_cast<size_t>(1 + p.nq + 1 + 2) * kTileBytes + 64 + 2 * 128 * sizeof(float);
-  static bool configured = false;
-  if (!configured) {
-    TT_CHECK_CUDA(cudaFuncSetAttribute(attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-    configured = true;
+  const size_t lsmem = 1024 + 6 * static_cast<size_t>(kTileBytes) + 48 + 2 * 128 * sizeof(float);
+  static bool lconfigured = false;
+  if (!lconfigured) {
+    TT_CHECK_CUDA(cudaFuncSetAttribute(attn_fwd_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lsmem));
+    lconfigured = true;
   }
-  TT_REQUIRE(smem <= 232448, "tt_attn_causal_fwd: shared memory %zu too large", smem);
-  TT_CHECK_CUDA(launch_k(attn_fwd_kernel, dim3(B * H * p.nq), dim3(256), smem, stream, tm, p));
+  TT_CHECK_CUDA(launch_k(attn_fwd_long_kernel, dim3(B * H * p.nq), dim3(256), lsmem, stream, tm, p));
   TT_LAUNCH_CHECK();
   return TT_OK;
 }

@@ -99,7 +99,7 @@ def test_attn_dropout_statistics():
 
 # More (sequence, head) items than SMs (a persistent CTA walks several items) and fewer; with and without dropout.
 REPEAT_SHAPES = [(160, 200, 4, 0.1), (150, 50, 4, 0.1), (40, 256, 2, 0.2), (37, 129, 4, 0.1), (3, 200, 4, 0.0),
-                 (2, 128, 4, 0.0)]
+                 (2, 128, 4, 0.0), (64, 384, 4, 0.1), (40, 512, 4, 0.1), (48, 300, 4, 0.0)]
 
 
 def _drop_mask(B, L, H, drop, seed, site):
@@ -168,8 +168,8 @@ def test_attn_bwd_repeated_launches_match_reference(B, L, H, drop):
 def test_attn_bwd_uses_the_forward_dropout_mask(B, L, H):
     """The backward re-creates the forward's dropout mask from the hash. Here the mask is READ OUT of the forward kernel
     (one-hot V blocks turn ctx into the dropped probabilities themselves) and a torch backward with exactly that mask
-    is the reference — for the two-tile (persistent) and the four-tile (L > 256) kernels, whose hash evaluation differs
-    (one word per 4 / 2 / 1 keys depending on alignment)."""
+    is the reference — for the persistent kernels (L <= 256) and for the tiled forward with the four-tile backward
+    (256 < L <= 512), whose hash evaluations differ (one word per 4 / 2 / 1 keys depending on alignment)."""
     from mrm_b200 import ops
     p_drop, seed, site = 0.3, 4242, 5
     D = H * 64

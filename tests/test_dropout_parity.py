@@ -217,7 +217,7 @@ def _attn_ref(qkv, B, L, H, mask, dctx):
 
 
 # odd B*H (and L = 50, 129, 300: every alignment of the index, so the quad, pair and single hash forms all run);
-# the persistent kernels for L <= 256, the four-tile per-item kernels for 256 < L <= 512
+# the persistent kernels for L <= 256, the tiled forward and the four-tile per-item backward for 256 < L <= 512
 ATTN_SHAPES = [(3, 50, 1), (1, 129, 3), (3, 200, 1), (2, 200, 4), (1, 256, 3), (3, 300, 1), (1, 512, 3)]
 
 

@@ -1,5 +1,6 @@
-"""Long listening histories: 512 < L <= 4096 through the tiled attention kernels, the single-query last layer, the
-training step, CUDA-graph replay and recommend_batch.
+"""Long listening histories: 512 < L <= 4096 through the tiled attention kernels (the tiled forward also serves
+256 < L <= 512, which tests/test_attention.py covers), the single-query last layer, the training step, CUDA-graph
+replay and recommend_batch.
 
 Attention references are the fp32 torch restatement of tests/test_attention.py on the same bf16 inputs, with its
 tolerances; dropout references apply the numpy mask of tests/_dropout_ref.drop_keep_k (64-bit element index

@@ -1,7 +1,7 @@
 """Times tt_attn_causal_fwd / tt_attn_causal_bwd alone with CUDA events, H = 4. By default over sequence lengths on
-both sides of the kernel switches at L = 256 and L = 512, at about the c2 step's token count (B*L ~ 51200); B and L
-in the environment time one shape instead. To compare two kernel variants, build two libraries and run this once
-with each (TT_B200_LIB selects the library)."""
+both sides of the kernel switches at L = 256 (forward and backward) and L = 512 (backward), at about the c2 step's
+token count (B*L ~ 51200); B and L in the environment time one shape instead. To compare two kernel variants, build
+two libraries and run this once with each (TT_B200_LIB selects the library)."""
 import os
 import sys
 

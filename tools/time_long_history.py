@@ -2,10 +2,10 @@
 """Long listening histories on the GPU, timed with CUDA events, one process:
 
   * attention forward / backward at dropout 0.1, H = 4: the tiled kernels at L = 1024, 2048, 4096 with
-    B * L = 131 072 tokens (B = 128, 64, 32), alternated round by round with the per-item kernels at B = 256,
-    L = 512. A 256 MB buffer is overwritten before every timed pass (L2 flushed). Microseconds (median of the
-    rounds) and algorithmic causal TFLOP/s: 2 (forward) or 5 (backward) products of 64 * L(L+1)/2 multiply-adds per
-    (sequence, head); recomputation does not count;
+    B * L = 131 072 tokens (B = 128, 64, 32), alternated round by round with B = 256, L = 512 (the tiled forward,
+    the four-tile per-item backward). A 256 MB buffer is overwritten before every timed pass (L2 flushed).
+    Microseconds (median of the rounds) and algorithmic causal TFLOP/s: 2 (forward) or 5 (backward) products of
+    64 * L(L+1)/2 multiply-adds per (sequence, head); recomputation does not count;
   * TrainStepRunner (CUDA-graph replay) at B = 64, L = 2048: ms per step and peak device memory;
   * recommend_batch at 10 000 users x 1 M items, L = 2048, K = 100: end-to-end ms, and the user tower alone.
 
@@ -74,7 +74,7 @@ def attention(rounds=15):
         for k, prods in (("fwd", 2), ("bwd", 5)):
             t = sorted(ts[((B, L), k)])[rounds // 2]
             row += [t * 1e3, 2 * prods * macs / (t * 1e-3) / 1e12]
-        kind = "per-item" if L <= 512 else "tiled"
+        kind = "fwd-tiled" if L <= 512 else "tiled"
         print(f"{kind:9s} {B:4d} {L:5d} {row[0]:9.1f} {row[1]:12.1f} {row[2]:9.1f} {row[3]:12.1f}")
     del bufs, flush
     torch.cuda.empty_cache()
