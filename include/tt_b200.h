@@ -218,6 +218,25 @@ int tt_concat4_bf16(const float* audio, const float* visual, const float* text, 
  * ids outside [0, V) are skipped. Rows not listed are left untouched (the caller zero-fills the table once). */
 int tt_index_rows(const float* y, int R, const float* ln_w, const float* ln_b, const int64_t* ids, int64_t V,
                   float* table, void* table_bf16, void* stream);
+/* Live catalog updates of a built index (retrieval.CatalogIndex.upsert / retire; the index holds rows
+ * [item_base, item_base + N) of a catalog of vocab_size ids, table / table_bf16 are its [N, 256] rows and
+ * retired_bits its bitmap in the layout of tt_score_topk_live). ids [n] int64 on the device; every id must lie in
+ * [1, vocab_size) and appear once: the launcher copies them to the host and checks that before it launches (one
+ * stream synchronisation). Ids outside this index's rows are skipped, so every shard can be handed the same batch.
+ * tt_index_rows_live : the tail of tt_index_rows with the same per-row arithmetic (one shared device function: the
+ *                      rows are bit-identical to a from-scratch indexing); writes row ids[r] - item_base, clears its
+ *                      retired bit (retired_bits may be NULL: no retired rows yet) and raises stats[0] / stats[1] to
+ *                      ||bf16(e) - e|| / ||bf16(e)|| of every written row (rounded up; integer atomicMax on the
+ *                      non-negative float bits, the caller zeroes stats). Serves the item-cache rebuild of
+ *                      src/evaluate_metrics.py:24-104 for a few rows instead of the whole catalog.
+ * tt_catalog_retire  : zeroes the fp32 and bf16 rows of the ids this index owns and sets their retired bits (a
+ *                      retired row equals an unlisted one of the cache of :92-104); retiring a retired id changes
+ *                      nothing. One warp per id. */
+int tt_index_rows_live(const float* y, int R, const float* ln_w, const float* ln_b, const int64_t* ids,
+                       int64_t vocab_size, int64_t item_base, int N, float* table, void* table_bf16,
+                       uint32_t* retired_bits, float* stats, void* stream);
+int tt_catalog_retire(const int64_t* ids, int n, int64_t vocab_size, int64_t item_base, int N, float* table,
+                      void* table_bf16, uint32_t* retired_bits, void* stream);
 
 /* BatchNorm1d + ReLU + Dropout on fp32 [B, C] -> bf16 (src/models/item_tower.py:124-126).
  * training != 0: batch statistics, running stats / num_batches_tracked updated (momentum 0.1,
@@ -384,6 +403,18 @@ int tt_logq_stream_update(const int64_t* ids, int n, int64_t* A, float* Bv, int 
  *                     tt_exclusions_build's output; NULL = tt_exact_topk).
  * tt_rank_metrics   : per-row Recall@k / NDCG@k (:159-185); gain_table[r] = 1/log2(r+2) comes
  *                     from the host so rows are bit-identical to the reference's; outputs [nk][U].
+ *
+ * Retired items (live catalog updates: songs taken down after the cache of :92-104 was built). retired_bits is one
+ * bit per row of this shard, bit r of word r / 32 = row r (global id item_base + r), 1 = retired; it holds
+ * ceil(N / 256) * 8 words (whole 256-item steps, the padding bits zero) and is 8-byte aligned. A zero-filled bitmap
+ * retires nothing. A retired row is never admitted as a candidate, so, as for exclusions, pruning, finalize, the
+ * certificate, the bounded shard protocol and the merges speak about live items only, and a user with fewer than K
+ * live admissible items gets a -1 / -inf tail. tt_topk_finalize, tt_topk_finalize_bounded and the merges need no
+ * bitmap: they only ever see admitted candidates.
+ * tt_score_topk_live : tt_score_topk_excl that never admits retired rows (retired_bits NULL = tt_score_topk_excl,
+ *                     which launches the kernels without the mask). The sample pass scores retired rows as -inf, so
+ *                     they own no chunk maximum: the start threshold can only fall.
+ * tt_exact_topk_live : tt_exact_topk_excl that never returns retired rows (NULL = tt_exact_topk_excl).
  */
 typedef struct tt_topk_plan {
   int32_t U, N, kprime, cap;
@@ -433,6 +464,13 @@ int tt_exact_topk_excl(const float* user_f32, const float* items_f32, int N, int
                        int32_t* out_idx, void* stream);
 int tt_rank_metrics(const int32_t* topk_idx, const int64_t* targets, int U, int K, const int32_t* k_list, int nk,
                     const float* gain_table, float* recall, float* ndcg, void* stream);
+int tt_score_topk_live(const void* users_bf16, const void* items_bf16, int item_base, const tt_topk_plan* plan,
+                       void* cand, int32_t* cand_cnt, void* thr, void* smax, int mask_item0, const int32_t* ex_ids,
+                       const int32_t* ex_cnt, const uint32_t* ex_bits, int ex_ld, const uint32_t* retired_bits,
+                       void* stream);
+int tt_exact_topk_live(const float* user_f32, const float* items_f32, int N, int item_base, int mask_item0, int K,
+                       const int32_t* ex_ids, const int32_t* ex_cnt, const uint32_t* retired_bits, void* key_scratch,
+                       float* out_score, int32_t* out_idx, void* stream);
 
 /* ---- diversified recommendations: maximal marginal relevance over each user's candidate pool ----
  * Extends the selection of src/inference.py:296-306 (masked scores, top k): instead of the k best scores, k picks

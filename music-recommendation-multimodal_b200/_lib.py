@@ -223,6 +223,13 @@ _SIGNATURES = {
                               c_void_p, c_void_p],
     "tt_inbatch_recall": [c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p],
     "tt_index_rows": [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, _I64, c_void_p, c_void_p, c_void_p],
+    "tt_score_topk_live": [c_void_p, c_void_p, c_int32, ctypes.POINTER(TopkPlan), c_void_p, c_void_p, c_void_p,
+                           c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p],
+    "tt_exact_topk_live": [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
+                           c_void_p, c_void_p, c_void_p, c_void_p],
+    "tt_index_rows_live": [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, _I64, _I64, c_int32, c_void_p, c_void_p,
+                           c_void_p, c_void_p, c_void_p],
+    "tt_catalog_retire": [c_void_p, c_int32, _I64, _I64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p],
 }
 
 _declare_base = _declare

@@ -76,6 +76,9 @@ struct TopkParams {
   const int* ex_cnt;         // [U]
   const uint32_t* ex_bits;   // [U][kExclWords] hashed bitmap: a clear bit proves an id is not excluded
   int ex_ld;
+  // score_topk_kernel<*, *, true>: one bit per row of this shard, 1 = retired (never scored as a candidate); a
+  // 64-bit word covers the 64 item columns an epilogue warp owns in one step. ceil(N / 256) * 4 words.
+  const unsigned long long* retired;
 };
 
 // Bit of the exclusion bitmap that stands for global id `id` (Fibonacci hashing: the top 12 bits of id * 2^32/phi).
@@ -186,10 +189,10 @@ __device__ __forceinline__ uint32_t chunk_group_mask(const uint32_t (&r)[32], fl
   return gm;
 }
 
-template <bool kExclude>
+template <bool kExclude, bool kLive>
 __device__ __forceinline__ void collect_groups(uint32_t gm, uint32_t t_chunk, int idx0, const TopkParams& p, int lane,
                                                int row, unsigned long long* buf, int& cnt,
-                                               unsigned long long& thr_key, float& thr_s) {
+                                               unsigned long long& thr_key, float& thr_s, uint64_t retired) {
   uint32_t wm = __reduce_or_sync(0xffffffffu, gm);   // groups in which ANY lane has a candidate (warp-uniform)
 #pragma unroll 1
   while (wm) {
@@ -205,7 +208,8 @@ __device__ __forceinline__ void collect_groups(uint32_t gm, uint32_t t_chunk, in
         if (s >= thr_s) {
           const int idx = idx0 + 4 * k + t;
           const uint32_t gidx = static_cast<uint32_t>(p.item_base + idx);
-          if (idx < p.N && !(p.mask_item0 && gidx == 0u)) {
+          const bool live = !kLive || !((retired >> (4 * k + t)) & 1ull);
+          if (idx < p.N && !(p.mask_item0 && gidx == 0u) && live) {
             const unsigned long long key = make_key(s, gidx);
             if (key > thr_key) buf[cnt++] = key;
           }
@@ -236,7 +240,10 @@ __device__ __forceinline__ void collect_groups(uint32_t gm, uint32_t t_chunk, in
 // kExclude (main pass only): the user's excluded items are removed from its candidate lists before every prune and
 // before the lists are handed over, so the pruning thresholds, finalize and its certificate all speak about the
 // admissible items only.
-template <bool kSample, bool kExclude>
+// kLive: rows whose bit in p.retired is set are never admitted (main pass) and never own a chunk maximum (sample
+// pass: their scores become -inf first, which can only lower a start threshold). A warp's 64 columns of a step share
+// one 64-bit word of the bitmap; it is loaded one step ahead, so the L2 round trip stays out of the chunk chain.
+template <bool kSample, bool kExclude, bool kLive>
 __global__ void __launch_bounds__(kTopkThreads, 1)
 score_topk_kernel(const __grid_constant__ CUtensorMap tmU, const __grid_constant__ CUtensorMap tmI,
                   const TopkParams p) {
@@ -365,7 +372,19 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmU, const __grid_constant
       unsigned long long thr_key = active ? p.thr[row] : ~0ull;
       float thr_s = thr_key == 0ull ? -INFINITY : (active ? key_score(thr_key) : INFINITY);
       int cnt = 0;
+      // word of the retired bitmap for this warp's 64 columns of step `tile` (sample pass: of physical step
+      // tile * tile_stride); the next step's word is in flight while this step is scanned
+      const auto retired_word = [&](int tile) -> uint64_t {
+        return __ldg(p.retired + static_cast<size_t>(tile) * p.tile_stride * (kIT / 64) + colq);
+      };
+      uint64_t rb_next = 0;
+      if constexpr (kLive) rb_next = tile0 < tile1 ? retired_word(tile0) : 0ull;
       for (int tile = tile0; tile < tile1; ++tile) {
+        uint64_t rb = 0;
+        if constexpr (kLive) {
+          rb = rb_next;
+          if (tile + 1 < tile1) rb_next = retired_word(tile + 1);
+        }
         mbar_wait(&t_full[acc], acc_phase);
         __syncwarp();
         tc_fence_after();
@@ -374,19 +393,39 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmU, const __grid_constant
         uint32_t r0[32], r1[32];
         tmem_ld32(t_base, r0);
         tmem_ld32(t_base + 32, r1);
+        uint32_t dead = 0;   // main pass: 4-score groups whose items are all retired (computed under the TMEM load)
+        if constexpr (kLive && !kSample) {
+          uint64_t x = rb & (rb >> 1);
+          x &= (x >> 2) & 0x1111111111111111ull;              // bit 4g: group g fully retired
+          x = (x | (x >> 3)) & 0x0303030303030303ull;
+          x = (x | (x >> 6)) & 0x000F000F000F000Full;
+          x = (x | (x >> 12)) & 0x000000FF000000FFull;
+          dead = static_cast<uint32_t>(x | (x >> 24)) & 0xFFFFu;
+        }
         if constexpr (kSample) {
           // sample pass: one float per (user, chunk) — the chunk's best score; layout [user][chunk]
           float* dst = p.smax + static_cast<size_t>(row) * (p.total_tiles * kChunks) + tile * kChunks + colq * 2;
           tmem_ld_wait();
+          if (kLive && rb != 0ull) {
+#pragma unroll
+            for (int t = 0; t < 32; ++t) {
+              if ((rb >> t) & 1ull) r0[t] = 0xFF800000u;          // -inf
+              if ((rb >> (32 + t)) & 1ull) r1[t] = 0xFF800000u;
+            }
+          }
           dst[0] = chunk_max(r0);
           dst[1] = chunk_max(r1);
         } else {
           tmem_ld_wait();
-          const uint32_t gm0 = chunk_group_mask(r0, thr_s);
-          const uint32_t gm1 = chunk_group_mask(r1, thr_s);
+          uint32_t gm0 = chunk_group_mask(r0, thr_s);
+          uint32_t gm1 = chunk_group_mask(r1, thr_s);
+          if constexpr (kLive) {   // fully retired groups leave the vote
+            gm0 &= ~dead & 0xFFu;
+            gm1 &= ~(dead >> 8);
+          }
           if (__any_sync(0xffffffffu, (gm0 | gm1) != 0u)) {
             const int idx0 = tile * kIT + colq * 64;
-            collect_groups<kExclude>(gm0 | (gm1 << 8), t_base, idx0, p, lane, row, buf, cnt, thr_key, thr_s);
+            collect_groups<kExclude, kLive>(gm0 | (gm1 << 8), t_base, idx0, p, lane, row, buf, cnt, thr_key, thr_s, rb);
           }
         }
         tc_fence_before();
@@ -779,8 +818,11 @@ __global__ void __launch_bounds__(256) topk_merge_kernel(const float* __restrict
 // Exact fallback for users whose certificate failed: brute-force fp64-accumulated scores over
 // the whole shard into a key array, then K-th largest by bitwise search + sort. Slow and rare.
 // --------------------------------------------------------------------------------------------
+// kLive: rows whose bit in `retired` is set get key 0, like item 0 under mask_item0.
+template <bool kLive>
 __global__ void __launch_bounds__(256) exact_keys_kernel(const float* __restrict__ user, const float* __restrict__ items,
                                                          int N, int item_base, int mask_item0,
+                                                         const uint32_t* __restrict__ retired,
                                                          unsigned long long* __restrict__ keys) {
   pdl_launch_dependents();
   pdl_wait();
@@ -805,7 +847,9 @@ __global__ void __launch_bounds__(256) exact_keys_kernel(const float* __restrict
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
     if (lane == 0) {
       const uint32_t gidx = static_cast<uint32_t>(item_base + i);
-      keys[i] = (mask_item0 && gidx == 0u) ? 0ull : make_key(static_cast<float>(acc), gidx);
+      bool drop = mask_item0 && gidx == 0u;
+      if constexpr (kLive) drop = drop || ((__ldg(retired + (i >> 5)) >> (i & 31)) & 1u);
+      keys[i] = drop ? 0ull : make_key(static_cast<float>(acc), gidx);
     }
   }
 }
@@ -1103,9 +1147,12 @@ static int launch_score_topk(const void* users_bf16, const void* items_bf16, Top
   const size_t smem = 1024 + (kKB + kBStages) * kTile16K + 256;
   static bool configured = false;
   if (!configured) {
-    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    TT_CHECK_CUDA(cudaFuncSetAttribute(score_topk_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
     configured = true;
   }
   const int units = p.n_ut * p.n_ranges;
@@ -1122,12 +1169,13 @@ static int launch_score_topk(const void* users_bf16, const void* items_bf16, Top
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
+  const bool live = p.retired != nullptr;
   if (p.smax != nullptr)
-    TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, score_topk_kernel<true, false>, tmU, tmI, p));
+    TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, live ? score_topk_kernel<true, false, true> : score_topk_kernel<true, false, false>, tmU, tmI, p));
   else if (p.ex_ids != nullptr)
-    TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, score_topk_kernel<false, true>, tmU, tmI, p));
+    TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, live ? score_topk_kernel<false, true, true> : score_topk_kernel<false, true, false>, tmU, tmI, p));
   else
-    TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, score_topk_kernel<false, false>, tmU, tmI, p));
+    TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, live ? score_topk_kernel<false, false, true> : score_topk_kernel<false, false, false>, tmU, tmI, p));
   TT_LAUNCH_CHECK();
   return TT_OK;
 }
@@ -1142,11 +1190,20 @@ extern "C" int tt_score_topk_excl(const void* users_bf16, const void* items_bf16
                                   const tt_topk_plan* plan, void* cand, int32_t* cand_cnt, void* thr, void* smax,
                                   int mask_item0, const int32_t* ex_ids, const int32_t* ex_cnt,
                                   const uint32_t* ex_bits, int ex_ld, void* stream_) {
+  return tt_score_topk_live(users_bf16, items_bf16, item_base, plan, cand, cand_cnt, thr, smax, mask_item0, ex_ids,
+                            ex_cnt, ex_bits, ex_ld, nullptr, stream_);
+}
+
+extern "C" int tt_score_topk_live(const void* users_bf16, const void* items_bf16, int item_base,
+                                  const tt_topk_plan* plan, void* cand, int32_t* cand_cnt, void* thr, void* smax,
+                                  int mask_item0, const int32_t* ex_ids, const int32_t* ex_cnt,
+                                  const uint32_t* ex_bits, int ex_ld, const uint32_t* retired_bits, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   TT_REQUIRE(users_bf16 && items_bf16 && plan && cand && cand_cnt && thr, "tt_score_topk: null pointer");
   const bool excl = ex_ids != nullptr;
   TT_REQUIRE(excl == (ex_cnt != nullptr) && excl == (ex_bits != nullptr) && (!excl || ex_ld >= 1),
              "tt_score_topk_excl: exclusion ids, counts and bits must be given together (ex_ld >= 1)");
+  TT_REQUIRE(reinterpret_cast<uintptr_t>(retired_bits) % 8 == 0, "tt_score_topk_live: retired_bits must be 8-byte aligned");
   TopkParams p;
   p.U = plan->U; p.N = plan->N; p.item_base = item_base;
   p.n_ut = plan->n_ut;
@@ -1158,6 +1215,7 @@ extern "C" int tt_score_topk_excl(const void* users_bf16, const void* items_bf16
   p.thr = static_cast<unsigned long long*>(thr);
   p.mask_item0 = mask_item0;
   p.ex_ids = ex_ids; p.ex_cnt = ex_cnt; p.ex_bits = ex_bits; p.ex_ld = ex_ld;
+  p.retired = reinterpret_cast<const unsigned long long*>(retired_bits);
   TT_CHECK_CUDA(cudaMemsetAsync(thr, 0, static_cast<size_t>(plan->thr_bytes), stream));
 
   // ---- sample pass: chunk maxima of every sample_stride-th item step -> per-user start thresholds
@@ -1267,13 +1325,23 @@ extern "C" int tt_exact_topk(const float* user_f32, const float* items_f32, int 
 extern "C" int tt_exact_topk_excl(const float* user_f32, const float* items_f32, int N, int item_base, int mask_item0,
                                   int K, const int32_t* ex_ids, const int32_t* ex_cnt, void* key_scratch,
                                   float* out_score, int32_t* out_idx, void* stream_) {
+  return tt_exact_topk_live(user_f32, items_f32, N, item_base, mask_item0, K, ex_ids, ex_cnt, nullptr, key_scratch,
+                            out_score, out_idx, stream_);
+}
+
+extern "C" int tt_exact_topk_live(const float* user_f32, const float* items_f32, int N, int item_base, int mask_item0,
+                                  int K, const int32_t* ex_ids, const int32_t* ex_cnt, const uint32_t* retired_bits,
+                                  void* key_scratch, float* out_score, int32_t* out_idx, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   TT_REQUIRE(user_f32 && items_f32 && key_scratch && out_score && out_idx && N > 0 && K > 0 && K <= 256,
              "tt_exact_topk: bad arguments");
   TT_REQUIRE((ex_ids != nullptr) == (ex_cnt != nullptr), "tt_exact_topk_excl: exclusion ids and count go together");
   int grid = (N + 7) / 8;
   if (grid > num_sms() * 8) grid = num_sms() * 8;
-  TT_CHECK_CUDA(launch_k(exact_keys_kernel, dim3(grid), dim3(256), 0, stream, user_f32, items_f32, N, item_base, mask_item0, static_cast<unsigned long long*>(key_scratch)));
+  if (retired_bits != nullptr)
+    TT_CHECK_CUDA(launch_k(exact_keys_kernel<true>, dim3(grid), dim3(256), 0, stream, user_f32, items_f32, N, item_base, mask_item0, retired_bits, static_cast<unsigned long long*>(key_scratch)));
+  else
+    TT_CHECK_CUDA(launch_k(exact_keys_kernel<false>, dim3(grid), dim3(256), 0, stream, user_f32, items_f32, N, item_base, mask_item0, retired_bits, static_cast<unsigned long long*>(key_scratch)));
   TT_LAUNCH_CHECK();
   if (ex_ids != nullptr) {
     TT_CHECK_CUDA(launch_k(exact_exclude_kernel, dim3(1), dim3(256), 0, stream, ex_ids, ex_cnt, N, item_base, static_cast<unsigned long long*>(key_scratch)));

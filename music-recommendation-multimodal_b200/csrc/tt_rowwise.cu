@@ -9,6 +9,7 @@
 // cross-warp parameter-gradient combine.
 #include "../../include/tt_b200.h"
 #include "tt_common.cuh"
+#include <vector>
 
 namespace tt {
 
@@ -755,6 +756,29 @@ __global__ void __launch_bounds__(256) adamw_kernel(float* __restrict__ p, float
 // identity, and +-inf cannot survive the first normalisation (inf / inf = NaN), so the per-element rule here
 // is the same function. One warp per item: 1 KB in, 1 KB + 512 B out.
 // --------------------------------------------------------------------------------------------
+// The row arithmetic of both indexing kernels: y row (one lane's 8 values) -> the cache row's values.
+__device__ __forceinline__ void index_row_values(const float* __restrict__ yrow, int lane, const float (&w)[8],
+                                                 const float (&b)[8], float (&v)[8]) {
+  constexpr int NV = 2, E = 8;
+  load_row<NV>(yrow, lane, v);
+  float mean, rstd;
+  ln_stats<NV>(v, 1e-5f, mean, rstd);
+  float s = 0.f;
+#pragma unroll
+  for (int i = 0; i < E; ++i) { v[i] = (v[i] - mean) * rstd * w[i] + b[i]; s += v[i] * v[i]; }
+  float inv = 1.f / fmaxf(sqrtf(warp_sum(s)), 1e-12f);
+  s = 0.f;
+#pragma unroll
+  for (int i = 0; i < E; ++i) {
+    v[i] *= inv;
+    if (v[i] != v[i]) v[i] = 0.f;
+    s += v[i] * v[i];
+  }
+  inv = 1.f / fmaxf(sqrtf(warp_sum(s)), 1e-8f);
+#pragma unroll
+  for (int i = 0; i < E; ++i) v[i] *= inv;
+}
+
 __global__ void __launch_bounds__(kRowThreads) index_rows_kernel(const float* __restrict__ y, int R,
                                                                  const float* __restrict__ ln_w,
                                                                  const float* __restrict__ ln_b,
@@ -773,25 +797,78 @@ __global__ void __launch_bounds__(kRowThreads) index_rows_kernel(const float* __
     const int64_t id = ids[row];
     if (id < 0 || id >= V) continue;             // out-of-table ids are dropped (the reference would raise)
     float v[E];
-    load_row<NV>(y + static_cast<size_t>(row) * W, lane, v);
-    float mean, rstd;
-    ln_stats<NV>(v, 1e-5f, mean, rstd);
-    float s = 0.f;
-#pragma unroll
-    for (int i = 0; i < E; ++i) { v[i] = (v[i] - mean) * rstd * w[i] + b[i]; s += v[i] * v[i]; }
-    float inv = 1.f / fmaxf(sqrtf(warp_sum(s)), 1e-12f);
-    s = 0.f;
-#pragma unroll
-    for (int i = 0; i < E; ++i) {
-      v[i] *= inv;
-      if (v[i] != v[i]) v[i] = 0.f;
-      s += v[i] * v[i];
-    }
-    inv = 1.f / fmaxf(sqrtf(warp_sum(s)), 1e-8f);
-#pragma unroll
-    for (int i = 0; i < E; ++i) v[i] *= inv;
+    index_row_values(y + static_cast<size_t>(row) * W, lane, w, b, v);
     store_row<NV>(table + static_cast<size_t>(id) * W, lane, v);
     if (table_bf16) store_row_bf16<NV>(table_bf16 + static_cast<size_t>(id) * W, lane, v);
+  }
+}
+
+// Live update of a built index (rows [item_base, item_base + N) of the catalog): the rows of index_rows_kernel for
+// the ids this index owns, their retired bits cleared, and the item-side terms of the retrieval certificate
+// (max ||bf16(e) - e||, max ||bf16(e)||) raised to cover them.
+__global__ void __launch_bounds__(kRowThreads) index_rows_live_kernel(const float* __restrict__ y, int R,
+                                                                      const float* __restrict__ ln_w,
+                                                                      const float* __restrict__ ln_b,
+                                                                      const int64_t* __restrict__ ids,
+                                                                      int64_t item_base, int N,
+                                                                      float* __restrict__ table,
+                                                                      __nv_bfloat16* __restrict__ table_bf16,
+                                                                      uint32_t* __restrict__ retired,
+                                                                      float* __restrict__ stats) {
+  pdl_launch_dependents();
+  pdl_wait();
+  constexpr int NV = 2, E = 8, W = 256;
+  const int lane = threadIdx.x & 31;
+  const int warps_total = (gridDim.x * blockDim.x) >> 5;
+  float w[E], b[E];
+  load_row<NV>(ln_w, lane, w);
+  load_row<NV>(ln_b, lane, b);
+  for (int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; row < R; row += warps_total) {
+    const int64_t local = ids[row] - item_base;
+    if (local < 0 || local >= N) continue;       // another shard's row
+    float v[E];
+    index_row_values(y + static_cast<size_t>(row) * W, lane, w, b, v);
+    store_row<NV>(table + static_cast<size_t>(local) * W, lane, v);
+    store_row_bf16<NV>(table_bf16 + static_cast<size_t>(local) * W, lane, v);
+    float d2 = 0.f, n2 = 0.f;
+#pragma unroll
+    for (int i = 0; i < E; i += 2) {
+      const float2 r = unpack_bf16(pack_bf16(v[i], v[i + 1]));
+      const float e0 = r.x - v[i], e1 = r.y - v[i + 1];
+      d2 += e0 * e0 + e1 * e1;
+      n2 += r.x * r.x + r.y * r.y;
+    }
+    d2 = warp_sum(d2);
+    n2 = warp_sum(n2);
+    if (lane == 0) {
+      if (retired) atomicAnd(retired + (local >> 5), ~(1u << (local & 31)));   // rows share words
+      // rounded up by a few ulps: these feed an upper bound
+      atomicMax(reinterpret_cast<int*>(stats), __float_as_int(sqrtf(d2) * 1.00001f));
+      atomicMax(reinterpret_cast<int*>(stats) + 1, __float_as_int(sqrtf(n2) * 1.00001f));
+    }
+  }
+}
+
+// Retire ids of this index: zero their fp32 and bf16 rows, set their retired bits. One warp per id.
+__global__ void __launch_bounds__(kRowThreads) catalog_retire_kernel(const int64_t* __restrict__ ids, int n,
+                                                                     int64_t item_base, int N,
+                                                                     float* __restrict__ table,
+                                                                     __nv_bfloat16* __restrict__ table_bf16,
+                                                                     uint32_t* __restrict__ retired) {
+  pdl_launch_dependents();
+  pdl_wait();
+  constexpr int NV = 2, E = 8, W = 256;
+  const int lane = threadIdx.x & 31;
+  const int warps_total = (gridDim.x * blockDim.x) >> 5;
+  float z[E];
+#pragma unroll
+  for (int i = 0; i < E; ++i) z[i] = 0.f;
+  for (int r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < n; r += warps_total) {
+    const int64_t local = ids[r] - item_base;
+    if (local < 0 || local >= N) continue;
+    store_row<NV>(table + static_cast<size_t>(local) * W, lane, z);
+    store_row_bf16<NV>(table_bf16 + static_cast<size_t>(local) * W, lane, z);
+    if (lane == 0) atomicOr(retired + (local >> 5), 1u << (local & 31));
   }
 }
 
@@ -1061,6 +1138,51 @@ extern "C" int tt_index_rows(const float* y, int R, const float* ln_w, const flo
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   TT_REQUIRE(y && ln_w && ln_b && ids && table && R > 0 && V > 0, "tt_index_rows: bad arguments");
   TT_CHECK_CUDA(launch_k(index_rows_kernel, dim3(row_grid(R)), dim3(kRowThreads), 0, stream, y, R, ln_w, ln_b, ids, V, table, static_cast<__nv_bfloat16*>(table_bf16)));
+  TT_LAUNCH_CHECK();
+  return TT_OK;
+}
+
+// The update id list on the host: every id in [1, vocab_size) and none twice, checked before any launch.
+static int check_update_ids(const int64_t* ids, int n, int64_t vocab_size, cudaStream_t stream, const char* what) {
+  std::vector<int64_t> h(static_cast<size_t>(n));
+  TT_CHECK_CUDA(cudaMemcpyAsync(h.data(), ids, static_cast<size_t>(n) * sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
+  TT_CHECK_CUDA(cudaStreamSynchronize(stream));
+  std::vector<uint64_t> seen(static_cast<size_t>((vocab_size + 63) / 64), 0ull);
+  for (int i = 0; i < n; ++i) {
+    const int64_t id = h[i];
+    TT_REQUIRE(id >= 1 && id < vocab_size, "%s: id %lld outside [1, %lld)", what, static_cast<long long>(id),
+               static_cast<long long>(vocab_size));
+    uint64_t& word = seen[static_cast<size_t>(id >> 6)];
+    TT_REQUIRE(!((word >> (id & 63)) & 1ull), "%s: id %lld appears twice", what, static_cast<long long>(id));
+    word |= 1ull << (id & 63);
+  }
+  return TT_OK;
+}
+
+extern "C" int tt_index_rows_live(const float* y, int R, const float* ln_w, const float* ln_b, const int64_t* ids,
+                                  int64_t vocab_size, int64_t item_base, int N, float* table, void* table_bf16,
+                                  uint32_t* retired_bits, float* stats, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  TT_REQUIRE(y && ln_w && ln_b && ids && table && table_bf16 && stats && R > 0 && N > 0,
+             "tt_index_rows_live: bad arguments");
+  TT_REQUIRE(item_base >= 0 && item_base + N <= vocab_size, "tt_index_rows_live: rows [%lld, %lld) outside the catalog of %lld",
+             static_cast<long long>(item_base), static_cast<long long>(item_base + N), static_cast<long long>(vocab_size));
+  const int rc = check_update_ids(ids, R, vocab_size, stream, "tt_index_rows_live");
+  if (rc) return rc;
+  TT_CHECK_CUDA(launch_k(index_rows_live_kernel, dim3(row_grid(R)), dim3(kRowThreads), 0, stream, y, R, ln_w, ln_b, ids, item_base, N, table, static_cast<__nv_bfloat16*>(table_bf16), retired_bits, stats));
+  TT_LAUNCH_CHECK();
+  return TT_OK;
+}
+
+extern "C" int tt_catalog_retire(const int64_t* ids, int n, int64_t vocab_size, int64_t item_base, int N, float* table,
+                                 void* table_bf16, uint32_t* retired_bits, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  TT_REQUIRE(ids && table && table_bf16 && retired_bits && n > 0 && N > 0, "tt_catalog_retire: bad arguments");
+  TT_REQUIRE(item_base >= 0 && item_base + N <= vocab_size, "tt_catalog_retire: rows [%lld, %lld) outside the catalog of %lld",
+             static_cast<long long>(item_base), static_cast<long long>(item_base + N), static_cast<long long>(vocab_size));
+  const int rc = check_update_ids(ids, n, vocab_size, stream, "tt_catalog_retire");
+  if (rc) return rc;
+  TT_CHECK_CUDA(launch_k(catalog_retire_kernel, dim3(row_grid(n)), dim3(kRowThreads), 0, stream, ids, n, item_base, N, table, static_cast<__nv_bfloat16*>(table_bf16), retired_bits));
   TT_LAUNCH_CHECK();
   return TT_OK;
 }

@@ -642,13 +642,16 @@ class TwoTowerEngine:
         return ws["in"]
 
     def index_items(self, features: Dict[str, torch.Tensor], item_ids: torch.Tensor, table: torch.Tensor,
-                    table_bf16: Optional[torch.Tensor] = None, batch_size: int = 131072) -> None:
+                    table_bf16: Optional[torch.Tensor] = None, batch_size: int = 131072, live=None) -> None:
         """Catalog indexing (src/evaluate_metrics.py:24-104) on device tensors: item tower in eval mode over
         ``features`` (four (n, 128) fp32 device tensors), NaN -> 0, re-normalise (eps 1e-8), rows scattered by
         ``item_ids`` into ``table`` fp32 (V, 256) (+ its bf16 copy). Eval-mode BatchNorm is an affine map per
         column, so it is folded into the first Linear once per call (W' = diag(gamma * rstd) W, b' = (b - mean)
         * gamma * rstd + beta): GEMM -> bias+ReLU epilogue -> bf16 replaces GEMM -> fp32 -> BatchNorm kernel, and
-        an item costs 9.5 KB of HBM traffic against the 3 KB (2 KB of features in, 1 KB of embedding out) it must."""
+        an item costs 9.5 KB of HBM traffic against the 3 KB (2 KB of features in, 1 KB of embedding out) it must.
+        ``live`` = (vocab_size, item_base, retired_bits, stats): update of a built index (`CatalogIndex.upsert`) —
+        ``table`` holds rows [item_base, item_base + len(table)) and the tail is tt_index_rows_live (same rows,
+        other ids skipped, retired bits cleared, certificate terms raised into ``stats``)."""
         p = self.p
         it = "item_tower.fusion_layer."
         n = item_ids.shape[0]
@@ -664,7 +667,12 @@ class TwoTowerEngine:
             ops.concat4_bf16(f[0][s0:s0 + r], f[1][s0:s0 + r], f[2][s0:s0 + r], f[3][s0:s0 + r], ws["xi"][:r])
             self._gemm(ws["xi"][:r], w_fold, bias=b_fold, relu=True, out_bf16=ws["a"][:r])
             self._gemm(ws["a"][:r], self.w[it + "4.weight"], bias=p[it + "4.bias"], out_f32=ws["y2"][:r])
-            ops.index_rows(ws["y2"][:r], p[it + "5.weight"], p[it + "5.bias"], item_ids[s0:s0 + r], table, table_bf16)
+            if live is None:
+                ops.index_rows(ws["y2"][:r], p[it + "5.weight"], p[it + "5.bias"], item_ids[s0:s0 + r], table,
+                               table_bf16)
+            else:
+                ops.index_rows_live(ws["y2"][:r], p[it + "5.weight"], p[it + "5.bias"], item_ids[s0:s0 + r], live[0],
+                                    live[1], table, table_bf16, live[2], live[3])
 
     # -- InfoNCE, written for data parallelism with all-gathered negatives --------------------
     # Rank r holds B local users/items and the G*B gathered ones; its positives sit at column

@@ -454,6 +454,32 @@ def index_rows(y, ln_w, ln_b, ids, table, table_bf16=None) -> None:
                               table.shape[0], table.data_ptr(), _ptr(table_bf16), _stream()), "tt_index_rows")
 
 
+def index_rows_live(y, ln_w, ln_b, ids, vocab_size: int, item_base: int, table, table_bf16, retired_bits, stats) -> None:
+    """index_rows into the rows [item_base, item_base + len(table)) of a built index: other ids are skipped, written
+    rows leave ``retired_bits`` (int32 bitmap or None) and raise ``stats`` = {max ||bf16(e) - e||, max ||bf16(e)||}
+    (tt_index_rows_live)."""
+    _require_cuda(y, ln_w, ln_b, ids, table, table_bf16, retired_bits, stats)
+    assert y.dtype == torch.float32 and y.is_contiguous() and y.shape[1] == 256
+    assert ids.dtype == torch.int64 and ids.is_contiguous() and ids.numel() == y.shape[0]
+    assert table.dtype == torch.float32 and table.is_contiguous() and table.shape[1] == 256
+    assert table_bf16.dtype == torch.bfloat16 and table_bf16.is_contiguous() and table_bf16.shape == table.shape
+    assert stats.dtype == torch.float32 and stats.numel() == 2
+    check(lib().tt_index_rows_live(y.data_ptr(), y.shape[0], ln_w.data_ptr(), ln_b.data_ptr(), ids.data_ptr(),
+                                   vocab_size, item_base, table.shape[0], table.data_ptr(), table_bf16.data_ptr(),
+                                   _ptr(retired_bits), stats.data_ptr(), _stream()), "tt_index_rows_live")
+
+
+def catalog_retire(ids, vocab_size: int, item_base: int, table, table_bf16, retired_bits) -> None:
+    """Zero the rows of ``ids`` (int64, the ones in [item_base, item_base + len(table))) and set their retired bits
+    (tt_catalog_retire)."""
+    _require_cuda(ids, table, table_bf16, retired_bits)
+    assert ids.dtype == torch.int64 and ids.is_contiguous() and ids.dim() == 1
+    assert table.dtype == torch.float32 and table_bf16.dtype == torch.bfloat16 and table_bf16.shape == table.shape
+    assert retired_bits.dtype == torch.int32
+    check(lib().tt_catalog_retire(ids.data_ptr(), ids.numel(), vocab_size, item_base, table.shape[0], table.data_ptr(),
+                                  table_bf16.data_ptr(), retired_bits.data_ptr(), _stream()), "tt_catalog_retire")
+
+
 # --------------------------------------------------------------------------------------
 # last-layer specialisation (one query row per sequence)
 # --------------------------------------------------------------------------------------

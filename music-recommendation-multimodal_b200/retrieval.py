@@ -8,6 +8,7 @@ import ctypes
 import os
 from typing import Dict, List, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 
 from . import ops
@@ -21,7 +22,17 @@ def _stream() -> int:
 class CatalogIndex:
     """Device-resident item table in the reference's cache layout: fp32 (V, 256), row i = embedding
     of item id i, row 0 = padding. ``shard`` = (first_row, num_rows) keeps only a contiguous slice
-    on this GPU (catalog sharding); indices returned by retrieval are always global."""
+    on this GPU (catalog sharding); indices returned by retrieval are always global.
+
+    A built index takes live catalog updates: `upsert` adds or re-embeds songs, `retire` removes them. No retrieval
+    call on the index (`retrieve_topk` and its exact fallback, `retrieve_candidates`, `sharded_topk`, and everything
+    built on them: recommendations with or without diversity, sessions, metrics) ever returns a retired song; that
+    combines with per-user `Exclusions` and ``mask_item0``, and a user with fewer than K live admissible songs gets
+    an id -1 / score -inf tail. The mask is a bitmap of one bit per row that the scoring kernel reads; it exists
+    from the first `retire` on (before that the index launches exactly the kernels of an index without updates).
+    Updates are ordered on the current stream like every other call on the index; updates concurrent with queries
+    on other streams are not supported. The index never grows: to leave room for new songs, build it with
+    ``vocab_size`` = the wanted capacity and retire the ids not yet in use."""
 
     def __init__(self, item_embeddings: torch.Tensor, device=None, shard: Optional[Tuple[int, int]] = None):
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
@@ -40,6 +51,8 @@ class CatalogIndex:
         self._error_terms()
         self._scratch: Dict[Tuple[int, int], Dict[str, torch.Tensor]] = {}
         self._plans: Dict[Tuple[int, int], TopkPlan] = {}
+        #: int32 bitmap, bit r = row r of this index is retired (tt_score_topk_live layout); None until `retire`
+        self.retired_bits: Optional[torch.Tensor] = None
 
     @classmethod
     def from_shard(cls, shard_rows: torch.Tensor, first_row: int, vocab_size: int, device=None) -> "CatalogIndex":
@@ -59,6 +72,7 @@ class CatalogIndex:
         self.table, self.table_bf16 = table, table_bf16
         self._error_terms()
         self._scratch, self._plans = {}, {}
+        self.retired_bits = None
         return self
 
     def _error_terms(self) -> None:
@@ -74,6 +88,94 @@ class CatalogIndex:
     @property
     def num_rows(self) -> int:
         return self.table.shape[0]
+
+    def _check_update_ids(self, item_ids, what: str) -> torch.Tensor:
+        """the ids of an update as a host int64 vector; ValueError (before any launch) for id 0, ids outside
+        [1, vocab_size) and ids that appear twice"""
+        if not torch.is_tensor(item_ids) or item_ids.dim() != 1 or item_ids.dtype.is_floating_point \
+                or item_ids.is_complex() or item_ids.dtype == torch.bool:
+            raise ValueError(f"{what}: item_ids must be a 1-D integer tensor")
+        ids = item_ids.to("cpu", torch.int64)
+        if ids.numel() and (int(ids.min()) < 1 or int(ids.max()) >= self.vocab_size):
+            raise ValueError(f"{what}: item ids must lie in [1, {self.vocab_size}) (id 0 is the padding row)")
+        s = np.sort(ids.numpy())                 # cheaper on the host than torch.unique
+        if (s[1:] == s[:-1]).any():
+            raise ValueError(f"{what}: duplicate item ids")
+        return ids
+
+    def _owned(self, ids: torch.Tensor) -> np.ndarray:
+        a = ids.numpy()
+        return (a >= self.item_base) & (a < self.item_base + self.num_rows)
+
+    def retire(self, item_ids: torch.Tensor) -> None:
+        """Remove songs from retrieval: their fp32 and bf16 rows become zero (so `table` stays the reference's cache
+        of the live catalog, a retired row indistinguishable from an unlisted one) and their retired bits are set.
+        ``item_ids``: integer tensor on any device; ids outside this index's rows are skipped (every shard may be
+        handed the same batch), retiring a retired id does nothing. The certificate terms ``de_max`` / ``ne_max`` are
+        never lowered: the bound stays valid, only conservative. The first call that retires a row of this index
+        allocates the bitmap (ceil(rows / 256) * 32 bytes)."""
+        ids = self._check_update_ids(item_ids, "retire")
+        own = torch.from_numpy(ids.numpy()[self._owned(ids)])
+        if own.numel() == 0:
+            return
+        dev = self.table.device
+        if self.retired_bits is None:
+            self.retired_bits = torch.zeros((self.num_rows + 255) // 256 * 8, device=dev, dtype=torch.int32)
+        ops.catalog_retire(own.to(dev), self.vocab_size, self.item_base, self.table, self.table_bf16,
+                           self.retired_bits)
+
+    def retired_ids(self) -> torch.Tensor:
+        """Global ids of this index's retired rows, int64, ascending, on the index's device (with `retire` the round
+        trip that persists the retired set)."""
+        dev = self.table.device
+        if self.retired_bits is None:
+            return torch.empty(0, device=dev, dtype=torch.int64)
+        bits = (self.retired_bits[:, None] >> torch.arange(32, device=dev, dtype=torch.int32)) & 1
+        return torch.nonzero(bits.flatten()[:self.num_rows]).flatten() + self.item_base
+
+    def upsert(self, model, item_features: Dict[str, torch.Tensor], item_ids: torch.Tensor,
+               batch_size: int = 131072) -> None:
+        """Add new songs or re-embed existing ones: the item tower runs in eval mode with the model's CURRENT weights
+        over ``item_features`` (the four (n, modality_dim) feature tensors of catalog indexing, any device) and row
+        ``item_ids[i]`` gets song i's embedding; the song is live afterwards, also when it had been retired. The
+        arithmetic is `TwoTowerEngine.index_items`' (folded BatchNorm, GEMM, GEMM, the index-rows tail), so a row is
+        bit-identical to the one a from-scratch `index_catalog_device` writes for the same song and weights. Ids
+        outside this index's rows are skipped; id 0, ids outside [1, vocab_size), duplicates and malformed features
+        raise ValueError before any launch. Ids at or above the MODEL's vocab_size can be upserted and recommended,
+        but the user tower cannot take them in a history (`UserSessions` rejects them).
+
+        The certificate terms ``de_max`` / ``ne_max`` are raised on the device and read back once: one host
+        synchronisation per call."""
+        ids = self._check_update_ids(item_ids, "upsert")
+        n = ids.numel()
+        keys = ("target_audio", "target_image", "target_input_ids", "target_tabular")
+        m = model.engine.cfg.modality_dim
+        if not isinstance(item_features, dict) or any(k not in item_features for k in keys):
+            raise ValueError(f"upsert: item_features must hold {keys}")
+        for k in keys:
+            f = item_features[k]
+            if not torch.is_tensor(f) or not f.dtype.is_floating_point or tuple(f.shape) != (n, m):
+                raise ValueError(f"upsert: item_features[{k!r}] must be a floating tensor of shape ({n}, {m})")
+        own = self._owned(ids)
+        if not bool(own.any()):
+            return
+        dev = self.table.device
+        if bool(own.all()):
+            feats = {k: item_features[k].to(dev, dtype=torch.float32).contiguous() for k in keys}
+        else:
+            sel = torch.from_numpy(np.nonzero(own)[0])
+            feats = {k: item_features[k][sel.to(item_features[k].device)].to(dev, dtype=torch.float32).contiguous()
+                     for k in keys}
+            ids = ids[sel]
+        eng = model.engine
+        model.eval()
+        if hasattr(model, "_sync_shadow"):
+            model._sync_shadow()
+        stats = torch.zeros(2, device=dev)
+        eng.index_items(feats, ids.to(dev), self.table, self.table_bf16, batch_size=batch_size,
+                        live=(self.vocab_size, self.item_base, self.retired_bits, stats))
+        de, ne = stats.tolist()
+        self.de_max, self.ne_max = max(self.de_max, de), max(self.ne_max, ne)
 
     def check_group(self, U: int, group=None) -> None:
         """Once per (group, U): the shards of the group's ranks must tile [0, vocab_size) without gaps or overlaps
@@ -241,10 +343,17 @@ def retrieve_topk(user_emb: torch.Tensor, index: CatalogIndex, K: int, kprime: i
             for u in bad:
                 ex_ids, ex_cnt = (None, None) if exclude is None else (exclude.ids[u].data_ptr(),
                                                                        exclude.cnt[u:].data_ptr())
-                check(lib().tt_exact_topk_excl(user_emb[u].data_ptr(), index.table.data_ptr(), index.num_rows,
-                                               index.item_base, int(mask_item0), K, ex_ids, ex_cnt,
-                                               sc["keys"].data_ptr(), out_score[u].data_ptr(), out_idx[u].data_ptr(),
-                                               _stream()), "tt_exact_topk_excl")
+                if index.retired_bits is None:
+                    check(lib().tt_exact_topk_excl(user_emb[u].data_ptr(), index.table.data_ptr(), index.num_rows,
+                                                   index.item_base, int(mask_item0), K, ex_ids, ex_cnt,
+                                                   sc["keys"].data_ptr(), out_score[u].data_ptr(),
+                                                   out_idx[u].data_ptr(), _stream()), "tt_exact_topk_excl")
+                else:
+                    check(lib().tt_exact_topk_live(user_emb[u].data_ptr(), index.table.data_ptr(), index.num_rows,
+                                                   index.item_base, int(mask_item0), K, ex_ids, ex_cnt,
+                                                   index.retired_bits.data_ptr(), sc["keys"].data_ptr(),
+                                                   out_score[u].data_ptr(), out_idx[u].data_ptr(), _stream()),
+                          "tt_exact_topk_live")
     return out_idx, out_score, n_fallback
 
 
@@ -262,10 +371,17 @@ def _score_pass(user_emb: torch.Tensor, index: "CatalogIndex", kprime: int, mask
                                  _stream()), "tt_users_prepare")
     ex = (None, None, None, 0) if exclude is None else (exclude.ids.data_ptr(), exclude.cnt.data_ptr(),
                                                          exclude.bits.data_ptr(), exclude.ld)
-    check(lib().tt_score_topk_excl(sc["users_bf16"].data_ptr(), index.table_bf16.data_ptr(), index.item_base,
-                                   ctypes.byref(plan), sc["cand"].data_ptr(), sc["cnt"].data_ptr(),
-                                   sc["thr"].data_ptr(), None if sc["smax"] is None else sc["smax"].data_ptr(),
-                                   int(mask_item0), *ex, _stream()), "tt_score_topk_excl")
+    smax = None if sc["smax"] is None else sc["smax"].data_ptr()
+    if index.retired_bits is None:
+        check(lib().tt_score_topk_excl(sc["users_bf16"].data_ptr(), index.table_bf16.data_ptr(), index.item_base,
+                                       ctypes.byref(plan), sc["cand"].data_ptr(), sc["cnt"].data_ptr(),
+                                       sc["thr"].data_ptr(), smax, int(mask_item0), *ex, _stream()),
+              "tt_score_topk_excl")
+    else:
+        check(lib().tt_score_topk_live(sc["users_bf16"].data_ptr(), index.table_bf16.data_ptr(), index.item_base,
+                                       ctypes.byref(plan), sc["cand"].data_ptr(), sc["cnt"].data_ptr(),
+                                       sc["thr"].data_ptr(), smax, int(mask_item0), *ex,
+                                       index.retired_bits.data_ptr(), _stream()), "tt_score_topk_live")
     return plan, sc
 
 
