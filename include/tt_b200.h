@@ -99,6 +99,9 @@ int tt_gemm_bf16(const tt_gemm_args* args, void* stream);
  * 256 < L <= 4096 runs the tiled online-softmax forward, which hashes the element index in 64 bits. The backward keeps
  * a sequence's dQ accumulators on chip up to L = 512; 512 < L <= 4096 runs the tiled backward (deterministic, in two
  * kernels: one per key tile for dK / dV and one per query tile for dQ; 64-bit element index). B*L <= 2^31 - 1.
+ * The kernels that keep a sequence on chip (forward L <= 256, backward L <= 512) hash a 32-bit element index, so with
+ * drop_p > 0 they require B*H*L*L <= 2^32 and return an error beyond it: above 2^32 their masks would repeat across
+ * sequences and differ from the 64-bit masks of the tiled kernels.
  */
 int tt_attn_causal_fwd(const void* qkv, void* ctx, float* lse, int B, int L, int H, float drop_p,
                        uint64_t drop_seed, const uint64_t* drop_seed_dev, uint32_t drop_site, void* stream);

@@ -1759,6 +1759,9 @@ extern "C" int tt_attn_causal_fwd(const void* qkv, void* ctx, float* lse, int B,
   TT_REQUIRE(static_cast<int64_t>(B) * L <= INT32_MAX, "tt_attn_causal_fwd: B*L=%lld rows too many",
              static_cast<long long>(B) * L);
   TT_REQUIRE(drop_p >= 0.f && drop_p < 1.f, "tt_attn_causal_fwd: drop_p out of range");
+  // the persistent kernel hashes a 32-bit element index ((b*H + h)*L + i)*L + j
+  TT_REQUIRE(!(drop_p > 0.f) || L > 2 * kTile || static_cast<uint64_t>(B) * H <= (1ull << 32) / (L * L),
+             "tt_attn_causal_fwd: dropout at L=%d needs B*H*L*L <= 2^32 (B=%d, H=%d)", L, B, H);
   const int D = H * kDh;
   AttnParams p;
   p.B = B; p.L = L; p.H = H;
@@ -1807,6 +1810,9 @@ extern "C" int tt_attn_causal_bwd(const void* qkv, const void* ctx, const void* 
   TT_REQUIRE(L <= kLongMaxL, "tt_attn_causal_bwd: L=%d > %d unsupported", L, kLongMaxL);
   TT_REQUIRE(static_cast<int64_t>(B) * L <= INT32_MAX, "tt_attn_causal_bwd: B*L=%lld rows too many",
              static_cast<long long>(B) * L);
+  // the persistent and per-item kernels hash a 32-bit element index ((b*H + h)*L + i)*L + j
+  TT_REQUIRE(!(drop_p > 0.f) || L > 4 * kTile || static_cast<uint64_t>(B) * H <= (1ull << 32) / (L * L),
+             "tt_attn_causal_bwd: dropout at L=%d needs B*H*L*L <= 2^32 (B=%d, H=%d)", L, B, H);
   const int D = H * kDh;
   AttnBwdParams p;
   p.B = B; p.L = L; p.H = H;

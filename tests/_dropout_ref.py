@@ -10,9 +10,11 @@ training step of the engine.
 All arithmetic is uint64 holding 32-bit values, masked with 0xFFFFFFFF after every product: a 32 x
 32-bit product overflows int64 (and torch has no uint64 arithmetic).
 
-Scope: element indices below 2^32. The kernels' quad / pair hash forms take the index as uint32
-while drop_keep_k takes it as uint64 and folds the high word into the hash; the two agree below 2^32
-only (the largest index a benchmarked shape forms is B*H*L*L = 256*4*200*200 < 2^26 at c2).
+Element indices are 64-bit. drop_keep_k here folds the high word into the hash as the kernels'
+drop_keep_k and their 64-bit quad / pair forms do (the tiled attention kernels, the single-query
+kernels), so it is right above 2^32 too: the long-history tests compare masks there. The 32-bit
+quad / pair forms of the kernels that keep a sequence on chip agree with it below 2^32 only, and
+tt_attn_causal_fwd / _bwd refuse dropout on those kernels once B*H*L*L passes 2^32.
 """
 from __future__ import annotations
 
@@ -53,7 +55,7 @@ def drop_key(seed: int, site: int) -> int:
 
 
 def drop_keep_k(key: int, idx, thresh: int) -> np.ndarray:
-    """Keep bit of every element index in ``idx`` (< 2^32, see the module docstring)."""
+    """Keep bit of every (64-bit) element index in ``idx``."""
     idx = _u64(idx)
     quad = idx >> np.uint64(2)
     x = (quad & _M32) ^ (((quad >> np.uint64(32)) * np.uint64(0x85EBCA6B)) & _M32)
@@ -79,7 +81,7 @@ def drop_scale(p: float) -> np.float32:
 
 def keep_bits(seed: int, site: int, n: int, p: float, start: int = 0) -> np.ndarray:
     """Keep bits of the element indices start .. start+n-1 at (seed, site) and rate p."""
-    assert start + n <= 1 << 32, "indices at or above 2^32 are out of scope"
+    assert 0 <= start and start + n <= 1 << 64
     thresh = drop_threshold(p)
     if thresh == 0:
         return np.ones(n, dtype=bool)
